@@ -2,11 +2,12 @@
 """Benchmark of the APAP hot path on B200 (BASELINE.json metric: moving-DLT cells/s and mesh-warp
 Mpix/s vs roofline, beside the reference's CPU path timed on the same box).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one synthetic pair.  Two stages are timed, each for
-exactly K steps after W warm-up steps, on the device with CUDA events, with the L2 flushed (a
-256 MiB write) before every step:
+exactly K steps after W warm-up steps (at least 3), on the device with CUDA events, with the L2 flushed (a
+256 MiB write) before every step (the side measurements below -- global warp, spectral weighting, matcher,
+c4 / c5 -- run K timed steps after W warm-up steps too):
   * moving DLT  = K1 (weights + Gram contraction) + K2 (9x9 Jacobi + de-normalise)  -> cells/s
     (the headline ``value``; ``ms_per_step`` is this stage)
   * mesh warp   = K3 (`local_warp`), plus K4 blend and the fused warp+blend          -> Mpix/s
@@ -16,10 +17,15 @@ rank per GPU): every rank runs its own c2-shaped pair (independent pairs, no dat
 "scaling": "weak"), and the c3 pass (8K, 20k keypoints, 400x400) is additionally run strong-scaled
 -- cell rows and canvas row bands sharded, NCCL all-gather to assemble the panorama -- and
 reported under ``"c3_sharded"``.  Times are max over ranks.  Prints ONE JSON line on rank 0.
+
+``--dump-outputs DIR`` writes, after the timed steps, what each timed path of rank 0 computed in its last step as
+``DIR/<name>.npy`` (see ``OutputDump``).  The inputs are seeded, so two builds run with the same arguments can be
+compared output for output.
 """
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import math
 import os
@@ -33,6 +39,7 @@ import numpy as np
 REPO = os.path.dirname(os.path.abspath(__file__))
 if REPO not in sys.path:
     sys.path.insert(0, REPO)
+sys.dont_write_bytecode = True          # the tree may be read-only: the bench writes nothing into it
 
 METRIC = "apap_moving_dlt_cells_per_s"
 UNIT = "cells/s"
@@ -74,6 +81,7 @@ class ClockSampler:
             self.proc = subprocess.Popen(
                 ["nvidia-smi", f"--id={self.index}", f"--query-gpu={self.FIELDS}", "--format=csv,noheader,nounits",
                  "-lms", "100"], stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self.proc.terminate)      # the sampler never outlives the bench, even one that fails
             self.thread = threading.Thread(target=self._pump, daemon=True)
             self.thread.start()
         except Exception:
@@ -365,6 +373,42 @@ class Pass:
         self.rt.blend_device(self.torch, self.canvas, self.pasted, out=self.canvas2)
 
 
+class OutputDump:
+    """``--dump-outputs DIR``: the arrays a caller of each timed path receives from its last timed step, written as
+    ``DIR/<name>.npy`` in float32 (float32 results, uint8 images) or float64 (float64 and integer results).  An array
+    larger than ``ARRAY_BYTES`` keeps a fixed seeded sample of its rows (first axis), the same rows in every run of
+    the same shape, so that the 20 or so arrays stay under 64 MB in all.  ``path`` None: nothing is kept.
+    Two runs of the same build give the same bits everywhere but in ``spectral_segment``: the power iteration sums
+    its norm with float64 atomics, so its last bits vary from run to run (4e-16 apart in two runs on a B200)."""
+
+    ARRAY_BYTES = 3 << 20
+    TOTAL_BYTES = 64 * 10 ** 6
+
+    def __init__(self, path):
+        self.path, self.arrays = path, {}
+
+    def add(self, name, value):
+        if self.path is None:
+            return
+        a = value.cpu().numpy() if hasattr(value, "cpu") else np.asarray(value)
+        dtype = np.float32 if a.dtype == np.float32 or a.dtype.itemsize <= 2 else np.float64
+        keep = self.ARRAY_BYTES // (a[:1].size * np.dtype(dtype).itemsize)
+        if a.shape[0] > keep:
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+        self.arrays[name] = a.astype(dtype)
+
+    def write(self):
+        if self.path is None:
+            return
+        total = sum(a.nbytes for a in self.arrays.values())
+        if total > self.TOTAL_BYTES:
+            raise RuntimeError(f"--dump-outputs: {total} bytes exceed {self.TOTAL_BYTES}")
+        os.makedirs(self.path, exist_ok=True)
+        for name, a in self.arrays.items():
+            np.save(os.path.join(self.path, name + ".npy"), a)
+        print(f"bench: {len(self.arrays)} outputs ({total / 1e6:.1f} MB) -> {self.path}", file=sys.stderr)
+
+
 def timed_steps(torch, flush, warmup, steps, body, n_marks):
     """Run ``body(mark)`` warmup+steps times; ``body`` calls ``mark()`` n_marks times.  Returns the
     per-interval mean milliseconds over the timed steps (list of n_marks-1 floats)."""
@@ -427,6 +471,7 @@ def run_ours(args):
     mufu_peak = rt.pipe_peak(rt.PROBE_MUFU, device) / 1e12                    # Tlane-op/s
     p = Pass(torch, device, name, seed=rank, gram_engine=args.gram_engine)
     sc = p.sc
+    dump = OutputDump(args.dump_outputs if rank == 0 else None)
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
@@ -438,6 +483,7 @@ def run_ours(args):
     t_gram, t_eig = timed_steps(torch, flush, W, K, dlt_body, 3)        # K1, K2 timed one by one (roofline attribution)
     barrier()
     (t_dlt,) = timed_steps(torch, flush, W, K, lambda mark: (mark(), p.dlt(), mark()), 2)   # the stage as the public call launches it
+    dump.add("h", p.h_out.reshape(-1, sc.mesh_cells, 3, 3))
     barrier()
     launches += 4 * K
     ms_dlt = max_over_ranks(t_dlt)
@@ -450,9 +496,13 @@ def run_ours(args):
     p.prepare_warp()
     barrier()
     (t_warp,) = timed_steps(torch, flush, W, K, lambda mark: (mark(), p.warp(False), mark()), 2)
+    dump.add("warp", p.canvas)
     (t_strip,) = timed_steps(torch, flush, W, K, lambda mark: (mark(), p.warp(False, legacy=True), mark()), 2)
+    dump.add("warp_strip", p.canvas)
     (t_fused,) = timed_steps(torch, flush, W, K, lambda mark: (mark(), p.warp(True), mark()), 2)
+    dump.add("warp_blend", p.canvas)
     (t_blend,) = timed_steps(torch, flush, W, K, lambda mark: (mark(), p.blend(), mark()), 2)
+    dump.add("blend", p.canvas2)
     barrier()
     launches += 4 * K
     ms_warp, ms_fused, ms_blend, ms_strip = (max_over_ranks(t) for t in (t_warp, t_fused, t_blend, t_strip))
@@ -471,6 +521,7 @@ def run_ours(args):
     for g_name, g_mode in (("warp_only", 0), ("paste", 1), ("mean_blend", 2)):
         (g_t,) = timed_steps(torch, flush, W, K, lambda mark: (mark(), putils.warp_perspective(
             p.img, g_m, (g_cw, g_ch), base=p.centre, offset=(g_tx, g_ty), mode=g_mode, out=g_out), mark()), 2)
+        dump.add("global_" + g_name, g_out)
         g_times[g_name] = max_over_ranks(g_t)
     launches += 3 * K
     barrier()
@@ -484,13 +535,17 @@ def run_ours(args):
     sp_bad = sp_rng.random(sp_n) < 0.3
     sp_c[sp_bad] += sp_rng.normal(0, 60, (int(sp_bad.sum()), 2)).astype(np.float32)
     sp_diag = 0.9 + 0.1 * sp_rng.random(sp_n)
-    psm.spectral_segment_device(sp_c, sp_o, sp_diag, 30.0, device=device)
-    torch.cuda.synchronize()
-    sp_t0 = time.perf_counter()
-    _, sp_info = psm.spectral_segment_device(sp_c, sp_o, sp_diag, 30.0, device=device, return_info=True)
-    torch.cuda.synchronize()
-    sp_ms = (time.perf_counter() - sp_t0) * 1e3
-    launches += 2 * (1 + sp_info["iterations"] + sp_info["iterations"] // 16)      # k_affinity, k_power_step per step, k_power_diff per 16
+    sp_times = []
+    for k in range(W + K):
+        torch.cuda.synchronize()
+        sp_t0 = time.perf_counter()
+        sp_seg, sp_info = psm.spectral_segment_device(sp_c, sp_o, sp_diag, 30.0, device=device, return_info=True)
+        torch.cuda.synchronize()
+        if k >= W:
+            sp_times.append((time.perf_counter() - sp_t0) * 1e3)
+    sp_ms = float(np.mean(sp_times))
+    dump.add("spectral_segment", sp_seg)
+    launches += (W + K) * (1 + sp_info["iterations"] + sp_info["iterations"] // 16)   # k_affinity, k_power_step per step, k_power_diff per 16
 
     # ---- e2e through the public API: pinned host buffers in, host arrays out -------------------
     src_pin = rt.pinned_empty(sc.src.shape, np.float32); src_pin[...] = sc.src
@@ -510,6 +565,8 @@ def run_ours(args):
         if k >= W:
             e2e_dlt.append(t1 - t0)
             e2e_warp.append(t2 - t1)
+    dump.add("e2e_h_inverted", h_host)                # local_warp leaves the per-cell inverses in the caller's grid
+    dump.add("e2e_warp", warped)
     # k_scale_anchors, k_condition, k_condition_mats, k_kp_rows, k_weight_bound, k_kp_blocks, k_gram_tc, k_eig;
     # k_inv_grid, k_warp_prep, k_tile_prep, k_warp_tile
     launches += 12 * K
@@ -523,17 +580,18 @@ def run_ours(args):
     # ---- c3 strong-scaled across ranks (cell rows + row bands, one all-gather) -----------------
     c3 = None
     if args.c3 and (world > 1 or args.c3 == "always"):
-        c3 = run_c3_sharded(torch, dist, device, rank, world, flush, W, K, max_over_ranks, barrier, args.gram_engine)
+        c3 = run_c3_sharded(torch, dist, device, rank, world, flush, W, K, max_over_ranks, barrier, dump, args.gram_engine)
         launches += c3.pop("_launches")
 
     extras = None
     if world == 1 and not args.no_extras:
-        extras = run_c4_c5(torch, device, flush, mufu_peak * 1e12)
+        extras = run_c4_c5(torch, device, flush, mufu_peak * 1e12, W, K, dump)
         launches += extras.pop("_launches")
-        extras["matcher"] = run_matcher(torch, device, flush, fp32_peak)
+        extras["matcher"] = run_matcher(torch, device, flush, fp32_peak, W, K, dump)
         launches += extras["matcher"].pop("_launches")
 
     clocks = sampler.stop() if rank == 0 else None
+    dump.write()
     if rank != 0:
         if world > 1:
             dist.destroy_process_group()
@@ -657,7 +715,7 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
-def run_c3_sharded(torch, dist, device, rank, world, flush, W, K, max_over_ranks, barrier, gram_engine="tcgen05"):
+def run_c3_sharded(torch, dist, device, rank, world, flush, W, K, max_over_ranks, barrier, dump, gram_engine="tcgen05"):
     """BASELINE config c3 split over the ranks: cell rows [m0, m1) and the canvas rows they own per
     rank, keypoints and source image replicated, one NCCL all-gather of the row bands."""
     from cvx_proj_b200 import sharding
@@ -676,10 +734,12 @@ def run_c3_sharded(torch, dist, device, rank, world, flush, W, K, max_over_ranks
     t_gram, t_eig = timed_steps(torch, flush, W, K, dlt_body, 3)
     barrier()
     (t_dlt,) = timed_steps(torch, flush, W, K, lambda mark: (mark(), p.dlt(), mark()), 2)
+    dump.add("c3_h", p.h_out.reshape(-1, cfg["mesh"], 3, 3))
     barrier()
     p.prepare_warp(px_rows=(me.px_row0, me.px_row1))
     barrier()
     (t_warp,) = timed_steps(torch, flush, W, K, lambda mark: (mark(), p.warp(False), mark()), 2)
+    dump.add("c3_warp", p.canvas)
     barrier()
     t_gather = 0.0
     if world > 1:
@@ -767,7 +827,7 @@ def run_c3_sharded(torch, dist, device, rank, world, flush, W, K, max_over_ranks
             "_launches": 5 * K + (3 * K if world > 1 else 0)}
 
 
-def run_matcher(torch, device, flush, fp32_peak):
+def run_matcher(torch, device, flush, fp32_peak, W, K, dump):
     """SURVEY 8f row N3, matcher step: exact 1-NN of 4000 x 4000 SIFT-like descriptors (the c2 keypoint count after
     border rejection), device-resident and host to host, next to OpenCV's exact and FLANN matchers on this box's CPU."""
     import time
@@ -779,24 +839,26 @@ def run_matcher(torch, device, flush, fp32_peak):
     query = np.clip(train[rng.permutation(nt)] + rng.integers(-6, 7, size=(nq, 128)), 0, 255).astype(np.float32)
     q_dev, t_dev = torch.from_numpy(query).to(device), torch.from_numpy(train).to(device)
     ts = []
-    for k in range(8):
+    for k in range(W + K):
         flush.add_(1)
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record(); match_descriptors(q_dev, t_dev); e1.record(); e1.synchronize()
-        if k >= 3:
+        if k >= W:
             ts.append(e0.elapsed_time(e1))
     ms_dev = float(np.median(ts))
     t0 = time.perf_counter()
-    for _ in range(5):
-        match_descriptors(query, train)
-    ms_host = (time.perf_counter() - t0) / 5 * 1e3
+    for _ in range(K):
+        idx, dist = match_descriptors(query, train)
+    ms_host = (time.perf_counter() - t0) / K * 1e3
+    dump.add("matcher_index", idx)
+    dump.add("matcher_distance", dist)
     out = {"what": "exact 1-nearest-neighbour descriptor matching (apap_match_nn) = cv.BFMatcher(NORM_L2).match, bit-identical on "
                    "SIFT descriptors; the reference calls FLANN's approximate matcher (pyviz/utils.py:149-150)",
            "queries": nq, "train": nt, "dim": 128, "ms_device": ms_dev, "ms_host_to_host": ms_host,
            "pairs_per_s": nq * nt / (ms_dev * 1e-3),
            "fp32_frac": 3.0 * nq * nt * 128 / (ms_dev * 1e-3) / 1e12 / fp32_peak,
            "fp32_note": "3 flop (subtract, multiply, add) per component of a (query, train) pair on the packed FP32x2 pipe, "
-                        "against the FFMA probe peak of this run", "_launches": 13 * 3}
+                        "against the FFMA probe peak of this run", "_launches": (W + 2 * K) * 3}
     try:
         import cv2 as cv
         t0 = time.perf_counter(); cv.BFMatcher(cv.NORM_L2).match(query, train); ms_bf = (time.perf_counter() - t0) * 1e3
@@ -807,19 +869,19 @@ def run_matcher(torch, device, flush, fp32_peak):
     return out
 
 
-def run_c4_c5(torch, device, flush, mufu_peak):
+def run_c4_c5(torch, device, flush, mufu_peak, W, K, dump):
     """BASELINE configs c4 (a batch of 64 1080p pairs, 2k keypoints, 100 x 100 grid, ONE launch of K1 + K2) and c5
     (keypoint sweep at a fixed 256 x 256 grid) on one GPU: device-resident, CUDA events, L2 flushed before every launch."""
     from cvx_proj_b200 import _runtime as rt, synth
     from cvx_proj_b200.apap import APAP, scale_anchors, weight_scale
 
-    def timed(fn, iters=5, warm=3):
+    def timed(fn):
         ts = []
-        for k in range(iters + warm):
+        for k in range(W + K):
             flush.add_(1)
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record(); fn(); e1.record(); e1.synchronize()
-            if k >= warm:
+            if k >= W:
                 ts.append(e0.elapsed_time(e1))
         return float(np.median(ts))
 
@@ -847,7 +909,8 @@ def run_c4_c5(torch, device, flush, mufu_peak):
                                                                 stream)))
         ms_both = timed(lambda: st.local_homography_device(t_dev, a_dev, m_dev, 1, cells, out_h=out_h, partials=partials,
                                                            t_bound=bound))
-        launches += 8 * 3
+        dump.add(f"c5_h_{n_kp}", out_h[0].reshape(sc.mesh_cells, sc.mesh_cells, 3, 3))
+        launches += (W + K) * 3
         sweep.append({"n_kp": n_kp, "cells": cells, "k_splits": ks, "gram_ms": ms_gram, "k1_k2_ms": ms_both,
                       "cells_per_s": cells / (ms_both * 1e-3), "xu_frac": 2.0 * cells * n_pad / (ms_gram * 1e-3) / mufu_peak})
     pairs = 64
@@ -866,7 +929,8 @@ def run_c4_c5(torch, device, flush, mufu_peak):
     bound = st.weight_bound_device(torch.from_numpy(raw).to(device), None, a_dev)
     ms_batch = timed(lambda: st.local_homography_device(t_dev, a_dev, m_dev, pairs, cells, out_h=out_h, partials=partials,
                                                         t_bound=bound))
-    launches += 8 * 2
+    dump.add("c4_h", out_h.reshape(pairs, scs[0].mesh_cells, scs[0].mesh_cells, 3, 3))
+    launches += (W + K) * 2
     c4 = {"workload": _workload_desc("c4") + f", batch of {pairs} pairs in one launch", "batch_ms": ms_batch,
           "cells_per_s": pairs * cells / (ms_batch * 1e-3),
           "xu_frac": 2.0 * pairs * cells * n_pad / (ms_batch * 1e-3) / mufu_peak}
@@ -886,7 +950,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the CPU baseline leg")
     ap.add_argument("--gram-engine", default="tcgen05", choices=["tcgen05", "ffma2"],
                     help="kernel of the moving-DLT contraction (default: tensor cores)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what each timed path computed in its last step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU arm's outputs (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

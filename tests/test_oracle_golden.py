@@ -148,15 +148,21 @@ def test_image_warping_oracle_reproduces_live_reference(golden):
 
 
 def test_spectral_oracle_reproduces_live_reference(golden):
-    """oracle/spectral_oracle.py against outputs of the live reference's calculate_M (oracle/gen_golden_spectral.py)."""
+    """oracle/spectral_oracle.py against outputs of the live reference's calculate_M (oracle/gen_golden_spectral.py).
+    The segment is |U[:, 0]| of LAPACK's SVD, whose last bits depend on the CPU (OpenBLAS picks its kernels at run
+    time) and on the thread count: it is held to 1e-12 of the reference's (the GPU path's gate is 1e-10), the ransac
+    mask (float32 copies of segment entries) as in the GPU test, the original mask bit for bit."""
     from oracle import spectral_oracle as so
     from oracle.gen_golden_spectral import CASES, OPTS, spectral_case
     g = golden("ref_spectral.npz")
     for name in ("s40", "s300", "s1000"):
         c, o, cf, of, fmat, hg = spectral_case(name)
         seg, rmask, omask = so.calculate_m(c, o, cf, of, fmat, hg, **OPTS)
-        assert np.array_equal(seg, g[name + "_segment"])
-        assert np.array_equal(rmask, g[name + "_ransac_mask"]) and np.array_equal(omask, g[name + "_original_mask"])
+        err = np.abs(seg - g[name + "_segment"]).max()
+        print(f"{name}: max |segment - reference| = {err:.2e}")
+        assert seg.dtype == np.float64 and seg.shape == g[name + "_segment"].shape and err <= 1e-12
+        assert np.allclose(rmask, g[name + "_ransac_mask"], rtol=0, atol=1e-7)
+        assert np.array_equal(omask, g[name + "_original_mask"])
     assert set(CASES) == {"s40", "s300", "s1000", "s2500"}
 
 
