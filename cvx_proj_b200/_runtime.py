@@ -62,6 +62,8 @@ SIGNATURES = {
     "apap_multicast_copy": (c_int, [c_void_p, c_void_p, c_size_t, c_void_p]),
     "apap_peer_copy": (c_int, [c_void_p, c_void_p, c_int, c_size_t, c_void_p]),
     "apap_match_nn": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "apap_sift_describe": (c_int, [c_void_p, c_int, c_int, c_void_p, c_int, c_void_p, c_int, c_float, c_void_p, c_void_p,
+                                   c_void_p]),
     "apap_invert_grid": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p]),
     "apap_kp_rows": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_double, c_void_p, c_void_p]),
     "apap_condition": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),

@@ -21,7 +21,8 @@ import numpy as np
 
 from . import _runtime as rt
 
-__all__ = ["image_warping", "warp_perspective", "warping_canvas", "invert3x3", "match_descriptors", "coarse_matching"]
+__all__ = ["image_warping", "warp_perspective", "warping_canvas", "invert3x3", "match_descriptors", "coarse_matching",
+           "sift_describe"]
 
 
 def invert3x3(m) -> np.ndarray:
@@ -132,19 +133,128 @@ def match_descriptors(feats_query, feats_train, device=None):
     return idx, dist
 
 
-def coarse_matching(c_img, o_img, raw_kpts_cp, raw_kpts_op, device=None):
+SIFT_DIM = 128
+_SIFT_TABLES = {}
+
+
+def sift_sample_table(size, angle, h, w):
+    """``(table float32 [n, 5], ori)`` of ``calcSIFTDescriptor`` (OpenCV 4.x) for keypoints of one ``size`` and ``angle`` on
+    an ``h x w`` image: ``(i, j, rbin, cbin, weight)`` of every sample of the ``(2 radius + 1)^2`` window (row offset ``i``
+    outer, column offset ``j`` inner) that passes the bin test, and ``ori = 360 - angle``.  float32 with OpenCV's operation
+    order; the weight is ``exp`` of its float32 argument rounded once to float32 (OpenCV's own ``exp32f`` may differ from
+    that in the last bit)."""
+    f = np.float32
+    size, angle = f(size), f(angle)
+    ori = f(360.0) - angle
+    if abs(ori - f(360.0)) < np.finfo(np.float32).eps:
+        ori = f(0.0)
+    hist_width = f(3.0) * (size * f(0.5))                              # SIFT_DESCR_SCL_FCTR * scl
+    radius = int(np.rint(hist_width * f(1.4142135623730951) * f(5.0) * f(0.5)))   # * (d + 1) * 0.5
+    radius = min(radius, int(np.sqrt(float(w) * w + float(h) * h)))
+    rad = ori * f(np.pi / 180)
+    cos_t = f(np.cos(np.float64(rad))) / hist_width
+    sin_t = f(np.sin(np.float64(rad))) / hist_width
+    i, j = np.meshgrid(np.arange(-radius, radius + 1, dtype=np.float32), np.arange(-radius, radius + 1, dtype=np.float32),
+                       indexing="ij")
+    i, j = i.ravel(), j.ravel()
+    c_rot = j * cos_t - i * sin_t
+    r_rot = j * sin_t + i * cos_t
+    rbin = r_rot + f(2.0) - f(0.5)                                     # + d / 2 - 0.5f
+    cbin = c_rot + f(2.0) - f(0.5)
+    keep = (rbin > -1) & (rbin < 4) & (cbin > -1) & (cbin < 4)
+    wgt = np.exp(((c_rot * c_rot + r_rot * r_rot) * f(-0.125)).astype(np.float64)).astype(np.float32)  # -1 / (d d 0.5)
+    table = np.stack([i, j, rbin, cbin, wgt], axis=1)[keep]
+    return np.ascontiguousarray(table, dtype=np.float32), ori
+
+
+def _keypoint_args(points, size, angle):
+    """``(xy float32 [K, 2] or tensor, size, angle)`` from an array / tensor of points or a list of ``cv.KeyPoint``."""
+    if isinstance(points, (list, tuple)) and points and hasattr(points[0], "pt"):
+        octaves = {int(kp.octave) for kp in points}
+        if octaves != {0}:
+            raise ValueError(f"sift_describe: keypoints of octave {sorted(octaves - {0})} are not supported (octave 0 only)")
+        sizes, angles = {float(kp.size) for kp in points}, {float(kp.angle) for kp in points}
+        if len(sizes) > 1:
+            raise ValueError("sift_describe: keypoints of mixed sizes are not supported (one size per call)")
+        if len(angles) > 1:
+            raise ValueError("sift_describe: keypoints of mixed angles are not supported (one angle per call)")
+        return np.array([kp.pt for kp in points], dtype=np.float32).reshape(-1, 2), sizes.pop(), angles.pop()
+    if isinstance(points, (list, tuple)):
+        points = np.asarray(points, dtype=np.float32).reshape(-1, 2)
+    return points, size, angle
+
+
+def sift_describe(image, points, size=1.0, angle=-1.0, device=None):
+    """SIFT descriptors at given keypoints on the GPU: ``cv.SIFT.create().compute(image, [cv.KeyPoint(x, y, size,
+    angle), ...])[1]`` (``apap_sift_describe``), ``float32 [K, 128]``, one row per point (a point with no sample inside
+    the image gives zeros, as in OpenCV).  Every component is within +-2 of OpenCV 4.x's and almost all are equal.
+
+    ``image``: ``uint8 [H, W, 3]`` BGR.  ``points``: ``[K, 2]`` (x, y), or a list of ``cv.KeyPoint`` of octave 0 sharing
+    one size and one angle (which then replace ``size`` / ``angle``).  ``angle`` is -1 (the reference's keypoints) or in
+    [0, 360).  numpy in -> numpy out; a CUDA tensor image -> the descriptors stay on its device."""
+    points, size, angle = _keypoint_args(points, size, angle)
+    if not (np.isfinite(size) and size > 0):
+        raise ValueError(f"sift_describe: size must be finite and > 0, got {size}")
+    if not (angle == -1.0 or 0.0 <= angle < 360.0):
+        raise ValueError(f"sift_describe: angle {angle} is not supported (-1 or [0, 360))")
+    on_device = not isinstance(image, np.ndarray)
+    torch, device = rt.torch_cuda(image.device if on_device else device)
+    lib = rt.load_library()
+    if image.ndim != 3 or image.shape[2] != 3 or image.dtype != (np.uint8 if not on_device else torch.uint8):
+        raise ValueError("sift_describe: expected a uint8 [H, W, 3] BGR image")
+    img = _device_image(torch, device, image)
+    h, w = int(img.shape[0]), int(img.shape[1])
+    if isinstance(points, np.ndarray) or not hasattr(points, "device"):
+        pts = rt.to_device(torch, device, np.asarray(points, dtype=np.float32).reshape(-1, 2))
+    else:
+        pts = points.to(device=device, dtype=torch.float32).reshape(-1, 2).contiguous()
+    k = int(pts.shape[0])
+    desc = torch.empty((k, SIFT_DIM), dtype=torch.float32, device=device)
+    if k:
+        key = (float(size), float(angle), h, w, device)
+        if key not in _SIFT_TABLES:
+            if len(_SIFT_TABLES) >= 64:
+                _SIFT_TABLES.clear()
+            table, ori = sift_sample_table(size, angle, h, w)
+            _SIFT_TABLES[key] = (rt.to_device(torch, device, table), float(ori))
+        table, ori = _SIFT_TABLES[key]
+        base = torch.empty((h, w), dtype=torch.float32, device=device)
+        with torch.cuda.device(device):
+            rt.check(lib.apap_sift_describe(img.data_ptr(), h, w, pts.data_ptr(), k, table.data_ptr(), int(table.shape[0]),
+                                            ori, base.data_ptr(), desc.data_ptr(), rt.stream_ptr(torch, device)),
+                     "apap_sift_describe")
+    return desc if on_device else rt.to_host(torch, desc)
+
+
+def coarse_matching(c_img, o_img, raw_kpts_cp, raw_kpts_op, device=None, describe="opencv"):
     """``coarse_matching`` of the reference (pyviz/utils.py:142-151) -- same arguments, same return tuple
     ``(kpts_cp, feats_cp, kpts_op, feats_op, matches)`` with ``matches`` a list of ``cv.DMatch`` (one per centre
-    keypoint, in query order).  SIFT descriptors at the given keypoints are OpenCV's own (``cv.SIFT.compute``, host:
-    un-vendored, no bit-level restatement exists); the matcher is the exact nearest neighbour on the GPU
-    (``match_descriptors``) where the reference asks FLANN's randomised kd-trees for an approximation of it."""
+    keypoint, in query order).  The matcher is the exact nearest neighbour on the GPU (``match_descriptors``) where the
+    reference asks FLANN's randomised kd-trees for an approximation of it.
+
+    ``describe`` picks the SIFT descriptors at the given keypoints:
+      ``"opencv"`` (default): OpenCV's own ``cv.SIFT.compute`` on the host, the reference's exact bytes;
+      ``"gpu"``: ``sift_describe`` -- each image is uploaded once, described on the device and matched there; every
+      component is within +-2 of OpenCV's (almost all equal), and only the descriptors come back for the tuple."""
     import cv2 as cv
 
     kpts_cp = [cv.KeyPoint(*pt, 1) for pt in raw_kpts_cp]
     kpts_op = [cv.KeyPoint(*pt, 1) for pt in raw_kpts_op]
-    extractor = cv.SIFT.create(nfeatures=128)
-    kpts_cp, feats_cp = extractor.compute(c_img, kpts_cp)
-    kpts_op, feats_op = extractor.compute(o_img, kpts_op)
-    idx, dist = match_descriptors(feats_cp, feats_op, device=device)
+    if describe == "opencv":
+        extractor = cv.SIFT.create(nfeatures=128)
+        kpts_cp, feats_cp = extractor.compute(c_img, kpts_cp)
+        kpts_op, feats_op = extractor.compute(o_img, kpts_op)
+        idx, dist = match_descriptors(feats_cp, feats_op, device=device)
+    elif describe == "gpu":
+        torch, device = rt.torch_cuda(device)
+        # the keypoints above are size 1, angle -1 (sift_describe's defaults) at the float32 points
+        dev_cp = sift_describe(_device_image(torch, device, c_img), np.asarray(raw_kpts_cp, dtype=np.float32).reshape(-1, 2))
+        dev_op = sift_describe(_device_image(torch, device, o_img), np.asarray(raw_kpts_op, dtype=np.float32).reshape(-1, 2))
+        idx, dist = match_descriptors(dev_cp, dev_op, device=device)
+        feats_cp, feats_op = rt.to_host(torch, dev_cp), rt.to_host(torch, dev_op)
+        idx, dist = rt.to_host(torch, idx).tolist(), rt.to_host(torch, dist).tolist()
+        kpts_cp, kpts_op = tuple(kpts_cp), tuple(kpts_op)
+    else:
+        raise ValueError(f"coarse_matching: describe must be 'opencv' or 'gpu', got {describe!r}")
     matches = [cv.DMatch(i, int(j), 0, float(d)) for i, (j, d) in enumerate(zip(idx, dist)) if j >= 0]
     return kpts_cp, feats_cp, kpts_op, feats_op, matches

@@ -338,6 +338,24 @@ int apap_match_nn(const float *query, const float *train, int nq, int nt, int di
                   int *idx, float *dist, void *stream);
 
 /*
+ * SIFT descriptors at given keypoints: cv.SIFT.compute(image, keypoints) of the reference's keypoint-pair producer
+ * (pyviz/utils.py:143-147; SURVEY 8f row N3) for keypoints of octave 0 that share one size and one angle -- the
+ * reference builds them as cv.KeyPoint(x, y, 1): size 1, angle -1.  Such keypoints read only the first image of
+ * OpenCV's pyramid, the gray image blurred once (sigma^2 = 1.6^2 - 0.5^2), so the call is two kernels: gray + 13-tap
+ * blur into base_scratch, then calcSIFTDescriptor per keypoint.  Every component is within +-2 of OpenCV 4.x and almost
+ * every one equal (the blur's and the norms' summation orders differ); a keypoint with no sample inside the image gives
+ * a zero row.
+ *   bgr   : uint8 [h][w][3] (device);  pts : float [n_kp][2] (x, y; device), rounded half to even like cvRound
+ *   table : float [n_samples][5] (device): (i, j, rbin, cbin, weight) of every window sample that passes the bin test,
+ *           i (row offset) outer and j inner -- what depends only on size and angle, built on the host in float32
+ *           exactly as calcSIFTDescriptor does (cvx_proj_b200.utils.sift_sample_table);  ori = 360 - angle
+ *           (0 within FLT_EPSILON of 360; 361 for angle -1), in [0, 361]
+ *   base_scratch : float [h][w] (device);  desc : out float [n_kp][128] (device), integers 0..255 as OpenCV returns
+ */
+int apap_sift_describe(const uint8_t *bgr, int h, int w, const float *pts, int n_kp, const float *table, int n_samples,
+                       float ori, float *base_scratch, float *desc, void *stream);
+
+/*
  * Panorama assembly of a sharded pass without an all-gather: broadcast `bytes` of device memory at `src` (this
  * rank's row band, already warped) into every GPU's panorama through an NVLS multicast mapping -- `multicast_dst` is
  * the band's address inside the multicast mapping of the panorama buffers (torch symmetric memory's multicast_ptr +
