@@ -64,6 +64,9 @@ SIGNATURES = {
     "apap_match_nn": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
     "apap_sift_describe": (c_int, [c_void_p, c_int, c_int, c_void_p, c_int, c_void_p, c_int, c_float, c_void_p, c_void_p,
                                    c_void_p]),
+    "apap_sift_describe_lut": (c_int, [c_void_p, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p, c_int, c_float, c_void_p,
+                                       c_void_p, c_void_p]),
+    "apap_equalize_hist": (c_int, [c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
     "apap_invert_grid": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p]),
     "apap_kp_rows": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_double, c_void_p, c_void_p]),
     "apap_condition": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),

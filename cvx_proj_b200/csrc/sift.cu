@@ -48,10 +48,18 @@ __device__ __forceinline__ void blur_run(const float (&x)[kBaseRun + 2 * kSiftR]
   }
 }
 
+// kLut: the image is seen through a per-channel LUT (lut: uint8 [3][256], B G R; staged in shared memory), the
+// equalised image of csrc/equalize.cu without materialising it.  k_sift_base<false> ignores lut.
+template <bool kLut>
 __global__ void __launch_bounds__(kBaseThreads) k_sift_base(const uint8_t *__restrict__ bgr, int h, int w,
-                                                            float *__restrict__ base) {
+                                                            float *__restrict__ base, const uint8_t *__restrict__ lut) {
   __shared__ __align__(16) float gray[kBaseInH][kBaseInW];
   __shared__ __align__(16) float horiz[kBaseInH][kBaseTW];
+  __shared__ uint8_t lut_s[kLut ? 3 * 256 : 1];
+  if constexpr (kLut) {
+    for (int i = threadIdx.x; i < 3 * 256; i += kBaseThreads) lut_s[i] = lut[i];
+    __syncthreads();
+  }
   const int x0 = blockIdx.x * kBaseTW, y0 = blockIdx.y * kBaseTH;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   for (int ty = warp; ty < kBaseInH; ty += kBaseThreads / 32) {
@@ -59,7 +67,10 @@ __global__ void __launch_bounds__(kBaseThreads) k_sift_base(const uint8_t *__res
     for (int tx = lane; tx < kBaseInW; tx += 32) {
       const uint8_t *p = row + (size_t)reflect101(x0 + tx - kSiftR, w) * 3;
       // cv.cvtColor(COLOR_BGR2GRAY) for 8-bit input: 15-bit coefficients, rounded
-      gray[ty][tx] = (float)((3735 * p[0] + 19235 * p[1] + 9798 * p[2] + (1 << 14)) >> 15);
+      if constexpr (kLut)
+        gray[ty][tx] = (float)((3735 * lut_s[p[0]] + 19235 * lut_s[256 + p[1]] + 9798 * lut_s[512 + p[2]] + (1 << 14)) >> 15);
+      else
+        gray[ty][tx] = (float)((3735 * p[0] + 19235 * p[1] + 9798 * p[2] + (1 << 14)) >> 15);
     }
   }
   __syncthreads();
@@ -215,11 +226,14 @@ __global__ void __launch_bounds__(kDescWarps * 32) k_sift_desc(const float *__re
   }
 }
 
-int launch_sift_describe(const uint8_t *bgr, int h, int w, const float *pts, int n_kp, const float *table, int n_samples,
-                         float ori, float *base, float *desc, cudaStream_t st) {
+int launch_sift_describe(const uint8_t *bgr, int h, int w, const uint8_t *lut, const float *pts, int n_kp,
+                         const float *table, int n_samples, float ori, float *base, float *desc, cudaStream_t st) {
   const dim3 grid((w + kBaseTW - 1) / kBaseTW, (h + kBaseTH - 1) / kBaseTH);
-  k_sift_base<<<grid, kBaseThreads, 0, st>>>(bgr, h, w, base);
-  int rc = check_cuda(cudaGetLastError(), "k_sift_base launch");
+  if (lut)
+    k_sift_base<true><<<grid, kBaseThreads, 0, st>>>(bgr, h, w, base, lut);
+  else
+    k_sift_base<false><<<grid, kBaseThreads, 0, st>>>(bgr, h, w, base, nullptr);
+  int rc = check_cuda(cudaGetLastError(), lut ? "k_sift_base<true> launch" : "k_sift_base launch");
   if (rc) return rc;
   k_sift_desc<<<(n_kp + kDescWarps - 1) / kDescWarps, kDescWarps * 32, 0, st>>>(base, h, w, pts, n_kp, table, n_samples,
                                                                                   ori, desc);
@@ -230,8 +244,10 @@ int launch_sift_describe(const uint8_t *bgr, int h, int w, const float *pts, int
 
 using namespace apap;
 
-extern "C" int apap_sift_describe(const uint8_t *bgr, int h, int w, const float *pts, int n_kp, const float *table,
-                                  int n_samples, float ori, float *base_scratch, float *desc, void *stream) {
+// the argument checks of both entry points; lut is null for the plain image
+static int sift_describe_checked(const uint8_t *bgr, int h, int w, const uint8_t *lut, const float *pts, int n_kp,
+                                 const float *table, int n_samples, float ori, float *base_scratch, float *desc,
+                                 void *stream) {
   if (n_kp < 0 || n_samples < 0) return fail(APAP_E_BADARG, "sift_describe: negative size");
   if (n_kp == 0) return 0;
   if (h <= 0 || w <= 0) return fail(APAP_E_BADARG, "sift_describe: image sizes must be > 0");
@@ -240,6 +256,18 @@ extern "C" int apap_sift_describe(const uint8_t *bgr, int h, int w, const float 
   if (!bgr || !pts || (!table && n_samples) || !base_scratch || !desc) return fail(APAP_E_BADARG, "sift_describe: null pointer");
   // ori = 360 - angle for angle in [-1, 360): keeps every trilinear slot inside the histogram
   if (!(ori >= 0.f && ori <= 361.f)) return fail(APAP_E_BADARG, "sift_describe: ori must be in [0, 361]");
-  return launch_sift_describe(bgr, h, w, pts, n_kp, table, n_samples, ori, base_scratch, desc,
+  return launch_sift_describe(bgr, h, w, lut, pts, n_kp, table, n_samples, ori, base_scratch, desc,
                               static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int apap_sift_describe(const uint8_t *bgr, int h, int w, const float *pts, int n_kp, const float *table,
+                                  int n_samples, float ori, float *base_scratch, float *desc, void *stream) {
+  return sift_describe_checked(bgr, h, w, nullptr, pts, n_kp, table, n_samples, ori, base_scratch, desc, stream);
+}
+
+extern "C" int apap_sift_describe_lut(const uint8_t *bgr, int h, int w, const uint8_t *lut, const float *pts, int n_kp,
+                                      const float *table, int n_samples, float ori, float *base_scratch, float *desc,
+                                      void *stream) {
+  if (!lut) return fail(APAP_E_BADARG, "sift_describe_lut: null lut");
+  return sift_describe_checked(bgr, h, w, lut, pts, n_kp, table, n_samples, ori, base_scratch, desc, stream);
 }

@@ -22,7 +22,7 @@ import numpy as np
 from . import _runtime as rt
 
 __all__ = ["image_warping", "warp_perspective", "warping_canvas", "invert3x3", "match_descriptors", "coarse_matching",
-           "sift_describe"]
+           "sift_describe", "equalize_hist", "keypoint_pairs"]
 
 
 def invert3x3(m) -> np.ndarray:
@@ -184,14 +184,19 @@ def _keypoint_args(points, size, angle):
     return points, size, angle
 
 
-def sift_describe(image, points, size=1.0, angle=-1.0, device=None):
+def sift_describe(image, points, size=1.0, angle=-1.0, device=None, equalize=False):
     """SIFT descriptors at given keypoints on the GPU: ``cv.SIFT.create().compute(image, [cv.KeyPoint(x, y, size,
     angle), ...])[1]`` (``apap_sift_describe``), ``float32 [K, 128]``, one row per point (a point with no sample inside
     the image gives zeros, as in OpenCV).  Every component is within +-2 of OpenCV 4.x's and almost all are equal.
 
     ``image``: ``uint8 [H, W, 3]`` BGR.  ``points``: ``[K, 2]`` (x, y), or a list of ``cv.KeyPoint`` of octave 0 sharing
     one size and one angle (which then replace ``size`` / ``angle``).  ``angle`` is -1 (the reference's keypoints) or in
-    [0, 360).  numpy in -> numpy out; a CUDA tensor image -> the descriptors stay on its device."""
+    [0, 360).  numpy in -> numpy out; a CUDA tensor image -> the descriptors stay on its device.
+
+    ``equalize=True`` describes the per-channel equalised image instead (the reference describes the output of
+    ``visualize_equalized_hist``, pyviz/apap.py:234-236): bit for bit ``sift_describe(equalize_hist(image), ...)``, but the
+    equalised image is never written -- the gray conversion reads the image through the equalisation LUT
+    (``apap_equalize_hist`` + ``apap_sift_describe_lut``)."""
     points, size, angle = _keypoint_args(points, size, angle)
     if not (np.isfinite(size) and size > 0):
         raise ValueError(f"sift_describe: size must be finite and > 0, got {size}")
@@ -220,10 +225,40 @@ def sift_describe(image, points, size=1.0, angle=-1.0, device=None):
         table, ori = _SIFT_TABLES[key]
         base = torch.empty((h, w), dtype=torch.float32, device=device)
         with torch.cuda.device(device):
-            rt.check(lib.apap_sift_describe(img.data_ptr(), h, w, pts.data_ptr(), k, table.data_ptr(), int(table.shape[0]),
-                                            ori, base.data_ptr(), desc.data_ptr(), rt.stream_ptr(torch, device)),
-                     "apap_sift_describe")
+            st = rt.stream_ptr(torch, device)
+            if equalize:
+                hist = torch.empty(3 * 256, dtype=torch.int32, device=device)
+                lut = torch.empty(3 * 256, dtype=torch.uint8, device=device)
+                rt.check(lib.apap_equalize_hist(img.data_ptr(), h, w, hist.data_ptr(), lut.data_ptr(), None, st),
+                         "apap_equalize_hist")
+                rt.check(lib.apap_sift_describe_lut(img.data_ptr(), h, w, lut.data_ptr(), pts.data_ptr(), k, table.data_ptr(),
+                                                    int(table.shape[0]), ori, base.data_ptr(), desc.data_ptr(), st),
+                         "apap_sift_describe_lut")
+            else:
+                rt.check(lib.apap_sift_describe(img.data_ptr(), h, w, pts.data_ptr(), k, table.data_ptr(),
+                                                int(table.shape[0]), ori, base.data_ptr(), desc.data_ptr(), st),
+                         "apap_sift_describe")
     return desc if on_device else rt.to_host(torch, desc)
+
+
+def equalize_hist(image, device=None):
+    """``cv.merge([cv.equalizeHist(c) for c in cv.split(image)])`` on the GPU, bit for bit (``apap_equalize_hist``): the
+    per-channel equalisation of the reference's ``visualize_equalized_hist`` (pyviz/utils.py:85-91).  ``image``: ``uint8
+    [H, W, 3]``; numpy in -> numpy out, a CUDA tensor (any byte offset) in -> the result stays on its device."""
+    on_device = not isinstance(image, np.ndarray)
+    torch, device = rt.torch_cuda(image.device if on_device else device)
+    lib = rt.load_library()
+    if image.ndim != 3 or image.shape[2] != 3 or image.dtype != (np.uint8 if not on_device else torch.uint8):
+        raise ValueError("equalize_hist: expected a uint8 [H, W, 3] image")
+    img = _device_image(torch, device, image)
+    h, w = int(img.shape[0]), int(img.shape[1])
+    hist = torch.empty(3 * 256, dtype=torch.int32, device=device)
+    lut = torch.empty(3 * 256, dtype=torch.uint8, device=device)
+    out = torch.empty_like(img)
+    with torch.cuda.device(device):
+        rt.check(lib.apap_equalize_hist(img.data_ptr(), h, w, hist.data_ptr(), lut.data_ptr(), out.data_ptr(),
+                                        rt.stream_ptr(torch, device)), "apap_equalize_hist")
+    return out if on_device else rt.to_host(torch, out)
 
 
 def coarse_matching(c_img, o_img, raw_kpts_cp, raw_kpts_op, device=None, describe="opencv"):
@@ -258,3 +293,36 @@ def coarse_matching(c_img, o_img, raw_kpts_cp, raw_kpts_op, device=None, describ
         raise ValueError(f"coarse_matching: describe must be 'opencv' or 'gpu', got {describe!r}")
     matches = [cv.DMatch(i, int(j), 0, float(d)) for i, (j, d) in enumerate(zip(idx, dist)) if j >= 0]
     return kpts_cp, feats_cp, kpts_op, feats_op, matches
+
+
+def keypoint_pairs(center_img, other_img, raw_kpts_cp, raw_kpts_op, *, equalize=True, device=None):
+    """``(final_src, final_dst, H)`` of the reference's ``visualize_feature_pairs(center, other, swap=True)``
+    (baseline_stitch_test.py:18-61, SURVEY 3.1) on arrays, without the ``.mat`` keypoint loading and the plots: what
+    ``driver.stitch_pair`` takes.  Each image is uploaded once, equalised per channel (``equalize``: the reference
+    describes ``visualize_equalized_hist``'s output, pyviz/apap.py:234-236) and described at ``float32(raw_kpts)``
+    with size 1 and angle -1 on the device; the centre descriptors are matched against the other image's
+    (``apap_match_nn``, exact nearest neighbour), and only the train indices come back.  Then, on the host:
+    ``H, mask = cv.findHomography(centre, other, cv.RANSAC, 5.0)``, ``H = inv(H)`` and ``(other[mask], centre[mask],
+    H)`` -- final_src are other-image points, final_dst centre-image points, and H maps other -> centre.  No
+    ``cv.KeyPoint`` or ``cv.DMatch`` is built.
+
+    ``equalize=False`` is for images that are already equalised (equalising twice is not the identity).  Fewer than 4
+    matches, or no homography from RANSAC, raise ``ValueError``."""
+    import cv2 as cv
+
+    torch, device = rt.torch_cuda(device if device is not None else
+                                  (center_img.device if not isinstance(center_img, np.ndarray) else None))
+    raw_cp = np.asarray(raw_kpts_cp, dtype=np.float32).reshape(-1, 2)
+    raw_op = np.asarray(raw_kpts_op, dtype=np.float32).reshape(-1, 2)
+    feats_cp = sift_describe(_device_image(torch, device, center_img), raw_cp, equalize=equalize)
+    feats_op = sift_describe(_device_image(torch, device, other_img), raw_op, equalize=equalize)
+    idx = rt.to_host(torch, match_descriptors(feats_cp, feats_op, device=device)[0])
+    q = np.flatnonzero(idx >= 0)
+    if len(q) < 4:
+        raise ValueError(f"keypoint_pairs: {len(q)} matches, a homography needs at least 4")
+    centre, other = raw_cp[q], raw_op[idx[q]]
+    h, mask = cv.findHomography(centre, other, cv.RANSAC, 5.0)
+    if h is None:
+        raise ValueError("keypoint_pairs: RANSAC found no homography")
+    mask = mask.ravel().astype(bool)
+    return other[mask], centre[mask], np.linalg.inv(h)

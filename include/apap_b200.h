@@ -356,6 +356,26 @@ int apap_sift_describe(const uint8_t *bgr, int h, int w, const float *pts, int n
                        float ori, float *base_scratch, float *desc, void *stream);
 
 /*
+ * apap_sift_describe of the image seen through a per-channel LUT: the descriptors of the image whose byte (y, x, c) is
+ * lut[c][bgr[y][x][c]], without that image being written (the LUT is read in the gray conversion).  With the LUT of
+ * apap_equalize_hist this describes the per-channel equalised image, as the reference does (pyviz/apap.py:234-236).
+ *   lut : uint8 [3][256] (device, B G R), not null;  every other argument as in apap_sift_describe
+ */
+int apap_sift_describe_lut(const uint8_t *bgr, int h, int w, const uint8_t *lut, const float *pts, int n_kp,
+                           const float *table, int n_samples, float ori, float *base_scratch, float *desc, void *stream);
+
+/*
+ * Per-channel histogram equalisation: cv.merge([cv.equalizeHist(c) for c in cv.split(image)]) of the reference's
+ * visualize_equalized_hist (pyviz/utils.py:85-91), bit for bit.  Histograms, then OpenCV's LUT per channel, then
+ * (when out is given) the equalised image.
+ *   bgr  : uint8 [h][w][3] (device), any byte alignment;  h, w > 0, h w <= INT_MAX
+ *   hist : uint32 [3][256] scratch (device), zeroed here;  out: the three histograms
+ *   lut  : out uint8 [3][256] (device): OpenCV's LUT per channel (entries below the first non-zero bin are 0)
+ *   out  : nullable out uint8 [h][w][3] (device): lut[c][bgr[y][x][c]]
+ */
+int apap_equalize_hist(const uint8_t *bgr, int h, int w, uint32_t *hist, uint8_t *lut, uint8_t *out, void *stream);
+
+/*
  * Panorama assembly of a sharded pass without an all-gather: broadcast `bytes` of device memory at `src` (this
  * rank's row band, already warped) into every GPU's panorama through an NVLS multicast mapping -- `multicast_dst` is
  * the band's address inside the multicast mapping of the panorama buffers (torch symmetric memory's multicast_ptr +
