@@ -29,6 +29,7 @@ EIG_JACOBI = 1
 WARP_FORCE_EXACT = 1
 WARP_LEGACY = 2
 WARP_TILE_FUSED = 4
+RANSAC_MAX_ITERS = 1 << 20
 
 # symbol -> (restype, argtypes); tests check every symbol of include/apap_b200.h is exported
 SIGNATURES = {
@@ -67,6 +68,9 @@ SIGNATURES = {
     "apap_sift_describe_lut": (c_int, [c_void_p, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p, c_int, c_float, c_void_p,
                                        c_void_p, c_void_p]),
     "apap_equalize_hist": (c_int, [c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "apap_ransac_workspace_bytes": (c_int, [c_int, POINTER(c_size_t)]),
+    "apap_ransac_homography": (c_int, [c_void_p, c_void_p, c_int, c_double, c_int, c_void_p, c_size_t, c_void_p, c_void_p,
+                                       c_void_p, c_void_p, c_void_p]),
     "apap_invert_grid": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p]),
     "apap_kp_rows": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_double, c_void_p, c_void_p]),
     "apap_condition": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
@@ -152,6 +156,18 @@ def to_host(torch, dev_tensor) -> np.ndarray:
     out.copy_(dev_tensor, non_blocking=True)
     torch.cuda.current_stream(dev_tensor.device).synchronize()
     return out.numpy()
+
+
+def to_host_many(torch, dev_tensors) -> list:
+    """D2H of several tensors of one device into fresh pinned memory with a single synchronise."""
+    outs = []
+    for t in dev_tensors:
+        out = torch.empty(t.shape, dtype=t.dtype, pin_memory=True)
+        out.copy_(t, non_blocking=True)
+        outs.append(out)
+    if dev_tensors:
+        torch.cuda.current_stream(dev_tensors[0].device).synchronize()
+    return [o.numpy() for o in outs]
 
 
 def pinned_empty(shape, dtype=np.uint8) -> np.ndarray:

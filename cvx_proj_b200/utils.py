@@ -16,13 +16,14 @@ No CPU fallback.
 from __future__ import annotations
 
 import ctypes
+import math
 
 import numpy as np
 
 from . import _runtime as rt
 
 __all__ = ["image_warping", "warp_perspective", "warping_canvas", "invert3x3", "match_descriptors", "coarse_matching",
-           "sift_describe", "equalize_hist", "keypoint_pairs"]
+           "sift_describe", "equalize_hist", "keypoint_pairs", "find_homography_ransac"]
 
 
 def invert3x3(m) -> np.ndarray:
@@ -295,7 +296,119 @@ def coarse_matching(c_img, o_img, raw_kpts_cp, raw_kpts_op, device=None, describ
     return kpts_cp, feats_cp, kpts_op, feats_op, matches
 
 
-def keypoint_pairs(center_img, other_img, raw_kpts_cp, raw_kpts_op, *, equalize=True, device=None):
+RANSAC_MODEL_POINTS = 4
+
+
+def _ransac_update_num_iters(p, ep, model_points, max_iters):
+    """OpenCV's ``RANSACUpdateNumIters``: the iterations that reach confidence ``p`` at outlier ratio ``ep``."""
+    p, ep = min(max(p, 0.0), 1.0), min(max(ep, 0.0), 1.0)
+    num = max(1.0 - p, np.finfo(np.float64).tiny)
+    denom = 1.0 - math.pow(1.0 - ep, model_points)
+    if denom < np.finfo(np.float64).tiny:
+        return 0
+    num, denom = math.log(num), math.log(denom)
+    return max_iters if denom >= 0 or -num >= max_iters * (-denom) else int(round(num / denom))   # cvRound
+
+
+def _inliers(src, dst, H, thr_sq):
+    """``computeError`` (float32, OpenCV's operation order, each step rounded on its own) ``<= thr_sq``."""
+    hf = np.asarray(H, np.float64).ravel()[:8].astype(np.float32)
+    x, y = src[:, 0], src[:, 1]
+    with np.errstate(all="ignore"):                     # non-finite points: NaN errors, never inliers (as in OpenCV)
+        ww = np.float32(1.0) / (hf[6] * x + hf[7] * y + np.float32(1.0))
+        dx = (hf[0] * x + hf[1] * y + hf[2]) * ww - dst[:, 0]
+        dy = (hf[3] * x + hf[4] * y + hf[5]) * ww - dst[:, 1]
+        return dx * dx + dy * dy <= thr_sq
+
+
+def find_homography_ransac(src, dst, threshold=5.0, *, confidence=0.995, max_iters=2000, device=None):
+    """``cv.findHomography(src, dst, cv.RANSAC, threshold, maxIters=max_iters, confidence=confidence)`` with its
+    hypothesis loop on the GPU (``apap_ransac_homography``): ``(H float64 [3, 3], mask uint8 [n, 1])``, or ``(None,
+    zeros)`` when OpenCV finds no model.  ``src`` / ``dst``: ``[n, 2]`` numpy arrays or CUDA tensors (float32 as OpenCV
+    converts them).
+
+    One device call draws OpenCV's subsets and fits and scores every hypothesis exactly as OpenCV does (its RNG, its
+    subset checks, ``runKernel`` with ``cv::eigen``'s Jacobi, the float32 error); one download brings back the subsets
+    and counts.  The adaptive stop is applied to the counts here, the chosen hypothesis is OpenCV's own fit of its 4
+    points (``cv.findHomography(4 points, 0)`` runs the same ``runKernel``), its inlier mask is computed in numpy
+    float32 in OpenCV's order, and ``cv.findHomography(src[mask], dst[mask], 0)`` -- ``runKernel`` + LM on the
+    inliers, which is what ``findHomography`` runs -- gives H; the returned mask is recomputed from that H.  H and
+    mask are OpenCV's bit for bit, except when the best hypothesis has exactly 4 inliers: OpenCV then refits and
+    LM-refines those 4 points, which ``findHomography(4 points, 0)`` does not, so H agrees to about 1e-12 relative
+    (the mask is still OpenCV's).  Fewer than 4 points raise ``ValueError`` (OpenCV raises ``cv.error``)."""
+    on_device = not isinstance(src, np.ndarray) and hasattr(src, "device")
+    torch, device = rt.torch_cuda(src.device if on_device else device)
+    if on_device:
+        s_dev = src.to(device=device, dtype=torch.float32).reshape(-1, 2).contiguous()
+        d_dev = dst.to(device=device, dtype=torch.float32).reshape(-1, 2).contiguous()
+        s_host = d_host = None
+    else:
+        s_host = np.ascontiguousarray(np.asarray(src, np.float32).reshape(-1, 2))
+        d_host = np.ascontiguousarray(np.asarray(dst, np.float32).reshape(-1, 2))
+        s_dev, d_dev = rt.to_device(torch, device, s_host), rt.to_device(torch, device, d_host)
+    return _ransac(torch, device, s_dev, d_dev, s_host, d_host, threshold, confidence, max_iters)
+
+
+def _ransac(torch, device, s_dev, d_dev, s_host, d_host, threshold, confidence, max_iters):
+    """``find_homography_ransac`` on float32 ``[n, 2]`` device points; ``s_host`` / ``d_host`` are their host copies,
+    or ``None`` to download them with the counts."""
+    import cv2 as cv
+
+    if not 0.0 < confidence < 1.0:
+        raise ValueError(f"find_homography_ransac: confidence must be in (0, 1), got {confidence}")
+    n = int(s_dev.shape[0])
+    if n < RANSAC_MODEL_POINTS or int(d_dev.shape[0]) != n:
+        raise ValueError(f"find_homography_ransac: needs at least 4 corresponding points, got {n} and {int(d_dev.shape[0])}")
+    if threshold <= 0:
+        threshold = 3.0                                 # OpenCV's defaultRANSACReprojThreshold
+    max_iters = max(int(max_iters), 1)
+    if max_iters > rt.RANSAC_MAX_ITERS:
+        raise ValueError(f"find_homography_ransac: max_iters must be <= {rt.RANSAC_MAX_ITERS}")
+    down = []
+    if n > RANSAC_MODEL_POINTS:
+        lib = rt.load_library()
+        ws_bytes = ctypes.c_size_t()
+        rt.check(lib.apap_ransac_workspace_bytes(max_iters, ctypes.byref(ws_bytes)), "apap_ransac_workspace_bytes")
+        ws = torch.empty(ws_bytes.value, dtype=torch.uint8, device=device)
+        out = torch.empty(5 * max_iters + 1, dtype=torch.int32, device=device)     # subsets | counts | n_sampled
+        hyps = torch.empty((max_iters, 9), dtype=torch.float64, device=device)
+        with torch.cuda.device(device):
+            rt.check(lib.apap_ransac_homography(s_dev.data_ptr(), d_dev.data_ptr(), n, float(threshold), max_iters,
+                                                ws.data_ptr(), ws_bytes.value, out.data_ptr(), hyps.data_ptr(),
+                                                out.data_ptr() + 16 * max_iters, out.data_ptr() + 20 * max_iters,
+                                                rt.stream_ptr(torch, device)), "apap_ransac_homography")
+        down.append(out)
+    if s_host is None:
+        down += [s_dev, d_dev]
+    down = rt.to_host_many(torch, down)
+    if s_host is None:
+        s_host, d_host = down[-2], down[-1]
+    if n == RANSAC_MODEL_POINTS:                        # findHomography: method 0 on the 4 points, mask all ones
+        H = cv.findHomography(s_host, d_host, 0)[0]
+        return H, (np.ones if H is not None else np.zeros)((n, 1), np.uint8)
+    subsets = down[0][:4 * max_iters].reshape(-1, 4)
+    counts, n_sampled = down[0][4 * max_iters:5 * max_iters], int(down[0][-1])
+    # RANSACPointSetRegistrator::run over the counts: a hypothesis is kept when it beats max(best, 3)
+    niters, best, max_good, it = max_iters, -1, 0, 0
+    while it < niters and it < n_sampled:
+        good = int(counts[it])
+        if good > max(max_good, RANSAC_MODEL_POINTS - 1):
+            best, max_good = it, good
+            niters = _ransac_update_num_iters(confidence, (n - good) / n, RANSAC_MODEL_POINTS, niters)
+        it += 1
+    if best < 0:
+        return None, np.zeros((n, 1), np.uint8)
+    thr_sq = np.float32(float(threshold) * float(threshold))
+    sub = subsets[best]
+    mask = _inliers(s_host, d_host, cv.findHomography(s_host[sub], d_host[sub], 0)[0], thr_sq)
+    if int(mask.sum()) != max_good:                     # the device fit and counts are OpenCV's: never expected
+        raise rt.ApapError(f"find_homography_ransac: hypothesis {best} has {max_good} inliers on the device but "
+                           f"{int(mask.sum())} under OpenCV's fit of the same subset")
+    H = cv.findHomography(s_host[mask], d_host[mask], 0)[0]
+    return H, _inliers(s_host, d_host, H, thr_sq).astype(np.uint8).reshape(-1, 1)
+
+
+def keypoint_pairs(center_img, other_img, raw_kpts_cp, raw_kpts_op, *, equalize=True, device=None, ransac="opencv"):
     """``(final_src, final_dst, H)`` of the reference's ``visualize_feature_pairs(center, other, swap=True)``
     (baseline_stitch_test.py:18-61, SURVEY 3.1) on arrays, without the ``.mat`` keypoint loading and the plots: what
     ``driver.stitch_pair`` takes.  Each image is uploaded once, equalised per channel (``equalize``: the reference
@@ -307,21 +420,36 @@ def keypoint_pairs(center_img, other_img, raw_kpts_cp, raw_kpts_op, *, equalize=
     ``cv.KeyPoint`` or ``cv.DMatch`` is built.
 
     ``equalize=False`` is for images that are already equalised (equalising twice is not the identity).  Fewer than 4
-    matches, or no homography from RANSAC, raise ``ValueError``."""
+    matches, or no homography from RANSAC, raise ``ValueError``.
+
+    ``ransac`` picks where the RANSAC runs: ``"opencv"`` (default) calls ``cv.findHomography`` on the host; ``"gpu"``
+    gathers the matched points on the device from the train indices the matcher left there and runs
+    ``find_homography_ransac`` on them -- the same ``(final_src, final_dst, H)`` bit for bit (see that function for
+    the one case where its H is only within ~1e-12 of OpenCV's)."""
     import cv2 as cv
 
+    if ransac not in ("opencv", "gpu"):
+        raise ValueError(f"keypoint_pairs: ransac must be 'opencv' or 'gpu', got {ransac!r}")
     torch, device = rt.torch_cuda(device if device is not None else
                                   (center_img.device if not isinstance(center_img, np.ndarray) else None))
     raw_cp = np.asarray(raw_kpts_cp, dtype=np.float32).reshape(-1, 2)
     raw_op = np.asarray(raw_kpts_op, dtype=np.float32).reshape(-1, 2)
-    feats_cp = sift_describe(_device_image(torch, device, center_img), raw_cp, equalize=equalize)
-    feats_op = sift_describe(_device_image(torch, device, other_img), raw_op, equalize=equalize)
-    idx = rt.to_host(torch, match_descriptors(feats_cp, feats_op, device=device)[0])
+    pts_cp, pts_op = rt.to_device(torch, device, raw_cp), rt.to_device(torch, device, raw_op)
+    feats_cp = sift_describe(_device_image(torch, device, center_img), pts_cp, equalize=equalize)
+    feats_op = sift_describe(_device_image(torch, device, other_img), pts_op, equalize=equalize)
+    idx_dev = match_descriptors(feats_cp, feats_op, device=device)[0]
+    idx = rt.to_host(torch, idx_dev)
     q = np.flatnonzero(idx >= 0)
     if len(q) < 4:
         raise ValueError(f"keypoint_pairs: {len(q)} matches, a homography needs at least 4")
     centre, other = raw_cp[q], raw_op[idx[q]]
-    h, mask = cv.findHomography(centre, other, cv.RANSAC, 5.0)
+    if ransac == "gpu":
+        q_dev = torch.nonzero(idx_dev >= 0).squeeze(1)
+        h, mask = _ransac(torch, device, pts_cp.index_select(0, q_dev),
+                          pts_op.index_select(0, idx_dev.index_select(0, q_dev).long()), centre, other, 5.0, 0.995,
+                          2000)
+    else:
+        h, mask = cv.findHomography(centre, other, cv.RANSAC, 5.0)
     if h is None:
         raise ValueError("keypoint_pairs: RANSAC found no homography")
     mask = mask.ravel().astype(bool)

@@ -376,6 +376,32 @@ int apap_sift_describe_lut(const uint8_t *bgr, int h, int w, const uint8_t *lut,
 int apap_equalize_hist(const uint8_t *bgr, int h, int w, uint32_t *hist, uint8_t *lut, uint8_t *out, void *stream);
 
 /*
+ * The hypothesis loop of cv.findHomography(src, dst, cv.RANSAC, threshold) (OpenCV 4.x RANSACPointSetRegistrator) in
+ * the reference's keypoint-pair producer (baseline_stitch_test.py:41): every hypothesis the loop can draw, up to
+ * max_iters, with its inlier count.  The subsets come from OpenCV's cv::RNG(0xFFFFFFFFFFFFFFFF) stream with its
+ * duplicate rejection, checkSubset and the 10000-attempt limit; the counts use computeError's float32 arithmetic, so
+ * subsets and counts are OpenCV's.  The caller applies the adaptive stop (RANSACUpdateNumIters) to the counts and
+ * refits the chosen hypothesis's inliers (cvx_proj_b200.utils.find_homography_ransac).
+ *   src, dst   : float [n][2] (device, 8-byte aligned), n >= 5;  threshold > 0 (pixels; inlier: err <= (float)(t t))
+ *   max_iters  : 1 .. APAP_RANSAC_MAX_ITERS;  workspace: device scratch of apap_ransac_workspace_bytes, 16-byte aligned
+ *   subsets    : out int32 [max_iters][4] (device, 16-byte aligned), the accepted subsets in draw order
+ *   hyps       : out double [max_iters][9] (device, 8-byte aligned): each subset's homography, OpenCV's runKernel
+ *                bit for bit (cv::eigen's Jacobi restated; H22 = 1; NaN when runKernel finds 0 models)
+ *   counts     : out int32 [max_iters] (device, 4-byte aligned): inliers of each hypothesis, -1 for 0 models
+ *   n_sampled  : out int32 [1] (device, 4-byte aligned): hypotheses filled; < max_iters when the attempt limit ended
+ *                the sequence (0: OpenCV finds no model)
+ * All max_iters subsets are drawn whatever the adaptive stop would do (the counts that decide it come after), so on
+ * degenerate data -- most candidates rejected by checkSubset -- the sampler can run up to 10000 candidates per
+ * subset, max_iters x 10000 in all, on one warp: about 16 us per 32 candidates on a B200, i.e. seconds at the
+ * default 2000.  OpenCV may stop after one hypothesis on such data.
+ */
+#define APAP_RANSAC_MAX_ITERS (1 << 20)
+int apap_ransac_workspace_bytes(int max_iters, size_t *bytes);
+int apap_ransac_homography(const float *src, const float *dst, int n, double threshold, int max_iters, void *workspace,
+                           size_t workspace_bytes, int *subsets, double *hyps, int *counts, int *n_sampled,
+                           void *stream);
+
+/*
  * Panorama assembly of a sharded pass without an all-gather: broadcast `bytes` of device memory at `src` (this
  * rank's row band, already warped) into every GPU's panorama through an NVLS multicast mapping -- `multicast_dst` is
  * the band's address inside the multicast mapping of the panorama buffers (torch symmetric memory's multicast_ptr +
