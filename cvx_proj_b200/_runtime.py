@@ -71,6 +71,9 @@ SIGNATURES = {
     "apap_ransac_workspace_bytes": (c_int, [c_int, POINTER(c_size_t)]),
     "apap_ransac_homography": (c_int, [c_void_p, c_void_p, c_int, c_double, c_int, c_void_p, c_size_t, c_void_p, c_void_p,
                                        c_void_p, c_void_p, c_void_p]),
+    "apap_ransac_batch_workspace_bytes": (c_int, [c_int, c_int, POINTER(c_size_t)]),
+    "apap_ransac_homography_batch": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_double, c_int, c_void_p,
+                                             c_size_t, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "apap_invert_grid": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p]),
     "apap_kp_rows": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_double, c_void_p, c_void_p]),
     "apap_condition": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),

@@ -868,7 +868,9 @@ class APAP:
     def local_homography_batch(self, src_points, dst_points, vertices):
         """Extension (no reference API; its multi-image mode is a shell loop, run_all.sh:15,29):
         several pairs in one launch.  ``vertices`` is one ``[mesh_n, pt_size, 2]`` array shared by
-        all pairs or a list of them (same shape).  Each item equals the single-pair call."""
+        all pairs or a list of them (same shape).  Each item equals the single-pair call when the pairs' keypoint
+        counts give the same Gram split plan (equal counts always do): the plan follows the largest count, so a
+        smaller pair's grid can otherwise differ from its single call in the last bits."""
         count = len(src_points)
         verts = vertices if isinstance(vertices, (list, tuple)) else [vertices] * count
         mesh_n, pt_size, _ = np.shape(verts[0])

@@ -5,13 +5,19 @@
 //   k_ransac_sample : one warp.  Lane 0 runs cv::RNG(0xFFFFFFFFFFFFFFFF) serially and draws 32 candidate subsets of 4
 //                     distinct indices (getSubset); the 32 lanes run checkSubset on them at once; lane 0 keeps the
 //                     accepted ones in draw order.  10000 rejected candidates in a row end the sequence (getSubset
-//                     fails: the loop breaks, or has no model when that happens on iteration 0).
+//                     fails: the loop breaks, or has no model when that happens on iteration 0).  One warp (CTA)
+//                     per pair, each pair on its own cv::RNG(0xFFFFFFFFFFFFFFFF) like a separate findHomography call.
 //   k_ransac_fit    : one thread per hypothesis: runKernel in float64 step by step (centroid, mean absolute
 //                     deviation, the DBL_EPSILON exit, LtL, cv::eigen's cyclic Jacobi, H = invHnorm V8 Hnorm2 / H22),
-//                     every operation rounded on its own, so each hypothesis is OpenCV's bit for bit.
-//   k_ransac_score  : a CTA takes 32 hypotheses and 1024 points: computeError in float32 with every operation rounded
-//                     on its own (no contraction), err <= (float)(thr * thr), integer counts by warp reductions and
-//                     atomics (exact in any order).  Invalid hypotheses (0 models) keep count -1.
+//                     every operation rounded on its own, so each hypothesis is OpenCV's bit for bit.  One thread per
+//                     (pair, hypothesis).
+//   k_ransac_score  : a CTA takes 32 hypotheses of one pair and walks that pair's points 1024 at a time with a grid
+//                     stride: computeError in float32 with every operation rounded on its own (no contraction),
+//                     err <= (float)(thr * thr), integer counts by warp reductions and atomics (exact in any order).
+//                     Invalid hypotheses (0 models) keep count -1.
+// A batch is independent point sets stored back to back, pair p at [offsets[p], offsets[p + 1]); every output is laid
+// out [batch][max_iters]..., and pair p's record is the record of a single call on its points.  The single call
+// (apap_ransac_homography) is a batch of one with offsets == nullptr: its pair is [0, max_n).
 #include <cfloat>
 
 #include "common.cuh"
@@ -26,6 +32,12 @@ constexpr int kScoreHyps = 32;                     // hypotheses per CTA
 constexpr int kScorePtsPerThread = 4;
 constexpr int kScorePts = kScoreThreads * kScorePtsPerThread;
 constexpr int kHf = 9;                             // workspace row: (float)H[0..7], valid flag
+constexpr int kMaxGridZ = 65535;                   // pairs per score launch
+
+// [begin, end) of pair p's points
+__device__ __forceinline__ int2 pair_range(const int *__restrict__ offsets, int p, int max_n) {
+  return offsets ? make_int2(offsets[p], offsets[p + 1]) : make_int2(0, max_n);
+}
 
 // ------------------------------------------------------------------------------------------------ checkSubset
 // haveCollinearPoints(m, 4): the last point against the line through each pair of the earlier three.  Point2f
@@ -71,10 +83,19 @@ __device__ __forceinline__ uint32_t rng_uniform(unsigned long long &state, uint3
 }
 
 __global__ void __launch_bounds__(32) k_ransac_sample(const float2 *__restrict__ src, const float2 *__restrict__ dst,
-                                                      int n, int max_iters, int4 *__restrict__ subsets,
-                                                      int *__restrict__ n_sampled) {
+                                                      const int *__restrict__ offsets, int max_n, int max_iters,
+                                                      int4 *__restrict__ subsets, int *__restrict__ n_sampled) {
   __shared__ int4 cand[32];
-  const int lane = threadIdx.x;
+  const int lane = threadIdx.x, pair = blockIdx.x;
+  const int2 r = pair_range(offsets, pair, max_n);
+  const int n = r.y - r.x;
+  if (n < 5) {                                      // 4 points are a single fit; fewer could never draw 4 distinct
+    if (lane == 0) n_sampled[pair] = 0;
+    return;
+  }
+  src += r.x;
+  dst += r.x;
+  subsets += (size_t)pair * max_iters;
   unsigned long long state = ~0ull;                 // lane 0's RNG
   int accepted = 0, run = 0;                        // run: rejected candidates since the last accepted one
   bool done = false;
@@ -116,7 +137,7 @@ __global__ void __launch_bounds__(32) k_ransac_sample(const float2 *__restrict__
     done = __shfl_sync(0xffffffffu, done, 0);
     __syncwarp();
   }
-  if (lane == 0) *n_sampled = accepted;
+  if (lane == 0) n_sampled[pair] = accepted;
 }
 
 // ------------------------------------------------------------------------------------------------ runKernel
@@ -238,19 +259,22 @@ __device__ __forceinline__ void mat3(const double (&a)[9], const double (&b)[9],
 
 __global__ void __launch_bounds__(kFitThreads) k_ransac_fit(const float2 *__restrict__ src,
                                                             const float2 *__restrict__ dst,
-                                                            const int4 *__restrict__ subsets,
+                                                            const int *__restrict__ offsets, int max_n, int batch,
+                                                            int max_iters, const int4 *__restrict__ subsets,
                                                             const int *__restrict__ n_sampled,
                                                             double *__restrict__ hyps, float *__restrict__ hf,
                                                             int *__restrict__ counts) {
-  const int h = blockIdx.x * kFitThreads + threadIdx.x;
-  if (h >= *n_sampled) return;
+  const int h = blockIdx.x * kFitThreads + threadIdx.x;   // (pair, hypothesis); batch * max_iters <= 2^20
+  const int pair = h / max_iters;
+  if (pair >= batch || h - pair * max_iters >= n_sampled[pair]) return;
+  const int base = pair_range(offsets, pair, max_n).x;
   const int4 q = subsets[h];
   const int id[4] = {q.x, q.y, q.z, q.w};
   float2 M[4], m[4];
 #pragma unroll
   for (int i = 0; i < 4; ++i) {
-    M[i] = src[id[i]];
-    m[i] = dst[id[i]];
+    M[i] = src[base + id[i]];
+    m[i] = dst[base + id[i]];
   }
   double cmx = 0, cmy = 0, cMx = 0, cMy = 0;
 #pragma unroll
@@ -314,65 +338,83 @@ __global__ void __launch_bounds__(kFitThreads) k_ransac_fit(const float2 *__rest
 
 // ------------------------------------------------------------------------------------------------ computeError
 __global__ void __launch_bounds__(kScoreThreads) k_ransac_score(const float2 *__restrict__ src,
-                                                                const float2 *__restrict__ dst, int n,
+                                                                const float2 *__restrict__ dst,
+                                                                const int *__restrict__ offsets, int max_n,
+                                                                int pair0, int max_iters,
                                                                 const float *__restrict__ hf,
                                                                 const int *__restrict__ n_sampled, float thr_sq,
                                                                 int *__restrict__ counts) {
   __shared__ float hs[kScoreHyps][kHf];
   __shared__ int cnt[kScoreHyps];
-  const int h0 = blockIdx.y * kScoreHyps;
-  const int nh = min(kScoreHyps, *n_sampled - h0);
+  const int pair = pair0 + blockIdx.z;
+  const size_t h0 = (size_t)pair * max_iters + blockIdx.y * kScoreHyps;   // first hypothesis of the CTA
+  const int nh = min(kScoreHyps, n_sampled[pair] - (int)blockIdx.y * kScoreHyps);
   if (nh <= 0) return;
-  for (int i = threadIdx.x; i < nh * kHf; i += kScoreThreads) hs[i / kHf][i % kHf] = hf[(size_t)h0 * kHf + i];
+  const int2 r = pair_range(offsets, pair, max_n);
+  const int n = r.y - r.x;
+  src += r.x;
+  dst += r.x;
+  for (int i = threadIdx.x; i < nh * kHf; i += kScoreThreads) hs[i / kHf][i % kHf] = hf[h0 * kHf + i];
   if (threadIdx.x < kScoreHyps) cnt[threadIdx.x] = 0;
   __syncthreads();
-  float2 M[kScorePtsPerThread], m[kScorePtsPerThread];
-  bool live[kScorePtsPerThread];
-  const int p0 = blockIdx.x * kScorePts + threadIdx.x;
-#pragma unroll
-  for (int k = 0; k < kScorePtsPerThread; ++k) {
-    const int p = p0 + k * kScoreThreads;
-    live[k] = p < n;
-    M[k] = live[k] ? src[p] : make_float2(0.f, 0.f);
-    m[k] = live[k] ? dst[p] : make_float2(0.f, 0.f);
-  }
   const int lane = threadIdx.x & 31;
-  for (int j = 0; j < nh; ++j) {
-    if (hs[j][8] == 0.f) continue;                  // invalid hypothesis: uniform across the CTA
-    const float *H = hs[j];
-    int c = 0;
+  for (int chunk = blockIdx.x; chunk * kScorePts < n; chunk += gridDim.x) {   // a pair beyond max_n is still counted
+    float2 M[kScorePtsPerThread], m[kScorePtsPerThread];
+    bool live[kScorePtsPerThread];
+    const int p0 = chunk * kScorePts + threadIdx.x;
 #pragma unroll
     for (int k = 0; k < kScorePtsPerThread; ++k) {
-      const float x = M[k].x, y = M[k].y;
-      const float ww = __fdiv_rn(1.f, __fadd_rn(__fadd_rn(__fmul_rn(H[6], x), __fmul_rn(H[7], y)), 1.f));
-      const float dx = __fsub_rn(__fmul_rn(__fadd_rn(__fadd_rn(__fmul_rn(H[0], x), __fmul_rn(H[1], y)), H[2]), ww), m[k].x);
-      const float dy = __fsub_rn(__fmul_rn(__fadd_rn(__fadd_rn(__fmul_rn(H[3], x), __fmul_rn(H[4], y)), H[5]), ww), m[k].y);
-      const float e = __fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy));
-      c += (live[k] && e <= thr_sq) ? 1 : 0;
+      const int p = p0 + k * kScoreThreads;
+      live[k] = p < n;
+      M[k] = live[k] ? src[p] : make_float2(0.f, 0.f);
+      m[k] = live[k] ? dst[p] : make_float2(0.f, 0.f);
     }
-    c = __reduce_add_sync(0xffffffffu, c);
-    if (lane == 0 && c) atomicAdd(&cnt[j], c);
+    for (int j = 0; j < nh; ++j) {
+      if (hs[j][8] == 0.f) continue;                // invalid hypothesis: uniform across the CTA
+      const float *H = hs[j];
+      int c = 0;
+#pragma unroll
+      for (int k = 0; k < kScorePtsPerThread; ++k) {
+        const float x = M[k].x, y = M[k].y;
+        const float ww = __fdiv_rn(1.f, __fadd_rn(__fadd_rn(__fmul_rn(H[6], x), __fmul_rn(H[7], y)), 1.f));
+        const float dx = __fsub_rn(__fmul_rn(__fadd_rn(__fadd_rn(__fmul_rn(H[0], x), __fmul_rn(H[1], y)), H[2]), ww), m[k].x);
+        const float dy = __fsub_rn(__fmul_rn(__fadd_rn(__fadd_rn(__fmul_rn(H[3], x), __fmul_rn(H[4], y)), H[5]), ww), m[k].y);
+        const float e = __fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy));
+        c += (live[k] && e <= thr_sq) ? 1 : 0;
+      }
+      c = __reduce_add_sync(0xffffffffu, c);
+      if (lane == 0 && c) atomicAdd(&cnt[j], c);
+    }
   }
   __syncthreads();
   if (threadIdx.x < nh && hs[threadIdx.x][8] != 0.f && cnt[threadIdx.x]) atomicAdd(counts + h0 + threadIdx.x, cnt[threadIdx.x]);
 }
 
-static size_t ransac_workspace(int max_iters) {
-  return ((size_t)max_iters * kHf * sizeof(float) + 255) & ~(size_t)255;
+static size_t ransac_workspace(size_t hyps) {
+  return (hyps * kHf * sizeof(float) + 255) & ~(size_t)255;
 }
 
-int launch_ransac(const float2 *src, const float2 *dst, int n, double threshold, int max_iters, float *hf, int4 *subsets,
-                  double *hyps, int *counts, int *n_sampled, cudaStream_t st) {
-  k_ransac_sample<<<1, 32, 0, st>>>(src, dst, n, max_iters, subsets, n_sampled);
+// offsets == nullptr: one pair of max_n points
+int launch_ransac(const float2 *src, const float2 *dst, const int *offsets, int batch, int max_n, double threshold,
+                  int max_iters, float *hf, int4 *subsets, double *hyps, int *counts, int *n_sampled, cudaStream_t st) {
+  k_ransac_sample<<<batch, 32, 0, st>>>(src, dst, offsets, max_n, max_iters, subsets, n_sampled);
   int rc = check_cuda(cudaGetLastError(), "k_ransac_sample launch");
   if (rc) return rc;
-  k_ransac_fit<<<(max_iters + kFitThreads - 1) / kFitThreads, kFitThreads, 0, st>>>(src, dst, subsets, n_sampled, hyps,
-                                                                                    hf, counts);
+  const int total = batch * max_iters;
+  k_ransac_fit<<<(total + kFitThreads - 1) / kFitThreads, kFitThreads, 0, st>>>(src, dst, offsets, max_n, batch, max_iters,
+                                                                                subsets, n_sampled, hyps, hf, counts);
   rc = check_cuda(cudaGetLastError(), "k_ransac_fit launch");
   if (rc) return rc;
-  const dim3 grid((n + kScorePts - 1) / kScorePts, (max_iters + kScoreHyps - 1) / kScoreHyps);
-  k_ransac_score<<<grid, kScoreThreads, 0, st>>>(src, dst, n, hf, n_sampled, (float)(threshold * threshold), counts);
-  return check_cuda(cudaGetLastError(), "k_ransac_score launch");
+  const float thr_sq = (float)(threshold * threshold);
+  for (int pair0 = 0; pair0 < batch; pair0 += kMaxGridZ) {
+    const dim3 grid(max((max_n + kScorePts - 1) / kScorePts, 1), (max_iters + kScoreHyps - 1) / kScoreHyps,
+                    min(batch - pair0, kMaxGridZ));
+    k_ransac_score<<<grid, kScoreThreads, 0, st>>>(src, dst, offsets, max_n, pair0, max_iters, hf, n_sampled, thr_sq,
+                                                   counts);
+    rc = check_cuda(cudaGetLastError(), "k_ransac_score launch");
+    if (rc) return rc;
+  }
+  return 0;
 }
 
 }  // namespace apap
@@ -387,12 +429,9 @@ extern "C" int apap_ransac_workspace_bytes(int max_iters, size_t *bytes) {
   return 0;
 }
 
-extern "C" int apap_ransac_homography(const float *src, const float *dst, int n, double threshold, int max_iters,
-                                      void *workspace, size_t workspace_bytes, int *subsets, double *hyps, int *counts,
-                                      int *n_sampled, void *stream) {
-  if (n < 5) return fail(APAP_E_BADARG, "ransac: n must be >= 5 (4 points are a single fit, no sampling)");
-  if (max_iters < 1 || max_iters > APAP_RANSAC_MAX_ITERS)
-    return fail(APAP_E_BADARG, "ransac: max_iters must be in [1, APAP_RANSAC_MAX_ITERS]");
+static int check_ransac_args(double threshold, const void *src, const void *dst, const void *workspace,
+                             size_t workspace_bytes, size_t hyps_total, const int *subsets, const double *hyps,
+                             const int *counts, const int *n_sampled) {
   if (!(threshold > 0.0) || !isfinite(threshold)) return fail(APAP_E_BADARG, "ransac: threshold must be finite and > 0");
   if (!src || !dst || !workspace || !subsets || !hyps || !counts || !n_sampled)
     return fail(APAP_E_BADARG, "ransac: null pointer");
@@ -403,8 +442,51 @@ extern "C" int apap_ransac_homography(const float *src, const float *dst, int n,
   if (reinterpret_cast<uintptr_t>(hyps) & 7u) return fail(APAP_E_BADARG, "ransac: hyps must be 8-byte aligned");
   if ((reinterpret_cast<uintptr_t>(counts) | reinterpret_cast<uintptr_t>(n_sampled)) & 3u)
     return fail(APAP_E_BADARG, "ransac: counts and n_sampled must be 4-byte aligned");
-  if (workspace_bytes < ransac_workspace(max_iters)) return fail(APAP_E_BADARG, "ransac: workspace too small");
-  return launch_ransac(reinterpret_cast<const float2 *>(src), reinterpret_cast<const float2 *>(dst), n, threshold,
-                       max_iters, static_cast<float *>(workspace), reinterpret_cast<int4 *>(subsets), hyps, counts,
-                       n_sampled, static_cast<cudaStream_t>(stream));
+  if (workspace_bytes < ransac_workspace(hyps_total)) return fail(APAP_E_BADARG, "ransac: workspace too small");
+  return 0;
+}
+
+extern "C" int apap_ransac_homography(const float *src, const float *dst, int n, double threshold, int max_iters,
+                                      void *workspace, size_t workspace_bytes, int *subsets, double *hyps, int *counts,
+                                      int *n_sampled, void *stream) {
+  if (n < 5) return fail(APAP_E_BADARG, "ransac: n must be >= 5 (4 points are a single fit, no sampling)");
+  if (max_iters < 1 || max_iters > APAP_RANSAC_MAX_ITERS)
+    return fail(APAP_E_BADARG, "ransac: max_iters must be in [1, APAP_RANSAC_MAX_ITERS]");
+  const int rc = check_ransac_args(threshold, src, dst, workspace, workspace_bytes, max_iters, subsets, hyps, counts,
+                                   n_sampled);
+  if (rc) return rc;
+  return launch_ransac(reinterpret_cast<const float2 *>(src), reinterpret_cast<const float2 *>(dst), nullptr, 1, n,
+                       threshold, max_iters, static_cast<float *>(workspace), reinterpret_cast<int4 *>(subsets), hyps,
+                       counts, n_sampled, static_cast<cudaStream_t>(stream));
+}
+
+static bool batch_fits(int batch, int max_iters) {
+  return batch >= 1 && max_iters >= 1 && (long long)batch * max_iters <= APAP_RANSAC_MAX_ITERS;
+}
+
+extern "C" int apap_ransac_batch_workspace_bytes(int batch, int max_iters, size_t *bytes) {
+  if (!batch_fits(batch, max_iters))
+    return fail(APAP_E_BADARG, "ransac batch: batch and max_iters must be >= 1 with batch * max_iters <= "
+                               "APAP_RANSAC_MAX_ITERS");
+  if (!bytes) return fail(APAP_E_BADARG, "ransac: null pointer");
+  *bytes = ransac_workspace((size_t)batch * max_iters);
+  return 0;
+}
+
+extern "C" int apap_ransac_homography_batch(const float *src, const float *dst, const int *offsets, int batch,
+                                            int max_n, double threshold, int max_iters, void *workspace,
+                                            size_t workspace_bytes, int *subsets, double *hyps, int *counts,
+                                            int *n_sampled, void *stream) {
+  if (!batch_fits(batch, max_iters))
+    return fail(APAP_E_BADARG, "ransac batch: batch and max_iters must be >= 1 with batch * max_iters <= "
+                               "APAP_RANSAC_MAX_ITERS");
+  if (max_n < 0) return fail(APAP_E_BADARG, "ransac batch: max_n must be >= 0");
+  if (!offsets) return fail(APAP_E_BADARG, "ransac: null pointer");
+  if (reinterpret_cast<uintptr_t>(offsets) & 3u) return fail(APAP_E_BADARG, "ransac batch: offsets must be 4-byte aligned");
+  const int rc = check_ransac_args(threshold, src, dst, workspace, workspace_bytes, (size_t)batch * max_iters, subsets,
+                                   hyps, counts, n_sampled);
+  if (rc) return rc;
+  return launch_ransac(reinterpret_cast<const float2 *>(src), reinterpret_cast<const float2 *>(dst), offsets, batch,
+                       max_n, threshold, max_iters, static_cast<float *>(workspace), reinterpret_cast<int4 *>(subsets),
+                       hyps, counts, n_sampled, static_cast<cudaStream_t>(stream));
 }

@@ -8,6 +8,7 @@ inverse + ``/[2, 2]`` + column-major ``[cells, 9]`` float64 layout of the ``.mat
   ``mat_layout``      pyviz/apap.py:250-254,263-264   (in place on the caller's grid, like the script)
   ``save2mat``        pyviz/utils.py:68-70
   ``stitch_pair``     pyviz/apap.py:238-265           (grid, H field, ``.mat`` matrix, stitched image)
+  ``stitch_case``     run_all.sh:15,29                (every image of a case against the centre, from raw keypoints)
 
 The keypoint-pair producer (``visualize_feature_pairs``) and the dataset IO stay with the caller
 (SURVEY.md section 8f, rows N3/N4): ``stitch_pair`` starts where the script has its matched
@@ -21,7 +22,7 @@ import numpy as np
 
 from .apap_utils import final_size, get_mesh, get_vertice
 
-__all__ = ["mat_layout", "save2mat", "stitch_pair", "StitchResult"]
+__all__ = ["mat_layout", "save2mat", "stitch_pair", "stitch_case", "StitchResult"]
 
 
 def mat_layout(local_homography: np.ndarray, stitcher=None) -> np.ndarray:
@@ -90,3 +91,54 @@ def stitch_pair(center_img, other_img, final_src, final_dst, project_h, *, mesh_
         blend_img = center_img if blend_img is None else blend_img
         stitched = stitcher.local_warp_blend(warp_img, local_h.copy(), mesh, blend_img)
     return StitchResult((final_w, final_h, offset_x, offset_y), mesh, vertices, local_h, mat, stitched)
+
+
+def stitch_case(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops, *, mesh_size: int = 100, gamma=0.5, sigma=100,
+                warp_imgs=None, blend_img=None, stitch: bool = True, equalize: bool = True, ransac: str = "opencv",
+                device=None) -> list:
+    """The reference's multi-image mode for one centre: ``pyviz/apap.py <case> <img>`` for every other image of a case
+    (run_all.sh:15,29), from the images and raw keypoints to one ``StitchResult`` per other image.  Element ``i`` is
+    field for field, bit for bit ``stitch_pair(center_img, other_imgs[i], *keypoint_pairs(center_img, other_imgs[i],
+    kc_i, raw_kpts_ops[i], equalize=equalize, ransac=ransac), ...)`` with ``warp_img=warp_imgs[i]``; ``raw_kpts_cp``
+    is one array for all pairs or a list with one per pair (``utils.keypoint_pairs_batch``).
+
+    The keypoint pairs come from ``keypoint_pairs_batch`` (the centre uploaded and described once, one RANSAC batch
+    with ``ransac="gpu"``), and the warp and blend read the images the producer already holds on the device: without
+    ``warp_imgs`` / ``blend_img`` each image crosses PCIe once.  The moving DLT runs per pair (``local_homography``):
+    ``local_homography_batch`` pads every pair to the largest keypoint count, which changes the Gram kernel's split
+    plan, so a smaller pair's grid could differ from ``stitch_pair``'s in the last bits.  ``warp_imgs`` (one per pair) and ``blend_img`` (one for all) are the de-hazed images the script warps
+    and pastes (pyviz/apap.py:245); each is uploaded once.  ``stitched`` comes back as a numpy array.  The ``.mat`` and
+    keypoint files stay with the caller, as for ``stitch_pair``."""
+    from . import _runtime as rt
+    from .apap import APAP
+    from .utils import _device_image, _keypoint_pairs_uploaded
+
+    if warp_imgs is not None and len(warp_imgs) != len(other_imgs):
+        raise ValueError(f"stitch_case: {len(other_imgs)} other images but {len(warp_imgs)} warp images")
+    pairs, centre_dev, other_devs = _keypoint_pairs_uploaded(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops,
+                                                              equalize, device, ransac)
+    if not pairs:
+        return []
+    torch, device = rt.torch_cuda(centre_dev.device)
+    stitchers, meshes, vertices = [], [], []
+    for other_img, (_, _, project_h) in zip(other_imgs, pairs):
+        final_w, final_h, offset_x, offset_y = final_size(center_img, other_img, project_h)
+        meshes.append(get_mesh((final_w, final_h), mesh_size + 1))
+        vertices.append(get_vertice((final_w, final_h), mesh_size, (offset_x, offset_y)))
+        stitchers.append(APAP(gamma, sigma, [final_w, final_h], [offset_x, offset_y], device=device))
+    # per pair, not local_homography_batch: a batch pads every pair to the largest keypoint count, and the Gram
+    # kernel's split plan follows that count, so a smaller pair's grid can differ from its single call in the last bits
+    grids = [st.local_homography(p[0], p[1], v)[0] for st, p, v in zip(stitchers, pairs, vertices)]
+    if stitch:
+        warp_devs = other_devs if warp_imgs is None else [_device_image(torch, device, img) for img in warp_imgs]
+        blend_dev = centre_dev if blend_img is None else _device_image(torch, device, blend_img)
+    results = []
+    for i, (st, local_h) in enumerate(zip(stitchers, grids)):
+        mat = mat_layout(local_h.copy(), st)
+        stitched = None
+        if stitch:
+            # the grid as local_homography returned it, as in stitch_pair
+            stitched = rt.to_host(torch, st.local_warp_blend(warp_devs[i], local_h.copy(), meshes[i], blend_dev))
+        results.append(StitchResult((st.final_width, st.final_height, st.offset_x, st.offset_y), meshes[i],
+                                    vertices[i], local_h, mat, stitched))
+    return results

@@ -23,7 +23,8 @@ import numpy as np
 from . import _runtime as rt
 
 __all__ = ["image_warping", "warp_perspective", "warping_canvas", "invert3x3", "match_descriptors", "coarse_matching",
-           "sift_describe", "equalize_hist", "keypoint_pairs", "find_homography_ransac"]
+           "sift_describe", "equalize_hist", "keypoint_pairs", "keypoint_pairs_batch", "find_homography_ransac",
+           "find_homography_ransac_batch"]
 
 
 def invert3x3(m) -> np.ndarray:
@@ -336,58 +337,117 @@ def find_homography_ransac(src, dst, threshold=5.0, *, confidence=0.995, max_ite
     mask are OpenCV's bit for bit, except when the best hypothesis has exactly 4 inliers: OpenCV then refits and
     LM-refines those 4 points, which ``findHomography(4 points, 0)`` does not, so H agrees to about 1e-12 relative
     (the mask is still OpenCV's).  Fewer than 4 points raise ``ValueError`` (OpenCV raises ``cv.error``)."""
-    on_device = not isinstance(src, np.ndarray) and hasattr(src, "device")
-    torch, device = rt.torch_cuda(src.device if on_device else device)
-    if on_device:
-        s_dev = src.to(device=device, dtype=torch.float32).reshape(-1, 2).contiguous()
-        d_dev = dst.to(device=device, dtype=torch.float32).reshape(-1, 2).contiguous()
-        s_host = d_host = None
-    else:
-        s_host = np.ascontiguousarray(np.asarray(src, np.float32).reshape(-1, 2))
-        d_host = np.ascontiguousarray(np.asarray(dst, np.float32).reshape(-1, 2))
-        s_dev, d_dev = rt.to_device(torch, device, s_host), rt.to_device(torch, device, d_host)
-    return _ransac(torch, device, s_dev, d_dev, s_host, d_host, threshold, confidence, max_iters)
+    return find_homography_ransac_batch([src], [dst], threshold, confidence=confidence, max_iters=max_iters,
+                                        device=device)[0]
 
 
-def _ransac(torch, device, s_dev, d_dev, s_host, d_host, threshold, confidence, max_iters):
-    """``find_homography_ransac`` on float32 ``[n, 2]`` device points; ``s_host`` / ``d_host`` are their host copies,
-    or ``None`` to download them with the counts."""
-    import cv2 as cv
+def find_homography_ransac_batch(srcs, dsts, threshold=5.0, *, confidence=0.995, max_iters=2000, device=None):
+    """``find_homography_ransac`` for several independent point sets: a list of ``(H, mask)``, element ``i`` bit for
+    bit ``find_homography_ransac(srcs[i], dsts[i], ...)``.  ``srcs`` / ``dsts``: lists of ``[n_i, 2]`` numpy arrays or
+    CUDA tensors.  Every set of 5 or more points goes to the device in one call (``apap_ransac_homography_batch``: the
+    sets concatenated on the device, one sampler warp per set) and one download brings back all subsets and counts;
+    sets of exactly 4 points are OpenCV's single fit; fewer than 4 raise ``ValueError`` naming the set.  The scan,
+    fit, mask and refit run per set on the host.  The batch waits for its slowest sampler (see
+    ``apap_ransac_homography_batch``)."""
+    if len(srcs) != len(dsts):
+        raise ValueError(f"find_homography_ransac_batch: {len(srcs)} source sets but {len(dsts)} target sets")
+    if not srcs:
+        return []
+    first = next((s for s in srcs if not isinstance(s, np.ndarray) and hasattr(s, "device")), None)
+    torch, device = rt.torch_cuda(first.device if first is not None else device)
+    s_devs, d_devs, s_hosts, d_hosts = [], [], [], []
+    for src, dst in zip(srcs, dsts):
+        if not isinstance(src, np.ndarray) and hasattr(src, "device"):
+            s_devs.append(src.to(device=device, dtype=torch.float32).reshape(-1, 2).contiguous())
+            d_devs.append(dst.to(device=device, dtype=torch.float32).reshape(-1, 2).contiguous())
+            s_hosts.append(None)
+            d_hosts.append(None)
+        else:
+            s_hosts.append(np.ascontiguousarray(np.asarray(src, np.float32).reshape(-1, 2)))
+            d_hosts.append(np.ascontiguousarray(np.asarray(dst, np.float32).reshape(-1, 2)))
+            s_devs.append(None)
+            d_devs.append(None)
+    return _ransac(torch, device, s_devs, d_devs, s_hosts, d_hosts, threshold, confidence, max_iters)
 
+
+def _ransac(torch, device, s_devs, d_devs, s_hosts, d_hosts, threshold, confidence, max_iters):
+    """``find_homography_ransac_batch`` on float32 ``[n, 2]`` point sets.  Per set, the device points, the host copies,
+    or both: a set without device points is uploaded when it is sampled, one without host copies is downloaded with
+    the counts."""
     if not 0.0 < confidence < 1.0:
         raise ValueError(f"find_homography_ransac: confidence must be in (0, 1), got {confidence}")
-    n = int(s_dev.shape[0])
-    if n < RANSAC_MODEL_POINTS or int(d_dev.shape[0]) != n:
-        raise ValueError(f"find_homography_ransac: needs at least 4 corresponding points, got {n} and {int(d_dev.shape[0])}")
+    ns = []
+    for i, (s_dev, d_dev, s_host, d_host) in enumerate(zip(s_devs, d_devs, s_hosts, d_hosts)):
+        n, m = (int(s_host.shape[0]), int(d_host.shape[0])) if s_host is not None else (int(s_dev.shape[0]),
+                                                                                         int(d_dev.shape[0]))
+        if n < RANSAC_MODEL_POINTS or m != n:
+            raise ValueError(f"find_homography_ransac: pair {i} needs at least 4 corresponding points, got {n} and {m}")
+        ns.append(n)
     if threshold <= 0:
         threshold = 3.0                                 # OpenCV's defaultRANSACReprojThreshold
     max_iters = max(int(max_iters), 1)
-    if max_iters > rt.RANSAC_MAX_ITERS:
-        raise ValueError(f"find_homography_ransac: max_iters must be <= {rt.RANSAC_MAX_ITERS}")
+    sampled = [i for i, n in enumerate(ns) if n > RANSAC_MODEL_POINTS]
+    if max(len(sampled), 1) * max_iters > rt.RANSAC_MAX_ITERS:
+        raise ValueError(f"find_homography_ransac: {len(sampled)} sets x max_iters {max_iters} must be <= "
+                         f"{rt.RANSAC_MAX_ITERS}")
+    for i in sampled:
+        if s_devs[i] is None:
+            s_devs[i], d_devs[i] = rt.to_device(torch, device, s_hosts[i]), rt.to_device(torch, device, d_hosts[i])
     down = []
-    if n > RANSAC_MODEL_POINTS:
+    if sampled:
         lib = rt.load_library()
+        b = len(sampled)
         ws_bytes = ctypes.c_size_t()
-        rt.check(lib.apap_ransac_workspace_bytes(max_iters, ctypes.byref(ws_bytes)), "apap_ransac_workspace_bytes")
+        rt.check(lib.apap_ransac_batch_workspace_bytes(b, max_iters, ctypes.byref(ws_bytes)),
+                 "apap_ransac_batch_workspace_bytes")
         ws = torch.empty(ws_bytes.value, dtype=torch.uint8, device=device)
-        out = torch.empty(5 * max_iters + 1, dtype=torch.int32, device=device)     # subsets | counts | n_sampled
-        hyps = torch.empty((max_iters, 9), dtype=torch.float64, device=device)
+        out = torch.empty(b * (5 * max_iters + 1), dtype=torch.int32, device=device)   # subsets | counts | n_sampled
+        hyps = torch.empty((b * max_iters, 9), dtype=torch.float64, device=device)
+        cnt_ptr, ns_ptr = out.data_ptr() + 16 * b * max_iters, out.data_ptr() + 20 * b * max_iters
         with torch.cuda.device(device):
-            rt.check(lib.apap_ransac_homography(s_dev.data_ptr(), d_dev.data_ptr(), n, float(threshold), max_iters,
-                                                ws.data_ptr(), ws_bytes.value, out.data_ptr(), hyps.data_ptr(),
-                                                out.data_ptr() + 16 * max_iters, out.data_ptr() + 20 * max_iters,
-                                                rt.stream_ptr(torch, device)), "apap_ransac_homography")
+            st = rt.stream_ptr(torch, device)
+            if b == 1:                                  # no offsets to upload
+                i = sampled[0]
+                rt.check(lib.apap_ransac_homography(s_devs[i].data_ptr(), d_devs[i].data_ptr(), ns[i], float(threshold),
+                                                    max_iters, ws.data_ptr(), ws_bytes.value, out.data_ptr(),
+                                                    hyps.data_ptr(), cnt_ptr, ns_ptr, st), "apap_ransac_homography")
+            else:
+                s_cat = torch.cat([s_devs[i] for i in sampled])
+                d_cat = torch.cat([d_devs[i] for i in sampled])
+                offsets = rt.to_device(torch, device, np.cumsum([0] + [ns[i] for i in sampled], dtype=np.int32))
+                rt.check(lib.apap_ransac_homography_batch(s_cat.data_ptr(), d_cat.data_ptr(), offsets.data_ptr(), b,
+                                                          max(ns[i] for i in sampled), float(threshold), max_iters,
+                                                          ws.data_ptr(), ws_bytes.value, out.data_ptr(), hyps.data_ptr(),
+                                                          cnt_ptr, ns_ptr, st), "apap_ransac_homography_batch")
         down.append(out)
-    if s_host is None:
-        down += [s_dev, d_dev]
+    missing = [i for i, s in enumerate(s_hosts) if s is None]
+    for i in missing:
+        down += [s_devs[i], d_devs[i]]
     down = rt.to_host_many(torch, down)
-    if s_host is None:
-        s_host, d_host = down[-2], down[-1]
-    if n == RANSAC_MODEL_POINTS:                        # findHomography: method 0 on the 4 points, mask all ones
+    first = 1 if sampled else 0
+    for k, i in enumerate(missing):
+        s_hosts[i], d_hosts[i] = down[first + 2 * k], down[first + 2 * k + 1]
+    records = [None] * len(ns)                          # None: 4 points, no sampling
+    if sampled:
+        b, rec = len(sampled), down[0]
+        subsets = rec[:4 * b * max_iters].reshape(b, max_iters, 4)
+        counts = rec[4 * b * max_iters:5 * b * max_iters].reshape(b, max_iters)
+        for k, i in enumerate(sampled):
+            records[i] = (subsets[k], counts[k], int(rec[5 * b * max_iters + k]))
+    return [_ransac_tail(s_hosts[i], d_hosts[i], records[i], threshold, confidence, max_iters) for i in range(len(ns))]
+
+
+def _ransac_tail(s_host, d_host, record, threshold, confidence, max_iters):
+    """The host end of ``find_homography_ransac`` for one set: OpenCV's single fit for 4 points (``record`` None),
+    else the adaptive-stop scan of the device's ``(subsets, counts, n_sampled)``, OpenCV's fit of the chosen subset,
+    the mask and the refit."""
+    import cv2 as cv
+
+    n = int(s_host.shape[0])
+    if record is None:                                  # findHomography: method 0 on the 4 points, mask all ones
         H = cv.findHomography(s_host, d_host, 0)[0]
         return H, (np.ones if H is not None else np.zeros)((n, 1), np.uint8)
-    subsets = down[0][:4 * max_iters].reshape(-1, 4)
-    counts, n_sampled = down[0][4 * max_iters:5 * max_iters], int(down[0][-1])
+    subsets, counts, n_sampled = record
     # RANSACPointSetRegistrator::run over the counts: a hypothesis is kept when it beats max(best, 3)
     niters, best, max_good, it = max_iters, -1, 0, 0
     while it < niters and it < n_sampled:
@@ -445,12 +505,92 @@ def keypoint_pairs(center_img, other_img, raw_kpts_cp, raw_kpts_op, *, equalize=
     centre, other = raw_cp[q], raw_op[idx[q]]
     if ransac == "gpu":
         q_dev = torch.nonzero(idx_dev >= 0).squeeze(1)
-        h, mask = _ransac(torch, device, pts_cp.index_select(0, q_dev),
-                          pts_op.index_select(0, idx_dev.index_select(0, q_dev).long()), centre, other, 5.0, 0.995,
-                          2000)
+        h, mask = _ransac(torch, device, [pts_cp.index_select(0, q_dev)],
+                          [pts_op.index_select(0, idx_dev.index_select(0, q_dev).long())], [centre], [other], 5.0,
+                          0.995, 2000)[0]
     else:
         h, mask = cv.findHomography(centre, other, cv.RANSAC, 5.0)
     if h is None:
         raise ValueError("keypoint_pairs: RANSAC found no homography")
     mask = mask.ravel().astype(bool)
     return other[mask], centre[mask], np.linalg.inv(h)
+
+
+def keypoint_pairs_batch(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops, *, equalize=True, device=None,
+                         ransac="opencv"):
+    """``keypoint_pairs`` of one centre image against several others -- the reference's multi-image mode, where
+    ``pyviz/apap.py`` runs once per image of a case against the fixed centre (run_all.sh:15,29): a list of
+    ``(final_src, final_dst, H)``, element ``i`` bit for bit ``keypoint_pairs(center_img, other_imgs[i], kc_i,
+    raw_kpts_ops[i], ...)`` in both ``ransac`` modes.  ``raw_kpts_cp`` is one ``[n, 2]`` array shared by all pairs
+    (``kc_i = raw_kpts_cp``), or a list or tuple with one array per pair.
+
+    The centre is uploaded, equalised and described once, at the concatenation of the pairs' centre keypoints
+    (descriptors are per keypoint, so each pair's slice has its own call's bytes); each other image is uploaded and
+    described once; the matches are launched back to back and all train indices come down in one copy.  With
+    ``ransac="gpu"`` the matched points are gathered on the device and go through one ``find_homography_ransac_batch``;
+    with ``"opencv"`` each pair calls ``cv.findHomography``.  A pair with fewer than 4 matches, or without a
+    homography, raises ``ValueError`` naming its index."""
+    return _keypoint_pairs_uploaded(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops, equalize, device, ransac)[0]
+
+
+def _keypoint_pairs_uploaded(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops, equalize, device, ransac):
+    """``keypoint_pairs_batch`` that also returns the images it uploaded: ``(pairs, centre [H, W, 3] uint8 device
+    tensor, [other device tensors])``, for callers that warp them next (``driver.stitch_case``)."""
+    import cv2 as cv
+
+    if ransac not in ("opencv", "gpu"):
+        raise ValueError(f"keypoint_pairs_batch: ransac must be 'opencv' or 'gpu', got {ransac!r}")
+    k = len(other_imgs)
+    shared = not isinstance(raw_kpts_cp, (list, tuple))
+    if len(raw_kpts_ops) != k or (not shared and len(raw_kpts_cp) != k):
+        raise ValueError(f"keypoint_pairs_batch: {k} other images need {k} keypoint sets, got {len(raw_kpts_ops)}"
+                         + ("" if shared else f" and {len(raw_kpts_cp)} centre sets"))
+    torch, device = rt.torch_cuda(device if device is not None else
+                                  (center_img.device if not isinstance(center_img, np.ndarray) else None))
+    if k == 0:
+        return [], None, []
+    raw_ops = [np.asarray(r, dtype=np.float32).reshape(-1, 2) for r in raw_kpts_ops]
+    raw_cps = ([np.asarray(raw_kpts_cp, dtype=np.float32).reshape(-1, 2)] if shared else
+               [np.asarray(r, dtype=np.float32).reshape(-1, 2) for r in raw_kpts_cp])
+    cp_start = np.cumsum([0] + [len(r) for r in raw_cps])
+    op_start = np.cumsum([0] + [len(r) for r in raw_ops])
+    pts_cp = rt.to_device(torch, device, np.concatenate(raw_cps))
+    pts_op = rt.to_device(torch, device, np.concatenate(raw_ops))
+    centre_dev = _device_image(torch, device, center_img)
+    feats_cp = sift_describe(centre_dev, pts_cp, equalize=equalize)
+    other_devs = [_device_image(torch, device, img) for img in other_imgs]
+    if shared:
+        raw_cps, cp_start = raw_cps * k, np.zeros(k + 1, np.int64)
+    idx_devs = []
+    for i, img in enumerate(other_devs):
+        feats_op = sift_describe(img, pts_op[op_start[i]:op_start[i + 1]], equalize=equalize)
+        idx_devs.append(match_descriptors(feats_cp[cp_start[i]:cp_start[i] + len(raw_cps[i])], feats_op,
+                                          device=device)[0])
+    idxs = rt.to_host_many(torch, idx_devs)
+    qs, centres, others = [], [], []
+    for i, idx in enumerate(idxs):
+        q = np.flatnonzero(idx >= 0)
+        if len(q) < 4:
+            raise ValueError(f"keypoint_pairs_batch: pair {i} has {len(q)} matches, a homography needs at least 4")
+        qs.append(q)
+        centres.append(raw_cps[i][q])
+        others.append(raw_ops[i][idx[q]])
+    if ransac == "gpu":
+        rows = np.concatenate([np.concatenate([cp_start[i] + q, op_start[i] + idx[q]])
+                               for i, (q, idx) in enumerate(zip(qs, idxs))]).astype(np.int64)
+        rows = rt.to_device(torch, device, rows)        # per pair: centre rows, then other rows
+        s_devs, d_devs, at = [], [], 0
+        for q in qs:
+            s_devs.append(pts_cp.index_select(0, rows[at:at + len(q)]))
+            d_devs.append(pts_op.index_select(0, rows[at + len(q):at + 2 * len(q)]))
+            at += 2 * len(q)
+        fits = _ransac(torch, device, s_devs, d_devs, centres, others, 5.0, 0.995, 2000)
+    else:
+        fits = [cv.findHomography(c, o, cv.RANSAC, 5.0) for c, o in zip(centres, others)]
+    pairs = []
+    for i, ((h, mask), centre, other) in enumerate(zip(fits, centres, others)):
+        if h is None:
+            raise ValueError(f"keypoint_pairs_batch: RANSAC found no homography for pair {i}")
+        mask = mask.ravel().astype(bool)
+        pairs.append((other[mask], centre[mask], np.linalg.inv(h)))
+    return pairs, centre_dev, other_devs

@@ -402,6 +402,28 @@ int apap_ransac_homography(const float *src, const float *dst, int n, double thr
                            void *stream);
 
 /*
+ * apap_ransac_homography for a batch of independent point sets in one launch per kernel (one sampler warp per pair,
+ * one fit thread per pair and hypothesis, score CTAs per pair): the reference's multi-image mode matches every image
+ * of a case against one centre, and the pairs' serial samplers run side by side on different SMs.  Pair p's record
+ * is exactly apap_ransac_homography's record of its points (each pair starts its own cv::RNG(0xFFFFFFFFFFFFFFFF)).
+ *   src, dst   : float [total][2] (device, 8-byte aligned), the pairs back to back
+ *   offsets    : int32 [batch + 1] (device, 4-byte aligned): pair p is [offsets[p], offsets[p + 1]); a pair of fewer
+ *                than 5 points is not sampled (n_sampled 0)
+ *   batch      : >= 1, with batch * max_iters <= APAP_RANSAC_MAX_ITERS;  max_n >= 0 sizes the score grid (the
+ *                largest pair; a larger pair is still scored completely, with fewer CTAs per hypothesis)
+ *   threshold, max_iters : as apap_ransac_homography;  workspace: apap_ransac_batch_workspace_bytes, 16-byte aligned
+ *   subsets    : out int32 [batch][max_iters][4] (16-byte aligned), indices local to the pair
+ *   hyps       : out double [batch][max_iters][9] (8-byte aligned);  counts: out int32 [batch][max_iters]
+ *   n_sampled  : out int32 [batch]
+ * The launch ends when its slowest sampler ends: one degenerate pair, most candidates rejected by checkSubset, holds
+ * the whole batch for up to max_iters x 10000 candidates (seconds at 2000), as it would hold a single call.
+ */
+int apap_ransac_batch_workspace_bytes(int batch, int max_iters, size_t *bytes);
+int apap_ransac_homography_batch(const float *src, const float *dst, const int *offsets, int batch, int max_n,
+                                 double threshold, int max_iters, void *workspace, size_t workspace_bytes,
+                                 int *subsets, double *hyps, int *counts, int *n_sampled, void *stream);
+
+/*
  * Panorama assembly of a sharded pass without an all-gather: broadcast `bytes` of device memory at `src` (this
  * rank's row band, already warped) into every GPU's panorama through an NVLS multicast mapping -- `multicast_dst` is
  * the band's address inside the multicast mapping of the panorama buffers (torch symmetric memory's multicast_ptr +
