@@ -30,6 +30,7 @@ WARP_FORCE_EXACT = 1
 WARP_LEGACY = 2
 WARP_TILE_FUSED = 4
 RANSAC_MAX_ITERS = 1 << 20
+BLEND_MAX_LAYERS = 256
 
 # symbol -> (restype, argtypes); tests check every symbol of include/apap_b200.h is exported
 SIGNATURES = {
@@ -55,6 +56,7 @@ SIGNATURES = {
     "apap_warp_tiles": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int,
                                 c_int, c_void_p, c_size_t, c_void_p]),
     "apap_blend": (c_int, [c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "apap_blend_layers": (c_int, [POINTER(ctypes.c_longlong), c_int, c_int, c_int, c_void_p, c_size_t, c_void_p]),
     "apap_pipe_probe": (c_int, [c_int, c_int, c_void_p, POINTER(c_double), c_void_p]),
     "apap_warp_perspective": (c_int, [c_void_p, c_int, c_int, POINTER(c_double), c_void_p, c_int, c_int, c_void_p, c_int,
                                       c_int, c_int, c_int, c_int, c_void_p]),

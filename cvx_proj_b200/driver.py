@@ -9,6 +9,7 @@ inverse + ``/[2, 2]`` + column-major ``[cells, 9]`` float64 layout of the ``.mat
   ``save2mat``        pyviz/utils.py:68-70
   ``stitch_pair``     pyviz/apap.py:238-265           (grid, H field, ``.mat`` matrix, stitched image)
   ``stitch_case``     run_all.sh:15,29                (every image of a case against the centre, from raw keypoints)
+  ``stitch_panorama`` (no reference counterpart)      (the same, blended into one panorama of the case)
 
 The keypoint-pair producer (``visualize_feature_pairs``) and the dataset IO stay with the caller
 (SURVEY.md section 8f, rows N3/N4): ``stitch_pair`` starts where the script has its matched
@@ -22,7 +23,8 @@ import numpy as np
 
 from .apap_utils import final_size, get_mesh, get_vertice
 
-__all__ = ["mat_layout", "save2mat", "stitch_pair", "stitch_case", "StitchResult"]
+__all__ = ["mat_layout", "save2mat", "stitch_pair", "stitch_case", "StitchResult", "panorama_size", "stitch_panorama",
+           "PanoramaResult"]
 
 
 def mat_layout(local_homography: np.ndarray, stitcher=None) -> np.ndarray:
@@ -110,25 +112,16 @@ def stitch_case(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops, *, mesh_size:
     and pastes (pyviz/apap.py:245); each is uploaded once.  ``stitched`` comes back as a numpy array.  The ``.mat`` and
     keypoint files stay with the caller, as for ``stitch_pair``."""
     from . import _runtime as rt
-    from .apap import APAP
-    from .utils import _device_image, _keypoint_pairs_uploaded
+    from .utils import _device_image
 
     if warp_imgs is not None and len(warp_imgs) != len(other_imgs):
         raise ValueError(f"stitch_case: {len(other_imgs)} other images but {len(warp_imgs)} warp images")
-    pairs, centre_dev, other_devs = _keypoint_pairs_uploaded(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops,
-                                                              equalize, device, ransac)
-    if not pairs:
+    front = _case_front(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops, mesh_size, gamma, sigma, equalize, ransac,
+                        device)
+    if front is None:
         return []
+    centre_dev, other_devs, stitchers, meshes, vertices, grids = front
     torch, device = rt.torch_cuda(centre_dev.device)
-    stitchers, meshes, vertices = [], [], []
-    for other_img, (_, _, project_h) in zip(other_imgs, pairs):
-        final_w, final_h, offset_x, offset_y = final_size(center_img, other_img, project_h)
-        meshes.append(get_mesh((final_w, final_h), mesh_size + 1))
-        vertices.append(get_vertice((final_w, final_h), mesh_size, (offset_x, offset_y)))
-        stitchers.append(APAP(gamma, sigma, [final_w, final_h], [offset_x, offset_y], device=device))
-    # per pair, not local_homography_batch: a batch pads every pair to the largest keypoint count, and the Gram
-    # kernel's split plan follows that count, so a smaller pair's grid can differ from its single call in the last bits
-    grids = [st.local_homography(p[0], p[1], v)[0] for st, p, v in zip(stitchers, pairs, vertices)]
     if stitch:
         warp_devs = other_devs if warp_imgs is None else [_device_image(torch, device, img) for img in warp_imgs]
         blend_dev = centre_dev if blend_img is None else _device_image(torch, device, blend_img)
@@ -142,3 +135,99 @@ def stitch_case(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops, *, mesh_size:
         results.append(StitchResult((st.final_width, st.final_height, st.offset_x, st.offset_y), meshes[i],
                                     vertices[i], local_h, mat, stitched))
     return results
+
+
+def _case_front(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops, mesh_size, gamma, sigma, equalize, ransac, device):
+    """What ``stitch_case`` and ``stitch_panorama`` share: the keypoint pairs of every other image against the centre
+    (``_keypoint_pairs_uploaded``), then per pair its canvas, mesh, anchors and grid.  ``None`` without other images,
+    else ``(centre device tensor, [other device tensors], [APAP], [mesh], [vertices], [grid])``."""
+    from . import _runtime as rt
+    from .apap import APAP
+    from .utils import _keypoint_pairs_uploaded
+
+    pairs, centre_dev, other_devs = _keypoint_pairs_uploaded(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops,
+                                                              equalize, device, ransac)
+    if not pairs:
+        return None
+    _, device = rt.torch_cuda(centre_dev.device)
+    stitchers, meshes, vertices = [], [], []
+    for other_img, (_, _, project_h) in zip(other_imgs, pairs):
+        final_w, final_h, offset_x, offset_y = final_size(center_img, other_img, project_h)
+        meshes.append(get_mesh((final_w, final_h), mesh_size + 1))
+        vertices.append(get_vertice((final_w, final_h), mesh_size, (offset_x, offset_y)))
+        stitchers.append(APAP(gamma, sigma, [final_w, final_h], [offset_x, offset_y], device=device))
+    # per pair, not local_homography_batch: a batch pads every pair to the largest keypoint count, and the Gram
+    # kernel's split plan follows that count, so a smaller pair's grid can differ from its single call in the last bits
+    grids = [st.local_homography(p[0], p[1], v)[0] for st, p, v in zip(stitchers, pairs, vertices)]
+    return centre_dev, other_devs, stitchers, meshes, vertices, grids
+
+
+def panorama_size(final_sizes):
+    """The panorama canvas of a case from its pairs' ``final_size`` tuples ``(W_k, H_k, ox_k, oy_k)``: pair k's canvas
+    covers ``[-ox_k, W_k - ox_k) x [-oy_k, H_k - oy_k)`` in centre coordinates, and the panorama is the union of those
+    rectangles.  Returns ``((W, H, OX, OY), origins)``: the centre lies at ``(OX, OY)`` of the panorama and pair k's
+    canvas at ``origins[k] = (OX - ox_k, OY - oy_k)`` (int64 ``[K, 2]``).  For one pair this is its own ``final_size``
+    with origin ``(0, 0)``.  Host arithmetic."""
+    fs = np.asarray(final_sizes, dtype=np.int64).reshape(-1, 4)
+    if len(fs) == 0:
+        raise ValueError("panorama_size: at least one final_size")
+    ox, oy = int(fs[:, 2].max()), int(fs[:, 3].max())
+    width = int((fs[:, 0] - fs[:, 2]).max()) + ox
+    height = int((fs[:, 1] - fs[:, 3]).max()) + oy
+    origins = np.stack([ox - fs[:, 2], oy - fs[:, 3]], axis=1)
+    return (width, height, ox, oy), origins
+
+
+class PanoramaResult(NamedTuple):
+    final_size: tuple        # (W, H, OX, OY): the panorama canvas, the centre at (OX, OY)
+    origins: np.ndarray      # [K, 2] int64 top-left panorama position of each pair's canvas
+    pairs: list              # one StitchResult per other image, stitched = None (stitch_case(..., stitch=False))
+    panorama: np.ndarray     # [H, W, 3] uint8
+
+
+def stitch_panorama(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops, *, mesh_size: int = 100, gamma=0.5, sigma=100,
+                    warp_imgs=None, blend_img=None, equalize: bool = True, ransac: str = "opencv",
+                    device=None) -> PanoramaResult:
+    """Every image of a case stitched against the centre into ONE panorama (the reference has no multi-image blend;
+    ``stitch_case`` returns one two-image canvas per pair, each in a frame of its own).
+
+    ``pairs[i]`` is ``stitch_case(..., stitch=False)[i]`` field for field.  Every pair's grid maps its canvas into the
+    centre's frame, so the panorama is the union of the pair canvases (``panorama_size``) with
+      - layer k: ``APAP.local_warp(warp_imgs[k], grid_k, mesh_k)`` on pair k's own canvas (nearest, as the reference),
+        placed at ``origins[k]`` -- not re-warped on a union mesh, the cell lookup belongs to the pair canvas;
+      - the centre layer: ``blend_img`` (default ``center_img``) at ``(OX, OY)``;
+    blended by ``utils.blend_layers``: per pixel the floor mean of the non-empty layers.  With one other image the
+    panorama is ``stitch_pair(...).stitched`` bit for bit; with none it is the centre image itself (``pairs == []``).
+
+    The layers are warped from the images the keypoint-pair producer already holds on the device and stay there; one
+    ``blend_layers`` launch and one download make the panorama.  At most 255 other images."""
+    from . import _runtime as rt
+    from .utils import _device_image, blend_layers
+
+    if warp_imgs is not None and len(warp_imgs) != len(other_imgs):
+        raise ValueError(f"stitch_panorama: {len(other_imgs)} other images but {len(warp_imgs)} warp images")
+    if len(other_imgs) >= rt.BLEND_MAX_LAYERS:
+        raise ValueError(f"stitch_panorama: at most {rt.BLEND_MAX_LAYERS - 1} other images, got {len(other_imgs)}")
+    front = _case_front(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops, mesh_size, gamma, sigma, equalize, ransac,
+                        device)
+    centre = center_img if blend_img is None else blend_img
+    if front is None:
+        h, w = centre.shape[0], centre.shape[1]
+        pano = blend_layers([centre], [(0, 0)], (w, h), device=device)
+        if not isinstance(pano, np.ndarray):
+            pano = rt.to_host(rt.torch_cuda(pano.device)[0], pano)
+        return PanoramaResult((int(w), int(h), 0, 0), np.zeros((0, 2), np.int64), [], pano)
+    centre_dev, other_devs, stitchers, meshes, vertices, grids = front
+    torch, device = rt.torch_cuda(centre_dev.device)
+    warp_devs = other_devs if warp_imgs is None else [_device_image(torch, device, img) for img in warp_imgs]
+    blend_dev = centre_dev if blend_img is None else _device_image(torch, device, blend_img)
+    pairs, layers = [], []
+    for i, (st, local_h) in enumerate(zip(stitchers, grids)):
+        mat = mat_layout(local_h.copy(), st)
+        pairs.append(StitchResult((st.final_width, st.final_height, st.offset_x, st.offset_y), meshes[i], vertices[i],
+                                  local_h, mat, None))
+        # the grid as local_homography returned it, as stitch_pair hands it to the fused warp
+        layers.append(st.local_warp(warp_devs[i], local_h.copy(), meshes[i]))
+    (width, height, ox, oy), origins = panorama_size([p.final_size for p in pairs])
+    pano = blend_layers(layers + [blend_dev], [tuple(o) for o in origins] + [(ox, oy)], (width, height))
+    return PanoramaResult((width, height, ox, oy), origins, pairs, rt.to_host(torch, pano))

@@ -24,7 +24,7 @@ from . import _runtime as rt
 
 __all__ = ["image_warping", "warp_perspective", "warping_canvas", "invert3x3", "match_descriptors", "coarse_matching",
            "sift_describe", "equalize_hist", "keypoint_pairs", "keypoint_pairs_batch", "find_homography_ransac",
-           "find_homography_ransac_batch"]
+           "find_homography_ransac_batch", "blend_layers"]
 
 
 def invert3x3(m) -> np.ndarray:
@@ -99,6 +99,59 @@ def image_warping(img_base, img2warp, H, direct_blend=True, device=None):
     cw, ch, tx, ty, m = warping_canvas(img_base.shape, img2warp.shape, H)
     return warp_perspective(img2warp, m, (cw, ch), base=img_base, offset=(tx, ty), mode=1 if direct_blend else 2,
                             device=device)
+
+
+def blend_layers(layers, origins, size, device=None):
+    """Mean blend of placed layers (``k_blend_layers``), the panorama blend of ``driver.stitch_panorama``.
+
+    ``layers`` are ``uint8 [h, w, 3]`` images, ``origins`` their top-left canvas positions ``[(x0, y0), ...]`` (may be
+    negative; a layer may stick out of the canvas and is clipped) and ``size = (width, height)`` the canvas.  Per
+    pixel, with ``n`` the number of layers that are non-empty there (any channel > 0) and ``s`` their per-channel
+    integer sum, the result is ``floor(s / n)``, 0 where ``n = 0`` -- for two equal layers at one origin exactly
+    ``uniform_blend``, and independent of the layer order.  1 to 256 layers.
+
+    All numpy in -> numpy out (uploaded to ``device``); all CUDA tensors (one device) in -> a tensor on that device.
+    Tensor layers are read in place when their pixels are packed (strides ``(pitch, 3, 1)``), so crops of a larger
+    image need no copy.  No CPU fallback."""
+    layers = list(layers)
+    origins = [tuple(o) for o in origins]
+    if not 1 <= len(layers) <= rt.BLEND_MAX_LAYERS:
+        raise ValueError(f"blend_layers: 1 to {rt.BLEND_MAX_LAYERS} layers, got {len(layers)}")
+    if len(origins) != len(layers) or any(len(o) != 2 for o in origins):
+        raise ValueError(f"blend_layers: one (x0, y0) origin per layer ({len(layers)} layers, {len(origins)} origins)")
+    width, height = (int(v) for v in size)
+    if width <= 0 or height <= 0:
+        raise ValueError(f"blend_layers: the canvas size must be positive, got {tuple(size)}")
+    numpy_in = [isinstance(img, np.ndarray) for img in layers]
+    if any(numpy_in) and not all(numpy_in):
+        raise ValueError("blend_layers: layers must be all numpy arrays or all CUDA tensors")
+    on_device = not numpy_in[0]
+    for k, img in enumerate(layers):
+        if on_device and not getattr(img, "is_cuda", False):
+            raise ValueError(f"blend_layers: layer {k} is neither a numpy array nor a CUDA tensor")
+        if len(img.shape) != 3 or img.shape[2] != 3 or img.shape[0] < 1 or img.shape[1] < 1:
+            raise ValueError(f"blend_layers: layer {k} must be [h, w, 3], got {tuple(img.shape)}")
+        if (img.dtype != np.uint8) if not on_device else (str(img.dtype) != "torch.uint8"):
+            raise ValueError(f"blend_layers: layer {k} must be uint8, got {img.dtype}")
+    if on_device:
+        devs = {img.device for img in layers}
+        if len(devs) != 1:
+            raise ValueError(f"blend_layers: all layers must be on one device, got {sorted(map(str, devs))}")
+        device = layers[0].device
+    torch, device = rt.torch_cuda(device)
+    lib = rt.load_library()
+    if on_device:
+        devs = [img if img.stride(2) == 1 and img.stride(1) == 3 and (img.shape[0] == 1 or img.stride(0) >= 3 * img.shape[1])
+                else img.contiguous() for img in layers]
+    else:
+        devs = [rt.to_device(torch, device, img) for img in layers]
+    desc = np.array([[img.data_ptr(), img.shape[0], img.shape[1], img.stride(0), x0, y0]
+                     for img, (x0, y0) in zip(devs, origins)], dtype=np.int64)
+    out = torch.empty((height, width, 3), dtype=torch.uint8, device=device)
+    with torch.cuda.device(device):
+        rt.check(lib.apap_blend_layers(desc.ctypes.data_as(ctypes.POINTER(ctypes.c_longlong)), len(devs), height, width,
+                                       out.data_ptr(), out.numel(), rt.stream_ptr(torch, device)), "apap_blend_layers")
+    return out if on_device else rt.to_host(torch, out)
 
 
 # ------------------------------------------------------------------ keypoint-pair producer (SURVEY 8f, row N3)

@@ -228,6 +228,22 @@ int apap_warp_bilinear(const uint8_t *src, int src_h, int src_w, const float *ce
 int apap_blend(const uint8_t *a, const uint8_t *b, uint8_t *out, size_t n_px, void *stream);
 
 /*
+ * Panorama blend of placed layers (driver.stitch_panorama): out [canvas_h][canvas_w][3] uint8 (device, any alignment,
+ * out_bytes >= canvas_h x canvas_w x 3) gets, per pixel, the per-channel floor((sum of the layers' pixels) / n), n =
+ * the number of layers whose pixel there is non-empty (any channel > 0), and 0 where n = 0.  With two equal layers at
+ * one origin this is apap_blend bit for bit; the result does not depend on the layer order.
+ *   layers   : HOST long long [n_layers][6] = {device address, h, w, row pitch in bytes, x0, y0}: an [h][w][3] uint8
+ *              image whose pixel (0, 0) lies at canvas (x0, y0).  Any address and any pitch >= 3 w (ignored for
+ *              h = 1), so crops of a larger image need no copy; origins may be negative and layers may stick out of
+ *              the canvas (clipped).  Sizes in [1, 2^30], origins in [-2^30, 2^30].
+ *   n_layers : 1 .. APAP_BLEND_MAX_LAYERS (255 x 256 fits the kernel's 16-bit sums)
+ * One kernel (k_blend_layers), one pass over the canvas; every layer byte inside the canvas is read once.
+ */
+#define APAP_BLEND_MAX_LAYERS 256
+int apap_blend_layers(const long long *layers, int n_layers, int canvas_h, int canvas_w, uint8_t *out,
+                      size_t out_bytes, void *stream);
+
+/*
  * Input preparation on the device (what the host layer used to build in numpy; both reproduce their
  * numpy restatements in cvx_proj_b200/apap.py bit for bit).
  *
