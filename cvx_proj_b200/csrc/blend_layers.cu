@@ -3,82 +3,21 @@
 // uniform_blend (K4) bit for bit.
 //
 // Bandwidth-bound byte work: every canvas byte is written once and every layer byte inside the canvas is read once.
-// A CTA owns a segment of kSegPx pixels of one canvas row, a thread 4 consecutive pixels (12 bytes).  The layer loop
-// runs over all descriptors (a __grid_constant__ parameter, read through the constant cache with a uniform index);
-// the row and segment tests are uniform per CTA.  A layer row's 12-byte groups all share one phase modulo 4 (12 is a
-// multiple of 4), so a thread reads its group as 3 or 4 aligned words -- each holding at least one byte of the group
-// -- and funnel-shifts them into place; the at most two groups that straddle a layer's left or right edge read byte
-// by byte.  Sums are packed 16-bit pairs in registers (255 x 256 < 2^16), counts too.  An empty pixel adds zero to
-// the sums, so only the count needs the non-empty test.  floor(s / n) is __umulhi(s, ceil(2^32 / n)) for n >= 2
-// (exact: s (m n - 2^32) < s n <= 255 x 256^2 < 2^32), s itself for n <= 1 (n = 0 means s = 0).
+// The segment and group shape and the layer reads are layers.cuh's.  The layer loop runs over all descriptors (a
+// __grid_constant__ parameter, read through the constant cache with a uniform index); the row and segment tests are
+// uniform per CTA.  Sums are packed 16-bit pairs in registers (255 x 256 < 2^16), counts too.  An empty pixel adds
+// zero to the sums, so only the count needs the non-empty test.  floor(s / n) is __umulhi(s, ceil(2^32 / n)) for
+// n >= 2 (exact: s (m n - 2^32) < s n <= 255 x 256^2 < 2^32), s itself for n <= 1 (n = 0 means s = 0).
 // The segment's bytes are staged in shared memory and leave as aligned 16-byte stores plus a byte-wise head and tail.
-#include "common.cuh"
+#include "layers.cuh"
 
 namespace apap {
-
-constexpr int kLayerThreads = 256;
-constexpr int kLayerGroupPx = 4;                         // pixels per thread
-constexpr int kSegPx = kLayerThreads * kLayerGroupPx;    // canvas pixels per CTA
-constexpr int kSegBytes = 3 * kSegPx;
-static_assert(kSegBytes / 16 <= kLayerThreads - 32, "the last warp writes the head and tail bytes");
-
-struct LayerDesc {
-  const uint8_t *addr;     // pixel (0, 0) of the layer
-  long long pitch;         // bytes from one layer row to the next
-  int h, w, x0, y0;        // size and canvas position of the top-left pixel (may be negative)
-};
 
 struct LayerParams {
   LayerDesc layer[APAP_BLEND_MAX_LAYERS];
   uint8_t *out;
   int n_layers, canvas_h, canvas_w, segs_per_row;
 };
-
-// one byte per pixel of a 12-byte group: the OR of its three channel bytes
-__device__ __forceinline__ uint32_t group_or(uint32_t w0, uint32_t w1, uint32_t w2) {
-  const uint32_t x = __byte_perm(__byte_perm(w0, w1, 0x0630), w2, 0x5210);   // bytes 0, 3, 6, 9
-  const uint32_t y = __byte_perm(__byte_perm(w0, w1, 0x0741), w2, 0x6210);   // bytes 1, 4, 7, 10
-  const uint32_t z = __byte_perm(__byte_perm(w0, w1, 0x0052), w2, 0x7410);   // bytes 2, 5, 8, 11
-  return x | y | z;
-}
-
-// bit 0 of every byte = that byte of v is non-zero, the other bits 0
-__device__ __forceinline__ uint32_t byte_nonzero(uint32_t v) {
-  return ((((v & 0x7f7f7f7fu) + 0x7f7f7f7fu) | v) >> 7) & 0x01010101u;
-}
-
-// the 12 bytes of layer l under this thread's group of canvas pixels [x, x + n_px) of row y, zeros where the layer is
-// absent (the row or the pixels outside the layer; an absent layer adds nothing to the sums and counts)
-__device__ __forceinline__ void fetch_group(const LayerParams &p, int l, int y, int seg0, int seg_px, int x, int n_px,
-                                            uint32_t (&w)[3]) {
-  w[0] = w[1] = w[2] = 0u;
-  const LayerDesc &L = p.layer[l];
-  const int ly = y - L.y0;
-  const int lx0 = seg0 - L.x0;                  // layer column of the segment's first pixel
-  if ((unsigned)ly >= (unsigned)L.h || lx0 >= L.w || lx0 + seg_px <= 0) return;   // uniform
-  const int lx = x - L.x0;
-  if (n_px <= 0 || lx >= L.w || lx + n_px <= 0) return;
-  const uint8_t *q = L.addr + (long long)ly * L.pitch + 3LL * lx;
-  if (n_px == kLayerGroupPx && lx >= 0 && lx + kLayerGroupPx <= L.w) {
-    const uint32_t phase = (uint32_t)reinterpret_cast<uintptr_t>(q) & 3u;   // uniform over the CTA
-    const uint32_t *a = reinterpret_cast<const uint32_t *>(q - phase);
-    const uint32_t a0 = __ldg(a), a1 = __ldg(a + 1), a2 = __ldg(a + 2), a3 = phase ? __ldg(a + 3) : 0u;
-    w[0] = __funnelshift_r(a0, a1, 8u * phase);
-    w[1] = __funnelshift_r(a1, a2, 8u * phase);
-    w[2] = __funnelshift_r(a2, a3, 8u * phase);
-  } else {                                      // the group straddles the layer's edge or the canvas end
-#pragma unroll
-    for (int k = 0; k < kLayerGroupPx; ++k) {
-      if (k < n_px && (unsigned)(lx + k) < (unsigned)L.w) {
-#pragma unroll
-        for (int c = 0; c < 3; ++c) {
-          const int b = 3 * k + c;
-          w[b >> 2] |= (uint32_t)__ldg(q + b) << (8 * (b & 3));
-        }
-      }
-    }
-  }
-}
 
 __global__ void __launch_bounds__(kLayerThreads) k_blend_layers(const __grid_constant__ LayerParams p) {
   __shared__ uint32_t recip[APAP_BLEND_MAX_LAYERS + 1];
@@ -96,7 +35,7 @@ __global__ void __launch_bounds__(kLayerThreads) k_blend_layers(const __grid_con
   uint32_t c01 = 0u, c23 = 0u;                 // non-empty counts of pixels 0, 1 and 2, 3 (16-bit halves)
   for (int l = 0; l < p.n_layers; ++l) {
     uint32_t w[3];
-    fetch_group(p, l, y, seg0, seg_px, x, n_px, w);
+    fetch_group(p.layer[l], y, seg0, seg_px, x, n_px, w);
     s[0] += __byte_perm(w[0], 0u, 0x4140); s[1] += __byte_perm(w[0], 0u, 0x4342);
     s[2] += __byte_perm(w[1], 0u, 0x4140); s[3] += __byte_perm(w[1], 0u, 0x4342);
     s[4] += __byte_perm(w[2], 0u, 0x4140); s[5] += __byte_perm(w[2], 0u, 0x4342);
@@ -148,15 +87,7 @@ __global__ void __launch_bounds__(kLayerThreads) k_blend_layers(const __grid_con
 int launch_blend_layers(const long long *layers, int n_layers, int canvas_h, int canvas_w, uint8_t *out,
                         cudaStream_t st) {
   LayerParams p;
-  for (int l = 0; l < n_layers; ++l) {
-    const long long *d = layers + 6 * l;
-    p.layer[l].addr = reinterpret_cast<const uint8_t *>(static_cast<uintptr_t>(d[0]));
-    p.layer[l].h = (int)d[1];
-    p.layer[l].w = (int)d[2];
-    p.layer[l].pitch = d[3];
-    p.layer[l].x0 = (int)d[4];
-    p.layer[l].y0 = (int)d[5];
-  }
+  for (int l = 0; l < n_layers; ++l) p.layer[l] = layer_desc(layers + 6 * l);
   p.out = out;
   p.n_layers = n_layers;
   p.canvas_h = canvas_h;

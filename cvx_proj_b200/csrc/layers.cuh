@@ -1,0 +1,106 @@
+// Placed uint8 [h][w][3] layers read and a canvas row segment written by the N-layer blends (blend_layers.cu,
+// feather.cu).  A CTA owns a segment of kSegPx pixels of one canvas row, a thread 4 consecutive pixels (12 bytes).
+// A layer row's 12-byte groups all share one phase modulo 4 (12 is a multiple of 4), so a thread reads its group as 3
+// or 4 aligned words -- each holding at least one byte of the group -- and funnel-shifts them into place; the at most
+// two groups that straddle a layer's left or right edge read byte by byte.  The segment's bytes are staged in shared
+// memory and leave as aligned 16-byte stores plus a byte-wise head and tail.
+#pragma once
+#include "common.cuh"
+
+namespace apap {
+
+constexpr int kLayerThreads = 256;
+constexpr int kLayerGroupPx = 4;                         // pixels per thread
+constexpr int kSegPx = kLayerThreads * kLayerGroupPx;    // canvas pixels per CTA
+constexpr int kSegBytes = 3 * kSegPx;
+static_assert(kSegBytes / 16 <= kLayerThreads - 32, "the last warp writes the head and tail bytes");
+
+struct LayerDesc {
+  const uint8_t *addr;     // pixel (0, 0) of the layer
+  long long pitch;         // bytes from one layer row to the next
+  int h, w, x0, y0;        // size and canvas position of the top-left pixel (may be negative)
+};
+
+// {device address, h, w, row pitch in bytes, x0, y0} of the C ABI
+inline LayerDesc layer_desc(const long long *d) {
+  LayerDesc L;
+  L.addr = reinterpret_cast<const uint8_t *>(static_cast<uintptr_t>(d[0]));
+  L.h = (int)d[1];
+  L.w = (int)d[2];
+  L.pitch = d[3];
+  L.x0 = (int)d[4];
+  L.y0 = (int)d[5];
+  return L;
+}
+
+// one byte per pixel of a 12-byte group: the OR of its three channel bytes
+__device__ __forceinline__ uint32_t group_or(uint32_t w0, uint32_t w1, uint32_t w2) {
+  const uint32_t x = __byte_perm(__byte_perm(w0, w1, 0x0630), w2, 0x5210);   // bytes 0, 3, 6, 9
+  const uint32_t y = __byte_perm(__byte_perm(w0, w1, 0x0741), w2, 0x6210);   // bytes 1, 4, 7, 10
+  const uint32_t z = __byte_perm(__byte_perm(w0, w1, 0x0052), w2, 0x7410);   // bytes 2, 5, 8, 11
+  return x | y | z;
+}
+
+// bit 0 of every byte = that byte of v is non-zero, the other bits 0
+__device__ __forceinline__ uint32_t byte_nonzero(uint32_t v) {
+  return ((((v & 0x7f7f7f7fu) + 0x7f7f7f7fu) | v) >> 7) & 0x01010101u;
+}
+
+// the 12 bytes of layer L under this thread's group of canvas pixels [x, x + n_px) of row y, zeros where the layer is
+// absent (the row or the pixels outside the layer); [seg0, seg0 + seg_px) is the CTA's segment
+__device__ __forceinline__ void fetch_group(const LayerDesc &L, int y, int seg0, int seg_px, int x, int n_px,
+                                            uint32_t (&w)[3]) {
+  w[0] = w[1] = w[2] = 0u;
+  const int ly = y - L.y0;
+  const int lx0 = seg0 - L.x0;                  // layer column of the segment's first pixel
+  if ((unsigned)ly >= (unsigned)L.h || lx0 >= L.w || lx0 + seg_px <= 0) return;   // uniform
+  const int lx = x - L.x0;
+  if (n_px <= 0 || lx >= L.w || lx + n_px <= 0) return;
+  const uint8_t *q = L.addr + (long long)ly * L.pitch + 3LL * lx;
+  if (n_px == kLayerGroupPx && lx >= 0 && lx + kLayerGroupPx <= L.w) {
+    const uint32_t phase = (uint32_t)reinterpret_cast<uintptr_t>(q) & 3u;   // uniform over the CTA
+    const uint32_t *a = reinterpret_cast<const uint32_t *>(q - phase);
+    const uint32_t a0 = __ldg(a), a1 = __ldg(a + 1), a2 = __ldg(a + 2), a3 = phase ? __ldg(a + 3) : 0u;
+    w[0] = __funnelshift_r(a0, a1, 8u * phase);
+    w[1] = __funnelshift_r(a1, a2, 8u * phase);
+    w[2] = __funnelshift_r(a2, a3, 8u * phase);
+  } else {                                      // the group straddles the layer's edge or the canvas end
+#pragma unroll
+    for (int k = 0; k < kLayerGroupPx; ++k) {
+      if (k < n_px && (unsigned)(lx + k) < (unsigned)L.w) {
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+          const int b = 3 * k + c;
+          w[b >> 2] |= (uint32_t)__ldg(q + b) << (8 * (b & 3));
+        }
+      }
+    }
+  }
+}
+
+// the segment's staged bytes [0, nb) go to dst: byte-wise head up to a 16-byte boundary, 16-byte units, byte-wise
+// tail; every thread of the CTA calls it after the stage is complete.  k_blend_layers keeps the same code inline:
+// calling this helper there compiles to a different schedule and register assignment (cuobjdump -sass), while the
+// inline copy leaves its SASS as it was before the helper existed.
+__device__ __forceinline__ void store_segment(const uint32_t (&stage)[kSegBytes / 4], uint8_t *dst, int nb) {
+  const int head = min(nb, (int)((16u - ((uint32_t)reinterpret_cast<uintptr_t>(dst) & 15u)) & 15u));
+  const int units = (nb - head) >> 4;
+  const int tail0 = head + 16 * units;
+  const uint8_t *stage8 = reinterpret_cast<const uint8_t *>(stage);
+  const int t = threadIdx.x;
+  if (t < units) {
+    const int off = head + 16 * t;              // a multiple of 4 plus (head & 3)
+    const int sh = off & 3;
+    const uint32_t *src = stage + (off >> 2);
+    const uint32_t a0 = src[0], a1 = src[1], a2 = src[2], a3 = src[3], a4 = sh ? src[4] : 0u;
+    reinterpret_cast<uint4 *>(dst + off)[0] =
+        make_uint4(__funnelshift_r(a0, a1, 8 * sh), __funnelshift_r(a1, a2, 8 * sh), __funnelshift_r(a2, a3, 8 * sh),
+                   __funnelshift_r(a3, a4, 8 * sh));
+  } else if (t >= kLayerThreads - 32) {         // one warp: head and tail bytes (fewer than 16 each)
+    const int k = t - (kLayerThreads - 32);
+    if (k < head) dst[k] = stage8[k];
+    else if (k >= 16 && tail0 + (k - 16) < nb) dst[tail0 + k - 16] = stage8[tail0 + k - 16];
+  }
+}
+
+}  // namespace apap

@@ -187,7 +187,7 @@ class PanoramaResult(NamedTuple):
 
 def stitch_panorama(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops, *, mesh_size: int = 100, gamma=0.5, sigma=100,
                     warp_imgs=None, blend_img=None, equalize: bool = True, ransac: str = "opencv",
-                    device=None) -> PanoramaResult:
+                    device=None, blend: str = "mean", sharpness=0.02) -> PanoramaResult:
     """Every image of a case stitched against the centre into ONE panorama (the reference has no multi-image blend;
     ``stitch_case`` returns one two-image canvas per pair, each in a frame of its own).
 
@@ -199,21 +199,40 @@ def stitch_panorama(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops, *, mesh_s
     blended by ``utils.blend_layers``: per pixel the floor mean of the non-empty layers.  With one other image the
     panorama is ``stitch_pair(...).stitched`` bit for bit; with none it is the centre image itself (``pairs == []``).
 
-    The layers are warped from the images the keypoint-pair producer already holds on the device and stay there; one
-    ``blend_layers`` launch and one download make the panorama.  At most 255 other images."""
-    from . import _runtime as rt
-    from .utils import _device_image, blend_layers
+    ``blend="feather"`` blends the same layers in the same order (the others, then the centre) by
+    ``utils.feather_blend(..., sharpness)``, OpenCV's ``FeatherBlender``: each layer's weight ramps up from its
+    boundary over about ``1 / sharpness`` pixels, so the seams along the layers' edges fade.  Every field but
+    ``panorama`` is the mean call's.  With no other image the panorama is ``feather_blend([centre])``, the centre less
+    1 where it is non-empty (OpenCV's ``trunc(v / 1.00001)``).  ``sharpness`` is used by ``"feather"`` only.
 
+    The layers are warped from the images the keypoint-pair producer already holds on the device and stay there; one
+    blend call and one download make the panorama.  At most 255 other images (127 with ``"feather"``); an unknown
+    ``blend``, too many images or a ``sharpness`` that ``feather_blend`` refuses for every canvas raise ``ValueError``
+    before any keypoint work."""
+    from . import _runtime as rt
+    from .utils import _device_image, _feather_sharpness, blend_layers, feather_blend
+
+    if blend not in ("mean", "feather"):
+        raise ValueError(f"stitch_panorama: blend must be 'mean' or 'feather', got {blend!r}")
     if warp_imgs is not None and len(warp_imgs) != len(other_imgs):
         raise ValueError(f"stitch_panorama: {len(other_imgs)} other images but {len(warp_imgs)} warp images")
-    if len(other_imgs) >= rt.BLEND_MAX_LAYERS:
-        raise ValueError(f"stitch_panorama: at most {rt.BLEND_MAX_LAYERS - 1} other images, got {len(other_imgs)}")
+    max_layers = rt.BLEND_MAX_LAYERS if blend == "mean" else rt.FEATHER_MAX_LAYERS
+    if len(other_imgs) >= max_layers:
+        raise ValueError(f"stitch_panorama: at most {max_layers - 1} other images with blend={blend!r}, "
+                         f"got {len(other_imgs)}")
+    if blend == "feather":
+        sharpness = _feather_sharpness("stitch_panorama", sharpness)
+
+        def blend_fn(layers, origins, size, device=None):
+            return feather_blend(layers, origins, size, sharpness, device=device)
+    else:
+        blend_fn = blend_layers
     front = _case_front(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops, mesh_size, gamma, sigma, equalize, ransac,
                         device)
     centre = center_img if blend_img is None else blend_img
     if front is None:
         h, w = centre.shape[0], centre.shape[1]
-        pano = blend_layers([centre], [(0, 0)], (w, h), device=device)
+        pano = blend_fn([centre], [(0, 0)], (w, h), device=device)
         if not isinstance(pano, np.ndarray):
             pano = rt.to_host(rt.torch_cuda(pano.device)[0], pano)
         return PanoramaResult((int(w), int(h), 0, 0), np.zeros((0, 2), np.int64), [], pano)
@@ -229,5 +248,5 @@ def stitch_panorama(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops, *, mesh_s
         # the grid as local_homography returned it, as stitch_pair hands it to the fused warp
         layers.append(st.local_warp(warp_devs[i], local_h.copy(), meshes[i]))
     (width, height, ox, oy), origins = panorama_size([p.final_size for p in pairs])
-    pano = blend_layers(layers + [blend_dev], [tuple(o) for o in origins] + [(ox, oy)], (width, height))
+    pano = blend_fn(layers + [blend_dev], [tuple(o) for o in origins] + [(ox, oy)], (width, height))
     return PanoramaResult((width, height, ox, oy), origins, pairs, rt.to_host(torch, pano))

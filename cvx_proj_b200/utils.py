@@ -24,7 +24,7 @@ from . import _runtime as rt
 
 __all__ = ["image_warping", "warp_perspective", "warping_canvas", "invert3x3", "match_descriptors", "coarse_matching",
            "sift_describe", "equalize_hist", "keypoint_pairs", "keypoint_pairs_batch", "find_homography_ransac",
-           "find_homography_ransac_batch", "blend_layers"]
+           "find_homography_ransac_batch", "blend_layers", "feather_blend"]
 
 
 def invert3x3(m) -> np.ndarray:
@@ -113,33 +113,106 @@ def blend_layers(layers, origins, size, device=None):
     All numpy in -> numpy out (uploaded to ``device``); all CUDA tensors (one device) in -> a tensor on that device.
     Tensor layers are read in place when their pixels are packed (strides ``(pitch, 3, 1)``), so crops of a larger
     image need no copy.  No CPU fallback."""
+    layers, origins, width, height, on_device, device = _check_layers("blend_layers", layers, origins, size,
+                                                                       rt.BLEND_MAX_LAYERS, device)
+    torch, device = rt.torch_cuda(device)
+    lib = rt.load_library()
+    devs, desc = _layer_descs(torch, device, layers, origins, on_device)
+    out = torch.empty((height, width, 3), dtype=torch.uint8, device=device)
+    with torch.cuda.device(device):
+        rt.check(lib.apap_blend_layers(desc.ctypes.data_as(ctypes.POINTER(ctypes.c_longlong)), len(devs), height, width,
+                                       out.data_ptr(), out.numel(), rt.stream_ptr(torch, device)), "apap_blend_layers")
+    return out if on_device else rt.to_host(torch, out)
+
+
+def feather_blend(layers, origins, size, sharpness=0.02, device=None):
+    """Feather blend of placed layers (``k_feather_rows``, ``k_feather_cols``, ``k_feather_blend``), bit for bit what
+    ``cv.detail.FeatherBlender(sharpness)`` gives after ``prepare((0, 0, W, H))``, ``feed(P_k.astype(int16), mask_k,
+    (0, 0))`` for every layer in the order given, and ``blend()``, converted to uint8 (``stitch_panorama(...,
+    blend="feather")``).
+
+    ``layers``, ``origins`` and ``size = (W, H)`` as for ``blend_layers``.  ``P_k`` is layer k pasted into a zero
+    ``H x W`` canvas (clipped) and ``mask_k`` its non-empty pixels (any channel > 0).  Each layer's weight rises as
+    ``min(D s, 1)`` (float32) with ``D`` the L1 distance to its nearest empty pixel -- pixels of the canvas outside the
+    layer count as empty, the canvas border does not -- so seams between layers fade over about ``1 / s`` pixels.
+    The weighted sum is kept as OpenCV keeps it (truncated int16 terms, float32 weights summed in layer order), so the
+    last bits depend on the layer order.  Where one layer alone has weight 1 the result is ``v - 1`` for ``v >= 1``
+    (``trunc(v / 1.00001)``): that is OpenCV's result, kept on purpose.
+
+    1 to 128 layers (OpenCV's int16 accumulator holds 128 x 255).  ``sharpness`` must be a finite float32 of at least
+    ``FLT_MIN`` (about 1.18e-38); below about 1.5e-5 the canvas must also have ``W + H <= 65536`` (distances are stored
+    in 16 bits).  ``ValueError`` before any launch otherwise.  Inputs and outputs as ``blend_layers``.  No CPU
+    fallback."""
+    layers, origins, width, height, on_device, device = _check_layers("feather_blend", layers, origins, size,
+                                                                       rt.FEATHER_MAX_LAYERS, device)
+    s = _feather_sharpness("feather_blend", sharpness)
+    lib = rt.load_library()
+    cap = ctypes.c_int()
+    rc = lib.apap_feather_distance_cap(s, height, width, ctypes.byref(cap))
+    if rc == rt.E_TOOBIG:
+        raise ValueError(f"feather_blend: sharpness {s} needs distances beyond 16 bits on a {width} x {height} canvas "
+                         "(a larger sharpness or W + H <= 65536)")
+    if rc != 0:
+        raise ValueError(f"feather_blend: {lib.apap_last_error().decode('utf-8', 'replace')}")
+    torch, device = rt.torch_cuda(device)
+    devs, desc = _layer_descs(torch, device, layers, origins, on_device)
+    desc_p = desc.ctypes.data_as(ctypes.POINTER(ctypes.c_longlong))
+    ws_bytes = ctypes.c_size_t()
+    rt.check(lib.apap_feather_workspace_bytes(desc_p, len(devs), height, width, ctypes.byref(ws_bytes)),
+             "apap_feather_workspace_bytes")
+    ws = torch.empty(max(ws_bytes.value, 16), dtype=torch.uint8, device=device)
+    out = torch.empty((height, width, 3), dtype=torch.uint8, device=device)
+    with torch.cuda.device(device):
+        rt.check(lib.apap_feather_blend(desc_p, len(devs), height, width, s, ws.data_ptr(), ws.numel(), out.data_ptr(),
+                                        out.numel(), rt.stream_ptr(torch, device)), "apap_feather_blend")
+    return out if on_device else rt.to_host(torch, out)
+
+
+def _feather_sharpness(what, sharpness):
+    """``sharpness`` as the float32 OpenCV's blender keeps, or ``ValueError``: it must be finite and at least
+    ``FLT_MIN``.  Below that (a subnormal), OpenCV gives a layer with no empty pixel the weight
+    ``min(fl(FLT_MAX s), 1)``, which can be < 1, and the kernels give it 1."""
+    with np.errstate(over="ignore"):
+        s = float(np.float32(sharpness))
+    if not (math.isfinite(s) and s >= np.finfo(np.float32).tiny):
+        raise ValueError(f"{what}: sharpness must be finite and >= FLT_MIN (a normal float32), got {sharpness}")
+    return s
+
+
+def _check_layers(what, layers, origins, size, max_layers, device):
+    """The argument checks ``blend_layers`` and ``feather_blend`` share (``ValueError`` named after ``what``).
+    Returns ``(layers, origins, width, height, on_device, device)``; ``device`` is the layers' own for tensors."""
     layers = list(layers)
     origins = [tuple(o) for o in origins]
-    if not 1 <= len(layers) <= rt.BLEND_MAX_LAYERS:
-        raise ValueError(f"blend_layers: 1 to {rt.BLEND_MAX_LAYERS} layers, got {len(layers)}")
+    if not 1 <= len(layers) <= max_layers:
+        raise ValueError(f"{what}: 1 to {max_layers} layers, got {len(layers)}")
     if len(origins) != len(layers) or any(len(o) != 2 for o in origins):
-        raise ValueError(f"blend_layers: one (x0, y0) origin per layer ({len(layers)} layers, {len(origins)} origins)")
+        raise ValueError(f"{what}: one (x0, y0) origin per layer ({len(layers)} layers, {len(origins)} origins)")
     width, height = (int(v) for v in size)
     if width <= 0 or height <= 0:
-        raise ValueError(f"blend_layers: the canvas size must be positive, got {tuple(size)}")
+        raise ValueError(f"{what}: the canvas size must be positive, got {tuple(size)}")
     numpy_in = [isinstance(img, np.ndarray) for img in layers]
     if any(numpy_in) and not all(numpy_in):
-        raise ValueError("blend_layers: layers must be all numpy arrays or all CUDA tensors")
+        raise ValueError(f"{what}: layers must be all numpy arrays or all CUDA tensors")
     on_device = not numpy_in[0]
     for k, img in enumerate(layers):
         if on_device and not getattr(img, "is_cuda", False):
-            raise ValueError(f"blend_layers: layer {k} is neither a numpy array nor a CUDA tensor")
+            raise ValueError(f"{what}: layer {k} is neither a numpy array nor a CUDA tensor")
         if len(img.shape) != 3 or img.shape[2] != 3 or img.shape[0] < 1 or img.shape[1] < 1:
-            raise ValueError(f"blend_layers: layer {k} must be [h, w, 3], got {tuple(img.shape)}")
+            raise ValueError(f"{what}: layer {k} must be [h, w, 3], got {tuple(img.shape)}")
         if (img.dtype != np.uint8) if not on_device else (str(img.dtype) != "torch.uint8"):
-            raise ValueError(f"blend_layers: layer {k} must be uint8, got {img.dtype}")
+            raise ValueError(f"{what}: layer {k} must be uint8, got {img.dtype}")
     if on_device:
         devs = {img.device for img in layers}
         if len(devs) != 1:
-            raise ValueError(f"blend_layers: all layers must be on one device, got {sorted(map(str, devs))}")
+            raise ValueError(f"{what}: all layers must be on one device, got {sorted(map(str, devs))}")
         device = layers[0].device
-    torch, device = rt.torch_cuda(device)
-    lib = rt.load_library()
+    return layers, origins, width, height, on_device, device
+
+
+def _layer_descs(torch, device, layers, origins, on_device):
+    """The layers on the device -- tensors in place when their pixels are packed (strides ``(pitch, 3, 1)``), numpy
+    uploaded -- and their C ABI descriptors ``int64 [n, 6] = {address, h, w, row pitch, x0, y0}``."""
     if on_device:
         devs = [img if img.stride(2) == 1 and img.stride(1) == 3 and (img.shape[0] == 1 or img.stride(0) >= 3 * img.shape[1])
                 else img.contiguous() for img in layers]
@@ -147,11 +220,7 @@ def blend_layers(layers, origins, size, device=None):
         devs = [rt.to_device(torch, device, img) for img in layers]
     desc = np.array([[img.data_ptr(), img.shape[0], img.shape[1], img.stride(0), x0, y0]
                      for img, (x0, y0) in zip(devs, origins)], dtype=np.int64)
-    out = torch.empty((height, width, 3), dtype=torch.uint8, device=device)
-    with torch.cuda.device(device):
-        rt.check(lib.apap_blend_layers(desc.ctypes.data_as(ctypes.POINTER(ctypes.c_longlong)), len(devs), height, width,
-                                       out.data_ptr(), out.numel(), rt.stream_ptr(torch, device)), "apap_blend_layers")
-    return out if on_device else rt.to_host(torch, out)
+    return devs, desc
 
 
 # ------------------------------------------------------------------ keypoint-pair producer (SURVEY 8f, row N3)

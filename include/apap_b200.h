@@ -244,6 +244,32 @@ int apap_blend_layers(const long long *layers, int n_layers, int canvas_h, int c
                       size_t out_bytes, void *stream);
 
 /*
+ * Feather blend of placed layers (utils.feather_blend, driver.stitch_panorama(blend="feather")): out [canvas_h]
+ * [canvas_w][3] uint8 (device, any alignment, out_bytes >= canvas_h x canvas_w x 3) is bit for bit what
+ * cv.detail.FeatherBlender(sharpness) gives after prepare((0, 0, canvas_w, canvas_h)), feed(P_k as int16, mask_k,
+ * (0, 0)) for every layer in order and blend(), converted to uint8.  P_k is layer k pasted into a zero canvas
+ * (clipped), mask_k its non-empty pixels (any channel > 0).  Per pixel and layer w = min(fl(D s), 1), D = the L1
+ * distance to the nearest empty pixel of P_k (the canvas border is not empty); acc += trunc(v w) per channel, wsum +=
+ * w in layer order; out = trunc(acc / (wsum + 1e-5)), 0 where wsum <= 1e-5.  Where one layer alone has weight 1 the
+ * result is v - 1 (v >= 1), as OpenCV's.
+ *   layers    : HOST long long [n_layers][6], as apap_blend_layers
+ *   n_layers  : 1 .. APAP_FEATHER_MAX_LAYERS (OpenCV's int16 accumulator holds 128 x 255)
+ *   sharpness : finite, >= FLT_MIN (a normal float), and apap_feather_distance_cap accepts it with this canvas
+ *   workspace : device scratch of apap_feather_workspace_bytes (2 bytes per layer pixel inside the canvas), 16-byte
+ *               aligned
+ * Three kernels (k_feather_rows, k_feather_cols, k_feather_blend) on `stream`.
+ * apap_feather_distance_cap: the distance the kernels store in place of larger ones (host only) -- the smallest
+ * integer d with fl(d s) >= 1, or canvas_h + canvas_w - 1 when that is smaller; APAP_E_TOOBIG when the cap exceeds
+ * 65535 (s below about 1.5e-5 on a canvas with canvas_h + canvas_w > 65536); APAP_E_BADARG for a sharpness that is
+ * not finite or below FLT_MIN.
+ */
+#define APAP_FEATHER_MAX_LAYERS 128
+int apap_feather_distance_cap(float sharpness, int canvas_h, int canvas_w, int *cap);
+int apap_feather_workspace_bytes(const long long *layers, int n_layers, int canvas_h, int canvas_w, size_t *bytes);
+int apap_feather_blend(const long long *layers, int n_layers, int canvas_h, int canvas_w, float sharpness,
+                       void *workspace, size_t workspace_bytes, uint8_t *out, size_t out_bytes, void *stream);
+
+/*
  * Input preparation on the device (what the host layer used to build in numpy; both reproduce their
  * numpy restatements in cvx_proj_b200/apap.py bit for bit).
  *
