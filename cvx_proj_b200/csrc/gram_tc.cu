@@ -49,8 +49,10 @@
 // MMA per keypoint block touches D1, and (b) every 256 keypoints (kSegKb blocks) the producers
 // drain D1 + D2 from TMEM (tcgen05.ld, SASS LDTM) into FP32 sums in shared memory and the MMAs
 // restart from zero; the per-split sums (<= 1024 keypoints, like the FFMA2 kernel) are written as
-// the same partial-sum layout and combined in float64 by K2.  Measured against a float64-accumulated
-// reference: 5e-7 mean / 7e-6 max of the largest sum per term (tools/gram_tc_lab.cu).
+// the same partial-sum layout and combined in float64 by K2.  Measured against the float64 reference of
+// tests/test_gram_reference.py, per partial entry and split, relative to its scale A = sum |w2 P_t| (B200, 1000 W,
+// over every case there): 2.8e-7 mean / 2.9e-6 max (the FFMA2 kernel: 8.7e-8 mean / 1.0e-5 max), at most 0.18 of
+// the test's bound (256 + 2 ln2 t) 2^-24 A.
 #include <type_traits>
 
 #include "common.cuh"

@@ -100,6 +100,10 @@ int apap_gram_partials(const float *kp_table, const float *anchors, int batch, i
  *   out_h  : float [batch][cells][9]
  *   out_sweeps : optional int32 [batch][cells]: > 0 Jacobi sweeps used, < 0 minus the number of
  *            inverse-iteration steps (NULL to skip)
+ * Planes scaled by a power of two give the same bits (K2 divides by sum(w^2) first).  A cell whose 24 sums are all
+ * zero (no weight at all) has the Gram matrix 0 / 0: it reports 0 Jacobi sweeps and stores T2inv e0 T1 divided by
+ * its [2][2] entry -- 0 for tmats whose last rows are [0 0 1] -- i.e. NaN where T2inv[:][0] T1[0][:] is 0, +-inf
+ * elsewhere.
  */
 #define APAP_EIG_AUTO   0
 #define APAP_EIG_JACOBI 1

@@ -206,7 +206,7 @@ def local_homography_svd(src_point, dst_point, vertices, gamma, sigma, cells=Non
     return out
 
 
-def local_homography_gram64(src_point, dst_point, vertices, gamma, sigma, chunk=2048):
+def local_homography_gram64(src_point, dst_point, vertices, gamma, sigma, chunk=2048, dtype=np.float32):
     """Fast float64 cross-check of pyviz/apap.py:147-168 for large grids.
 
     ``(WA)^T (WA) = A^T W^2 A``: the smallest right singular vector of the row-weighted
@@ -214,6 +214,7 @@ def local_homography_gram64(src_point, dst_point, vertices, gamma, sigma, chunk=
     a_2i+1 a_2i+1^T)``.  Float64 throughout; validated against ``local_homography_svd``
     in tests (agreement ~1e-7 on the size-normalised metric) -- it is a checker for
     sizes the per-cell SVD loop cannot finish, not a restatement of the SVD itself.
+    ``dtype=np.float64`` returns H before the final rounding (comparisons finer than a float32 ulp).
     """
     m, p, _ = vertices.shape
     n1, n2, c1, c2, aa = _prepare(src_point, dst_point)
@@ -226,7 +227,7 @@ def local_homography_gram64(src_point, dst_point, vertices, gamma, sigma, chunk=
     t2 = np.linalg.inv(n2).astype(np.float64) @ np.linalg.inv(c2).astype(np.float64)
     t1 = c1.astype(np.float64) @ n1.astype(np.float64)
     src64 = src_point.astype(np.float64)
-    out = np.empty((m * p, 3, 3), dtype=np.float32)
+    out = np.empty((m * p, 3, 3), dtype=dtype)
     for s in range(0, m * p, chunk):
         v = verts[s:s + chunk]
         d = np.sqrt((v[:, None, 0] - src64[None, :, 0]) ** 2 + (v[:, None, 1] - src64[None, :, 1]) ** 2)
@@ -235,7 +236,7 @@ def local_homography_gram64(src_point, dst_point, vertices, gamma, sigma, chunk=
         _, vecs = np.linalg.eigh(g)
         h = vecs[:, :, 0].reshape(-1, 3, 3)
         h = t2 @ h @ t1
-        out[s:s + chunk] = (h / h[:, 2:3, 2:3]).astype(np.float32)
+        out[s:s + chunk] = (h / h[:, 2:3, 2:3]).astype(dtype)
     return out.reshape(m, p, 3, 3)
 
 
