@@ -11,15 +11,14 @@ from ctypes import POINTER, c_char_p, c_double, c_float, c_int, c_size_t, c_void
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# APAP_B200_LIB: lab builds of the same library (tools/variants.sh); the product is the in-tree file
-LIB_PATH = os.environ.get("APAP_B200_LIB") or os.path.join(_HERE, "libapap_b200.so")
+LIB_PATH = os.path.join(_HERE, "libapap_b200.so")
 
 GRAM_TERMS = 24
 KP_ROW = 28
 KP_CHUNK = 128
 HINV_ROW = 12
 WARP_BLOCK_ROWS = 4
-ABI_VERSION = 22
+ABI_VERSION = 23
 KP_BLOCK = 8
 KP_BLOCK_FLOATS = 528
 GRAM_TCGEN05 = 0
@@ -28,7 +27,6 @@ EIG_AUTO = 0
 EIG_JACOBI = 1
 WARP_FORCE_EXACT = 1
 WARP_LEGACY = 2
-WARP_TILE_FUSED = 4
 RANSAC_MAX_ITERS = 1 << 20
 BLEND_MAX_LAYERS = 256
 FEATHER_MAX_LAYERS = 128

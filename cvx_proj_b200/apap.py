@@ -942,14 +942,13 @@ class APAP:
                           views[2].view(torch.int32), tiles, int(blocks.shape[0]), int(row0), int(row1))
 
     def warp_device(self, src_dev, tables, grid_cols, centre_dev=None, out=None, force_exact=False, multicast_ptr=None,
-                    legacy=False, tile_fused=False):
+                    legacy=False):
         """Device-resident K3 (optionally fused with K4): writes the canvas rows ``[tables.row0,
         tables.row1)`` into ``out`` (``[row1-row0, final_width, 3]`` uint8, allocated when None).
         ``multicast_ptr``: address of canvas row ``tables.row0`` inside an NVLS multicast mapping of a panorama buffer
         that every GPU of the group holds (``sharding.SymmetricPanorama``): the band is stored into all of them by
         the kernel itself and ``out`` is not written.  ``legacy``: round 1's strip kernel instead of the tile engine
-        (A/B timing and tests; same bytes).  ``tile_fused``: with ``centre_dev``, the tile engine's fused variant instead
-        of the strip kernel's (measured slower; A/B and tests)."""
+        (A/B timing and tests; same bytes).  With ``centre_dev`` the strip kernel runs either way."""
         torch, device = rt.torch_cuda(src_dev.device)
         lib = rt.load_library()
         fw = int(self.final_width)
@@ -965,8 +964,7 @@ class APAP:
                 tables.row0, tables.row1, centre_dev.data_ptr() if centre_dev is not None else None, ch, cw,
                 int(multicast_ptr) if multicast_ptr is not None else out.data_ptr(),
                 n_bytes if multicast_ptr is not None else out.numel(),
-                (rt.WARP_FORCE_EXACT if force_exact else 0) | (rt.WARP_LEGACY if legacy else 0)
-                | (rt.WARP_TILE_FUSED if tile_fused else 0),
+                (rt.WARP_FORCE_EXACT if force_exact else 0) | (rt.WARP_LEGACY if legacy else 0),
                 1 if multicast_ptr is not None else 0,
                 tables.tiles.data_ptr() if tables.tiles is not None else None,
                 rt.stream_ptr(torch, device)), "apap_warp")

@@ -115,7 +115,7 @@ int apap_warp(const uint8_t *src, int src_h, int src_w, const float *cell_fast, 
               int off_y, int row0, int row1, const uint8_t *centre, int centre_h, int centre_w, uint8_t *out_band,
               size_t out_band_bytes, int flags, int multicast, const void *tiles, void *stream) {
   if (!src || !cell_fast || !cell_hinv || !col_lut || !out_band) return fail(APAP_E_BADARG, "null pointer");
-  if (flags & ~(APAP_WARP_FORCE_EXACT | APAP_WARP_LEGACY | APAP_WARP_TILE_FUSED)) return fail(APAP_E_BADARG, "warp: unknown flag");
+  if (flags & ~(APAP_WARP_FORCE_EXACT | APAP_WARP_LEGACY)) return fail(APAP_E_BADARG, "warp: unknown flag");
   if (n_blocks < 0 || (n_blocks > 0 && !row_blocks)) return fail(APAP_E_BADARG, "warp: bad row blocks");
   if (src_h <= 0 || src_w <= 0 || canvas_w <= 0 || grid_cols <= 0) return fail(APAP_E_BADARG, "warp: sizes must be > 0");
   if (centre && (centre_h <= 0 || centre_w <= 0)) return fail(APAP_E_BADARG, "warp: bad centre image size");

@@ -17,16 +17,10 @@ constexpr int kHinvRow = APAP_HINV_ROW;     // 12 floats = 48 B per cell
 // Longest FP32 accumulation chain the Gram kernel runs before its sum leaves the register
 // (SURVEY.md finding 8: <= 1024 sequential FP32 terms, then a float64 combine, keeps the
 // per-cell H inside the 1e-4 gate; a single chain over all N does not).
-#ifndef APAP_MAX_CHAIN_CHUNKS
-#define APAP_MAX_CHAIN_CHUNKS 8
-#endif
-constexpr int kMaxChainChunks = APAP_MAX_CHAIN_CHUNKS;   // FFMA2 engine: 8 x 128 = 1024 keypoints per split
+constexpr int kMaxChainChunks = 8;   // FFMA2 engine: 8 x 128 = 1024 keypoints per split
 // The tensor-core engine never runs an FP32 chain longer than a 256-keypoint segment (its splits only exist for
 // parallelism), so its splits may be longer: fewer partial planes for K2 to read (c3: 311 -> 156 MB).
-#ifndef APAP_MAX_SPLIT_CHUNKS_TC
-#define APAP_MAX_SPLIT_CHUNKS_TC 16
-#endif
-constexpr int kMaxSplitChunksTc = APAP_MAX_SPLIT_CHUNKS_TC;   // 16 x 128 = 2048 keypoints per split.  32 (4096) was measured in round 2:
+constexpr int kMaxSplitChunksTc = 16;   // 16 x 128 = 2048 keypoints per split.  32 (4096) was measured in round 2:
 // c3 on one GPU 1.734 -> 1.709 ms (K2 reads half the planes), but an eighth of c3 is then 1.8 waves of CTAs instead of 3.5
 // and the 8-GPU shard goes from 0.251 to 0.270 ms -- the plan is a function of N only, so the sharded case decides
 

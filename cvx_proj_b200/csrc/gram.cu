@@ -42,13 +42,11 @@ int sm_count_cached() {
   return g_sm_count;
 }
 
-#ifndef APAP_SPLIT_DIV
-#define APAP_SPLIT_DIV 4     // lab knob: target number of keypoint splits
-#endif
+constexpr int kSplitDiv = 4;   // target number of keypoint splits
 GramPlan make_gram_plan(int cells, int n_kp_padded, int engine) {
   GramPlan p;
   const int n_chunks = n_kp_padded / kChunk;
-  int cps = (n_chunks + APAP_SPLIT_DIV - 1) / APAP_SPLIT_DIV;   // a function of N only (see header comment)
+  int cps = (n_chunks + kSplitDiv - 1) / kSplitDiv;   // a function of N only (see header comment)
   if (cps < 1) cps = 1;
   const int cap = engine == APAP_GRAM_TCGEN05 ? kMaxSplitChunksTc : kMaxChainChunks;
   if (cps > cap) cps = cap;

@@ -23,7 +23,7 @@
 //     a_full/a_empty (producers <-> MMA: two A slots in TMEM, slot h owned by the warps of parity h),
 //     d_full/d_empty (segment drains).
 //
-// What bounds it (in-kernel trace of the lab build, profiles/r01_gram_tc_trace.txt).  2 MUFU per weight at
+// What bounds it (in-kernel clock trace, profiles/r01_gram_tc_trace.txt).  2 MUFU per weight at
 // 16 lanes/clk/SM make the XU pipe the bound; a warp issues the MUFU of its step in order (8 cycles of XU
 // time each) and then spends ~600 cycles on work the XU does not see (split, STTM, tcgen05.wait::st,
 // fences, mbarrier round trips of ~90 cycles each), while the rest of the step needs ~60 % of the issue
@@ -59,23 +59,6 @@
 
 namespace apap {
 
-// lab knobs (tools/variants.sh builds the library with -D...; the defaults are the product)
-#ifndef APAP_TC_NOMUFU
-#define APAP_TC_NOMUFU 0         // 1: diagnostic, weights without the two MUFU operations (wrong results)
-#endif
-#ifndef APAP_TC_SMEM_STAGES
-#define APAP_TC_SMEM_STAGES 4
-#endif
-#ifndef APAP_TC_POLY
-#define APAP_TC_POLY 2           // weight pairs per k-block (of 4) whose 2^-t runs on the FMA pipe when gamma^2 >= 1/4
-#endif
-#ifndef APAP_TC_UNROLL
-#define APAP_TC_UNROLL 8          // producer loop unrolled over the ring positions and slot phases: addresses and parities are immediates (1: 131 us, 4: 128, 8: 125, 16: 126 at c2)
-#endif
-#ifndef APAP_TC_EARLY_PROBE
-#define APAP_TC_EARLY_PROBE 1    // 0: wait for the A slot before the step's arithmetic (A/B timing)
-#endif
-
 constexpr int kKB = APAP_KP_BLOCK;                 // keypoints per k-block = K of one TF32 MMA
 constexpr int kNT = 32;                            // accumulator columns (24 terms padded to the MMA N)
 constexpr int kKbFloats = APAP_KP_BLOCK_FLOATS;    // [Ph | Pl] tile 512, s*kx[8], s*ky[8]
@@ -83,21 +66,19 @@ constexpr int kKbBytes = kKbFloats * 4;            // 2112
 constexpr int kStepKb = 2;                         // k-blocks per producer/MMA hand-over ("step" = 16 keypoints)
 constexpr int kStageKb = 4;                        // k-blocks per shared-memory stage (2 steps: one per producer parity)
 constexpr int kStageBytesTc = kStageKb * kKbBytes; // 8448
-constexpr int kSmemStages = APAP_TC_SMEM_STAGES;
-constexpr int kUnroll = APAP_TC_UNROLL;
+constexpr int kSmemStages = 4;
+constexpr int kUnroll = 8;                         // producer loop unrolled over the ring positions and slot phases: addresses and parities are immediates (1: 131 us, 4: 128, 8: 125, 16: 126 at c2)
+constexpr int kPolyPairs = 2;                      // k_gram_tc's kPoly when gamma^2 >= 1/4 (the share measured best: above)
 constexpr int kSlots = 2;                          // A slots in TMEM: slot h = steps of parity h, 2 k-blocks x (8 hi + 8 lo columns)
 constexpr int kTmemCols = 128;                     // 32 (D1) + 32 (D2) + 2 * 32 (A)
 constexpr int kSegKb = 32;                         // k-blocks per accumulation segment (256 keypoints)
 constexpr int kSegSteps = kSegKb / kStepKb;
-#ifndef APAP_TC_PARITIES
-#define APAP_TC_PARITIES 2       // producer warps per lane quarter (1: 4 CTAs x 6 warps per SM, 2: 3 CTAs x 10 warps)
-#endif
-constexpr int kParities = APAP_TC_PARITIES;        // warps of a lane quarter take the steps s = h (mod kParities)
+constexpr int kParities = 2;                       // producer warps per lane quarter: they take the steps s = h (mod 2)
 constexpr int kProducerWarps = 4 * kParities;
 constexpr int kMmaWarp = kProducerWarps, kTmaWarp = kProducerWarps + 1;
 constexpr int kTcThreads = (kProducerWarps + 2) * 32;
-constexpr int kTcCtasPerSm = kParities == 1 ? 4 : 3;
-static_assert(kParities == 2 && kParities == kSlots, "two producer warps per lane quarter, each with its own A slot");
+constexpr int kTcCtasPerSm = 3;
+static_assert(kParities == kSlots, "each producer warp of a lane quarter has its own A slot");
 static_assert((kSmemStages & (kSmemStages - 1)) == 0, "the ring position is a mask of the stage index");
 static_assert(kKbFloats == 2 * kNT * kKB + 2 * kKB, "k-block layout");
 static_assert((kChunk / kKB) % kStageKb == 0, "a split is a whole number of stages");
@@ -221,16 +202,6 @@ __host__ __device__ constexpr uint32_t idesc_tf32(int n) {
   return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
 }
 
-// ------------------------------------------------------------------------------------------ lab trace
-#ifdef APAP_TC_TRACE
-__device__ long long g_trace[4][160][4];           // [role][step][mark] SM clock of CTA (APAP_TC_TRACE, 0, 0)
-__device__ long long g_cta[8192][4];               // per CTA: SM id, globaltimer at entry, after the TMEM allocation, at exit
-__device__ __forceinline__ long long gtimer() { long long t; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t)); return t; }
-#define TRACE(role, step, mark) do { if (blockIdx.y == APAP_TC_TRACE && blockIdx.x == 0 && (step) < 160) g_trace[role][step][mark] = clock64(); } while (0)
-#else
-#define TRACE(role, step, mark) do { } while (0)
-#endif
-
 // ------------------------------------------------------------------------------------------ kernel
 struct TcSmem {
   alignas(128) float stage[kSmemStages][kStageBytesTc / 4];
@@ -276,13 +247,6 @@ __global__ void __launch_bounds__(kTcThreads, kTcCtasPerSm) k_gram_tc(const floa
   anchors += (size_t)scene * cells * 2;
   partials += (size_t)scene * k_splits * kTerms * cells_padded;
 
-#ifdef APAP_TC_TRACE
-  const int cta_lin = blockIdx.y * gridDim.x + blockIdx.x;   // launch order
-  if (tid == 0 && cta_lin < 8192) {
-    uint32_t smid; asm volatile("mov.u32 %0, %smid;" : "=r"(smid));
-    g_cta[cta_lin][0] = smid; g_cta[cta_lin][1] = gtimer();
-  }
-#endif
   if (tid == 0) {
     for (int s = 0; s < kSmemStages; ++s) { mbar_init(&sm.smem_full[s], 1); mbar_init(&sm.smem_empty[s], 1); }
     for (int s = 0; s < kSlots; ++s) { mbar_init(&sm.a_full[s], 4); mbar_init(&sm.a_empty[s], 1); }
@@ -294,9 +258,6 @@ __global__ void __launch_bounds__(kTcThreads, kTcCtasPerSm) k_gram_tc(const floa
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
-#ifdef APAP_TC_TRACE
-  if (tid == 0 && cta_lin < 8192) g_cta[cta_lin][2] = gtimer();
-#endif
   const uint32_t tmem = sm.tmem_base;
   const uint32_t tmem_d = tmem;                    // columns [0, 32): hi x Ph sums; [32, 64): the two cross terms
   const uint32_t tmem_a = tmem + 2 * kNT;          // columns [64, 128): slot h, k-block e -> hi at 32 h + 16 e, lo + 8
@@ -309,26 +270,23 @@ __global__ void __launch_bounds__(kTcThreads, kTcCtasPerSm) k_gram_tc(const floa
     const float2 av = reinterpret_cast<const float2 *>(anchors)[min(c, cells - 1)];
     const float2 ax2 = make_float2(av.x, av.x), ay2 = make_float2(av.y, av.y);
     const uint32_t lane_base = (uint32_t)(q * 32) << 16;
-    // the terms this warp drains and writes: all 24, or half of them when two warps share the quarter
-    const int t0 = kParities == 1 ? 0 : 16 * h, nt = kParities == 1 ? kTerms : (h ? kTerms - 16 : 16);
+    // the terms this warp drains and writes: the first 16 (h = 0) or the last 8 (h = 1)
+    const int t0 = 16 * h, nt = h ? kTerms - 16 : 16;
     const float t_max = fminf(-__log2f(gamma_sq), 2.f);   // 2^-t_max = the clamp (polynomial path)
     int seg_done = 0;
     auto drain = [&]() {                           // add the finished segment's TMEM sums into the split's sums
       mbar_wait(&sm.d_full, seg_done & 1);
       tc_fence_after();
+      uint32_t v[16], u[16];
+      tmem_ld16(tmem_d + lane_base + t0, v);
+      tmem_ld16(tmem_d + lane_base + kNT + t0, u);
+      tmem_wait_ld();
 #pragma unroll
-      for (int half = 0; half < 2 / kParities; ++half) {
-        uint32_t v[16], u[16];
-        tmem_ld16(tmem_d + lane_base + t0 + 16 * half, v);
-        tmem_ld16(tmem_d + lane_base + kNT + t0 + 16 * half, u);
-        tmem_wait_ld();
-#pragma unroll
-        for (int t = 0; t < 16; ++t) {
-          if (16 * half + t < nt) {
-            const float add = __uint_as_float(v[t]) + __uint_as_float(u[t]);
-            float &dst = sm.acc[t0 + 16 * half + t][row];
-            dst = seg_done ? dst + add : add;
-          }
+      for (int t = 0; t < 16; ++t) {
+        if (t < nt) {
+          const float add = __uint_as_float(v[t]) + __uint_as_float(u[t]);
+          float &dst = sm.acc[t0 + t][row];
+          dst = seg_done ? dst + add : add;
         }
       }
       tc_fence_before();
@@ -351,13 +309,9 @@ __global__ void __launch_bounds__(kTcThreads, kTcCtasPerSm) k_gram_tc(const floa
 #pragma unroll kUnroll
     for (int it = 0; it < n_stage; ++it) {
       const uint32_t ss = (uint32_t)it & (kSmemStages - 1);
-      if (q == 0 && lane == 0) TRACE(h, it, 0);
       mbar_wait_at(bar_full0 + 8 * ss, ((uint32_t)it / kSmemStages) & 1);
       const uint32_t a_par = (it & 1) ^ 1;         // first use of the slot: free
-#if APAP_TC_EARLY_PROBE
       const uint32_t slot_free = mbar_test_at(bar_a_empty, a_par);   // consumed after the arithmetic
-#endif
-      if (q == 0 && lane == 0) TRACE(h, it, 1);
       uint32_t co = co0 + ss * kStageBytesTc;
       float w[kStepKb * 8];
 #pragma unroll
@@ -372,10 +326,6 @@ __global__ void __launch_bounds__(kTcThreads, kTcCtasPerSm) k_gram_tc(const floa
           const float2 dx = __fadd2_rn(ax2, make_float2(-kx[k].x, -kx[k].y));
           const float2 dy = __fadd2_rn(ay2, make_float2(-ky[k].x, -ky[k].y));
           const float2 d2 = __ffma2_rn(dy, dy, __fmul2_rn(dx, dx));
-#if APAP_TC_NOMUFU
-          w[8 * e + 2 * k] = fmaxf(1.f - d2.x, gamma_sq);
-          w[8 * e + 2 * k + 1] = fmaxf(1.f - d2.y, gamma_sq);
-#else
           if (kPoly > 0 && k >= 4 - kPoly) {
             // 2^-min(t, t_max) by a degree-7 polynomial in u = t - 1 on [-1, 1] (max relative error 1.6e-7)
             const float2 u = __fadd2_rn(kNoClamp ? make_float2(sqrt_approx(d2.x), sqrt_approx(d2.y))
@@ -394,16 +344,10 @@ __global__ void __launch_bounds__(kTcThreads, kTcCtasPerSm) k_gram_tc(const floa
             w[8 * e + 2 * k] = kNoClamp ? ex2_approx(-sqrt_approx(d2.x)) : fmaxf(ex2_approx(-sqrt_approx(d2.x)), gamma_sq);
             w[8 * e + 2 * k + 1] = kNoClamp ? ex2_approx(-sqrt_approx(d2.y)) : fmaxf(ex2_approx(-sqrt_approx(d2.y)), gamma_sq);
           }
-#endif
         }
       }
-#if APAP_TC_EARLY_PROBE
       if (!slot_free) mbar_wait_at(bar_a_empty, a_par);
-#else
-      mbar_wait_at(bar_a_empty, a_par);
-#endif
       tc_fence_after();
-      if (q == 0 && lane == 0) TRACE(h, it, 2);
 #pragma unroll
       for (int e = 0; e < kStepKb; ++e) {
         uint32_t hl[16];                               // TF32 heads, then tails: the 16 A columns of k-block e
@@ -422,7 +366,6 @@ __global__ void __launch_bounds__(kTcThreads, kTcCtasPerSm) k_gram_tc(const floa
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive_at(bar_a_full);
-      if (q == 0 && lane == 0) TRACE(h, it, 3);
       // a segment behind: its MMAs have had a step's worth of time to retire
       if ((it & (kSegKb / kStageKb - 1)) == 0 && it) drain();
     }
@@ -501,9 +444,6 @@ __global__ void __launch_bounds__(kTcThreads, kTcCtasPerSm) k_gram_tc(const floa
   if (warp == 0) tmem_dealloc(tmem, kTmemCols);
   // one more split of this tile is complete (release: every writer fenced before the barrier above)
   if (tid == 0 && tile_done) atomicAdd(tile_done + (size_t)scene * gridDim.y + tile, 1);
-#ifdef APAP_TC_TRACE
-  if (tid == 0 && cta_lin < 8192) g_cta[cta_lin][3] = gtimer();
-#endif
 }
 
 int launch_gram_tc(const float *kp_blocks, const float *anchors, int batch, int cells, int n_kp_padded, float gamma_sq,
@@ -513,18 +453,13 @@ int launch_gram_tc(const float *kp_blocks, const float *anchors, int batch, int 
   const int kb_per_split = p.chunks_per_split * (kChunk / kKB);
   dim3 grid(p.k_splits, (cells + 127) / 128, batch);
   if (grid.y > 65535 || batch > 65535) return fail(APAP_E_TOOBIG, "gram: more than 65535 cell tiles (8.3 M cells) or scenes per launch");
-  if (APAP_TC_POLY > 0 && gamma_sq >= 0.25f && gamma_sq <= 1.f)   // the polynomial covers 2^-t for t in [0, 2]
-    k_gram_tc<APAP_TC_POLY><<<grid, kTcThreads, sizeof(TcSmem), st>>>(kp_blocks, anchors, cells, p.cells_padded, n_kb,
-                                                                      kb_per_split, p.k_splits, gamma_sq, t_bound, partials, tile_done);
+  if (gamma_sq >= 0.25f && gamma_sq <= 1.f)   // the polynomial covers 2^-t for t in [0, 2]
+    k_gram_tc<kPolyPairs><<<grid, kTcThreads, sizeof(TcSmem), st>>>(kp_blocks, anchors, cells, p.cells_padded, n_kb,
+                                                                    kb_per_split, p.k_splits, gamma_sq, t_bound, partials, tile_done);
   else
     k_gram_tc<0><<<grid, kTcThreads, sizeof(TcSmem), st>>>(kp_blocks, anchors, cells, p.cells_padded, n_kb, kb_per_split,
                                                            p.k_splits, gamma_sq, t_bound, partials, tile_done);
   return check_cuda(cudaGetLastError(), "k_gram_tc launch");
 }
-
-#ifdef APAP_TC_TRACE
-extern "C" int apap_lab_trace(long long *out) { return (int)cudaMemcpyFromSymbol(out, g_trace, sizeof(g_trace)); }
-extern "C" int apap_lab_cta_trace(long long *out) { return (int)cudaMemcpyFromSymbol(out, g_cta, sizeof(g_cta)); }
-#endif
 
 }  // namespace apap

@@ -13,8 +13,9 @@
 //      bytes: 1-2 L1 wavefronts per byte plane);
 //   3. combine, blend, re-pack the warp's 96 output bytes of a row into 24 aligned 32-bit stores
 //      with two shuffles + one byte-permute.
-// The loop is software pipelined: phases 1-2 of block t+1 are issued before phase 3 of block t, so
-// two blocks' gathers are in flight per lane while the previous block is stored.
+// A warp visits two consecutive blocks at a time and finishes the first before it issues the second
+// (both blocks' gathers in flight before the first store: the same plain, +13 % fused at c2 --
+// profiles/r01_warp_variants.txt).
 //
 // Pixel selection must equal the reference's float64 arithmetic (float32 H^-1 promoted to
 // float64, divide, strict bounds, truncate).  The float32 fast path works in cell-relative
@@ -30,12 +31,8 @@
 
 namespace apap {
 
-#ifndef APAP_WARP_PIPELINE
-#define APAP_WARP_PIPELINE 0     // 1: the gathers of both blocks of a visit in flight before the first is stored
-#endif
-#ifndef APAP_WARP_CTAS
-#define APAP_WARP_CTAS 4         // resident CTAs per SM the kernel is compiled for (register cap 64 / 85 / 128)
-#endif
+constexpr int kWarpCtas = 4;     // resident CTAs per SM the kernel is compiled for: register cap 64 (3 CTAs, cap 85:
+                                 // c2 36.9 against 32.8 us -- profiles/r01_warp_variants.txt)
 constexpr int kWarpThreads = 256;
 constexpr int kWarpsPerCta = kWarpThreads / 32;
 // Phases 1 + 2 of one row block of one lane: the source pixel index of every row, then all byte
@@ -172,7 +169,7 @@ __device__ __forceinline__ void prefetch_l1(const void *ptr) {
 // column state stays loop invariant.  The cell record of the next visit is prefetched into L1
 // while the current visit's gathers are in flight.
 template <bool kBlend, bool kWords>
-__global__ void __launch_bounds__(kWarpThreads, APAP_WARP_CTAS) k_warp(const WarpParams p) {
+__global__ void __launch_bounds__(kWarpThreads, kWarpCtas) k_warp(const WarpParams p) {
   const int lane = threadIdx.x & 31;
   const int chunk = blockIdx.x * kWarpsPerCta + (threadIdx.x >> 5);
   if (chunk >= p.chunks_per_row) return;           // warp-uniform
@@ -220,19 +217,10 @@ __global__ void __launch_bounds__(kWarpThreads, APAP_WARP_CTAS) k_warp(const War
         prefetch_l1(rec);
         prefetch_l1(rec + 32);
       }
-#if APAP_WARP_PIPELINE
-      // both blocks' gathers in flight before the first block is packed and stored
-      uint32_t b0[kBlockRows], b1[kBlockRows], b2[kBlockRows], cb0[kBlockRows], cb1[kBlockRows], cb2[kBlockRows];
-      enter_cell_row(p, cl, dxf, (int)(cur1.y & 0xffffu), c);
-      block_issue<kBlend, true>(p, src, i0b, nb, (float)(cur1.y >> 16), x, col_ok, c, b0, b1, b2, cb0, cb1, cb2);
-      block_store<kBlend, kWords, true>(p, i0a, na, a0, a1, a2, ca0, ca1, ca2, lane_off, pitch, lane_a, lane_b, sel, store_ok);
-      block_store<kBlend, kWords, true>(p, i0b, nb, b0, b1, b2, cb0, cb1, cb2, lane_off, pitch, lane_a, lane_b, sel, store_ok);
-#else
       block_store<kBlend, kWords, true>(p, i0a, na, a0, a1, a2, ca0, ca1, ca2, lane_off, pitch, lane_a, lane_b, sel, store_ok);
       enter_cell_row(p, cl, dxf, (int)(cur1.y & 0xffffu), c);
       block_issue<kBlend, true>(p, src, i0b, nb, (float)(cur1.y >> 16), x, col_ok, c, a0, a1, a2, ca0, ca1, ca2);
       block_store<kBlend, kWords, true>(p, i0b, nb, a0, a1, a2, ca0, ca1, ca2, lane_off, pitch, lane_a, lane_b, sel, store_ok);
-#endif
     } else {                                       // partial blocks (cell rows shorter than 4 canvas rows, band end)
       enter_cell_row(p, cl, dxf, (int)(cur0.y & 0xffffu), c);
       block_issue<kBlend, false>(p, src, i0a, na, (float)(cur0.y >> 16), x, col_ok, c, a0, a1, a2, ca0, ca1, ca2);
@@ -297,10 +285,6 @@ __device__ __forceinline__ void blend_tail(const uint8_t *__restrict__ a8, const
   }
 }
 
-#ifndef APAP_BLEND_TMA
-#define APAP_BLEND_TMA 1         // 0 (lab): every thread loads and stores its own 48 bytes straight from / to global memory
-#endif
-
 // CTA = 256 units of 16 pixels = 12 KB per image.  One thread moves the CTA's slice of both images into shared memory
 // with two TMA bulk copies and the result back with one (whole 128-byte lines on the wire, no per-thread address
 // arithmetic); the threads read their 48 bytes as three LDS.128 (stride 48 B: conflict-free per quarter warp) and
@@ -313,7 +297,6 @@ struct BlendSmem {
 
 __global__ void __launch_bounds__(kBlendThreads) k_blend(const uint8_t *__restrict__ a8, const uint8_t *__restrict__ b8,
                                                           uint8_t *__restrict__ out8, long long n_vec3, long long n_px) {
-#if APAP_BLEND_TMA
   __shared__ __align__(128) BlendSmem sm;
   const long long unit0 = (long long)blockIdx.x * kBlendThreads;
   const long long left = n_vec3 - unit0;
@@ -351,27 +334,6 @@ __global__ void __launch_bounds__(kBlendThreads) k_blend(const uint8_t *__restri
     bulk_s2g(out8 + unit0 * 48, sm.a, bytes);
     bulk_commit_wait_read();
   }
-#else
-  const uint4 *a = reinterpret_cast<const uint4 *>(a8), *b = reinterpret_cast<const uint4 *>(b8);
-  uint4 *out = reinterpret_cast<uint4 *>(out8);
-  const long long gid = (long long)blockIdx.x * kBlendThreads + threadIdx.x;
-  if (gid < n_vec3) {
-    uint32_t wa[12], wb[12], wo[12];
-#pragma unroll
-    for (int v = 0; v < 3; ++v) {
-      const uint4 x = __ldcs(a + gid * 3 + v);
-      const uint4 y = __ldcs(b + gid * 3 + v);
-      wa[4 * v + 0] = x.x; wa[4 * v + 1] = x.y; wa[4 * v + 2] = x.z; wa[4 * v + 3] = x.w;
-      wb[4 * v + 0] = y.x; wb[4 * v + 1] = y.y; wb[4 * v + 2] = y.z; wb[4 * v + 3] = y.w;
-    }
-    blend16(wa, wb, wo);
-#pragma unroll
-    for (int v = 0; v < 3; ++v)
-      __stcs(out + gid * 3 + v, make_uint4(wo[4 * v], wo[4 * v + 1], wo[4 * v + 2], wo[4 * v + 3]));
-  } else if (gid == n_vec3) {
-    blend_tail(a8, b8, out8, n_vec3 * 16, n_px);
-  }
-#endif
 }
 
 int launch_warp(const uint8_t *src, int src_h, int src_w, const float *cell_fast, const float *cell_hinv,
@@ -397,24 +359,20 @@ int launch_warp(const uint8_t *src, int src_h, int src_w, const float *cell_fast
   p.src_h = src_h; p.src_w = src_w; p.grid_cols = grid_cols; p.canvas_w = canvas_w;
   p.off_x = off_x; p.off_y = off_y; p.centre_h = centre_h; p.centre_w = centre_w; p.force_exact = force_exact;
   p.multicast = multicast;
-#ifdef APAP_WARP_NOWORDS
-  const bool words = false;                        // lab: byte stores always
-#else
   const bool words = (canvas_w % 4 == 0) && !(reinterpret_cast<uintptr_t>(out_band) & 3u);
-#endif
   if (multicast && (!words || canvas_w % 16 != 0 || (reinterpret_cast<uintptr_t>(out_band) & 15u)))
     return fail(APAP_E_ALIGN, "warp: multicast stores need canvas_w % 16 == 0 and a 16-byte aligned band");
-  // the tile engine (csrc/warp_tile.cu) when the caller built tile records and the source rows are 16-byte aligned
-  // (plain warp by default: fused with the blend, the strip kernel's batched centre loads are faster -- c2 49 us against
-  // 65 us, c3 169 against 198 --; APAP_WARP_TILE_FUSED asks for the tile engine's fused variant all the same, for the A/B)
-  if (tiles && (!centre || (flags & APAP_WARP_TILE_FUSED)) && !(flags & APAP_WARP_LEGACY) && warp_tile_usable(p)) {
+  // the tile engine (csrc/warp_tile.cu) for the plain warp when the caller built tile records and the source rows are
+  // 16-byte aligned.  Fused with the blend, the warp runs on the strip kernel: its batched centre loads are faster than
+  // centre gathers inside the tile loop (c2 49 us against 65 us, c3 169 against 198)
+  if (tiles && !centre && !(flags & APAP_WARP_LEGACY) && warp_tile_usable(p)) {
     if (reinterpret_cast<uintptr_t>(tiles) & 15u) return fail(APAP_E_ALIGN, "warp: tiles must be 16-byte aligned");
     return launch_warp_tile(p, words, tiles, st);
   }
   // legacy strip kernel.  One resident wave: grid.x CTAs side by side cover the canvas width, grid.y of them share its height
   const int gx = (p.chunks_per_row + kWarpsPerCta - 1) / kWarpsPerCta;
   const int visits = (n_blocks + 1) / 2;           // a visit = two consecutive row blocks
-  int gy = (sm_count_cached() * APAP_WARP_CTAS) / gx;   // APAP_WARP_CTAS CTAs of 8 warps resident per SM (launch bounds)
+  int gy = (sm_count_cached() * kWarpCtas) / gx;   // kWarpCtas CTAs of 8 warps resident per SM (launch bounds)
   if (gy < 1) gy = 1;
   if (gy > visits) gy = visits;
   if (gy > 65535) gy = 65535;

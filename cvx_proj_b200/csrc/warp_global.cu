@@ -66,14 +66,8 @@ struct SegRec {
   float eps;                // error bound of the float32 sum; < 0: every pixel of the segment takes the float64 path
 };
 
-#ifndef APAP_GW_TILE_H
-#define APAP_GW_TILE_H 16    // lab knob: canvas rows per CTA tile (even, <= 32: one thread per (row, segment) in phase 1)
-#endif
-#ifndef APAP_GW_PREFETCH
-#define APAP_GW_PREFETCH 0   // lab knob: L2 prefetch of the next pass's source rows
-#endif
-__device__ __forceinline__ void prefetch_l2(const void *ptr) { asm volatile("prefetch.global.L2 [%0];" ::"l"(ptr)); }
-constexpr int kTileW = 256, kTileH = APAP_GW_TILE_H, kSegs = kTileW / 32;
+// kTileH: canvas rows per CTA tile (even, <= 32: one thread per (row, segment) in phase 1)
+constexpr int kTileW = 256, kTileH = 16, kSegs = kTileW / 32;
 
 __device__ __forceinline__ SegRec make_segment(const GlobalWarpParams &p, int xs, int y) {
   SegRec r;
@@ -207,14 +201,6 @@ __global__ void __launch_bounds__(256) k_warp_global(const GlobalWarpParams p) {
         const uint8_t *q1 = q + src_pitch;
 #pragma unroll
         for (int e = 0; e < 6; ++e) { v[k][e] = __ldg(q + e); v[k][6 + e] = __ldg(q1 + e); }
-#if APAP_GW_PREFETCH
-        if (k == 1) {                                // the source rows the next pass of this warp will read
-          const uint8_t *last = p.src + (size_t)(p.src_h - 1) * src_pitch;
-          const uint8_t *n0 = q1 + src_pitch, *n1 = q1 + 2 * src_pitch;
-          prefetch_l2(n0 < last ? n0 : last);
-          prefetch_l2(n1 < last ? n1 : last);
-        }
-#endif
       }
 #pragma unroll
       for (int k = 0; k < 2; ++k) {

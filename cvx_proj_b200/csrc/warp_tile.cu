@@ -1,5 +1,7 @@
 // K3, tile engine -- mesh warp through shared-memory tiles (reference APAP.local_warp pixel loop,
-// pyviz/apap.py:206-215), optionally fused with K4 (pyviz/apap_utils.py:75-88, pyviz/apap.py:259-261).
+// pyviz/apap.py:206-215).  The plain warp only: fused with K4, the warp runs on the strip kernel of
+// csrc/warp_blend.cu, whose batched centre loads beat centre gathers inside the tile loop (c2 49 us against 65 us:
+// profiles/r02_warp_tile_history.md).  The engine reads no environment: its schedule is the constants below.
 //
 // A tile is 128 canvas columns x 8 consecutive row blocks (<= 32 rows).
 //
@@ -39,7 +41,6 @@
 #include <atomic>
 #include <limits.h>
 #include <stddef.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include "common.cuh"
@@ -47,42 +48,29 @@
 
 namespace apap {
 
-#ifndef APAP_TILE_CTAS
-#define APAP_TILE_CTAS 3
-#endif
-#ifndef APAP_TILE_STAGES
-#define APAP_TILE_STAGES 2       // source-box stages of the ring (3 stages x 24-row tiles measured the same: profiles/)
-#endif
-#ifndef APAP_TILE_BLOCKS
-#define APAP_TILE_BLOCKS 8       // row blocks per tile (8 -> 32 rows, 20 KB box; 6 -> 24 rows, 16 KB box)
-#endif
-#ifndef APAP_TILE_BOX_KB
-#define APAP_TILE_BOX_KB (APAP_TILE_BLOCKS == 8 ? 20 : 16)
-#endif
-#ifndef APAP_TILE_GROUP
-#define APAP_TILE_GROUP 4
-#endif
+constexpr int kTileCtas = 3;                              // resident CTAs per SM, 2 stages each: 6 boxes in flight per SM
 constexpr int kWorkerWarps = 8;
 constexpr int kWorkerThreads = kWorkerWarps * 32;
 constexpr int kTileThreads = kWorkerThreads + 32;         // + the producer warp
 constexpr int kTileCols = 128;                            // 4 chunks of 32 columns
-constexpr int kStages = APAP_TILE_STAGES;
-constexpr int kTileBlocks = APAP_TILE_BLOCKS;             // row blocks per tile
+// source-box stages of the ring x row blocks per tile: 2 x 8 (32 rows, 20 KB box); 3 x 6 (24 rows, 16 KB box) measured
+// the same (profiles/r02_warp_tile_history.md)
+constexpr int kStages = 2;
+constexpr int kTileBlocks = 8;                            // row blocks per tile
 constexpr int kTileRows = kTileBlocks * kBlockRows;       // 32
 constexpr int kWarpRows = kTileRows / 2;                  // 16 canvas rows per worker warp
 static_assert(kTileBlocks <= 8 && kTileBlocks % 2 == 0 && kStages >= 2, "tile shape");
 constexpr int kWarpPitch = 32 * 3;                        // 96 B: a worker warp's 32 columns
 constexpr int kWarpOutBytes = kWarpRows * kWarpPitch;     // 1536 B: a warp's dense output block
-constexpr int kBoxBytes = APAP_TILE_BOX_KB * 1024;        // staged source box
+constexpr int kBoxBytes = 20 * 1024;                      // staged source box
 constexpr uint32_t kFlagOff = kBoxBytes + 4;              // staged mode, "guard band" marker: reads the zero word behind the box
 constexpr uint32_t kNoPixel = 0xffffffffu;                // global mode: "leave black"
 constexpr uint32_t kFlagPixel = 0xfffffffeu;              // global mode: guard band
 constexpr int kMaxCellCols = 32;                          // footprint: at most this many cell columns per tile
 constexpr int kCounterSlots = 64;                         // tile counters: launch n uses slot n % 64
-constexpr int kGroupRows = APAP_TILE_GROUP;               // rows a lane processes per loop iteration (independent gathers in flight)
-static_assert(kGroupRows == 4 || kGroupRows == 8, "row group");
+constexpr int kGroupRows = 4;                             // rows a lane processes per loop iteration (independent gathers in flight)
 constexpr int kRecRuns = 4;                               // cell rows of a tile whose records are staged ...
-constexpr int kRecCols = kStages > 2 ? 7 : 16;            // ... for at most this many cell columns (else global loads)
+constexpr int kRecCols = 16;                              // ... for at most this many cell columns (else global loads)
 
 enum TileMode : int { kBlack = 0, kStagedMode = 1, kGlobal = 3, kDone = 4 };
 
@@ -129,7 +117,7 @@ struct TileSmem {
 
 static_assert(offsetof(Stage, zero) == kBoxBytes, "the zero word sits right behind the staged box");
 static_assert(box_w(0) * box_h(0) <= kBoxBytes && box_w(1) * box_h(1) <= kBoxBytes && box_w(2) * box_h(2) <= kBoxBytes, "box shapes");
-static_assert(sizeof(TileSmem) * APAP_TILE_CTAS + 1024 * APAP_TILE_CTAS <= 227 * 1024, "shared memory of the resident CTAs");
+static_assert(sizeof(TileSmem) * kTileCtas + 1024 * kTileCtas <= 227 * 1024, "shared memory of the resident CTAs");
 
 __device__ unsigned int g_tile_next[kCounterSlots];       // tiles handed out beyond the first gridDim.x
 __device__ unsigned int g_tile_done[kCounterSlots];       // CTAs that have stopped claiming (the last one resets the slot)
@@ -142,7 +130,6 @@ struct TileParams {
   int store_mode;                // 0 bytes, 1 words, 2 TMA (one tensor-map store per warp block), 3 multimem
   int tiles_x, n_tiles;
   int slot;                      // which pair of tile counters this launch uses
-  int lab;                       // timing experiments only (APAP_TILE_LAB): 1 workers skip the pixel work, 2 no L2 prefetch
   TileInfo *tiles;               // [n_tiles]: written by k_tile_prep (apap_warp_tiles), streamed by the producer warps
 };
 
@@ -177,30 +164,16 @@ __device__ __forceinline__ void bulk_wait_read_all() { asm volatile("cp.async.bu
 __device__ __forceinline__ void bulk_wait_read_but_one() { asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory"); }
 __device__ __forceinline__ void prefetch_l2(const void *ptr) { asm volatile("prefetch.global.L2 [%0];" ::"l"(ptr)); }
 
-// uniform_blend of one pixel packed as b0 | b1 << 8 | b2 << 16 with the centre image's pixel (0 = none)
-__device__ __forceinline__ uint32_t blend_px(uint32_t val, uint32_t cv) {
-  if (cv != 0) val = (val != 0) ? __vhaddu4(val, cv) : cv;
-  return val;
-}
-
-__device__ __forceinline__ uint32_t centre_px(const WarpParams &p, int cx, int cy, bool col_ok) {
-  if ((unsigned)cy < (unsigned)p.centre_h && (unsigned)cx < (unsigned)p.centre_w && col_ok) {
-    const uint8_t *q = p.centre + ((size_t)cy * p.centre_w + cx) * 3;
-    return (uint32_t)__ldg(q) | ((uint32_t)__ldg(q + 1) << 8) | ((uint32_t)__ldg(q + 2) << 16);
-  }
-  return 0u;
-}
-
-// kRows (1, 2, 4 or 8) consecutive canvas rows of one lane (same cell): gather offsets on the float32 fast path --
+// kRows (1, 2 or 4) consecutive canvas rows of one lane (same cell): gather offsets on the float32 fast path --
 // packed FP32x2, two rows per instruction; same arithmetic and decisions as block_issue of csrc/warp_blend.cu --,
-// gathers, blend, bytes into the warp's output block; then the float64 path for the rows whose quotient lies inside
+// gathers, bytes into the warp's output block; then the float64 path for the rows whose quotient lies inside
 // the guard band.  All kRows pixels are independent: that many gathers are in flight per lane.
 //   kStaged: the shared-memory address of the pixel comes straight from the float bits of the floors
 //   (address = ty_bits * pitch + tx_bits * 3 + kbase), no bounds test: whatever the tile can pick is inside
 //   the staged box and the box is zero outside the image;  else: test against the image, gather from global memory.
-template <bool kStaged, bool kBlend, int kRows>
+template <bool kStaged, int kRows>
 __device__ __forceinline__ void tile_rows(const WarpParams &p, const CellState &c, int pitch, int kbase, uint32_t guard_addr,
-                                          uint8_t *__restrict__ orow, float dy0, int x, int y, bool col_ok) {
+                                          uint8_t *__restrict__ orow, float dy0, int x, int y) {
   constexpr int kPairs = (kRows + 1) / 2;
   const uint32_t guard = kStaged ? guard_addr : kFlagPixel;
   const float2 km = make_float2(kMagic, kMagic), nkm = make_float2(-kMagic, -kMagic), nh = make_float2(-0.5f, -0.5f);
@@ -241,11 +214,6 @@ __device__ __forceinline__ void tile_rows(const WarpParams &p, const CellState &
       so[2 * k + e] = clear ? off : guard;
     }
   }
-  uint32_t cv[kBlend ? kRows : 1];              // fused blend: the centre image's pixels, all loads in flight before the gathers
-  if (kBlend) {
-#pragma unroll
-    for (int k = 0; k < kRows; ++k) cv[k] = centre_px(p, x, y + k, col_ok);
-  }
   bool any_guard = false;
 #pragma unroll
   for (int k = 0; k < kRows; ++k) {
@@ -263,10 +231,6 @@ __device__ __forceinline__ void tile_rows(const WarpParams &p, const CellState &
         b0 = __ldg(q); b1 = __ldg(q + 1); b2 = __ldg(q + 2);
       }
     }
-    if (kBlend) {
-      const uint32_t val = blend_px(b0 | (b1 << 8) | (b2 << 16), cv[k]);
-      b0 = val & 0xffu; b1 = (val >> 8) & 0xffu; b2 = val >> 16;
-    }
     uint8_t *dst = orow + k * kWarpPitch;
     dst[0] = (uint8_t)b0; dst[1] = (uint8_t)b1; dst[2] = (uint8_t)b2;
   }
@@ -282,7 +246,6 @@ __device__ __forceinline__ void tile_rows(const WarpParams &p, const CellState &
         const uint8_t *q = p.src + (size_t)(unsigned)idx * 3;
         val = (uint32_t)__ldg(q) | ((uint32_t)__ldg(q + 1) << 8) | ((uint32_t)__ldg(q + 2) << 16);
       }
-      if (kBlend) val = blend_px(val, cv[k]);
       uint8_t *dst = orow + k * kWarpPitch;
       dst[0] = (uint8_t)val; dst[1] = (uint8_t)(val >> 8); dst[2] = (uint8_t)(val >> 16);
     }
@@ -292,10 +255,10 @@ __device__ __forceinline__ void tile_rows(const WarpParams &p, const CellState &
 // A worker warp's share of one tile: 32 columns x the canvas rows [row_lo, row_hi].  The tile's rows come as runs of
 // one cell row each; per run the lane's cell record is set up once (from shared memory, where the producer staged
 // it), then the rows go by four at a time.
-template <bool kStaged, bool kBlend>
+template <bool kStaged>
 __device__ __forceinline__ void tile_warp_rows(const WarpParams &p, const TileInfo &f, const Stage &stg,
-                                               uint8_t *__restrict__ warp_out, const uint2 cl, int x, bool col_ok,
-                                               int lane, int row_lo, int row_hi) {
+                                               uint8_t *__restrict__ warp_out, const uint2 cl, int x, int lane, int row_lo,
+                                               int row_hi) {
   // tile-invariant values into registers once (the byte stores into the output block could alias them for the compiler)
   const int x_lo = f.x_lo, y_lo = f.y_lo, bpitch = f.pitch, shift = f.shift, rec_ok = f.rec_ok, n_runs = f.n_runs;
   const int rec_col = (int)cl.x - f.c_lo, grid_cols = p.grid_cols, off_y = p.off_y, force = p.force_exact;
@@ -334,26 +297,18 @@ __device__ __forceinline__ void tile_warp_rows(const WarpParams &p, const TileIn
     uint8_t *orow = out_lane + lo * kWarpPitch;
     int y = lo - off_y;
     if (__all_sync(0xffffffffu, c.outside)) {   // every pixel of these rows stays black under this warp
-      for (; lo <= hi; ++lo, ++y, orow += kWarpPitch) {
-        uint32_t val = 0;
-        if (kBlend) val = centre_px(p, x, y, col_ok);
-        orow[0] = (uint8_t)val; orow[1] = (uint8_t)(val >> 8); orow[2] = (uint8_t)(val >> 16);
-      }
+      for (; lo <= hi; ++lo, orow += kWarpPitch) { orow[0] = 0; orow[1] = 0; orow[2] = 0; }
       continue;
     }
     float dyf = (float)(run.w + lo - run.x);
 #pragma unroll 1
     for (; lo + kGroupRows <= hi + 1; lo += kGroupRows, y += kGroupRows, orow += kGroupRows * kWarpPitch, dyf += (float)kGroupRows)
-      tile_rows<kStaged, kBlend, kGroupRows>(p, c, bpitch, kbase, guard_addr, orow, dyf, x, y, col_ok);
-    if (kGroupRows > 4 && lo + 4 <= hi + 1) {
-      tile_rows<kStaged, kBlend, 4>(p, c, bpitch, kbase, guard_addr, orow, dyf, x, y, col_ok);
-      lo += 4; y += 4; orow += 4 * kWarpPitch; dyf += 4.f;
-    }
-    if (lo + 2 <= hi + 1) {
-      tile_rows<kStaged, kBlend, 2>(p, c, bpitch, kbase, guard_addr, orow, dyf, x, y, col_ok);
+      tile_rows<kStaged, kGroupRows>(p, c, bpitch, kbase, guard_addr, orow, dyf, x, y);
+    if (lo + 2 <= hi + 1) {                     // the last 0 .. 3 rows
+      tile_rows<kStaged, 2>(p, c, bpitch, kbase, guard_addr, orow, dyf, x, y);
       lo += 2; y += 2; orow += 2 * kWarpPitch; dyf += 2.f;
     }
-    if (lo == hi) tile_rows<kStaged, kBlend, 1>(p, c, bpitch, kbase, guard_addr, orow, dyf, x, y, col_ok);
+    if (lo == hi) tile_rows<kStaged, 1>(p, c, bpitch, kbase, guard_addr, orow, dyf, x, y);
   }
 }
 
@@ -473,8 +428,7 @@ __global__ void __launch_bounds__(256) k_tile_prep(const __grid_constant__ TileP
   }
 }
 
-template <bool kBlend>
-__global__ void __launch_bounds__(kTileThreads, APAP_TILE_CTAS) k_warp_tile(const __grid_constant__ TileParams tp) {
+__global__ void __launch_bounds__(kTileThreads, kTileCtas) k_warp_tile(const __grid_constant__ TileParams tp) {
   extern __shared__ __align__(128) uint8_t smem_raw[];
   TileSmem &sm = *reinterpret_cast<TileSmem *>(smem_raw);
   const WarpParams &p = tp.w;
@@ -538,8 +492,7 @@ __global__ void __launch_bounds__(kTileThreads, APAP_TILE_CTAS) k_warp_tile(cons
       const int bpitch = __shfl_sync(0xffffffffu, (int)rec.z, 0);
       const int mode = __shfl_sync(0xffffffffu, (int)rec.x, 1);          // uint4 #1 = {mode, r_first, n_rows, c_lo}
       const int c_lo = __shfl_sync(0xffffffffu, (int)rec.w, 1);
-      int rec_ok = __shfl_sync(0xffffffffu, (int)rec.x, 2);              // uint4 #2 = {rec_ok, n_runs, j0, jw}
-      if (tp.lab & 8) rec_ok = 0;                                        // LAB: no record staging (workers load from global)
+      const int rec_ok = __shfl_sync(0xffffffffu, (int)rec.x, 2);        // uint4 #2 = {rec_ok, n_runs, j0, jw}
       const int n_runs = __shfl_sync(0xffffffffu, (int)rec.y, 2);
       const int shape = __shfl_sync(0xffffffffu, (int)rec.x, 3);         // uint4 #3 = {shape, c0, ncc, pad}
       const int c0 = __shfl_sync(0xffffffffu, (int)rec.y, 3);
@@ -552,7 +505,6 @@ __global__ void __launch_bounds__(kTileThreads, APAP_TILE_CTAS) k_warp_tile(cons
 
       mbar_wait(&sm.empty[s], ring_par ^ 1u);                // the workers have left this stage
       if (lane < 12) reinterpret_cast<uint4 *>(&f)[lane] = cur;
-      if ((tp.lab & 8) && lane == 0) f.rec_ok = 0;
 #pragma unroll
       for (int q = 0; q < kTileCols / 32; ++q) sm.st[s].lut[lane + 32 * q] = cur_lut[q];
       __syncwarp();
@@ -569,7 +521,7 @@ __global__ void __launch_bounds__(kTileThreads, APAP_TILE_CTAS) k_warp_tile(cons
       // The next tile's record has arrived by now: pull the lines of its box into L2 through the LSU path.  The copy
       // into the stage cannot start before the workers free the stage, a tile from now; a cold box then took 2.5-3.4 us
       // to arrive (a tile is 2 us of work) although the same copy from L2 takes 0.4 us (tools/tma_lab.cu).
-      if (tile_next < tp.n_tiles && !(tp.lab & 2)) {
+      if (tile_next < tp.n_tiles) {
         const int nshape = __shfl_sync(0xffffffffu, (int)rec.x, 3), nc0 = __shfl_sync(0xffffffffu, (int)rec.y, 3);
         const int ny = __shfl_sync(0xffffffffu, (int)rec.y, 0);
         if (nshape >= 0) {
@@ -603,30 +555,19 @@ __global__ void __launch_bounds__(kTileThreads, APAP_TILE_CTAS) k_warp_tile(cons
     const int mode = f.mode;
     if (mode == kDone) break;
     const int r_first = f.r_first, n_rows = f.n_rows, j0 = f.j0, jw = f.jw;
-    const bool col_ok = lane_col < jw;
     const uint2 cl = sm.st[s].lut[lane_col];
-    const int x = j0 + lane_col - p.off_x;
+    const int x = j0 + lane_col - p.off_x;                 // lanes at or past jw: bytes that are never stored
     // the two warps of a column chunk share the tile's rows: the first 16 and the last 16 (a tile of 31 rows has its
     // middle row computed by both, same bytes), so that every warp's block is one whole 16-row store; a tile of fewer
     // than 16 rows (end of a band) is all the first warp's
     const int row_lo = (half && n_rows >= kWarpRows) ? r_first + n_rows - kWarpRows : r_first + half * kWarpRows;
     const int row_hi = half ? r_first + n_rows - 1 : min(r_first + kWarpRows, r_first + n_rows) - 1;
-    if (tp.lab & 1) {                                         // LAB: no pixel work
-      for (int q = lane; q < kWarpOutBytes / 16; q += 32) reinterpret_cast<uint4 *>(warp_out)[q] = make_uint4(0u, 0u, 0u, 0u);
-    } else if (mode == kStagedMode) {
-      tile_warp_rows<true, kBlend>(p, f, sm.st[s], warp_out, cl, x, col_ok, lane, row_lo, row_hi);
+    if (mode == kStagedMode) {
+      tile_warp_rows<true>(p, f, sm.st[s], warp_out, cl, x, lane, row_lo, row_hi);
     } else if (mode == kGlobal) {
-      tile_warp_rows<false, kBlend>(p, f, sm.st[s], warp_out, cl, x, col_ok, lane, row_lo, row_hi);
-    } else {                                                  // kBlack: clear (or fill with the centre image) the block
-      if (!kBlend) {
-        for (int q = lane; q < kWarpOutBytes / 16; q += 32) reinterpret_cast<uint4 *>(warp_out)[q] = make_uint4(0u, 0u, 0u, 0u);
-      } else {
-        for (int r = row_lo; r <= row_hi; ++r) {
-          const uint32_t val = centre_px(p, x, r - p.off_y, col_ok);
-          uint8_t *d = warp_out + (r - row_lo) * kWarpPitch + lane * 3;
-          d[0] = (uint8_t)val; d[1] = (uint8_t)(val >> 8); d[2] = (uint8_t)(val >> 16);
-        }
-      }
+      tile_warp_rows<false>(p, f, sm.st[s], warp_out, cl, x, lane, row_lo, row_hi);
+    } else {                                                  // kBlack: clear the block
+      for (int q = lane; q < kWarpOutBytes / 16; q += 32) reinterpret_cast<uint4 *>(warp_out)[q] = make_uint4(0u, 0u, 0u, 0u);
     }
     __syncwarp();
     if (lane == 0) mbar_arrive(&sm.empty[s]);                // this warp no longer reads the stage (f is dead from here)
@@ -751,7 +692,6 @@ int launch_warp_tile(const WarpParams &w, bool words, const void *tiles, cudaStr
   TileParams tp;
   memset(&tp, 0, sizeof(tp));
   tp.w = w;
-  tp.lab = getenv("APAP_TILE_LAB") ? atoi(getenv("APAP_TILE_LAB")) : 0;
   const size_t src_pitch = (size_t)w.src_w * 3;
   for (int m = 0; m < kBoxShapes; ++m)                     // the source as uint32 [src_h][src_w * 3 / 4], three box shapes
     if (!encode_u32_rows(&tp.maps[m], w.src, src_pitch, w.src_h, box_w(m), box_h(m), CU_TENSOR_MAP_L2_PROMOTION_L2_128B))
@@ -770,17 +710,14 @@ int launch_warp_tile(const WarpParams &w, bool words, const void *tiles, cudaStr
   cudaError_t e = cudaGetDevice(&dev);
   if (e != cudaSuccess) return check_cuda(e, "cudaGetDevice");
   if (dev < 0 || dev >= 64 || !configured[dev]) {
-    e = cudaFuncSetAttribute(k_warp_tile<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e == cudaSuccess)
-      e = cudaFuncSetAttribute(k_warp_tile<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    e = cudaFuncSetAttribute(k_warp_tile, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return check_cuda(e, "k_warp_tile shared memory opt-in");
     if (dev >= 0 && dev < 64) configured[dev] = true;
   }
-  const int grid = min(tp.n_tiles, sm_count_cached() * APAP_TILE_CTAS);
+  const int grid = min(tp.n_tiles, sm_count_cached() * kTileCtas);
   static std::atomic<unsigned> launch_seq{0};              // concurrent launches (other streams) get different counters
   tp.slot = (int)(launch_seq.fetch_add(1u) % kCounterSlots);
-  if (w.centre) k_warp_tile<true><<<grid, kTileThreads, smem, st>>>(tp);
-  else k_warp_tile<false><<<grid, kTileThreads, smem, st>>>(tp);
+  k_warp_tile<<<grid, kTileThreads, smem, st>>>(tp);
   return check_cuda(cudaGetLastError(), "k_warp_tile launch");
 }
 

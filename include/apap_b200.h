@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define APAP_ABI_VERSION 22
+#define APAP_ABI_VERSION 23
 
 /* Layout constants shared with the host layer. */
 #define APAP_GRAM_TERMS 24   /* distinct non-zero sums of the 9x9 Gram matrix (4 sym. 3x3 blocks) */
@@ -175,9 +175,8 @@ int apap_local_weight(const double *anchors, const double *kp_xy, int cells, int
  *               NULL = plain warp
  *   flags     : APAP_WARP_FORCE_EXACT = every pixel takes the float64 path (validation switch);
  *               APAP_WARP_LEGACY = the strip kernel even when `tiles` is given
- *               APAP_WARP_TILE_FUSED = the tile engine also when `centre` is given (default there: the strip kernel, measured faster)
- *   tiles     : the band's tile records from apap_warp_tiles (same tables, same band), or NULL.  With tiles, and a
- *               source whose rows are 16-byte aligned (src % 16 == 0, src_w * 3 % 16 == 0), the TILE ENGINE runs
+ *   tiles     : the band's tile records from apap_warp_tiles (same tables, same band), or NULL.  With tiles, no centre
+ *               and a source whose rows are 16-byte aligned (src % 16 == 0, src_w * 3 % 16 == 0), the TILE ENGINE runs
  *               (csrc/warp_tile.cu): persistent warp-specialised CTAs; per 128 x 32 canvas tile the source box the
  *               tile can pick from is staged in shared memory by one tensor-map TMA copy (zero outside the image),
  *               gathers are LDS, the output leaves as 16-row tensor-map TMA stores when the band is 16-byte aligned
@@ -192,7 +191,6 @@ int apap_local_weight(const double *anchors, const double *kp_xy, int cells, int
  */
 #define APAP_WARP_FORCE_EXACT 1
 #define APAP_WARP_LEGACY      2
-#define APAP_WARP_TILE_FUSED  4
 int apap_warp(const uint8_t *src, int src_h, int src_w, const float *cell_fast, const float *cell_hinv,
               const uint32_t *col_lut, const uint32_t *row_blocks, int n_blocks,
               int grid_cols, int canvas_w, int off_x, int off_y, int row0, int row1,

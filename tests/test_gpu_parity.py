@@ -452,7 +452,7 @@ def test_local_warp_c2_full_size_vs_oracle():
     assert diff.size == 0, f"{diff.size} pixels differ, first {diff[:5]}"
 
 
-def _device_warp(st, sc, img, inv, centre=None, legacy=False, rows=None, tile_fused=False):
+def _device_warp(st, sc, img, inv, centre=None, legacy=False, rows=None):
     """K3 through warp_tables_device + warp_device on cuda tensors (``legacy`` = round 1's strip kernel)."""
     import torch
     dev = torch.device("cuda", torch.cuda.current_device())
@@ -460,14 +460,15 @@ def _device_warp(st, sc, img, inv, centre=None, legacy=False, rows=None, tile_fu
     col, row = cell_lookup_tables(sc.mesh, sc.final_w, sc.final_h, gr, gc)
     r0, r1 = rows if rows is not None else (0, sc.final_h)
     tabs = st.warp_tables_device(inv, col, row, img.shape[1], img.shape[0], dev, r0, r1)
-    out = st.warp_device(torch.from_numpy(img).to(dev), tabs, gc, legacy=legacy, tile_fused=tile_fused,
+    out = st.warp_device(torch.from_numpy(img).to(dev), tabs, gc, legacy=legacy,
                          centre_dev=torch.from_numpy(centre).to(dev) if centre is not None else None)
     return out.cpu().numpy()
 
 
 def test_tile_engine_equals_legacy_strip_kernel_c2():
     """The tile engine (TMA-staged source boxes, LDS gathers, bulk row stores) and round 1's strip kernel pick the same
-    bytes on the full c2 canvas, plain and fused with the blend, and on a row band that starts mid-cell-row."""
+    bytes on the full c2 canvas and on a row band that starts mid-cell-row; fused with the blend (always the strip
+    kernel) the default call and ``legacy`` agree."""
     sc = synth.make_scene("c2")
     img = sc.image(1)
     centre = synth.make_image(sc.width, sc.height, seed=2)
@@ -480,7 +481,6 @@ def test_tile_engine_equals_legacy_strip_kernel_c2():
     fa = _device_warp(st, sc, img, inv, centre=centre)
     fb = _device_warp(st, sc, img, inv, centre=centre, legacy=True)
     assert np.array_equal(fa, fb)
-    assert np.array_equal(_device_warp(st, sc, img, inv, centre=centre, tile_fused=True), fb)   # the tile engine's fused variant
     band = _device_warp(st, sc, img, inv, rows=(1001, 1777))
     assert np.array_equal(band, a[1001:1777])
 

@@ -297,7 +297,11 @@ def test_library_exports_every_declared_symbol():
     raw = ctypes.CDLL(rt.LIB_PATH)
     for name in declared:
         assert hasattr(raw, name), name
-    assert lib.apap_abi_version() == rt.ABI_VERSION == 22
+    assert lib.apap_abi_version() == rt.ABI_VERSION == 23
+    # flag 4 (a fused tile-engine variant up to ABI 22) is refused before any pointer is used: dummy pointers are safe
+    d = 256
+    assert (lib.apap_warp(d, 1, 1, d, d, d, d, 1, 1, 1, 0, 0, 0, 1, None, 0, 0, d, 3, 4, 0, None, None) == -1   # APAP_E_BADARG
+            and b"unknown flag" in lib.apap_last_error())
     m = re.search(r"#define\s+APAP_KP_ROW\s+(\d+)", header)
     assert int(m.group(1)) == rt.KP_ROW
 

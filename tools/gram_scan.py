@@ -15,7 +15,6 @@ torch.cuda.set_device(0)
 dev = torch.device("cuda", 0)
 lib = rt.load_library()
 flush = torch.zeros(256 << 20, dtype=torch.uint8, device=dev)
-tag = os.path.basename(os.environ.get("APAP_B200_LIB", "product"))
 for spec in sys.argv[1:]:
     cells, n_kp = (int(v) for v in spec.split(":"))
     src, dst, _ = synth.make_keypoints(3840, 2160, n_kp, seed=0)
@@ -40,43 +39,5 @@ for spec in sys.argv[1:]:
         if k >= 3:
             ts.append(e0.elapsed_time(e1) * 1e3)
     ctas = ((cells + 127) // 128) * ks
-    print(f"{tag:24s} cells={cells:7d} n_kp={n_kp:6d} splits={ks:3d} ctas={ctas:6d} ({ctas / 592:6.2f} waves)  "
+    print(f"cells={cells:7d} n_kp={n_kp:6d} splits={ks:3d} ctas={ctas:6d} ({ctas / 592:6.2f} waves)  "
           f"{np.median(ts):8.1f} us (min {np.min(ts):8.1f})  {2.0 * cells * n_pad / np.median(ts) / 1e6:6.2f} T MUFU/s", flush=True)
-try:
-    import ctypes
-    fn2 = lib.apap_lab_cta_trace
-    fn2.argtypes = [ctypes.c_void_p]
-    cta = np.zeros((8192, 4), dtype=np.int64)
-    fn2(cta.ctypes.data)
-    n = min(ctas, 8192)
-    cta = cta[:n]
-    t0 = cta[:, 1].min()
-    start, alloc, end = (cta[:, 1] - t0) / 1e3, (cta[:, 2] - t0) / 1e3, (cta[:, 3] - t0) / 1e3
-    print(f"per-CTA timeline (us since the first CTA started), {n} CTAs: kernel span {end.max():.1f} us")
-    print(f"  start: min {start.min():.1f} median {np.median(start):.1f} max {start.max():.1f};  alloc wait: median {np.median(alloc - start):.2f} max {(alloc - start).max():.2f};"
-          f"  lifetime: min {(end - start).min():.1f} median {np.median(end - start):.1f} max {(end - start).max():.1f}")
-    for smid in (0, 1, 73, 147):
-        idx = np.flatnonzero(cta[:, 0] == smid)
-        print(f"  SM {smid:3d}: " + " ".join(f"[{start[i]:5.1f}-{end[i]:5.1f}]" for i in idx[np.argsort(start[idx])]))
-    hist = np.histogram(start, bins=np.arange(0, end.max() + 5, 5))[0]
-    print("  CTA starts per 5 us bin:", hist.tolist())
-    conc = [(int(((start <= t) & (end > t)).sum())) for t in np.arange(0, end.max(), 5)]
-    print("  resident CTAs at t = 0, 5, 10 ... us:", conc)
-except AttributeError:
-    pass
-try:
-    fn = lib.apap_lab_trace
-    fn.argtypes = [ctypes.c_void_p]
-    buf = np.zeros((4, 160, 4), dtype=np.int64)
-    fn(buf.ctypes.data)
-    t0 = buf[buf > 0].min()
-    rel = np.where(buf > 0, buf - t0, -1)
-    print("trace of the last launch, CTA x = TRACE id, split 0 (SM clock cycles since the first mark)")
-    print("producer parity 0 | parity 1 (quarter 0): start, stage landed + probe issued, slot acquired, arrived;  MMA: wait, a_full seen, issued")
-    for it in range(0, 40):
-        if rel[0, it, 0] < 0:
-            break
-        print(f"  it {it:3d}: " + " ".join(f"{v:7d}" for v in rel[0, it]) + "  |" + " ".join(f"{v:7d}" for v in rel[1, it])
-              + f"   MMA step {2 * it}: " + " ".join(f"{v:7d}" for v in rel[2, 2 * it, :3]) + f"  step {2 * it + 1}: " + " ".join(f"{v:7d}" for v in rel[2, 2 * it + 1, :3]))
-except AttributeError:
-    pass

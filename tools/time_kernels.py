@@ -1,8 +1,8 @@
 #!/usr/bin/env python
-"""Quick device timing of the pass's kernels (CUDA events, L2 flushed before every launch) for lab
-builds: APAP_B200_LIB=<variant.so> python tools/time_kernels.py [workload] [iters] [what]
+"""Quick device timing of the pass's kernels (CUDA events, L2 flushed before every launch):
+python tools/time_kernels.py [workload] [iters] [what]
 what = comma list of gram,eig,warp,fused,blend (default all).  Also checks the H grid against the
-float64 Gram oracle of the default library run (max normalised error), so a variant that breaks the
+one the first run on this machine saved (max normalised error), so a change that breaks the
 numbers shows up next to its time."""
 import os
 import sys
@@ -47,7 +47,6 @@ for w in what:
             ts.append(e0.elapsed_time(e1) * 1e3)
     res[w] = (float(np.median(ts)), float(np.min(ts)))
 h = p.h_out.cpu().numpy().astype(np.float64)
-tag = os.path.basename(os.environ.get("APAP_B200_LIB", "product"))
 ref_path = f"/tmp/h_ref_{name}.npy"
 err = ""
 if os.path.exists(ref_path):
@@ -59,4 +58,4 @@ if os.path.exists(ref_path):
     err = f" | H vs first run: {np.abs(d).max(axis=(1, 2)).max() / 1.0:.2e} (norm by max|ref| per cell: {(np.abs(d).max(axis=(1, 2)) / np.abs(r).max(axis=(1, 2))).max():.2e})"
 else:
     np.save(ref_path, h)
-print(f"{tag:28s} {name} " + " ".join(f"{w}={m:7.1f}us(min {mn:6.1f})" for w, (m, mn) in res.items()) + err, flush=True)
+print(f"{name} " + " ".join(f"{w}={m:7.1f}us(min {mn:6.1f})" for w, (m, mn) in res.items()) + err, flush=True)

@@ -1,6 +1,7 @@
 #!/usr/bin/env python
-"""LAB: K3 timing, tile engine vs round 1's strip kernel, cold (L2 flushed) vs warm (source and canvas
-L2-resident, no launch gap), plain and fused with the blend; checks both engines write the same bytes."""
+"""LAB: K3 timing, cold (L2 flushed) vs warm (source and canvas L2-resident, no launch gap): the plain warp on the
+tile engine and on round 1's strip kernel, and the warp fused with the blend (strip kernel); checks both engines write
+the same bytes."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -12,7 +13,7 @@ p = bench.Pass(torch, dev, name)
 p.gram(); p.eig(); p.prepare_warp()
 flush = torch.zeros(256 << 20, dtype=torch.uint8, device=dev)
 def call(legacy, fused):
-    p.st.warp_device(p.img, p.tables, p.sc.mesh_cells, out=p.canvas, legacy=legacy, tile_fused=fused,
+    p.st.warp_device(p.img, p.tables, p.sc.mesh_cells, out=p.canvas, legacy=legacy,
                      centre_dev=p.centre if fused else None)
 def run(legacy, fused, warm, reps=20):
     ts = []
@@ -27,14 +28,13 @@ def run(legacy, fused, warm, reps=20):
         ts.append(e0.elapsed_time(e1) * 1e3)
     ts = ts[3:]
     return sum(ts) / len(ts), min(ts)
-for fused in (False, True):
-    outs = []
-    for legacy in (False, True):
-        call(legacy, fused); outs.append(p.canvas.clone())
-    print(f"{name} {'fused' if fused else 'plain'}: engines agree = {bool(torch.equal(outs[0], outs[1]))}, "
-          f"non-black {float((outs[0].amax(-1) > 0).float().mean()):.3f}")
-    for legacy in (False, True):
-        for warm in (False, True):
-            avg, best = run(legacy, fused, warm)
-            print(f"{name} {'fused' if fused else 'plain'} {'strip' if legacy else 'tile '} "
-                  f"{'warm L2' if warm else 'cold   '} avg {avg:7.2f} us  best {best:7.2f} us")
+outs = []
+for legacy in (False, True):
+    call(legacy, False); outs.append(p.canvas.clone())
+print(f"{name} plain: engines agree = {bool(torch.equal(outs[0], outs[1]))}, "
+      f"non-black {float((outs[0].amax(-1) > 0).float().mean()):.3f}")
+for legacy, fused in ((False, False), (True, False), (True, True)):
+    for warm in (False, True):
+        avg, best = run(legacy, fused, warm)
+        print(f"{name} {'fused' if fused else 'plain'} {'strip' if legacy else 'tile '} "
+              f"{'warm L2' if warm else 'cold   '} avg {avg:7.2f} us  best {best:7.2f} us")
