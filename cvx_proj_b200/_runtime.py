@@ -30,6 +30,7 @@ WARP_LEGACY = 2
 RANSAC_MAX_ITERS = 1 << 20
 BLEND_MAX_LAYERS = 256
 FEATHER_MAX_LAYERS = 128
+GAIN_MAX_LAYERS = 256
 E_TOOBIG = -3           # APAP_E_TOOBIG
 
 # symbol -> (restype, argtypes); tests check every symbol of include/apap_b200.h is exported
@@ -61,6 +62,12 @@ SIGNATURES = {
     "apap_feather_workspace_bytes": (c_int, [POINTER(ctypes.c_longlong), c_int, c_int, c_int, POINTER(c_size_t)]),
     "apap_feather_blend": (c_int, [POINTER(ctypes.c_longlong), c_int, c_int, c_int, c_float, c_void_p, c_size_t,
                                    c_void_p, c_size_t, c_void_p]),
+    "apap_gain_stats_bytes": (c_int, [c_int, POINTER(c_size_t)]),
+    "apap_gain_stats": (c_int, [POINTER(ctypes.c_longlong), c_int, c_int, c_int, c_void_p, c_size_t, c_void_p]),
+    "apap_blend_layers_gain": (c_int, [POINTER(ctypes.c_longlong), c_int, c_int, c_int, c_void_p, c_void_p, c_size_t,
+                                       c_void_p]),
+    "apap_feather_blend_gain": (c_int, [POINTER(ctypes.c_longlong), c_int, c_int, c_int, c_float, c_void_p, c_void_p,
+                                        c_size_t, c_void_p, c_size_t, c_void_p]),
     "apap_pipe_probe": (c_int, [c_int, c_int, c_void_p, POINTER(c_double), c_void_p]),
     "apap_warp_perspective": (c_int, [c_void_p, c_int, c_int, POINTER(c_double), c_void_p, c_int, c_int, c_void_p, c_int,
                                       c_int, c_int, c_int, c_int, c_void_p]),

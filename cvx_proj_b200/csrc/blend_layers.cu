@@ -9,6 +9,8 @@
 // zero to the sums, so only the count needs the non-empty test.  floor(s / n) is __umulhi(s, ceil(2^32 / n)) for
 // n >= 2 (exact: s (m n - 2^32) < s n <= 255 x 256^2 < 2^32), s itself for n <= 1 (n = 0 means s = 0).
 // The segment's bytes are staged in shared memory and leave as aligned 16-byte stores plus a byte-wise head and tail.
+// kGains (apap_blend_layers_gain): layer l's bytes go through its exposure-gain table lut[l][256] before they are
+// summed; the non-empty test still reads the raw bytes, and compensated bytes are <= 255, so the bound above holds.
 #include "layers.cuh"
 
 namespace apap {
@@ -19,7 +21,9 @@ struct LayerParams {
   int n_layers, canvas_h, canvas_w, segs_per_row;
 };
 
-__global__ void __launch_bounds__(kLayerThreads) k_blend_layers(const __grid_constant__ LayerParams p) {
+template <bool kGains>
+__global__ void __launch_bounds__(kLayerThreads) k_blend_layers(const __grid_constant__ LayerParams p,
+                                                                const uint8_t *__restrict__ lut) {
   __shared__ uint32_t recip[APAP_BLEND_MAX_LAYERS + 1];
   __shared__ __align__(16) uint32_t stage[kSegBytes / 4];
   for (int i = threadIdx.x; i <= APAP_BLEND_MAX_LAYERS; i += kLayerThreads)
@@ -36,9 +40,11 @@ __global__ void __launch_bounds__(kLayerThreads) k_blend_layers(const __grid_con
   for (int l = 0; l < p.n_layers; ++l) {
     uint32_t w[3];
     fetch_group(p.layer[l], y, seg0, seg_px, x, n_px, w);
-    s[0] += __byte_perm(w[0], 0u, 0x4140); s[1] += __byte_perm(w[0], 0u, 0x4342);
-    s[2] += __byte_perm(w[1], 0u, 0x4140); s[3] += __byte_perm(w[1], 0u, 0x4342);
-    s[4] += __byte_perm(w[2], 0u, 0x4140); s[5] += __byte_perm(w[2], 0u, 0x4342);
+    uint32_t v[3] = {w[0], w[1], w[2]};
+    if constexpr (kGains) gain_group(lut + 256 * l, v);
+    s[0] += __byte_perm(v[0], 0u, 0x4140); s[1] += __byte_perm(v[0], 0u, 0x4342);
+    s[2] += __byte_perm(v[1], 0u, 0x4140); s[3] += __byte_perm(v[1], 0u, 0x4342);
+    s[4] += __byte_perm(v[2], 0u, 0x4140); s[5] += __byte_perm(v[2], 0u, 0x4342);
     const uint32_t nz = byte_nonzero(group_or(w[0], w[1], w[2]));
     c01 += __byte_perm(nz, 0u, 0x4140);
     c23 += __byte_perm(nz, 0u, 0x4342);
@@ -84,8 +90,8 @@ __global__ void __launch_bounds__(kLayerThreads) k_blend_layers(const __grid_con
   }
 }
 
-int launch_blend_layers(const long long *layers, int n_layers, int canvas_h, int canvas_w, uint8_t *out,
-                        cudaStream_t st) {
+int launch_blend_layers(const long long *layers, int n_layers, int canvas_h, int canvas_w, const uint8_t *lut,
+                        uint8_t *out, cudaStream_t st) {
   LayerParams p;
   for (int l = 0; l < n_layers; ++l) p.layer[l] = layer_desc(layers + 6 * l);
   p.out = out;
@@ -95,7 +101,8 @@ int launch_blend_layers(const long long *layers, int n_layers, int canvas_h, int
   p.segs_per_row = (canvas_w + kSegPx - 1) / kSegPx;
   const long long blocks = (long long)p.segs_per_row * canvas_h;
   if (blocks > 2147483647LL) return fail(APAP_E_TOOBIG, "blend_layers: canvas too large");
-  k_blend_layers<<<(unsigned)blocks, kLayerThreads, 0, st>>>(p);
+  if (lut) k_blend_layers<true><<<(unsigned)blocks, kLayerThreads, 0, st>>>(p, lut);
+  else k_blend_layers<false><<<(unsigned)blocks, kLayerThreads, 0, st>>>(p, nullptr);
   return check_cuda(cudaGetLastError(), "k_blend_layers launch");
 }
 
@@ -103,24 +110,30 @@ int launch_blend_layers(const long long *layers, int n_layers, int canvas_h, int
 
 using namespace apap;
 
-extern "C" int apap_blend_layers(const long long *layers, int n_layers, int canvas_h, int canvas_w, uint8_t *out,
-                                 size_t out_bytes, void *stream) {
+namespace {
+
+int check_blend_layers(const long long *layers, int n_layers, int canvas_h, int canvas_w, const uint8_t *out,
+                       size_t out_bytes) {
   if (!layers || !out) return fail(APAP_E_BADARG, "blend_layers: null pointer");
-  if (n_layers < 1 || n_layers > APAP_BLEND_MAX_LAYERS)
-    return fail(APAP_E_BADARG, "blend_layers: 1 <= n_layers <= APAP_BLEND_MAX_LAYERS");
-  if (canvas_h <= 0 || canvas_w <= 0 || canvas_w > (1 << 30) || canvas_h > (1 << 30))
-    return fail(APAP_E_BADARG, "blend_layers: canvas sizes must be in [1, 2^30]");
+  if (int rc = check_layer_count_canvas("blend_layers", n_layers, APAP_BLEND_MAX_LAYERS, "APAP_BLEND_MAX_LAYERS",
+                                        canvas_h, canvas_w))
+    return rc;
   if (out_bytes < (size_t)canvas_h * (size_t)canvas_w * 3)
     return fail(APAP_E_BADARG, "blend_layers: out is smaller than canvas_h x canvas_w x 3 bytes");
-  for (int l = 0; l < n_layers; ++l) {
-    const long long *d = layers + 6 * l;
-    const long long h = d[1], w = d[2], pitch = d[3], x0 = d[4], y0 = d[5];
-    if (!d[0]) return fail(APAP_E_BADARG, "blend_layers: null layer address");
-    if (h < 1 || w < 1 || h > (1 << 30) || w > (1 << 30))
-      return fail(APAP_E_BADARG, "blend_layers: layer sizes must be in [1, 2^30]");
-    if (h > 1 && pitch < 3 * w) return fail(APAP_E_BADARG, "blend_layers: layer pitch is smaller than 3 x width");
-    if (x0 < -(1LL << 30) || x0 > (1LL << 30) || y0 < -(1LL << 30) || y0 > (1LL << 30))
-      return fail(APAP_E_BADARG, "blend_layers: layer origin outside [-2^30, 2^30]");
-  }
-  return launch_blend_layers(layers, n_layers, canvas_h, canvas_w, out, static_cast<cudaStream_t>(stream));
+  return check_layer_descs("blend_layers", layers, n_layers);
+}
+
+}  // namespace
+
+extern "C" int apap_blend_layers(const long long *layers, int n_layers, int canvas_h, int canvas_w, uint8_t *out,
+                                 size_t out_bytes, void *stream) {
+  if (int rc = check_blend_layers(layers, n_layers, canvas_h, canvas_w, out, out_bytes)) return rc;
+  return launch_blend_layers(layers, n_layers, canvas_h, canvas_w, nullptr, out, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int apap_blend_layers_gain(const long long *layers, int n_layers, int canvas_h, int canvas_w,
+                                      const uint8_t *lut, uint8_t *out, size_t out_bytes, void *stream) {
+  if (!lut) return fail(APAP_E_BADARG, "blend_layers_gain: null gain table");
+  if (int rc = check_blend_layers(layers, n_layers, canvas_h, canvas_w, out, out_bytes)) return rc;
+  return launch_blend_layers(layers, n_layers, canvas_h, canvas_w, lut, out, static_cast<cudaStream_t>(stream));
 }

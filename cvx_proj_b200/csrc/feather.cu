@@ -15,7 +15,9 @@
 //                   (the values a downward and an upward min(h, prev + 1) scan leave at its ends), the segments
 //                   exchange those in shared memory, then each thread scans its segment down and up with the carries.
 //   k_feather_blend one CTA per kSegPx-pixel canvas row segment, 4 pixels per thread (layers.cuh): a layer that does
-//                   not cover the segment adds exactly +0.0f and 0 and is skipped (uniform test).
+//                   not cover the segment adds exactly +0.0f and 0 and is skipped (uniform test).  kGains
+//                   (apap_feather_blend_gain): layer l's bytes go through its exposure-gain table lut[l][256]
+//                   first; the distances, made from the raw bytes, are unchanged.
 // Distances are stored as min(D, cap) (apap_feather_distance_cap): cap is either the smallest integer with
 // fl(cap s) >= 1 -- float multiplication by s > 0 is monotone, so every D >= cap has weight 1 -- or, when that is
 // larger, W + H - 1, more than any finite distance in the canvas, so that only a layer with no empty pixel in the
@@ -199,7 +201,9 @@ __global__ void __launch_bounds__(kColThreadsX * kColSegs) k_feather_cols(const 
   }
 }
 
-__global__ void __launch_bounds__(kLayerThreads) k_feather_blend(const __grid_constant__ FeatherParams p) {
+template <bool kGains>
+__global__ void __launch_bounds__(kLayerThreads) k_feather_blend(const __grid_constant__ FeatherParams p,
+                                                                 const uint8_t *__restrict__ lut) {
   __shared__ __align__(16) uint32_t stage[kSegBytes / 4];
   const int y = blockIdx.x / p.segs_per_row;
   const int seg0 = (blockIdx.x - y * p.segs_per_row) * kSegPx;
@@ -219,6 +223,7 @@ __global__ void __launch_bounds__(kLayerThreads) k_feather_blend(const __grid_co
     if ((unsigned)r >= (unsigned)R.ch || seg0 + seg_px <= R.cx0 || seg0 >= R.cx0 + R.cw) continue;   // uniform
     uint32_t v[3];
     fetch_group(p.layer[l], y, seg0, seg_px, x, n_px, v);
+    if constexpr (kGains) gain_group(lut + 256 * l, v);
     const uint16_t *row = R.dist + (size_t)r * (size_t)R.cw;
 #pragma unroll
     for (int k = 0; k < kLayerGroupPx; ++k) {
@@ -274,21 +279,10 @@ size_t dist_bytes(const FeatherRect &R) { return ((size_t)R.cw * (size_t)R.ch * 
 
 int check_layers(const long long *layers, int n_layers, int canvas_h, int canvas_w) {
   if (!layers) return fail(APAP_E_BADARG, "feather: null pointer");
-  if (n_layers < 1 || n_layers > APAP_FEATHER_MAX_LAYERS)
-    return fail(APAP_E_BADARG, "feather: 1 <= n_layers <= APAP_FEATHER_MAX_LAYERS");
-  if (canvas_h <= 0 || canvas_w <= 0 || canvas_w > (1 << 30) || canvas_h > (1 << 30))
-    return fail(APAP_E_BADARG, "feather: canvas sizes must be in [1, 2^30]");
-  for (int l = 0; l < n_layers; ++l) {
-    const long long *d = layers + 6 * l;
-    const long long h = d[1], w = d[2], pitch = d[3], x0 = d[4], y0 = d[5];
-    if (!d[0]) return fail(APAP_E_BADARG, "feather: null layer address");
-    if (h < 1 || w < 1 || h > (1 << 30) || w > (1 << 30))
-      return fail(APAP_E_BADARG, "feather: layer sizes must be in [1, 2^30]");
-    if (h > 1 && pitch < 3 * w) return fail(APAP_E_BADARG, "feather: layer pitch is smaller than 3 x width");
-    if (x0 < -(1LL << 30) || x0 > (1LL << 30) || y0 < -(1LL << 30) || y0 > (1LL << 30))
-      return fail(APAP_E_BADARG, "feather: layer origin outside [-2^30, 2^30]");
-  }
-  return 0;
+  if (int rc = check_layer_count_canvas("feather", n_layers, APAP_FEATHER_MAX_LAYERS, "APAP_FEATHER_MAX_LAYERS",
+                                        canvas_h, canvas_w))
+    return rc;
+  return check_layer_descs("feather", layers, n_layers);
 }
 
 int distance_cap(float s, int canvas_h, int canvas_w, int *cap) {
@@ -337,9 +331,9 @@ extern "C" int apap_feather_workspace_bytes(const long long *layers, int n_layer
   return 0;
 }
 
-extern "C" int apap_feather_blend(const long long *layers, int n_layers, int canvas_h, int canvas_w, float sharpness,
-                                  void *workspace, size_t workspace_bytes, uint8_t *out, size_t out_bytes,
-                                  void *stream) {
+static int feather_blend(const long long *layers, int n_layers, int canvas_h, int canvas_w, float sharpness,
+                         const uint8_t *lut, void *workspace, size_t workspace_bytes, uint8_t *out,
+                         size_t out_bytes, cudaStream_t st) {
   if (!out || !workspace) return fail(APAP_E_BADARG, "feather_blend: null pointer");
   if (int rc = check_layers(layers, n_layers, canvas_h, canvas_w)) return rc;
   if (out_bytes < (size_t)canvas_h * (size_t)canvas_w * 3)
@@ -369,7 +363,6 @@ extern "C" int apap_feather_blend(const long long *layers, int n_layers, int can
   p.segs_per_row = (canvas_w + kSegPx - 1) / kSegPx;
   const long long blocks = (long long)p.segs_per_row * canvas_h;
   if (blocks > 2147483647LL) return fail(APAP_E_TOOBIG, "feather_blend: canvas too large");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (max_ch > 0) {
     k_feather_rows<<<dim3((unsigned)max_ch, (unsigned)n_layers), kLayerThreads, 0, st>>>(p);
     if (int rc = check_cuda(cudaGetLastError(), "k_feather_rows launch")) return rc;
@@ -377,6 +370,22 @@ extern "C" int apap_feather_blend(const long long *layers, int n_layers, int can
                      dim3(kColThreadsX, kColSegs), 0, st>>>(p);
     if (int rc = check_cuda(cudaGetLastError(), "k_feather_cols launch")) return rc;
   }
-  k_feather_blend<<<(unsigned)blocks, kLayerThreads, 0, st>>>(p);
+  if (lut) k_feather_blend<true><<<(unsigned)blocks, kLayerThreads, 0, st>>>(p, lut);
+  else k_feather_blend<false><<<(unsigned)blocks, kLayerThreads, 0, st>>>(p, nullptr);
   return check_cuda(cudaGetLastError(), "k_feather_blend launch");
+}
+
+extern "C" int apap_feather_blend(const long long *layers, int n_layers, int canvas_h, int canvas_w, float sharpness,
+                                  void *workspace, size_t workspace_bytes, uint8_t *out, size_t out_bytes,
+                                  void *stream) {
+  return feather_blend(layers, n_layers, canvas_h, canvas_w, sharpness, nullptr, workspace, workspace_bytes, out,
+                       out_bytes, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int apap_feather_blend_gain(const long long *layers, int n_layers, int canvas_h, int canvas_w,
+                                       float sharpness, const uint8_t *lut, void *workspace, size_t workspace_bytes,
+                                       uint8_t *out, size_t out_bytes, void *stream) {
+  if (!lut) return fail(APAP_E_BADARG, "feather_blend_gain: null gain table");
+  return feather_blend(layers, n_layers, canvas_h, canvas_w, sharpness, lut, workspace, workspace_bytes, out,
+                       out_bytes, static_cast<cudaStream_t>(stream));
 }

@@ -1,10 +1,13 @@
-// Placed uint8 [h][w][3] layers read and a canvas row segment written by the N-layer blends (blend_layers.cu,
-// feather.cu).  A CTA owns a segment of kSegPx pixels of one canvas row, a thread 4 consecutive pixels (12 bytes).
+// Placed uint8 [h][w][3] layers read and a canvas row segment written by the N-layer kernels (blend_layers.cu,
+// feather.cu, gain.cu).  A CTA owns a segment of kSegPx pixels of one canvas row, a thread 4 consecutive pixels
+// (12 bytes).
 // A layer row's 12-byte groups all share one phase modulo 4 (12 is a multiple of 4), so a thread reads its group as 3
 // or 4 aligned words -- each holding at least one byte of the group -- and funnel-shifts them into place; the at most
 // two groups that straddle a layer's left or right edge read byte by byte.  The segment's bytes are staged in shared
 // memory and leave as aligned 16-byte stores plus a byte-wise head and tail.
 #pragma once
+#include <cstdio>
+
 #include "common.cuh"
 
 namespace apap {
@@ -31,6 +34,43 @@ inline LayerDesc layer_desc(const long long *d) {
   L.x0 = (int)d[4];
   L.y0 = (int)d[5];
   return L;
+}
+
+// Argument checks the placed-layer entry points share (apap_blend_layers*, apap_feather_*, apap_gain_stats), in two
+// steps so that each entry keeps its own order of checks; every message starts with `what`.
+// The layer count (1 .. max_layers, named max_name in the message) and the canvas sizes.
+inline int check_layer_count_canvas(const char *what, int n_layers, int max_layers, const char *max_name, int canvas_h,
+                                    int canvas_w) {
+  char msg[160];
+  if (n_layers < 1 || n_layers > max_layers) {
+    snprintf(msg, sizeof(msg), "%s: 1 <= n_layers <= %s", what, max_name);
+    return fail(APAP_E_BADARG, msg);
+  }
+  if (canvas_h <= 0 || canvas_w <= 0 || canvas_w > (1 << 30) || canvas_h > (1 << 30)) {
+    snprintf(msg, sizeof(msg), "%s: canvas sizes must be in [1, 2^30]", what);
+    return fail(APAP_E_BADARG, msg);
+  }
+  return 0;
+}
+
+// every descriptor {device address, h, w, row pitch in bytes, x0, y0} of the C ABI
+inline int check_layer_descs(const char *what, const long long *layers, int n_layers) {
+  char msg[160];
+  for (int l = 0; l < n_layers; ++l) {
+    const long long *d = layers + 6 * l;
+    const long long h = d[1], w = d[2], pitch = d[3], x0 = d[4], y0 = d[5];
+    const char *err = nullptr;
+    if (!d[0]) err = "null layer address";
+    else if (h < 1 || w < 1 || h > (1 << 30) || w > (1 << 30)) err = "layer sizes must be in [1, 2^30]";
+    else if (h > 1 && pitch < 3 * w) err = "layer pitch is smaller than 3 x width";
+    else if (x0 < -(1LL << 30) || x0 > (1LL << 30) || y0 < -(1LL << 30) || y0 > (1LL << 30))
+      err = "layer origin outside [-2^30, 2^30]";
+    if (err) {
+      snprintf(msg, sizeof(msg), "%s: %s", what, err);
+      return fail(APAP_E_BADARG, msg);
+    }
+  }
+  return 0;
 }
 
 // one byte per pixel of a 12-byte group: the OR of its three channel bytes
@@ -75,6 +115,17 @@ __device__ __forceinline__ void fetch_group(const LayerDesc &L, int y, int seg0,
         }
       }
     }
+  }
+}
+
+// exposure gain of one group (the blends' kGains instantiations): every byte v becomes lut[v], the layer's
+// saturate(rint(v g)) table of apap_blend_layers_gain; lut[0] is 0, so absent pixels stay 0
+__device__ __forceinline__ void gain_group(const uint8_t *__restrict__ lut, uint32_t (&v)[3]) {
+#pragma unroll
+  for (int i = 0; i < 3; ++i) {
+    const uint32_t u = v[i];
+    v[i] = (uint32_t)__ldg(lut + (u & 0xffu)) | (uint32_t)__ldg(lut + ((u >> 8) & 0xffu)) << 8 |
+           (uint32_t)__ldg(lut + ((u >> 16) & 0xffu)) << 16 | (uint32_t)__ldg(lut + (u >> 24)) << 24;
   }
 }
 

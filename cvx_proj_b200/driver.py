@@ -187,7 +187,7 @@ class PanoramaResult(NamedTuple):
 
 def stitch_panorama(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops, *, mesh_size: int = 100, gamma=0.5, sigma=100,
                     warp_imgs=None, blend_img=None, equalize: bool = True, ransac: str = "opencv",
-                    device=None, blend: str = "mean", sharpness=0.02) -> PanoramaResult:
+                    device=None, blend: str = "mean", sharpness=0.02, exposure: str = "none") -> PanoramaResult:
     """Every image of a case stitched against the centre into ONE panorama (the reference has no multi-image blend;
     ``stitch_case`` returns one two-image canvas per pair, each in a frame of its own).
 
@@ -205,15 +205,23 @@ def stitch_panorama(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops, *, mesh_s
     ``panorama`` is the mean call's.  With no other image the panorama is ``feather_blend([centre])``, the centre less
     1 where it is non-empty (OpenCV's ``trunc(v / 1.00001)``).  ``sharpness`` is used by ``"feather"`` only.
 
+    ``exposure="gain"`` evens out the brightness of the layers before either blend, as OpenCV's stitching pipeline
+    runs ``cv.detail.GainCompensator`` in front of its blender: ``utils.exposure_gains`` over the same layers in the
+    same order gives one gain per layer, and the blend gets them (``gains=``), compensating each layer's bytes while
+    keeping its original mask.  With no other image it equals ``"none"``.  The gains are not part of the result; a
+    caller who wants them calls ``exposure_gains`` on the layers.
+
     The layers are warped from the images the keypoint-pair producer already holds on the device and stay there; one
     blend call and one download make the panorama.  At most 255 other images (127 with ``"feather"``); an unknown
-    ``blend``, too many images or a ``sharpness`` that ``feather_blend`` refuses for every canvas raise ``ValueError``
-    before any keypoint work."""
+    ``blend``, an unknown ``exposure``, too many images or a ``sharpness`` that ``feather_blend`` refuses for every
+    canvas raise ``ValueError`` before any keypoint work."""
     from . import _runtime as rt
-    from .utils import _device_image, _feather_sharpness, blend_layers, feather_blend
+    from .utils import _device_image, _feather_sharpness, blend_layers, exposure_gains, feather_blend
 
     if blend not in ("mean", "feather"):
         raise ValueError(f"stitch_panorama: blend must be 'mean' or 'feather', got {blend!r}")
+    if exposure not in ("none", "gain"):
+        raise ValueError(f"stitch_panorama: exposure must be 'none' or 'gain', got {exposure!r}")
     if warp_imgs is not None and len(warp_imgs) != len(other_imgs):
         raise ValueError(f"stitch_panorama: {len(other_imgs)} other images but {len(warp_imgs)} warp images")
     max_layers = rt.BLEND_MAX_LAYERS if blend == "mean" else rt.FEATHER_MAX_LAYERS
@@ -223,8 +231,8 @@ def stitch_panorama(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops, *, mesh_s
     if blend == "feather":
         sharpness = _feather_sharpness("stitch_panorama", sharpness)
 
-        def blend_fn(layers, origins, size, device=None):
-            return feather_blend(layers, origins, size, sharpness, device=device)
+        def blend_fn(layers, origins, size, device=None, gains=None):
+            return feather_blend(layers, origins, size, sharpness, device=device, gains=gains)
     else:
         blend_fn = blend_layers
     front = _case_front(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops, mesh_size, gamma, sigma, equalize, ransac,
@@ -248,5 +256,9 @@ def stitch_panorama(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops, *, mesh_s
         # the grid as local_homography returned it, as stitch_pair hands it to the fused warp
         layers.append(st.local_warp(warp_devs[i], local_h.copy(), meshes[i]))
     (width, height, ox, oy), origins = panorama_size([p.final_size for p in pairs])
-    pano = blend_fn(layers + [blend_dev], [tuple(o) for o in origins] + [(ox, oy)], (width, height))
+    layers, places = layers + [blend_dev], [tuple(o) for o in origins] + [(ox, oy)]
+    if exposure == "gain":
+        pano = blend_fn(layers, places, (width, height), gains=exposure_gains(layers, places, (width, height)))
+    else:
+        pano = blend_fn(layers, places, (width, height))
     return PanoramaResult((width, height, ox, oy), origins, pairs, rt.to_host(torch, pano))

@@ -24,7 +24,7 @@ from . import _runtime as rt
 
 __all__ = ["image_warping", "warp_perspective", "warping_canvas", "invert3x3", "match_descriptors", "coarse_matching",
            "sift_describe", "equalize_hist", "keypoint_pairs", "keypoint_pairs_batch", "find_homography_ransac",
-           "find_homography_ransac_batch", "blend_layers", "feather_blend"]
+           "find_homography_ransac_batch", "blend_layers", "feather_blend", "exposure_gains"]
 
 
 def invert3x3(m) -> np.ndarray:
@@ -101,7 +101,7 @@ def image_warping(img_base, img2warp, H, direct_blend=True, device=None):
                             device=device)
 
 
-def blend_layers(layers, origins, size, device=None):
+def blend_layers(layers, origins, size, device=None, gains=None):
     """Mean blend of placed layers (``k_blend_layers``), the panorama blend of ``driver.stitch_panorama``.
 
     ``layers`` are ``uint8 [h, w, 3]`` images, ``origins`` their top-left canvas positions ``[(x0, y0), ...]`` (may be
@@ -110,22 +110,34 @@ def blend_layers(layers, origins, size, device=None):
     integer sum, the result is ``floor(s / n)``, 0 where ``n = 0`` -- for two equal layers at one origin exactly
     ``uniform_blend``, and independent of the layer order.  1 to 256 layers.
 
+    ``gains`` (one finite float per layer, e.g. from ``exposure_gains``): layer k's bytes ``v`` become
+    ``saturate(rint(v g_k))`` before they are summed, as ``cv.detail.GainCompensator.apply`` does; ``n`` still counts
+    the layers non-empty before compensation.  ``None`` leaves the bytes as they are.
+
     All numpy in -> numpy out (uploaded to ``device``); all CUDA tensors (one device) in -> a tensor on that device.
     Tensor layers are read in place when their pixels are packed (strides ``(pitch, 3, 1)``), so crops of a larger
     image need no copy.  No CPU fallback."""
     layers, origins, width, height, on_device, device = _check_layers("blend_layers", layers, origins, size,
                                                                        rt.BLEND_MAX_LAYERS, device)
+    lut = None if gains is None else _gain_table("blend_layers", gains, len(layers))
     torch, device = rt.torch_cuda(device)
     lib = rt.load_library()
     devs, desc = _layer_descs(torch, device, layers, origins, on_device)
+    desc_p = desc.ctypes.data_as(ctypes.POINTER(ctypes.c_longlong))
     out = torch.empty((height, width, 3), dtype=torch.uint8, device=device)
     with torch.cuda.device(device):
-        rt.check(lib.apap_blend_layers(desc.ctypes.data_as(ctypes.POINTER(ctypes.c_longlong)), len(devs), height, width,
-                                       out.data_ptr(), out.numel(), rt.stream_ptr(torch, device)), "apap_blend_layers")
+        st = rt.stream_ptr(torch, device)
+        if lut is None:
+            rt.check(lib.apap_blend_layers(desc_p, len(devs), height, width, out.data_ptr(), out.numel(), st),
+                     "apap_blend_layers")
+        else:
+            lut_dev = rt.to_device(torch, device, lut)
+            rt.check(lib.apap_blend_layers_gain(desc_p, len(devs), height, width, lut_dev.data_ptr(), out.data_ptr(),
+                                                out.numel(), st), "apap_blend_layers_gain")
     return out if on_device else rt.to_host(torch, out)
 
 
-def feather_blend(layers, origins, size, sharpness=0.02, device=None):
+def feather_blend(layers, origins, size, sharpness=0.02, device=None, gains=None):
     """Feather blend of placed layers (``k_feather_rows``, ``k_feather_cols``, ``k_feather_blend``), bit for bit what
     ``cv.detail.FeatherBlender(sharpness)`` gives after ``prepare((0, 0, W, H))``, ``feed(P_k.astype(int16), mask_k,
     (0, 0))`` for every layer in the order given, and ``blend()``, converted to uint8 (``stitch_panorama(...,
@@ -141,11 +153,15 @@ def feather_blend(layers, origins, size, sharpness=0.02, device=None):
 
     1 to 128 layers (OpenCV's int16 accumulator holds 128 x 255).  ``sharpness`` must be a finite float32 of at least
     ``FLT_MIN`` (about 1.18e-38); below about 1.5e-5 the canvas must also have ``W + H <= 65536`` (distances are stored
-    in 16 bits).  ``ValueError`` before any launch otherwise.  Inputs and outputs as ``blend_layers``.  No CPU
-    fallback."""
+    in 16 bits).  ``ValueError`` before any launch otherwise.  Inputs and outputs as ``blend_layers``.
+
+    ``gains`` as for ``blend_layers``: the blender is fed the compensated ``P_k`` with the raw ``mask_k``, as OpenCV's
+    stitching pipeline feeds it after ``GainCompensator.apply``; the distances, and so the weights, are unchanged.
+    No CPU fallback."""
     layers, origins, width, height, on_device, device = _check_layers("feather_blend", layers, origins, size,
                                                                        rt.FEATHER_MAX_LAYERS, device)
     s = _feather_sharpness("feather_blend", sharpness)
+    lut = None if gains is None else _gain_table("feather_blend", gains, len(layers))
     lib = rt.load_library()
     cap = ctypes.c_int()
     rc = lib.apap_feather_distance_cap(s, height, width, ctypes.byref(cap))
@@ -163,9 +179,106 @@ def feather_blend(layers, origins, size, sharpness=0.02, device=None):
     ws = torch.empty(max(ws_bytes.value, 16), dtype=torch.uint8, device=device)
     out = torch.empty((height, width, 3), dtype=torch.uint8, device=device)
     with torch.cuda.device(device):
-        rt.check(lib.apap_feather_blend(desc_p, len(devs), height, width, s, ws.data_ptr(), ws.numel(), out.data_ptr(),
-                                        out.numel(), rt.stream_ptr(torch, device)), "apap_feather_blend")
+        st = rt.stream_ptr(torch, device)
+        if lut is None:
+            rt.check(lib.apap_feather_blend(desc_p, len(devs), height, width, s, ws.data_ptr(), ws.numel(),
+                                            out.data_ptr(), out.numel(), st), "apap_feather_blend")
+        else:
+            lut_dev = rt.to_device(torch, device, lut)
+            rt.check(lib.apap_feather_blend_gain(desc_p, len(devs), height, width, s, lut_dev.data_ptr(), ws.data_ptr(),
+                                                 ws.numel(), out.data_ptr(), out.numel(), st), "apap_feather_blend_gain")
     return out if on_device else rt.to_host(torch, out)
+
+
+def exposure_gains(layers, origins, size, device=None) -> np.ndarray:
+    """Exposure-compensation gains of placed layers, float64 ``[n]``: what ``cv.detail.GainCompensator()`` (one feed,
+    no similarity mask) returns from ``getMatGains()`` after ``feed([(0, 0)] * n, [P_k], [mask_k])``, with ``P_k``
+    and ``mask_k`` as for ``feather_blend``.  Pass them as ``gains=`` to ``blend_layers`` / ``feather_blend``.
+
+    The pass over every layer pixel runs on the GPU (``k_gain_stats``): per pair of layers the count of pixels both
+    cover and, exactly, the sums of ``norm(P_i) = sqrt(b^2 + g^2 + r^2)`` over them -- the sums are the correctly
+    rounded ``math.fsum`` of the norms, so the result does not depend on the schedule.  The small linear system is
+    OpenCV's (``alpha = 0.01``, ``beta = 100``, layers that meet no other get gain 1), built in its loop order and
+    solved with ``cv.solve`` on the host, as an OpenCV build without Eigen solves it.
+
+    1 to 256 layers; ``layers``, ``origins``, ``size`` and the device rules as for ``blend_layers`` (tensor crops are
+    read in place).  One launch and one download.  No CPU fallback."""
+    layers, origins, width, height, on_device, device = _check_layers("exposure_gains", layers, origins, size,
+                                                                       rt.GAIN_MAX_LAYERS, device)
+    torch, device = rt.torch_cuda(device)
+    lib = rt.load_library()
+    devs, desc = _layer_descs(torch, device, layers, origins, on_device)
+    desc_p = desc.ctypes.data_as(ctypes.POINTER(ctypes.c_longlong))
+    n = len(devs)
+    nbytes = ctypes.c_size_t()
+    rt.check(lib.apap_gain_stats_bytes(n, ctypes.byref(nbytes)), "apap_gain_stats_bytes")
+    stats = torch.empty(nbytes.value // 8, dtype=torch.int64, device=device)
+    with torch.cuda.device(device):
+        rt.check(lib.apap_gain_stats(desc_p, n, height, width, stats.data_ptr(), stats.numel() * 8,
+                                     rt.stream_ptr(torch, device)), "apap_gain_stats")
+    count, sums = gain_stats_ints(rt.to_host(torch, stats), n)
+    return solve_gains(count, sums)
+
+
+def gain_stats_ints(stats, n):
+    """``apap_gain_stats``' uint64 ``[4][n][n]`` as Python ints: ``(count, sums)`` with ``count[i][j]`` for ``i <= j``
+    and ``sums[i][j] = word1 + word2 2^32 + word3 2^64`` (the sum of ``sqrt(q) 2^52`` over the intersection)."""
+    w = np.asarray(stats).view(np.uint64).reshape(4, n, n)
+    count = [[int(v) for v in row] for row in w[0]]
+    sums = [[int(a) + (int(b) << 32) + (int(c) << 64) for a, b, c in zip(*rows)] for rows in zip(w[1], w[2], w[3])]
+    return count, sums
+
+
+def solve_gains(count, sums):
+    """``GainCompensator::singleFeed``'s system from the statistics: ``N(i, j) = max(1, count)``, ``I(i, j) =
+    round(sums[i][j]) 2^-52 / N(i, j)`` for pairs that meet, ``A`` and ``b`` in OpenCV's loop order over the layers
+    that meet another, ``cv.solve`` (LU in double); gain 1 for the rest."""
+    import cv2 as cv
+
+    alpha, beta = 0.01, 100.0
+    n = len(count)
+    N = [[1] * n for _ in range(n)]
+    inten = [[0.0] * n for _ in range(n)]
+    skip = [True] * n
+    for i in range(n):
+        for j in range(i, n):
+            c = count[i][j]
+            N[i][j] = N[j][i] = max(1, c)
+            if c == 0:
+                continue
+            if i != j:
+                skip[i] = skip[j] = False
+            inten[i][j] = float(sums[i][j]) * 2.0 ** -52 / N[i][j]
+            inten[j][i] = float(sums[j][i]) * 2.0 ** -52 / N[i][j]
+    keep = [i for i in range(n) if not skip[i]]
+    gains = np.ones(n)
+    if not keep:
+        return gains
+    A = np.zeros((len(keep), len(keep)))
+    b = np.zeros((len(keep), 1))
+    for ki, i in enumerate(keep):
+        for kj, j in enumerate(keep):
+            nij = float(N[i][j])
+            b[ki, 0] += beta * nij
+            A[ki, ki] += beta * nij
+            if j != i:
+                A[ki, ki] += 2 * alpha * inten[i][j] * inten[i][j] * nij
+                A[ki, kj] -= 2 * alpha * inten[i][j] * inten[j][i] * nij
+    _, sol = cv.solve(A, b)
+    gains[keep] = sol[:, 0]
+    return gains
+
+
+def _gain_table(what, gains, n):
+    """``uint8 [n, 256]``: row k maps a byte ``v`` to ``saturate(rint(v g_k))`` in float64 (ties to even), what
+    ``GainCompensator.apply`` gives; ``ValueError`` unless ``gains`` holds one finite number per layer."""
+    try:
+        g = np.asarray(gains, dtype=np.float64)
+    except (TypeError, ValueError):
+        raise ValueError(f"{what}: gains must be {n} finite numbers") from None
+    if g.shape != (n,) or not np.isfinite(g).all():
+        raise ValueError(f"{what}: gains must be {n} finite numbers (one per layer), got shape {g.shape}")
+    return np.clip(np.rint(np.arange(256, dtype=np.float64)[None, :] * g[:, None]), 0, 255).astype(np.uint8)
 
 
 def _feather_sharpness(what, sharpness):

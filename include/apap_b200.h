@@ -272,6 +272,35 @@ int apap_feather_blend(const long long *layers, int n_layers, int canvas_h, int 
                        void *workspace, size_t workspace_bytes, uint8_t *out, size_t out_bytes, void *stream);
 
 /*
+ * Exposure compensation of placed layers (utils.exposure_gains, driver.stitch_panorama(exposure="gain")), as
+ * cv.detail.GainCompensator (DESIGN.md section 3).
+ *
+ * apap_gain_stats: the overlap statistics of its single feed, exact.  stats (device, 8-byte aligned, stats_bytes >=
+ * apap_gain_stats_bytes) gets uint64 [4][n_layers][n_layers]:
+ *   plane 0 [i][j], i <= j : |mask_i & mask_j|, mask_k = the non-empty pixels of layer k (any channel > 0)
+ *   planes 1..3 [i][j], i != j: S(i, j) = word1 + word2 2^32 + word3 2^64, the exact sum over mask_i & mask_j of
+ *              sqrt(b^2 + g^2 + r^2) 2^52 of layer i's pixels (sqrt correctly rounded in double: integers < 2^61)
+ *   the other entries are 0.  The result does not depend on the schedule.
+ *   layers   : HOST long long [n_layers][6], as apap_blend_layers
+ *   n_layers : 1 .. APAP_GAIN_MAX_LAYERS
+ * One memset and one kernel (k_gain_stats) on `stream`.
+ *
+ * apap_blend_layers_gain / apap_feather_blend_gain: apap_blend_layers / apap_feather_blend with layer k's bytes v
+ * replaced by lut[k][v] before they are summed or weighted; which pixels count as non-empty (the mean's n, the
+ * feather distances) still follows the raw bytes, as OpenCV's pipeline feeds the blender the original masks.
+ *   lut : device uint8 [n_layers][256], lut[k][0] = 0; for a gain g_k, saturate(rint(v g_k)) in double (ties to even)
+ */
+#define APAP_GAIN_MAX_LAYERS 256
+int apap_gain_stats_bytes(int n_layers, size_t *bytes);
+int apap_gain_stats(const long long *layers, int n_layers, int canvas_h, int canvas_w, void *stats, size_t stats_bytes,
+                    void *stream);
+int apap_blend_layers_gain(const long long *layers, int n_layers, int canvas_h, int canvas_w, const uint8_t *lut,
+                           uint8_t *out, size_t out_bytes, void *stream);
+int apap_feather_blend_gain(const long long *layers, int n_layers, int canvas_h, int canvas_w, float sharpness,
+                            const uint8_t *lut, void *workspace, size_t workspace_bytes, uint8_t *out, size_t out_bytes,
+                            void *stream);
+
+/*
  * Input preparation on the device (what the host layer used to build in numpy; both reproduce their
  * numpy restatements in cvx_proj_b200/apap.py bit for bit).
  *
