@@ -31,6 +31,8 @@ RANSAC_MAX_ITERS = 1 << 20
 BLEND_MAX_LAYERS = 256
 FEATHER_MAX_LAYERS = 128
 GAIN_MAX_LAYERS = 256
+MULTIBAND_MAX_LAYERS = 127
+MULTIBAND_MAX_HEIGHT = 524280  # 65535 tiles of 8 rows: apap_multiband_* return APAP_E_TOOBIG above
 E_TOOBIG = -3           # APAP_E_TOOBIG
 
 # symbol -> (restype, argtypes); tests check every symbol of include/apap_b200.h is exported
@@ -68,6 +70,12 @@ SIGNATURES = {
                                        c_void_p]),
     "apap_feather_blend_gain": (c_int, [POINTER(ctypes.c_longlong), c_int, c_int, c_int, c_float, c_void_p, c_void_p,
                                         c_size_t, c_void_p, c_size_t, c_void_p]),
+    "apap_multiband_workspace_bytes": (c_int, [POINTER(ctypes.c_longlong), c_int, c_int, c_int, c_int,
+                                               POINTER(c_size_t)]),
+    "apap_multiband_blend": (c_int, [POINTER(ctypes.c_longlong), c_int, c_int, c_int, c_int, c_void_p, c_size_t,
+                                     c_void_p, c_size_t, c_void_p]),
+    "apap_multiband_blend_gain": (c_int, [POINTER(ctypes.c_longlong), c_int, c_int, c_int, c_int, c_void_p, c_void_p,
+                                          c_size_t, c_void_p, c_size_t, c_void_p]),
     "apap_pipe_probe": (c_int, [c_int, c_int, c_void_p, POINTER(c_double), c_void_p]),
     "apap_warp_perspective": (c_int, [c_void_p, c_int, c_int, POINTER(c_double), c_void_p, c_int, c_int, c_void_p, c_int,
                                       c_int, c_int, c_int, c_int, c_void_p]),

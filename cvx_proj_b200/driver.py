@@ -187,7 +187,8 @@ class PanoramaResult(NamedTuple):
 
 def stitch_panorama(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops, *, mesh_size: int = 100, gamma=0.5, sigma=100,
                     warp_imgs=None, blend_img=None, equalize: bool = True, ransac: str = "opencv",
-                    device=None, blend: str = "mean", sharpness=0.02, exposure: str = "none") -> PanoramaResult:
+                    device=None, blend: str = "mean", sharpness=0.02, exposure: str = "none",
+                    bands: int = 5) -> PanoramaResult:
     """Every image of a case stitched against the centre into ONE panorama (the reference has no multi-image blend;
     ``stitch_case`` returns one two-image canvas per pair, each in a frame of its own).
 
@@ -205,26 +206,36 @@ def stitch_panorama(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops, *, mesh_s
     ``panorama`` is the mean call's.  With no other image the panorama is ``feather_blend([centre])``, the centre less
     1 where it is non-empty (OpenCV's ``trunc(v / 1.00001)``).  ``sharpness`` is used by ``"feather"`` only.
 
-    ``exposure="gain"`` evens out the brightness of the layers before either blend, as OpenCV's stitching pipeline
+    ``blend="multiband"`` blends the same layers in the same order by ``utils.multiband_blend(..., bands)``, OpenCV's
+    ``MultiBandBlender`` with int16 weights (``cv.detail_MultiBandBlender(0, bands, cv.CV_16S)``), the blender
+    OpenCV's stitcher runs by default: each Laplacian band is blended over a width matched to its scale, so low
+    frequencies mix over a wide seam while edges switch over a few pixels.  Every field but ``panorama`` is the mean
+    call's.  With no other image the panorama is ``multiband_blend([centre])``.  ``bands`` is used by
+    ``"multiband"`` only.
+
+    ``exposure="gain"`` evens out the brightness of the layers before any blend, as OpenCV's stitching pipeline
     runs ``cv.detail.GainCompensator`` in front of its blender: ``utils.exposure_gains`` over the same layers in the
     same order gives one gain per layer, and the blend gets them (``gains=``), compensating each layer's bytes while
     keeping its original mask.  With no other image it equals ``"none"``.  The gains are not part of the result; a
     caller who wants them calls ``exposure_gains`` on the layers.
 
     The layers are warped from the images the keypoint-pair producer already holds on the device and stay there; one
-    blend call and one download make the panorama.  At most 255 other images (127 with ``"feather"``); an unknown
-    ``blend``, an unknown ``exposure``, too many images or a ``sharpness`` that ``feather_blend`` refuses for every
-    canvas raise ``ValueError`` before any keypoint work."""
+    blend call and one download make the panorama.  At most 255 other images (127 with ``"feather"``, 126 with
+    ``"multiband"``); an unknown ``blend``, an unknown ``exposure``, too many images, a ``sharpness`` that
+    ``feather_blend`` refuses for every canvas or (with ``"multiband"``) a ``bands`` that ``multiband_blend`` refuses
+    raise ``ValueError`` before any keypoint work."""
     from . import _runtime as rt
-    from .utils import _device_image, _feather_sharpness, blend_layers, exposure_gains, feather_blend
+    from .utils import (_device_image, _feather_sharpness, _multiband_bands, blend_layers, exposure_gains,
+                        feather_blend, multiband_blend)
 
-    if blend not in ("mean", "feather"):
-        raise ValueError(f"stitch_panorama: blend must be 'mean' or 'feather', got {blend!r}")
+    if blend not in ("mean", "feather", "multiband"):
+        raise ValueError(f"stitch_panorama: blend must be 'mean', 'feather' or 'multiband', got {blend!r}")
     if exposure not in ("none", "gain"):
         raise ValueError(f"stitch_panorama: exposure must be 'none' or 'gain', got {exposure!r}")
     if warp_imgs is not None and len(warp_imgs) != len(other_imgs):
         raise ValueError(f"stitch_panorama: {len(other_imgs)} other images but {len(warp_imgs)} warp images")
-    max_layers = rt.BLEND_MAX_LAYERS if blend == "mean" else rt.FEATHER_MAX_LAYERS
+    max_layers = {"mean": rt.BLEND_MAX_LAYERS, "feather": rt.FEATHER_MAX_LAYERS,
+                  "multiband": rt.MULTIBAND_MAX_LAYERS}[blend]
     if len(other_imgs) >= max_layers:
         raise ValueError(f"stitch_panorama: at most {max_layers - 1} other images with blend={blend!r}, "
                          f"got {len(other_imgs)}")
@@ -233,6 +244,11 @@ def stitch_panorama(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops, *, mesh_s
 
         def blend_fn(layers, origins, size, device=None, gains=None):
             return feather_blend(layers, origins, size, sharpness, device=device, gains=gains)
+    elif blend == "multiband":
+        bands = _multiband_bands("stitch_panorama", bands)
+
+        def blend_fn(layers, origins, size, device=None, gains=None):
+            return multiband_blend(layers, origins, size, bands, device=device, gains=gains)
     else:
         blend_fn = blend_layers
     front = _case_front(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops, mesh_size, gamma, sigma, equalize, ransac,

@@ -24,7 +24,7 @@ from . import _runtime as rt
 
 __all__ = ["image_warping", "warp_perspective", "warping_canvas", "invert3x3", "match_descriptors", "coarse_matching",
            "sift_describe", "equalize_hist", "keypoint_pairs", "keypoint_pairs_batch", "find_homography_ransac",
-           "find_homography_ransac_batch", "blend_layers", "feather_blend", "exposure_gains"]
+           "find_homography_ransac_batch", "blend_layers", "feather_blend", "multiband_blend", "exposure_gains"]
 
 
 def invert3x3(m) -> np.ndarray:
@@ -188,6 +188,60 @@ def feather_blend(layers, origins, size, sharpness=0.02, device=None, gains=None
             rt.check(lib.apap_feather_blend_gain(desc_p, len(devs), height, width, s, lut_dev.data_ptr(), ws.data_ptr(),
                                                  ws.numel(), out.data_ptr(), out.numel(), st), "apap_feather_blend_gain")
     return out if on_device else rt.to_host(torch, out)
+
+
+def multiband_blend(layers, origins, size, bands=5, device=None, gains=None):
+    """Multi-band blend of placed layers (``k_mb_down``, ``k_mb_band``), bit for bit what
+    ``cv.detail_MultiBandBlender(0, bands, cv.CV_16S)`` gives after ``prepare((0, 0, W, H))``, ``feed(P_k.astype(int16),
+    mask_k, (0, 0))`` for every layer and ``blend()``, converted to uint8 with saturation (``stitch_panorama(...,
+    blend="multiband")``).  ``P_k`` and ``mask_k`` as for ``feather_blend``.
+
+    Each layer is split into Laplacian bands, and band ``i`` is blended with the mask blurred down to that band's
+    scale: low frequencies mix over a wide seam, edges switch over a few pixels.  ``bands`` is any int >= 0; OpenCV
+    caps it at ``ceil(log2(max(W, H)))``.  The weights are OpenCV's int16 ones (``weight_type=CV_16S``), so the blend
+    is integer arithmetic throughout and does not depend on the layer order or the CPU; to compare with OpenCV, build
+    its blender with ``cv.CV_16S``.  The default float32 weights (``cv.detail.MultiBandBlender()``) give a different
+    blend, by tens of levels at some pixels, and are not what this computes.
+
+    1 to 127 layers (128 would wrap OpenCV's int16 weight sums).  ``bands`` that is not an int, a bool or negative,
+    too many layers and a canvas taller than 524 280 rows raise ``ValueError`` before any launch.  ``gains`` as for
+    ``feather_blend``: the pyramids are built from the compensated bytes, the masks from the raw ones.  Inputs,
+    outputs and the device rules as ``blend_layers`` (tensor crops are read in place).  No CPU fallback."""
+    layers, origins, width, height, on_device, device = _check_layers("multiband_blend", layers, origins, size,
+                                                                       rt.MULTIBAND_MAX_LAYERS, device)
+    bands = _multiband_bands("multiband_blend", bands)
+    if height > rt.MULTIBAND_MAX_HEIGHT:
+        raise ValueError(f"multiband_blend: the canvas height must be <= {rt.MULTIBAND_MAX_HEIGHT}, got {height}")
+    lut = None if gains is None else _gain_table("multiband_blend", gains, len(layers))
+    torch, device = rt.torch_cuda(device)
+    lib = rt.load_library()
+    devs, desc = _layer_descs(torch, device, layers, origins, on_device)
+    desc_p = desc.ctypes.data_as(ctypes.POINTER(ctypes.c_longlong))
+    ws_bytes = ctypes.c_size_t()
+    rt.check(lib.apap_multiband_workspace_bytes(desc_p, len(devs), height, width, bands, ctypes.byref(ws_bytes)),
+             "apap_multiband_workspace_bytes")
+    ws = torch.empty(max(ws_bytes.value, 16), dtype=torch.uint8, device=device)
+    out = torch.empty((height, width, 3), dtype=torch.uint8, device=device)
+    with torch.cuda.device(device):
+        st = rt.stream_ptr(torch, device)
+        if lut is None:
+            rt.check(lib.apap_multiband_blend(desc_p, len(devs), height, width, bands, ws.data_ptr(), ws.numel(),
+                                              out.data_ptr(), out.numel(), st), "apap_multiband_blend")
+        else:
+            lut_dev = rt.to_device(torch, device, lut)
+            rt.check(lib.apap_multiband_blend_gain(desc_p, len(devs), height, width, bands, lut_dev.data_ptr(),
+                                                   ws.data_ptr(), ws.numel(), out.data_ptr(), out.numel(), st),
+                     "apap_multiband_blend_gain")
+    return out if on_device else rt.to_host(torch, out)
+
+
+def _multiband_bands(what, bands):
+    """``bands`` as an int >= 0, or ``ValueError`` (a bool, a non-integer or a negative value)."""
+    if isinstance(bands, (bool, np.bool_)) or not isinstance(bands, (int, np.integer)):
+        raise ValueError(f"{what}: bands must be an int >= 0, got {bands!r}")
+    if bands < 0:
+        raise ValueError(f"{what}: bands must be >= 0, got {bands}")
+    return min(int(bands), 1 << 20)                     # far above the cap of any canvas
 
 
 def exposure_gains(layers, origins, size, device=None) -> np.ndarray:

@@ -301,6 +301,32 @@ int apap_feather_blend_gain(const long long *layers, int n_layers, int canvas_h,
                             void *stream);
 
 /*
+ * Multi-band blend of placed layers (utils.multiband_blend, driver.stitch_panorama(blend="multiband")): out [canvas_h]
+ * [canvas_w][3] uint8 (device, any alignment, out_bytes >= canvas_h x canvas_w x 3) is bit for bit what
+ * cv.detail.MultiBandBlender(0, bands, CV_16S) gives after prepare((0, 0, canvas_w, canvas_h)), feed(P_k as int16,
+ * mask_k, (0, 0)) for every layer and blend(), converted to uint8 with saturation.  P_k is layer k pasted into a zero
+ * canvas (clipped), mask_k its non-empty pixels (any channel > 0).  The int16-weight blender is integer arithmetic
+ * throughout (DESIGN.md section 3), so the result does not depend on the layer order.
+ *   layers    : HOST long long [n_layers][6], as apap_blend_layers
+ *   n_layers  : 1 .. APAP_MULTIBAND_MAX_LAYERS (128 layers would wrap OpenCV's int16 weight sums)
+ *   bands     : >= 0; OpenCV's cap ceil(log2(max(canvas_w, canvas_h))) applies
+ *   canvas_h  : at most 524280 (APAP_E_TOOBIG above)
+ *   workspace : device scratch of apap_multiband_workspace_bytes (the layers' int16 pyramids above level 0 on boxes
+ *               around their rectangles, and one blended pyramid), 16-byte aligned
+ * nb k_mb_down and nb + 1 k_mb_band launches on `stream`.
+ * apap_multiband_blend_gain: layer k's bytes v replaced by lut[k][v] (as apap_blend_layers_gain) before the pyramids
+ * are built; mask_k still follows the raw bytes, as OpenCV's pipeline feeds the blender the original masks.
+ */
+#define APAP_MULTIBAND_MAX_LAYERS 127
+int apap_multiband_workspace_bytes(const long long *layers, int n_layers, int canvas_h, int canvas_w, int bands,
+                                   size_t *bytes);
+int apap_multiband_blend(const long long *layers, int n_layers, int canvas_h, int canvas_w, int bands, void *workspace,
+                         size_t workspace_bytes, uint8_t *out, size_t out_bytes, void *stream);
+int apap_multiband_blend_gain(const long long *layers, int n_layers, int canvas_h, int canvas_w, int bands,
+                              const uint8_t *lut, void *workspace, size_t workspace_bytes, uint8_t *out,
+                              size_t out_bytes, void *stream);
+
+/*
  * Input preparation on the device (what the host layer used to build in numpy; both reproduce their
  * numpy restatements in cvx_proj_b200/apap.py bit for bit).
  *
