@@ -225,38 +225,26 @@ def stitch_panorama(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops, *, mesh_s
     ``feather_blend`` refuses for every canvas or (with ``"multiband"``) a ``bands`` that ``multiband_blend`` refuses
     raise ``ValueError`` before any keypoint work."""
     from . import _runtime as rt
-    from .utils import (_device_image, _feather_sharpness, _multiband_bands, blend_layers, exposure_gains,
-                        feather_blend, multiband_blend)
+    from .utils import _BLENDERS, _device_image, exposure_gains
 
-    if blend not in ("mean", "feather", "multiband"):
+    if blend not in tuple(_BLENDERS):                   # a tuple: an unhashable blend is a ValueError too
         raise ValueError(f"stitch_panorama: blend must be 'mean', 'feather' or 'multiband', got {blend!r}")
     if exposure not in ("none", "gain"):
         raise ValueError(f"stitch_panorama: exposure must be 'none' or 'gain', got {exposure!r}")
     if warp_imgs is not None and len(warp_imgs) != len(other_imgs):
         raise ValueError(f"stitch_panorama: {len(other_imgs)} other images but {len(warp_imgs)} warp images")
-    max_layers = {"mean": rt.BLEND_MAX_LAYERS, "feather": rt.FEATHER_MAX_LAYERS,
-                  "multiband": rt.MULTIBAND_MAX_LAYERS}[blend]
+    blend_fn, max_layers, param, check_param = _BLENDERS[blend]
     if len(other_imgs) >= max_layers:
         raise ValueError(f"stitch_panorama: at most {max_layers - 1} other images with blend={blend!r}, "
                          f"got {len(other_imgs)}")
-    if blend == "feather":
-        sharpness = _feather_sharpness("stitch_panorama", sharpness)
-
-        def blend_fn(layers, origins, size, device=None, gains=None):
-            return feather_blend(layers, origins, size, sharpness, device=device, gains=gains)
-    elif blend == "multiband":
-        bands = _multiband_bands("stitch_panorama", bands)
-
-        def blend_fn(layers, origins, size, device=None, gains=None):
-            return multiband_blend(layers, origins, size, bands, device=device, gains=gains)
-    else:
-        blend_fn = blend_layers
+    options = {"sharpness": sharpness, "bands": bands}
+    params = {} if param is None else {param: check_param("stitch_panorama", options[param])}
     front = _case_front(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops, mesh_size, gamma, sigma, equalize, ransac,
                         device)
     centre = center_img if blend_img is None else blend_img
     if front is None:
         h, w = centre.shape[0], centre.shape[1]
-        pano = blend_fn([centre], [(0, 0)], (w, h), device=device)
+        pano = blend_fn([centre], [(0, 0)], (w, h), device=device, **params)
         if not isinstance(pano, np.ndarray):
             pano = rt.to_host(rt.torch_cuda(pano.device)[0], pano)
         return PanoramaResult((int(w), int(h), 0, 0), np.zeros((0, 2), np.int64), [], pano)
@@ -273,8 +261,6 @@ def stitch_panorama(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops, *, mesh_s
         layers.append(st.local_warp(warp_devs[i], local_h.copy(), meshes[i]))
     (width, height, ox, oy), origins = panorama_size([p.final_size for p in pairs])
     layers, places = layers + [blend_dev], [tuple(o) for o in origins] + [(ox, oy)]
-    if exposure == "gain":
-        pano = blend_fn(layers, places, (width, height), gains=exposure_gains(layers, places, (width, height)))
-    else:
-        pano = blend_fn(layers, places, (width, height))
+    gains = exposure_gains(layers, places, (width, height)) if exposure == "gain" else None
+    pano = blend_fn(layers, places, (width, height), gains=gains, **params)
     return PanoramaResult((width, height, ox, oy), origins, pairs, rt.to_host(torch, pano))

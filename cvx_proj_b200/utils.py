@@ -120,21 +120,7 @@ def blend_layers(layers, origins, size, device=None, gains=None):
     layers, origins, width, height, on_device, device = _check_layers("blend_layers", layers, origins, size,
                                                                        rt.BLEND_MAX_LAYERS, device)
     lut = None if gains is None else _gain_table("blend_layers", gains, len(layers))
-    torch, device = rt.torch_cuda(device)
-    lib = rt.load_library()
-    devs, desc = _layer_descs(torch, device, layers, origins, on_device)
-    desc_p = desc.ctypes.data_as(ctypes.POINTER(ctypes.c_longlong))
-    out = torch.empty((height, width, 3), dtype=torch.uint8, device=device)
-    with torch.cuda.device(device):
-        st = rt.stream_ptr(torch, device)
-        if lut is None:
-            rt.check(lib.apap_blend_layers(desc_p, len(devs), height, width, out.data_ptr(), out.numel(), st),
-                     "apap_blend_layers")
-        else:
-            lut_dev = rt.to_device(torch, device, lut)
-            rt.check(lib.apap_blend_layers_gain(desc_p, len(devs), height, width, lut_dev.data_ptr(), out.data_ptr(),
-                                                out.numel(), st), "apap_blend_layers_gain")
-    return out if on_device else rt.to_host(torch, out)
+    return _blend("apap_blend_layers", (), None, layers, origins, width, height, on_device, device, lut)
 
 
 def feather_blend(layers, origins, size, sharpness=0.02, device=None, gains=None):
@@ -162,32 +148,9 @@ def feather_blend(layers, origins, size, sharpness=0.02, device=None, gains=None
                                                                        rt.FEATHER_MAX_LAYERS, device)
     s = _feather_sharpness("feather_blend", sharpness)
     lut = None if gains is None else _gain_table("feather_blend", gains, len(layers))
-    lib = rt.load_library()
-    cap = ctypes.c_int()
-    rc = lib.apap_feather_distance_cap(s, height, width, ctypes.byref(cap))
-    if rc == rt.E_TOOBIG:
-        raise ValueError(f"feather_blend: sharpness {s} needs distances beyond 16 bits on a {width} x {height} canvas "
-                         "(a larger sharpness or W + H <= 65536)")
-    if rc != 0:
-        raise ValueError(f"feather_blend: {lib.apap_last_error().decode('utf-8', 'replace')}")
-    torch, device = rt.torch_cuda(device)
-    devs, desc = _layer_descs(torch, device, layers, origins, on_device)
-    desc_p = desc.ctypes.data_as(ctypes.POINTER(ctypes.c_longlong))
-    ws_bytes = ctypes.c_size_t()
-    rt.check(lib.apap_feather_workspace_bytes(desc_p, len(devs), height, width, ctypes.byref(ws_bytes)),
-             "apap_feather_workspace_bytes")
-    ws = torch.empty(max(ws_bytes.value, 16), dtype=torch.uint8, device=device)
-    out = torch.empty((height, width, 3), dtype=torch.uint8, device=device)
-    with torch.cuda.device(device):
-        st = rt.stream_ptr(torch, device)
-        if lut is None:
-            rt.check(lib.apap_feather_blend(desc_p, len(devs), height, width, s, ws.data_ptr(), ws.numel(),
-                                            out.data_ptr(), out.numel(), st), "apap_feather_blend")
-        else:
-            lut_dev = rt.to_device(torch, device, lut)
-            rt.check(lib.apap_feather_blend_gain(desc_p, len(devs), height, width, s, lut_dev.data_ptr(), ws.data_ptr(),
-                                                 ws.numel(), out.data_ptr(), out.numel(), st), "apap_feather_blend_gain")
-    return out if on_device else rt.to_host(torch, out)
+    _feather_distance_cap(s, width, height)
+    return _blend("apap_feather_blend", (s,), ("apap_feather_workspace_bytes", ()), layers, origins, width, height,
+                  on_device, device, lut)
 
 
 def multiband_blend(layers, origins, size, bands=5, device=None, gains=None):
@@ -213,26 +176,8 @@ def multiband_blend(layers, origins, size, bands=5, device=None, gains=None):
     if height > rt.MULTIBAND_MAX_HEIGHT:
         raise ValueError(f"multiband_blend: the canvas height must be <= {rt.MULTIBAND_MAX_HEIGHT}, got {height}")
     lut = None if gains is None else _gain_table("multiband_blend", gains, len(layers))
-    torch, device = rt.torch_cuda(device)
-    lib = rt.load_library()
-    devs, desc = _layer_descs(torch, device, layers, origins, on_device)
-    desc_p = desc.ctypes.data_as(ctypes.POINTER(ctypes.c_longlong))
-    ws_bytes = ctypes.c_size_t()
-    rt.check(lib.apap_multiband_workspace_bytes(desc_p, len(devs), height, width, bands, ctypes.byref(ws_bytes)),
-             "apap_multiband_workspace_bytes")
-    ws = torch.empty(max(ws_bytes.value, 16), dtype=torch.uint8, device=device)
-    out = torch.empty((height, width, 3), dtype=torch.uint8, device=device)
-    with torch.cuda.device(device):
-        st = rt.stream_ptr(torch, device)
-        if lut is None:
-            rt.check(lib.apap_multiband_blend(desc_p, len(devs), height, width, bands, ws.data_ptr(), ws.numel(),
-                                              out.data_ptr(), out.numel(), st), "apap_multiband_blend")
-        else:
-            lut_dev = rt.to_device(torch, device, lut)
-            rt.check(lib.apap_multiband_blend_gain(desc_p, len(devs), height, width, bands, lut_dev.data_ptr(),
-                                                   ws.data_ptr(), ws.numel(), out.data_ptr(), out.numel(), st),
-                     "apap_multiband_blend_gain")
-    return out if on_device else rt.to_host(torch, out)
+    return _blend("apap_multiband_blend", (bands,), ("apap_multiband_workspace_bytes", (bands,)), layers, origins,
+                  width, height, on_device, device, lut)
 
 
 def _multiband_bands(what, bands):
@@ -247,7 +192,8 @@ def _multiband_bands(what, bands):
 def exposure_gains(layers, origins, size, device=None) -> np.ndarray:
     """Exposure-compensation gains of placed layers, float64 ``[n]``: what ``cv.detail.GainCompensator()`` (one feed,
     no similarity mask) returns from ``getMatGains()`` after ``feed([(0, 0)] * n, [P_k], [mask_k])``, with ``P_k``
-    and ``mask_k`` as for ``feather_blend``.  Pass them as ``gains=`` to ``blend_layers`` / ``feather_blend``.
+    and ``mask_k`` as for ``feather_blend``.  Pass them as ``gains=`` to ``blend_layers``, ``feather_blend`` or
+    ``multiband_blend``.
 
     The pass over every layer pixel runs on the GPU (``k_gain_stats``): per pair of layers the count of pixels both
     cover and, exactly, the sums of ``norm(P_i) = sqrt(b^2 + g^2 + r^2)`` over them -- the sums are the correctly
@@ -259,10 +205,7 @@ def exposure_gains(layers, origins, size, device=None) -> np.ndarray:
     read in place).  One launch and one download.  No CPU fallback."""
     layers, origins, width, height, on_device, device = _check_layers("exposure_gains", layers, origins, size,
                                                                        rt.GAIN_MAX_LAYERS, device)
-    torch, device = rt.torch_cuda(device)
-    lib = rt.load_library()
-    devs, desc = _layer_descs(torch, device, layers, origins, on_device)
-    desc_p = desc.ctypes.data_as(ctypes.POINTER(ctypes.c_longlong))
+    torch, device, lib, devs, desc_p = _placed_layers(layers, origins, on_device, device)
     n = len(devs)
     nbytes = ctypes.c_size_t()
     rt.check(lib.apap_gain_stats_bytes(n, ctypes.byref(nbytes)), "apap_gain_stats_bytes")
@@ -346,9 +289,23 @@ def _feather_sharpness(what, sharpness):
     return s
 
 
+def _feather_distance_cap(s, width, height):
+    """``ValueError`` unless the feather kernels can store the distances of sharpness ``s`` (a checked float32) on a
+    ``width x height`` canvas (``apap_feather_distance_cap``, host only)."""
+    lib = rt.load_library()
+    cap = ctypes.c_int()
+    rc = lib.apap_feather_distance_cap(s, height, width, ctypes.byref(cap))
+    if rc == rt.E_TOOBIG:
+        raise ValueError(f"feather_blend: sharpness {s} needs distances beyond 16 bits on a {width} x {height} canvas "
+                         "(a larger sharpness or W + H <= 65536)")
+    if rc != 0:
+        raise ValueError(f"feather_blend: {lib.apap_last_error().decode('utf-8', 'replace')}")
+
+
 def _check_layers(what, layers, origins, size, max_layers, device):
-    """The argument checks ``blend_layers`` and ``feather_blend`` share (``ValueError`` named after ``what``).
-    Returns ``(layers, origins, width, height, on_device, device)``; ``device`` is the layers' own for tensors."""
+    """The argument checks of the placed-layer functions, the three blends and ``exposure_gains`` (``ValueError``
+    named after ``what``).  Returns ``(layers, origins, width, height, on_device, device)``; ``device`` is the layers'
+    own for tensors."""
     layers = list(layers)
     origins = [tuple(o) for o in origins]
     if not 1 <= len(layers) <= max_layers:
@@ -388,6 +345,47 @@ def _layer_descs(torch, device, layers, origins, on_device):
     desc = np.array([[img.data_ptr(), img.shape[0], img.shape[1], img.stride(0), x0, y0]
                      for img, (x0, y0) in zip(devs, origins)], dtype=np.int64)
     return devs, desc
+
+
+def _placed_layers(layers, origins, on_device, device):
+    """``(torch, device, lib, devs, desc_p)`` for a placed-layer call whose arguments are checked: the layers on the
+    device (``_layer_descs``) and a ctypes pointer to their descriptors, which keeps the descriptor array alive."""
+    torch, device = rt.torch_cuda(device)
+    lib = rt.load_library()
+    devs, desc = _layer_descs(torch, device, layers, origins, on_device)
+    return torch, device, lib, devs, desc.ctypes.data_as(ctypes.POINTER(ctypes.c_longlong))
+
+
+def _blend(entry, params, workspace, layers, origins, width, height, on_device, device, lut):
+    """A placed-layer blend after its checks: the layers described (``_placed_layers``), the workspace (``None``: the
+    blender needs none; else ``(query, its scalars)``), the canvas, and one call of ``entry`` -- or of ``entry +
+    "_gain"`` with the gain table ``lut`` uploaded when it is not ``None``.  The entries share one argument layout,
+    ``(desc, n, h, w, *params, [lut], [ws, ws_bytes], out, out_bytes, stream)`` with ``params`` the blender's
+    scalars (none, ``sharpness`` or ``bands``), and the workspace queries ``(desc, n, h, w, *scalars, &bytes)``.
+    numpy layers in -> numpy out, tensors in -> a tensor on their device."""
+    torch, device, lib, devs, desc_p = _placed_layers(layers, origins, on_device, device)
+    head = (desc_p, len(devs), height, width)
+    ws_args = lut_args = ()
+    if workspace is not None:
+        query, scalars = workspace
+        ws_bytes = ctypes.c_size_t()
+        rt.check(getattr(lib, query)(*head, *scalars, ctypes.byref(ws_bytes)), query)
+        ws = torch.empty(max(ws_bytes.value, 16), dtype=torch.uint8, device=device)
+        ws_args = (ws.data_ptr(), ws.numel())
+    out = torch.empty((height, width, 3), dtype=torch.uint8, device=device)
+    with torch.cuda.device(device):
+        st = rt.stream_ptr(torch, device)
+        if lut is not None:
+            lut_dev = rt.to_device(torch, device, lut)
+            entry, lut_args = entry + "_gain", (lut_dev.data_ptr(),)
+        rt.check(getattr(lib, entry)(*head, *params, *lut_args, *ws_args, out.data_ptr(), out.numel(), st), entry)
+    return out if on_device else rt.to_host(torch, out)
+
+
+# stitch_panorama's blend= names: (function, most layers, name of its one parameter, the parameter's validator)
+_BLENDERS = {"mean": (blend_layers, rt.BLEND_MAX_LAYERS, None, None),
+             "feather": (feather_blend, rt.FEATHER_MAX_LAYERS, "sharpness", _feather_sharpness),
+             "multiband": (multiband_blend, rt.MULTIBAND_MAX_LAYERS, "bands", _multiband_bands)}
 
 
 # ------------------------------------------------------------------ keypoint-pair producer (SURVEY 8f, row N3)

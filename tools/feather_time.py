@@ -29,6 +29,7 @@ import torch  # noqa: E402
 
 from cvx_proj_b200 import _runtime as rt  # noqa: E402
 from cvx_proj_b200.driver import stitch_panorama  # noqa: E402
+from cvx_proj_b200.utils import _layer_descs  # noqa: E402
 from oracle import feather_oracle as fo  # noqa: E402
 from oracle import panorama_oracle as po  # noqa: E402
 from panorama_time import HBM_TBS, case_layers, synthetic_layers  # noqa: E402
@@ -54,8 +55,7 @@ def model_bytes(layers, origins, size):
 
 def calls(lib, dev, layers, origins, size):
     width, height = size
-    desc = np.array([[t.data_ptr(), t.shape[0], t.shape[1], t.stride(0), x0, y0]
-                     for t, (x0, y0) in zip(layers, origins)], dtype=np.int64)
+    _, desc = _layer_descs(torch, dev, layers, origins, True)     # packed device layers: described in place
     ptr = desc.ctypes.data_as(ctypes.POINTER(ctypes.c_longlong))
     ws_bytes = ctypes.c_size_t()
     rt.check(lib.apap_feather_workspace_bytes(ptr, len(layers), height, width, ctypes.byref(ws_bytes)), "ws bytes")

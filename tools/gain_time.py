@@ -30,7 +30,7 @@ import torch  # noqa: E402
 
 from cvx_proj_b200 import _runtime as rt  # noqa: E402
 from cvx_proj_b200.driver import stitch_panorama  # noqa: E402
-from cvx_proj_b200.utils import _gain_table, exposure_gains, gain_stats_ints  # noqa: E402
+from cvx_proj_b200.utils import _gain_table, _layer_descs, exposure_gains, gain_stats_ints  # noqa: E402
 from feather_time import event_us  # noqa: E402
 from oracle import feather_oracle as fo  # noqa: E402
 from oracle import gain_oracle as go  # noqa: E402
@@ -53,8 +53,7 @@ def layer_px(layers, origins, size):
 def calls(lib, dev, layers, origins, size, gains):
     width, height = size
     n = len(layers)
-    desc = np.array([[t.data_ptr(), t.shape[0], t.shape[1], t.stride(0), x0, y0]
-                     for t, (x0, y0) in zip(layers, origins)], dtype=np.int64)
+    _, desc = _layer_descs(torch, dev, layers, origins, True)     # packed device layers: described in place
     ptr = desc.ctypes.data_as(ctypes.POINTER(ctypes.c_longlong))
     nb = ctypes.c_size_t()
     rt.check(lib.apap_gain_stats_bytes(n, ctypes.byref(nb)), "stats bytes")

@@ -29,7 +29,7 @@ import torch  # noqa: E402
 
 from cvx_proj_b200 import _runtime as rt  # noqa: E402
 from cvx_proj_b200.driver import stitch_panorama  # noqa: E402
-from cvx_proj_b200.utils import _gain_table, exposure_gains, multiband_blend  # noqa: E402
+from cvx_proj_b200.utils import _gain_table, _layer_descs, exposure_gains, multiband_blend  # noqa: E402
 from feather_time import event_us  # noqa: E402
 from gain_time import layer_px  # noqa: E402
 from oracle import feather_oracle as fo  # noqa: E402
@@ -45,8 +45,7 @@ KERNELS = ("k_mb_down", "k_mb_band")
 def calls(lib, dev, layers, origins, size, gains):
     width, height = size
     n = len(layers)
-    desc = np.array([[t.data_ptr(), t.shape[0], t.shape[1], t.stride(0), x0, y0]
-                     for t, (x0, y0) in zip(layers, origins)], dtype=np.int64)
+    _, desc = _layer_descs(torch, dev, layers, origins, True)     # packed device layers: described in place
     ptr = desc.ctypes.data_as(ctypes.POINTER(ctypes.c_longlong))
     ws_bytes = ctypes.c_size_t()
     rt.check(lib.apap_multiband_workspace_bytes(ptr, n, height, width, BANDS, ctypes.byref(ws_bytes)), "ws bytes")

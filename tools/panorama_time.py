@@ -29,6 +29,7 @@ import torch  # noqa: E402
 from cvx_proj_b200 import _runtime as rt  # noqa: E402
 from cvx_proj_b200.apap import APAP  # noqa: E402
 from cvx_proj_b200.driver import panorama_size, stitch_case, stitch_panorama  # noqa: E402
+from cvx_proj_b200.utils import _layer_descs  # noqa: E402
 from oracle import panorama_oracle as po  # noqa: E402
 from sift_time import host_ms  # noqa: E402
 from tests.test_case import _scene  # noqa: E402
@@ -75,8 +76,7 @@ def moved_bytes(layers, origins, size):
 
 def kernel_us(lib, dev, layers, origins, size, reps, flush):
     width, height = size
-    desc = np.array([[t.data_ptr(), t.shape[0], t.shape[1], t.stride(0), x0, y0]
-                     for t, (x0, y0) in zip(layers, origins)], dtype=np.int64)
+    _, desc = _layer_descs(torch, dev, layers, origins, True)     # packed device layers: described in place
     out = torch.empty((height, width, 3), dtype=torch.uint8, device=dev)
     st = rt.stream_ptr(torch, dev)
     ptr = desc.ctypes.data_as(ctypes.POINTER(ctypes.c_longlong))
