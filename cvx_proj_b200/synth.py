@@ -122,3 +122,44 @@ def make_scene(name: str = "c1", seed: int = 0, **override) -> Scene:
                  final_w=fw, final_h=fh, offset_x=ox, offset_y=oy,
                  mesh=get_mesh((fw, fh), mesh + 1),
                  vertices=get_vertice((fw, fh), mesh, (ox, oy)))
+
+
+def make_pair(name: str):
+    """A synthetic pair of the bench shape ``name``: centre image, the other view warped by the scene's homography,
+    centre keypoints and their (noisy) images in the other view."""
+    import cv2 as cv
+
+    sc = make_scene(name)
+    rng = np.random.default_rng(1)
+    img_c = make_image(sc.width, sc.height, seed=2)
+    hinv = np.linalg.inv(sc.h_gt)
+    img_o = cv.warpPerspective(img_c, hinv, (sc.width, sc.height))
+    raw_c = sc.dst.astype(np.float32)
+    raw_o = cv.perspectiveTransform(raw_c[None].astype(np.float64), hinv)[0].astype(np.float32)
+    keep = np.all((raw_o > 8) & (raw_o < [sc.width - 8, sc.height - 8]) & (raw_c > 8) & (raw_c < [sc.width - 8, sc.height - 8]),
+                  axis=1)
+    raw_c, raw_o = raw_c[keep], raw_o[keep]
+    raw_o = raw_o + rng.normal(0, 0.3, raw_o.shape).astype(np.float32)
+    return img_c, img_o, raw_c, raw_o
+
+
+def make_case(name: str, k: int):
+    """A centre image of the bench shape ``name`` and ``k`` others warped from it by different homographies (rotation,
+    shift, a little perspective), with the centre keypoints and their noisy images in each other view."""
+    import cv2 as cv
+
+    cfg = CONFIGS[name]
+    w, h = cfg["width"], cfg["height"]
+    centre = make_image(w, h, seed=2)
+    r = np.random.default_rng(5)
+    raw_c = (r.random((cfg["n_kp"], 2)) * [w - 48, h - 48] + 24).astype(np.float32)
+    others, raw_os = [], []
+    for j in range(k):
+        a = 0.015 * (j + 1) * (-1) ** j
+        hom = np.array([[np.cos(a), -np.sin(a), 0.02 * w * (j + 1)], [np.sin(a), np.cos(a), -0.015 * h * (j + 1)],
+                        [2e-6 * (j + 1), -3e-6 * j, 1.0]])
+        hinv = np.linalg.inv(hom)
+        others.append(cv.warpPerspective(centre, hinv, (w, h)))
+        raw_o = cv.perspectiveTransform(raw_c[None].astype(np.float64), hinv)[0].astype(np.float32)
+        raw_os.append(raw_o + r.normal(0, 0.3, raw_o.shape).astype(np.float32))
+    return centre, others, raw_c, raw_os

@@ -17,25 +17,7 @@ pytestmark = pytest.mark.gpu
 
 
 # ----------------------------------------------------------------------------------------------- fixtures
-@functools.lru_cache(maxsize=None)
-def _scene(name, k):
-    """A centre image of the bench shape ``name`` and ``k`` others warped from it by different homographies (rotation,
-    shift, a little perspective), with the centre keypoints and their noisy images in each other view."""
-    cfg = synth.CONFIGS[name]
-    w, h = cfg["width"], cfg["height"]
-    centre = synth.make_image(w, h, seed=2)
-    r = np.random.default_rng(5)
-    raw_c = (r.random((cfg["n_kp"], 2)) * [w - 48, h - 48] + 24).astype(np.float32)
-    others, raw_os = [], []
-    for j in range(k):
-        a = 0.015 * (j + 1) * (-1) ** j
-        hom = np.array([[np.cos(a), -np.sin(a), 0.02 * w * (j + 1)], [np.sin(a), np.cos(a), -0.015 * h * (j + 1)],
-                        [2e-6 * (j + 1), -3e-6 * j, 1.0]])
-        hinv = np.linalg.inv(hom)
-        others.append(cv.warpPerspective(centre, hinv, (w, h)))
-        raw_o = cv.perspectiveTransform(raw_c[None].astype(np.float64), hinv)[0].astype(np.float32)
-        raw_os.append(raw_o + r.normal(0, 0.3, raw_o.shape).astype(np.float32))
-    return centre, others, raw_c, raw_os
+_scene = functools.lru_cache(maxsize=None)(synth.make_case)
 
 
 def _per_pair_centres(raw_c, k):

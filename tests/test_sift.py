@@ -32,22 +32,7 @@ def _cv_describe(img, pts, size=1.0, angle=-1.0):
     return feats if feats is not None else np.zeros((0, 128), np.float32)
 
 
-@functools.lru_cache(maxsize=None)
-def _pair(name):
-    """A synthetic pair of the bench shape ``name`` (tools/n3_host_cost.py): centre image, the other view warped by the
-    scene's homography, centre keypoints and their (noisy) images in the other view."""
-    sc = synth.make_scene(name)
-    rng = np.random.default_rng(1)
-    img_c = synth.make_image(sc.width, sc.height, seed=2)
-    hinv = np.linalg.inv(sc.h_gt)
-    img_o = cv.warpPerspective(img_c, hinv, (sc.width, sc.height))
-    raw_c = sc.dst.astype(np.float32)
-    raw_o = cv.perspectiveTransform(raw_c[None].astype(np.float64), hinv)[0].astype(np.float32)
-    keep = np.all((raw_o > 8) & (raw_o < [sc.width - 8, sc.height - 8]) & (raw_c > 8) & (raw_c < [sc.width - 8, sc.height - 8]),
-                  axis=1)
-    raw_c, raw_o = raw_c[keep], raw_o[keep]
-    raw_o = raw_o + rng.normal(0, 0.3, raw_o.shape).astype(np.float32)
-    return img_c, img_o, raw_c, raw_o
+_pair = functools.lru_cache(maxsize=None)(synth.make_pair)
 
 
 def _border_points(h, w):

@@ -2,7 +2,7 @@
 """Cost of the multi-image mode (one centre against K images, run_all.sh:15,29) on the batched paths against the
 per-pair loop.  One run prints:
   - the card's name, power limit and top SM clock (queries only);
-  - batched RANSAC on K in {1, 4, 16, 64} c2 match sets (the 3 975 pairs of tests.test_sift._pair("c2"), each with its
+  - batched RANSAC on K in {1, 4, 16, 64} c2 match sets (the 3 975 pairs of synth.make_pair("c2"), each with its
     own seeded draw of uniform-noise targets at 17 % -- the exact matcher's own rate on that pair -- and at 80 %):
       one apap_ransac_homography_batch call by CUDA events, and k_ransac_sample / k_ransac_fit / k_ransac_score by
       torch.profiler (a run of its own);
@@ -10,7 +10,7 @@ per-pair loop.  One run prints:
       scan, OpenCV's fit of the chosen subset, mask, refit);
       a loop of find_homography_ransac and a loop of cv.findHomography(RANSAC) on the host cores;
   - end to end on a c2-size case (centre + 4 others) and a c4-size case (centre + 16 others), the images and keypoints
-    of tests/test_case.py: keypoint_pairs_batch against a loop of keypoint_pairs, and stitch_case against a loop of
+    of synth.make_case: keypoint_pairs_batch against a loop of keypoint_pairs, and stitch_case against a loop of
     keypoint_pairs + stitch_pair, in both ransac modes, the outputs checked equal in the same run.
 
     python tools/case_time.py [--reps 20] [--out FILE]
@@ -20,7 +20,6 @@ import ctypes
 import functools
 import json
 import os
-import subprocess
 import sys
 import time
 
@@ -32,22 +31,21 @@ import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 from cvx_proj_b200 import _runtime as rt  # noqa: E402
-from cvx_proj_b200 import utils  # noqa: E402
+from cvx_proj_b200 import synth, utils  # noqa: E402
 from cvx_proj_b200.driver import stitch_case, stitch_pair  # noqa: E402
 from cvx_proj_b200.utils import (find_homography_ransac, find_homography_ransac_batch, keypoint_pairs,  # noqa: E402
                                  keypoint_pairs_batch)
-from sift_time import c2_pair, host_ms  # noqa: E402
-from tests.test_case import _scene  # noqa: E402
+from timing import card, event_us, host_ms, kernel_times, name_in, say, write_out  # noqa: E402
 
 KERNELS = ("k_ransac_sample", "k_ransac_fit", "k_ransac_score")
 MAX_ITERS = 2000
 THR = 5.0
-_c2_pair = functools.lru_cache(maxsize=None)(c2_pair)
+_c2_pair = functools.lru_cache(maxsize=None)(synth.make_pair)
 
 
 def c2_sets(k, share):
     """``k`` copies of the c2 correspondences, each with its own seeded share of targets replaced by uniform noise."""
-    img_c, _, raw_c, raw_o = _c2_pair()
+    img_c, _, raw_c, raw_o = _c2_pair("c2")
     h, w = img_c.shape[:2]
     sets = []
     for j in range(k):
@@ -92,35 +90,6 @@ def kernel_call(lib, dev, sets):
     return call
 
 
-def event_us(call, reps):
-    for _ in range(3):
-        call()
-    torch.cuda.synchronize()
-    ts = []
-    for _ in range(reps):
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        call()
-        e1.record()
-        e1.synchronize()
-        ts.append(e0.elapsed_time(e1) * 1e3)
-    return float(np.median(ts)), float(np.min(ts))
-
-
-def profiled_us(call, reps):
-    from torch.profiler import ProfilerActivity, profile
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        for _ in range(reps):
-            call()
-        torch.cuda.synchronize()
-    kern = {}
-    for e in prof.key_averages():
-        for name in KERNELS:
-            if name in e.key:
-                kern[name] = (getattr(e, "device_time_total", None) or e.cuda_time_total) / max(e.count, 1)
-    return kern
-
-
 def batch_with_tails(sets, reps):
     """find_homography_ransac_batch host to host, and the summed time of its per-pair host tails, per call."""
     tails, orig = [], utils._ransac_tail
@@ -147,19 +116,10 @@ def main():
     ap.add_argument("--reps", type=int, default=20)
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
-    lines = []
-
-    def say(s):
-        print(s, flush=True)
-        lines.append(s)
-
     _, dev = rt.torch_cuda()
     lib = rt.load_library()
-    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
-                       capture_output=True, text=True)
-    say(f"card: {torch.cuda.get_device_name(dev)} | nvidia-smi: {q.stdout.strip() or q.stderr.strip()}")
+    res = {**card(dev), "ransac": [], "e2e": []}
     say(f"host cores: {os.cpu_count()}, cv.getNumThreads() = {cv.getNumThreads()}, OpenCV {cv.__version__}")
-    res = {"card": torch.cuda.get_device_name(dev), "nvidia_smi": q.stdout.strip(), "ransac": [], "e2e": []}
     say(f"== batched RANSAC: c2 match sets, max_iters {MAX_ITERS}, threshold {THR}")
     for share in (0.17, 0.8):
         for k in (1, 4, 16, 64):
@@ -167,7 +127,7 @@ def main():
             reps = max(3, args.reps // k)
             call = kernel_call(lib, dev, sets)
             call_us = event_us(call, args.reps)
-            kern = profiled_us(call, args.reps)
+            kern = {n: float(np.mean(v)) for n, v in kernel_times([call], name_in(KERNELS), args.reps).items()}
             (batch_ms, batch_min), tails_ms = batch_with_tails(sets, reps)
             loop_ms = host_ms(lambda: [find_homography_ransac(s, d, THR) for s, d in sets], reps)
             cv_ms = host_ms(lambda: [cv.findHomography(s, d, cv.RANSAC, THR) for s, d in sets], reps)
@@ -187,7 +147,7 @@ def main():
                                   "tails_ms": tails_ms, "loop_ms": loop_ms[0], "cv_loop_ms": cv_ms[0],
                                   "equal_loop": eq_loop, "equal_cv": eq_cv})
     for name, k in (("c2", 4), ("c4", 16)):
-        centre, others, raw_c, raw_os = _scene(name, k)
+        centre, others, raw_c, raw_os = synth.make_case(name, k)
         say(f"== end to end: {name} ({centre.shape[1]} x {centre.shape[0]}), centre + {k} others, {len(raw_c)} "
             f"keypoints, mesh 100")
         for mode in ("opencv", "gpu"):
@@ -210,10 +170,7 @@ def main():
             res["e2e"].append({"case": name, "k": k, "ransac": mode, "kp_batch_ms": t_kb[0], "kp_loop_ms": t_kl[0],
                                "stitch_case_ms": t_sc[0], "stitch_loop_ms": t_sl[0], "equal_kp": eq_kp, "equal": eq})
     say(json.dumps(res))
-    if args.out:
-        os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
-        with open(args.out, "w") as f:
-            f.write("\n".join(lines) + "\n")
+    write_out(args.out)
 
 
 if __name__ == "__main__":

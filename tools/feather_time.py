@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Cost of the feather blend (utils.feather_blend, stitch_panorama(blend="feather")).  One run prints:
   - the card's name, power limit and top SM clock (queries only);
-  - on the layer sets of tools/panorama_time.py (the c4-size case, centre + 16; the c2-size case, centre + 4; 64
+  - on the layer sets of timing.LAYER_SETS (the c4-size case, centre + 16; the c2-size case, centre + 4; 64
     synthetic 1920 x 1080 layers), each call preceded by a 256 MiB write that flushes L2:
       the whole apap_feather_blend call by CUDA events, and each of its kernels (k_feather_rows, k_feather_cols,
       k_feather_blend) from torch.profiler in a separate pass, with the bytes each must move over its time against
@@ -16,7 +16,6 @@ import argparse
 import ctypes
 import json
 import os
-import subprocess
 import sys
 import time
 
@@ -28,13 +27,13 @@ import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 from cvx_proj_b200 import _runtime as rt  # noqa: E402
+from cvx_proj_b200 import synth  # noqa: E402
 from cvx_proj_b200.driver import stitch_panorama  # noqa: E402
 from cvx_proj_b200.utils import _layer_descs  # noqa: E402
 from oracle import feather_oracle as fo  # noqa: E402
 from oracle import panorama_oracle as po  # noqa: E402
-from panorama_time import HBM_TBS, case_layers, synthetic_layers  # noqa: E402
-from sift_time import host_ms  # noqa: E402
-from tests.test_case import _scene  # noqa: E402
+from timing import (HBM_TBS, LAYER_SETS, card, clipped_px, event_us, host_ms, kernel_times, l2_flush,  # noqa: E402
+                    name_in, say, write_out)
 
 SHARPNESS = 0.02
 KERNELS = ("k_feather_rows", "k_feather_cols", "k_feather_blend", "k_blend_layers")
@@ -43,12 +42,8 @@ KERNELS = ("k_feather_rows", "k_feather_cols", "k_feather_blend", "k_blend_layer
 def model_bytes(layers, origins, size):
     """Bytes each kernel must move at least: rows read the layer and write 2-byte distances, cols read and write
     them, the blend reads layer and distances and writes the canvas; the mean blend reads layers, writes the canvas."""
-    width, height = size
-    px = 0
-    for t, (x0, y0) in zip(layers, origins):
-        h, w = t.shape[:2]
-        px += max(0, min(x0 + w, width) - max(x0, 0)) * max(0, min(y0 + h, height) - max(y0, 0))
-    canvas = 3 * width * height
+    px = clipped_px(layers, origins, size)
+    canvas = 3 * size[0] * size[1]
     return {"k_feather_rows": 5 * px, "k_feather_cols": 4 * px, "k_feather_blend": 5 * px + canvas,
             "k_blend_layers": 3 * px + canvas, "call": 14 * px + canvas}, px
 
@@ -74,39 +69,6 @@ def calls(lib, dev, layers, origins, size):
     return feather, mean, out_f, out_m, ws_bytes.value
 
 
-def event_us(fn, reps, flush):
-    for _ in range(3):
-        fn()
-    torch.cuda.synchronize()
-    ts = []
-    for _ in range(reps):
-        flush.fill_(1)
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        fn()
-        e1.record()
-        e1.synchronize()
-        ts.append(e0.elapsed_time(e1) * 1e3)
-    return float(np.median(ts)), float(np.min(ts))
-
-
-def profiled_us(fns, reps, flush):
-    """Median device time of every kernel named in KERNELS over ``reps`` flushed calls of each fn."""
-    from torch.profiler import ProfilerActivity, profile
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        for _ in range(reps):
-            for fn in fns:
-                flush.fill_(1)
-                fn()
-        torch.cuda.synchronize()
-    per = {k: [] for k in KERNELS}
-    for ev in prof.events():
-        for k in KERNELS:
-            if k in ev.name and ev.device_type.name == "CUDA":
-                per[k].append(ev.device_time_total if hasattr(ev, "device_time_total") else ev.cuda_time_total)
-    return {k: float(np.median(v)) for k, v in per.items() if v}
-
-
 def opencv_ms(layers_np, origins, size, reps):
     def run():
         blender = cv.detail.FeatherBlender(SHARPNESS)
@@ -124,32 +86,22 @@ def main():
     ap.add_argument("--reps", type=int, default=100)
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
-    lines = []
-
-    def say(s):
-        print(s, flush=True)
-        lines.append(s)
-
     _, dev = rt.torch_cuda()
     lib = rt.load_library()
-    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
-                       capture_output=True, text=True)
-    say(f"card: {torch.cuda.get_device_name(dev)} | nvidia-smi: {q.stdout.strip() or q.stderr.strip()}")
+    res = {**card(dev), "sets": [], "e2e": []}
     say(f"cv2 {cv.__version__}, {os.cpu_count()} host cores, sharpness {SHARPNESS}")
-    res = {"card": torch.cuda.get_device_name(dev), "nvidia_smi": q.stdout.strip(), "sets": [], "e2e": []}
-    flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
+    flush = l2_flush(dev)
     say(f"== every call after a 256 MiB L2-flushing write; whole call by CUDA events over {args.reps} calls (median), "
         f"kernels by torch.profiler over {args.reps} calls (median); bytes: rows 5 B, cols 4 B, blend 5 B per layer "
         f"pixel in the canvas + 3 B per canvas pixel; share of {HBM_TBS} TB/s")
-    sets = [("c4 centre + 16", lambda: case_layers(dev, "c4", 16)), ("c2 centre + 4", lambda: case_layers(dev, "c2", 4)),
-            ("64 synthetic 1920 x 1080", lambda: synthetic_layers(dev))]
-    for name, make in sets:
-        layers, origins, size = make()
+    for name, make in LAYER_SETS:
+        layers, origins, size = make(dev)
         nbytes, px = model_bytes(layers, origins, size)
         feather, mean, out_f, out_m, ws_bytes = calls(lib, dev, layers, origins, size)
         call_us = event_us(feather, args.reps, flush)
         mean_us = event_us(mean, args.reps, flush)
-        kern = profiled_us([feather, mean], args.reps, flush)
+        times = kernel_times([feather, mean], name_in(KERNELS), args.reps, flush)
+        kern = {k: float(np.median(times[k])) for k in KERNELS if k in times}
         layers_np = [t.cpu().numpy() for t in layers]
         t0 = time.perf_counter()
         want = fo.feather_blend(layers_np, origins, size, SHARPNESS)
@@ -178,7 +130,7 @@ def main():
                             "mean_equal_oracle": ok_m})
         del layers, out_f, out_m
     for name, k in (("c4", 16), ("c2", 4)):
-        centre, others, raw_c, raw_os = _scene(name, k)
+        centre, others, raw_c, raw_os = synth.make_case(name, k)
         fe = stitch_panorama(centre, others, raw_c, raw_os, ransac="gpu", blend="feather")
         me = stitch_panorama(centre, others, raw_c, raw_os, ransac="gpu")
         same = fe.final_size == me.final_size and np.array_equal(fe.origins, me.origins)
@@ -188,10 +140,7 @@ def main():
             f"blend='mean' {t_m[0]:.1f} ms (3 reps, medians; same canvas and origins: {same})")
         res["e2e"].append({"case": name, "k": k, "feather_ms": t_f[0], "mean_ms": t_m[0], "same_layout": bool(same)})
     say(json.dumps(res))
-    if args.out:
-        os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
-        with open(args.out, "w") as f:
-            f.write("\n".join(lines) + "\n")
+    write_out(args.out)
 
 
 if __name__ == "__main__":

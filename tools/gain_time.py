@@ -2,7 +2,7 @@
 """Cost of exposure compensation (utils.exposure_gains, the blends with gains, stitch_panorama(exposure="gain")).
 One run prints:
   - the card's name, power limit and top SM clock (queries only);
-  - on the layer sets of tools/feather_time.py (the c4-size case, centre + 16; the c2-size case, centre + 4; 64
+  - on the layer sets of timing.LAYER_SETS (the c4-size case, centre + 16; the c2-size case, centre + 4; 64
     synthetic 1920 x 1080 layers), each call preceded by a 256 MiB write that flushes L2, by CUDA events:
       apap_gain_stats (memset + k_gain_stats) against its floor of 3 B per layer pixel in the canvas at 7.7 TB/s;
       apap_blend_layers and apap_feather_blend with gains against without;
@@ -17,9 +17,7 @@ import argparse
 import ctypes
 import json
 import os
-import subprocess
 import sys
-import time
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -29,25 +27,14 @@ import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 from cvx_proj_b200 import _runtime as rt  # noqa: E402
+from cvx_proj_b200 import synth  # noqa: E402
 from cvx_proj_b200.driver import stitch_panorama  # noqa: E402
 from cvx_proj_b200.utils import _gain_table, _layer_descs, exposure_gains, gain_stats_ints  # noqa: E402
-from feather_time import event_us  # noqa: E402
 from oracle import feather_oracle as fo  # noqa: E402
 from oracle import gain_oracle as go  # noqa: E402
-from panorama_time import HBM_TBS, case_layers, synthetic_layers  # noqa: E402
-from sift_time import host_ms  # noqa: E402
-from tests.test_case import _scene  # noqa: E402
+from timing import HBM_TBS, LAYER_SETS, card, clipped_px, event_us, host_ms, l2_flush, say, write_out  # noqa: E402
 
 SHARPNESS = 0.02
-
-
-def layer_px(layers, origins, size):
-    width, height = size
-    px = 0
-    for t, (x0, y0) in zip(layers, origins):
-        h, w = t.shape[:2]
-        px += max(0, min(x0 + w, width) - max(x0, 0)) * max(0, min(y0 + h, height) - max(y0, 0))
-    return px
 
 
 def calls(lib, dev, layers, origins, size, gains):
@@ -96,27 +83,16 @@ def main():
     ap.add_argument("--reps", type=int, default=50)
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
-    lines = []
-
-    def say(s):
-        print(s, flush=True)
-        lines.append(s)
-
     _, dev = rt.torch_cuda()
     lib = rt.load_library()
-    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
-                       capture_output=True, text=True)
-    say(f"card: {torch.cuda.get_device_name(dev)} | nvidia-smi: {q.stdout.strip() or q.stderr.strip()}")
+    res = {**card(dev), "sets": [], "e2e": []}
     say(f"cv2 {cv.__version__}, {os.cpu_count()} host cores, feather sharpness {SHARPNESS}")
-    res = {"card": torch.cuda.get_device_name(dev), "nvidia_smi": q.stdout.strip(), "sets": [], "e2e": []}
-    flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
+    flush = l2_flush(dev)
     say(f"== every kernel call after a 256 MiB L2-flushing write, CUDA events over {args.reps} calls (median); "
         f"stats floor: 3 B per layer pixel in the canvas at {HBM_TBS} TB/s")
-    sets = [("c4 centre + 16", lambda: case_layers(dev, "c4", 16)), ("c2 centre + 4", lambda: case_layers(dev, "c2", 4)),
-            ("64 synthetic 1920 x 1080", lambda: synthetic_layers(dev))]
-    for name, make in sets:
-        layers, origins, size = make()
-        px = layer_px(layers, origins, size)
+    for name, make in LAYER_SETS:
+        layers, origins, size = make(dev)
+        px = clipped_px(layers, origins, size)
         g = exposure_gains(layers, origins, size)
         fns, stats = calls(lib, dev, layers, origins, size, g)
         us = {k: event_us(fn, args.reps, flush) for k, fn in fns.items()}
@@ -150,7 +126,7 @@ def main():
                             "rel_gap_opencv": rel})
         del layers, stats
     for name, k in (("c4", 16), ("c2", 4)):
-        centre, others, raw_c, raw_os = _scene(name, k)
+        centre, others, raw_c, raw_os = synth.make_case(name, k)
         row = {"case": name, "k": k}
         for blend in ("mean", "feather"):
             for exposure in ("none", "gain"):
@@ -162,10 +138,7 @@ def main():
             f"with gains {row['feather_gain_ms']:.1f} ms")
         res["e2e"].append(row)
     say(json.dumps(res))
-    if args.out:
-        os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
-        with open(args.out, "w") as f:
-            f.write("\n".join(lines) + "\n")
+    write_out(args.out)
 
 
 if __name__ == "__main__":

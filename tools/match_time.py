@@ -2,14 +2,16 @@
 """LAB: device time of the exact matcher (apap_match_nn), 4000 x 4000 x 128, L2 flushed."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 import numpy as np, torch
 from cvx_proj_b200.utils import match_descriptors
+from timing import l2_flush
 dev = torch.device("cuda", 0)
 rng = np.random.default_rng(0)
 for nq, nt in ((4000, 4000), (500, 500), (20000, 20000)):
     t = torch.from_numpy(np.rint(rng.uniform(0, 255, (nt, 128))).astype(np.float32)).to(dev)
     q = torch.from_numpy(np.rint(rng.uniform(0, 255, (nq, 128))).astype(np.float32)).to(dev)
-    flush = torch.zeros(256 << 20, dtype=torch.uint8, device=dev)
+    flush = l2_flush(dev)
     ts = []
     for k in range(10):
         flush.add_(1)

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Cost of the multi-band blend (utils.multiband_blend, stitch_panorama(blend="multiband")).  One run prints:
   - the card's name, power limit and top SM clock (queries only);
-  - on the layer sets of tools/feather_time.py (the c4-size case, centre + 16; the c2-size case, centre + 4; 64
+  - on the layer sets of timing.LAYER_SETS (the c4-size case, centre + 16; the c2-size case, centre + 4; 64
     synthetic 1920 x 1080 layers), each call preceded by a 256 MiB write that flushes L2:
       apap_multiband_blend at 5 bands, without and with gains, by CUDA events (median), against its floor: the layer
       bytes in the canvas read once plus the canvas written, at 7.7 TB/s;
@@ -17,7 +17,6 @@ import ctypes
 import json
 import multiprocessing as mp
 import os
-import subprocess
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -28,15 +27,13 @@ import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 from cvx_proj_b200 import _runtime as rt  # noqa: E402
+from cvx_proj_b200 import synth  # noqa: E402
 from cvx_proj_b200.driver import stitch_panorama  # noqa: E402
 from cvx_proj_b200.utils import _gain_table, _layer_descs, exposure_gains, multiband_blend  # noqa: E402
-from feather_time import event_us  # noqa: E402
-from gain_time import layer_px  # noqa: E402
 from oracle import feather_oracle as fo  # noqa: E402
 from oracle import multiband_oracle as mo  # noqa: E402
-from panorama_time import HBM_TBS, case_layers, synthetic_layers  # noqa: E402
-from sift_time import host_ms  # noqa: E402
-from tests.test_case import _scene  # noqa: E402
+from timing import (HBM_TBS, LAYER_SETS, card, clipped_px, event_us, host_ms, kernel_times, l2_flush,  # noqa: E402
+                    name_in, say, write_out)
 
 BANDS = 5
 KERNELS = ("k_mb_down", "k_mb_band")
@@ -66,20 +63,10 @@ def calls(lib, dev, layers, origins, size, gains):
 
 def kernel_us(fn, reps, flush):
     """Per call, the summed device time of every launch of each kernel in KERNELS (mean over ``reps`` calls)."""
-    from torch.profiler import ProfilerActivity, profile
     fn()
     torch.cuda.synchronize()
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        for _ in range(reps):
-            flush.fill_(1)
-            fn()
-        torch.cuda.synchronize()
-    per = {k: [] for k in KERNELS}
-    for ev in prof.events():
-        for k in KERNELS:
-            if k in ev.name and ev.device_type.name == "CUDA":
-                per[k].append(ev.device_time_total if hasattr(ev, "device_time_total") else ev.cuda_time_total)
-    return {k: float(np.sum(v)) / reps for k, v in per.items() if v}
+    times = kernel_times([fn], name_in(KERNELS), reps, flush)
+    return {k: float(np.sum(times[k])) / reps for k in KERNELS if k in times}
 
 
 def _accumulate(args):
@@ -122,28 +109,17 @@ def main():
     ap.add_argument("--procs", type=int, default=8, help="host processes for the oracle check")
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
-    lines = []
-
-    def say(s):
-        print(s, flush=True)
-        lines.append(s)
-
     _, dev = rt.torch_cuda()
     lib = rt.load_library()
-    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
-                       capture_output=True, text=True)
-    say(f"card: {torch.cuda.get_device_name(dev)} | nvidia-smi: {q.stdout.strip() or q.stderr.strip()}")
+    res = {**card(dev), "sets": [], "e2e": []}
     say(f"cv2 {cv.__version__}, {os.cpu_count()} host cores, bands {BANDS}")
-    res = {"card": torch.cuda.get_device_name(dev), "nvidia_smi": q.stdout.strip(), "sets": [], "e2e": []}
-    flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
+    flush = l2_flush(dev)
     say(f"== every call after a 256 MiB L2-flushing write; CUDA events over {args.reps} calls (median); per kernel: "
         f"torch.profiler, summed over a call's launches; floor: 3 B per layer pixel in the canvas + 3 B per canvas "
         f"pixel at {HBM_TBS} TB/s")
-    sets = [("c4 centre + 16", lambda: case_layers(dev, "c4", 16)), ("c2 centre + 4", lambda: case_layers(dev, "c2", 4)),
-            ("64 synthetic 1920 x 1080", lambda: synthetic_layers(dev))]
-    for name, make in sets:
-        layers, origins, size = make()
-        px = layer_px(layers, origins, size)
+    for name, make in LAYER_SETS:
+        layers, origins, size = make(dev)
+        px = clipped_px(layers, origins, size)
         g = exposure_gains(layers, origins, size)
         fns, outs, ws_bytes = calls(lib, dev, layers, origins, size, g)
         us = {k: event_us(fn, args.reps, flush) for k, fn in fns.items()}
@@ -179,7 +155,7 @@ def main():
                             "opencv_ms": cv_ms, "equal_oracle": ok, "equal_opencv": ok_cv})
         del layers, fns, outs
     for name, k in (("c4", 16), ("c2", 4)):
-        centre, others, raw_c, raw_os = _scene(name, k)
+        centre, others, raw_c, raw_os = synth.make_case(name, k)
         row = {"case": name, "k": k}
         for blend in ("mean", "feather", "multiband"):
             stitch_panorama(centre, others, raw_c, raw_os, ransac="gpu", blend=blend)
@@ -189,10 +165,7 @@ def main():
             f"feather {row['feather_ms']:.1f} ms, multiband {row['multiband_ms']:.1f} ms")
         res["e2e"].append(row)
     say(json.dumps(res))
-    if args.out:
-        os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
-        with open(args.out, "w") as f:
-            f.write("\n".join(lines) + "\n")
+    write_out(args.out)
 
 
 if __name__ == "__main__":

@@ -26,17 +26,8 @@ def timed(fn, reps=3):
 
 
 for name in (sys.argv[1:] or ["c1", "c2"]):
-    sc = synth.make_scene(name)
-    rng = np.random.default_rng(1)
-    img_c = synth.make_image(sc.width, sc.height, seed=2)
     # the other view = the centre image warped by the scene's ground-truth homography (so descriptors do match)
-    img_o = cv.warpPerspective(img_c, np.linalg.inv(sc.h_gt), (sc.width, sc.height))
-    raw_c = sc.dst.astype(np.float32)             # centre-image keypoints; their images under inv(h_gt) in the other view
-    raw_o = cv.perspectiveTransform(raw_c[None].astype(np.float64), np.linalg.inv(sc.h_gt))[0].astype(np.float32)
-    keep = (raw_o[:, 0] > 8) & (raw_o[:, 0] < sc.width - 8) & (raw_o[:, 1] > 8) & (raw_o[:, 1] < sc.height - 8) & \
-           (raw_c[:, 0] > 8) & (raw_c[:, 0] < sc.width - 8) & (raw_c[:, 1] > 8) & (raw_c[:, 1] < sc.height - 8)
-    raw_c, raw_o = raw_c[keep], raw_o[keep]
-    raw_o = raw_o + rng.normal(0, 0.3, raw_o.shape).astype(np.float32)
+    img_c, img_o, raw_c, raw_o = synth.make_pair(name)
     kc = [cv.KeyPoint(float(x), float(y), 1) for x, y in raw_c]
     ko = [cv.KeyPoint(float(x), float(y), 1) for x, y in raw_o]
     ext = cv.SIFT.create(nfeatures=128)
@@ -50,7 +41,7 @@ for name in (sys.argv[1:] or ["c1", "c2"]):
     src = np.float32([kc2[m.queryIdx].pt for m in m_flann])
     dst = np.float32([ko2[m.trainIdx].pt for m in m_flann])
     t_ransac, (h, mask) = timed(lambda: cv.findHomography(src, dst, cv.RANSAC, 5.0), reps=5)
-    print(f"{name}: {sc.width}x{sc.height}, {len(kc)} keypoints given (size 1, as the reference builds them)")
+    print(f"{name}: {img_c.shape[1]}x{img_c.shape[0]}, {len(kc)} keypoints given (size 1, as the reference builds them)")
     print(f"  SIFT.compute at the given keypoints     {t_desc:9.1f} ms per image (Gaussian pyramid of the whole image + 128-d descriptors)")
     print(f"  FlannBasedMatcher().match (reference)   {t_flann:9.1f} ms   {len(m_flann)} matches")
     print(f"  BFMatcher(NORM_L2).match  (exact 1-NN)  {t_bf:9.1f} ms   FLANN agrees with the exact neighbour on {same} of {len(m_bf)} "

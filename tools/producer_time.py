@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Cost of the histogram equalisation (csrc/equalize.cu) and of the array-level keypoint-pair producer
-(utils.keypoint_pairs) at the bench shape c2 (3840 x 2160, the tools/sift_time.py pair).  One run prints:
+(utils.keypoint_pairs) at the bench shape c2 (3840 x 2160, synth.make_pair("c2")).  One run prints:
   - the card's name and power limit (queries only);
   - k_eq_hist, k_eq_lut and k_eq_apply from torch.profiler, the L2 flushed by a 256 MiB write before every launch, with
     bytes over time against the data-sheet HBM bandwidth; k_eq_hist again on a flat image (every byte of a channel in
@@ -16,7 +16,6 @@
 import argparse
 import json
 import os
-import subprocess
 import sys
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -26,9 +25,10 @@ import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 from cvx_proj_b200 import _runtime as rt  # noqa: E402
+from cvx_proj_b200 import synth  # noqa: E402
 from cvx_proj_b200.utils import (coarse_matching, equalize_hist, keypoint_pairs, sift_describe,  # noqa: E402
                                  sift_sample_table)
-from sift_time import HBM_TBPS, c2_pair, host_ms  # noqa: E402
+from timing import HBM_TBS, card, host_ms, kernel_times, l2_flush  # noqa: E402
 
 
 def cv_equalize(img):
@@ -44,20 +44,9 @@ def kernel_name(key):
     return None
 
 
-def profiled(fn, flush, reps=50):
-    """{kernel: mean device us} of ``reps`` launches of ``fn``, each after an L2 flush."""
-    from torch.profiler import ProfilerActivity, profile
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        for _ in range(reps):
-            flush.fill_(1)
-            fn()
-        torch.cuda.synchronize()
-    out = {}
-    for e in prof.key_averages():
-        n = kernel_name(e.key)
-        if n:
-            out[n] = (getattr(e, "device_time_total", None) or e.cuda_time_total) / max(e.count, 1)
-    return out
+def profiled(fns, flush, reps=50):
+    """{kernel: mean device us per launch} of ``reps`` rounds over ``fns``, each call after an L2 flush."""
+    return {n: float(np.mean(v)) for n, v in kernel_times(fns, kernel_name, reps, flush).items()}
 
 
 def main():
@@ -66,18 +55,16 @@ def main():
     args = ap.parse_args()
     torch_, dev = rt.torch_cuda()
     lib = rt.load_library()
-    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
-                       capture_output=True, text=True)
-    print(f"card: {torch.cuda.get_device_name(dev)} | nvidia-smi: {q.stdout.strip() or q.stderr.strip()}")
-    img_c, img_o, raw_c, raw_o = c2_pair()
+    res = card(dev)
+    img_c, img_o, raw_c, raw_o = synth.make_pair("c2")
     h, w = img_c.shape[:2]
     px = h * w
     k = len(raw_c)
     print(f"c2: {w}x{h} ({3 * px / 1e6:.1f} MB per image), {k} keypoints")
-    res = {"card": torch.cuda.get_device_name(dev), "nvidia_smi": q.stdout.strip(), "w": w, "h": h, "keypoints": k}
+    res.update(w=w, h=h, keypoints=k)
 
     st = rt.stream_ptr(torch_, dev)
-    flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
+    flush = l2_flush(dev)
     d_img = torch.from_numpy(img_c).to(dev)
     d_flat = torch.full_like(d_img, 128)
     hist = torch.empty(768, dtype=torch.int32, device=dev)
@@ -91,6 +78,8 @@ def main():
         eq(d_img, out.data_ptr())
         eq(d_flat, None)
     torch.cuda.synchronize()
+    # All launches are queued and their events read after one synchronise.  A synchronise after every call, as
+    # timing.event_us does, adds about 0.9 us to the median of these 20-35 us calls (measured on a B200 at 1000 W).
     for label, fn in (("apap_equalize_hist (hist + LUT)", lambda: eq(d_img, None)),
                       ("apap_equalize_hist (hist + LUT + apply)", lambda: eq(d_img, out.data_ptr()))):
         evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(args.iters)]
@@ -104,17 +93,17 @@ def main():
         print(f"{label} device time (L2 flushed, {args.iters} launches): median {np.median(us):.1f} us, min {us.min():.1f} us")
         res["eq_call_us" if "apply" not in label else "eq_call_apply_us"] = float(np.median(us))
 
-    floor = lambda b: b / (HBM_TBPS * 1e12) * 1e6  # noqa: E731
-    kern = profiled(lambda: eq(d_img, out.data_ptr()), flush)
+    floor = lambda b: b / (HBM_TBS * 1e12) * 1e6  # noqa: E731
+    kern = profiled([lambda: eq(d_img, out.data_ptr())], flush)
     for name, nbytes, what in (("k_eq_hist", 3 * px, "3 px read"), ("k_eq_lut", 768 * 4 + 768, "hist read + LUT written"),
                                ("k_eq_apply", 6 * px, "3 px read + 3 px written")):
         if name in kern:
             t = kern[name]
             gbs = nbytes / (t * 1e-6) / 1e9
             print(f"{name} (profiler, 50 launches): {t:.2f} us; {nbytes / 1e6:.3g} MB ({what}) -> {gbs:.0f} GB/s = "
-                  f"{gbs / (HBM_TBPS * 1e3) * 100:.1f} % of {HBM_TBPS} TB/s (floor {floor(nbytes):.2f} us)")
+                  f"{gbs / (HBM_TBS * 1e3) * 100:.1f} % of {HBM_TBS} TB/s (floor {floor(nbytes):.2f} us)")
             res[f"{name}_us"] = t
-    kflat = profiled(lambda: eq(d_flat, None), flush)
+    kflat = profiled([lambda: eq(d_flat, None)], flush)
     if "k_eq_hist" in kflat:
         t = kflat["k_eq_hist"]
         print(f"k_eq_hist on a flat image (every byte of a channel in one bin): {t:.2f} us = "
@@ -128,15 +117,17 @@ def main():
     desc = torch.empty((k, 128), dtype=torch.float32, device=dev)
     eq(d_img, None)
 
-    def both():
+    def plain():
         rt.check(lib.apap_sift_describe(d_img.data_ptr(), h, w, d_pts.data_ptr(), k, d_tab.data_ptr(), table.shape[0],
                                         float(ori), base.data_ptr(), desc.data_ptr(), st), "apap_sift_describe")
-        flush.fill_(1)
+
+    def through_lut():
         rt.check(lib.apap_sift_describe_lut(d_img.data_ptr(), h, w, lut.data_ptr(), d_pts.data_ptr(), k, d_tab.data_ptr(),
                                             table.shape[0], float(ori), base.data_ptr(), desc.data_ptr(), st),
                  "apap_sift_describe_lut")
-    both()
-    kb = profiled(both, flush)
+    plain()
+    through_lut()
+    kb = profiled([plain, through_lut], flush)
     if "k_sift_base" in kb and "k_sift_base_lut" in kb:
         print(f"k_sift_base (profiler, 50 launches each, alternating): plain {kb['k_sift_base']:.1f} us, through the LUT "
               f"{kb['k_sift_base_lut']:.1f} us")

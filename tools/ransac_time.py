@@ -1,6 +1,6 @@
 #!/usr/bin/env python
-"""Cost of the GPU RANSAC (csrc/ransac.cu, utils.find_homography_ransac) at the bench shape c2 (3840 x 2160, the
-tools/sift_time.py pair).  The match set is the exact matcher's on that pair (what keypoint_pairs hands to RANSAC);
+"""Cost of the GPU RANSAC (csrc/ransac.cu, utils.find_homography_ransac) at the bench shape c2 (3840 x 2160,
+synth.make_pair("c2")).  The match set is the exact matcher's on that pair (what keypoint_pairs hands to RANSAC);
 for the higher outlier shares a seeded part of its targets is replaced by uniform noise over the image.  One run
 prints:
   - the card's name, power limit and top SM clock (queries only);
@@ -15,7 +15,6 @@ import argparse
 import ctypes
 import json
 import os
-import subprocess
 import sys
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -25,9 +24,10 @@ import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 from cvx_proj_b200 import _runtime as rt  # noqa: E402
+from cvx_proj_b200 import synth  # noqa: E402
 from cvx_proj_b200.utils import (find_homography_ransac, keypoint_pairs, match_descriptors,  # noqa: E402
                                  sift_describe)
-from sift_time import c2_pair, host_ms  # noqa: E402
+from timing import card, event_us, host_ms, kernel_times, name_in, say, write_out  # noqa: E402
 
 KERNELS = ("k_ransac_sample", "k_ransac_fit", "k_ransac_score")
 MAX_ITERS = 2000
@@ -49,26 +49,18 @@ def main():
     ap.add_argument("--reps", type=int, default=50)
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
-    lines = []
-
-    def say(s):
-        print(s, flush=True)
-        lines.append(s)
-
     torch_, dev = rt.torch_cuda()
     lib = rt.load_library()
-    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
-                       capture_output=True, text=True)
-    say(f"card: {torch.cuda.get_device_name(dev)} | nvidia-smi: {q.stdout.strip() or q.stderr.strip()}")
+    res = card(dev)
     say(f"host cores: {os.cpu_count()}, cv.getNumThreads() = {cv.getNumThreads()}, OpenCV {cv.__version__}")
-    img_c, img_o, raw_c, raw_o = c2_pair()
+    img_c, img_o, raw_c, raw_o = synth.make_pair("c2")
     idx, _ = match_descriptors(sift_describe(img_c, raw_c, equalize=True), sift_describe(img_o, raw_o, equalize=True))
     qi = np.flatnonzero(idx >= 0)
     centre, other0 = raw_c[qi], raw_o[idx[qi]]
     n = len(centre)
     wrong = int(np.sum(idx[qi] != qi))
     say(f"c2: {n} matches, {wrong} ({100 * wrong / n:.0f} %) not the generating pair")
-    res = {"card": torch.cuda.get_device_name(dev), "nvidia_smi": q.stdout.strip(), "matches": n, "cases": []}
+    res.update(matches=n, cases=[])
     st = rt.stream_ptr(torch_, dev)
     nb = ctypes.c_size_t()
     rt.check(lib.apap_ransac_workspace_bytes(MAX_ITERS, ctypes.byref(nb)), "apap_ransac_workspace_bytes")
@@ -92,29 +84,10 @@ def main():
             rt.check(lib.apap_ransac_homography(s_dev.data_ptr(), d_dev.data_ptr(), n, 5.0, MAX_ITERS, ws.data_ptr(),
                                                 nb.value, sub.data_ptr(), hyps.data_ptr(), cnt.data_ptr(),
                                                 ns.data_ptr(), st), "apap_ransac_homography")
-        for _ in range(5):
-            call()
-        torch.cuda.synchronize()
-        ts = []
-        for _ in range(args.reps):
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record()
-            call()
-            e1.record()
-            e1.synchronize()
-            ts.append(e0.elapsed_time(e1) * 1e3)
+        call_us = event_us(call, args.reps, warmup=5)
         n_s = int(ns.item())
         its = iterations_run(cnt.cpu().numpy(), n_s, n)
-        from torch.profiler import ProfilerActivity, profile
-        with profile(activities=[ProfilerActivity.CUDA]) as prof:
-            for _ in range(args.reps):
-                call()
-            torch.cuda.synchronize()
-        kern = {}
-        for e in prof.key_averages():
-            for name in KERNELS:
-                if name in e.key:
-                    kern[name] = (getattr(e, "device_time_total", None) or e.cuda_time_total) / max(e.count, 1)
+        kern = {k: float(np.mean(v)) for k, v in kernel_times([call], name_in(KERNELS), args.reps).items()}
         want = cv.findHomography(centre, other, cv.RANSAC, 5.0)
         got = find_homography_ransac(centre, other, 5.0)
         same = np.array_equal(got[0], want[0]) and np.array_equal(got[1], want[1])
@@ -124,15 +97,15 @@ def main():
                            args.reps)
         inl = int(got[1].sum())
         say(f"{label}: {inl} inliers, OpenCV's loop runs {its} of {n_s} sampled hypotheses")
-        say(f"  apap_ransac_homography device time (CUDA events, {args.reps} calls): median {np.median(ts):.1f} us, "
-            f"min {np.min(ts):.1f} us")
+        say(f"  apap_ransac_homography device time (CUDA events, {args.reps} calls): median {call_us[0]:.1f} us, "
+            f"min {call_us[1]:.1f} us")
         say("  " + ", ".join(f"{k} {kern.get(k, float('nan')):.1f} us" for k in KERNELS) +
             f" (profiler, {args.reps} calls)")
         say(f"  find_homography_ransac host to host: median {gpu_ms[0]:.3f} ms (min {gpu_ms[1]:.3f}); "
             f"cv.findHomography(RANSAC): median {cv_ms[0]:.3f} ms (min {cv_ms[1]:.3f}); "
             f"of which the refit cv.findHomography(inliers, 0): {refit_ms[0]:.3f} ms; equal: {same}")
         res["cases"].append({"case": label, "inliers": inl, "iterations": its, "sampled": n_s,
-                             "call_us": float(np.median(ts)), **{k + "_us": v for k, v in kern.items()},
+                             "call_us": call_us[0], **{k + "_us": v for k, v in kern.items()},
                              "gpu_h2h_ms": gpu_ms[0], "cv_ms": cv_ms[0], "refit_ms": refit_ms[0], "equal": bool(same)})
     for mode in ("opencv", "gpu"):
         keypoint_pairs(img_c, img_o, raw_c, raw_o, ransac=mode)
@@ -140,10 +113,7 @@ def main():
         say(f"keypoint_pairs(ransac={mode!r}) host to host: median {t[0]:.2f} ms, min {t[1]:.2f} ms")
         res[f"keypoint_pairs_{mode}_ms"] = t[0]
     say(json.dumps(res))
-    if args.out:
-        os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
-        with open(args.out, "w") as f:
-            f.write("\n".join(lines) + "\n")
+    write_out(args.out)
 
 
 if __name__ == "__main__":
