@@ -70,12 +70,19 @@ SIGNATURES = {
                                        c_void_p]),
     "apap_feather_blend_gain": (c_int, [POINTER(ctypes.c_longlong), c_int, c_int, c_int, c_float, c_void_p, c_void_p,
                                         c_size_t, c_void_p, c_size_t, c_void_p]),
+    "apap_channel_stats": (c_int, [POINTER(ctypes.c_longlong), c_int, c_int, c_int, c_void_p, c_size_t, c_void_p]),
+    "apap_blend_layers_channels": (c_int, [POINTER(ctypes.c_longlong), c_int, c_int, c_int, c_void_p, c_void_p,
+                                           c_size_t, c_void_p]),
+    "apap_feather_blend_channels": (c_int, [POINTER(ctypes.c_longlong), c_int, c_int, c_int, c_float, c_void_p,
+                                            c_void_p, c_size_t, c_void_p, c_size_t, c_void_p]),
     "apap_multiband_workspace_bytes": (c_int, [POINTER(ctypes.c_longlong), c_int, c_int, c_int, c_int,
                                                POINTER(c_size_t)]),
     "apap_multiband_blend": (c_int, [POINTER(ctypes.c_longlong), c_int, c_int, c_int, c_int, c_void_p, c_size_t,
                                      c_void_p, c_size_t, c_void_p]),
     "apap_multiband_blend_gain": (c_int, [POINTER(ctypes.c_longlong), c_int, c_int, c_int, c_int, c_void_p, c_void_p,
                                           c_size_t, c_void_p, c_size_t, c_void_p]),
+    "apap_multiband_blend_channels": (c_int, [POINTER(ctypes.c_longlong), c_int, c_int, c_int, c_int, c_void_p,
+                                              c_void_p, c_size_t, c_void_p, c_size_t, c_void_p]),
     "apap_pipe_probe": (c_int, [c_int, c_int, c_void_p, POINTER(c_double), c_void_p]),
     "apap_warp_perspective": (c_int, [c_void_p, c_int, c_int, POINTER(c_double), c_void_p, c_int, c_int, c_void_p, c_int,
                                       c_int, c_int, c_int, c_int, c_void_p]),

@@ -11,6 +11,7 @@
 // The segment's bytes are staged in shared memory and leave as aligned 16-byte stores plus a byte-wise head and tail.
 // kGains (apap_blend_layers_gain): layer l's bytes go through its exposure-gain table lut[l][256] before they are
 // summed; the non-empty test still reads the raw bytes, and compensated bytes are <= 255, so the bound above holds.
+// kChannels (apap_blend_layers_channels): the table is lut[l][3][256], one row per channel.
 #include "layers.cuh"
 
 namespace apap {
@@ -21,7 +22,7 @@ struct LayerParams {
   int n_layers, canvas_h, canvas_w, segs_per_row;
 };
 
-template <bool kGains>
+template <bool kGains, bool kChannels>
 __global__ void __launch_bounds__(kLayerThreads) k_blend_layers(const __grid_constant__ LayerParams p,
                                                                 const uint8_t *__restrict__ lut) {
   __shared__ uint32_t recip[APAP_BLEND_MAX_LAYERS + 1];
@@ -41,7 +42,8 @@ __global__ void __launch_bounds__(kLayerThreads) k_blend_layers(const __grid_con
     uint32_t w[3];
     fetch_group(p.layer[l], y, seg0, seg_px, x, n_px, w);
     uint32_t v[3] = {w[0], w[1], w[2]};
-    if constexpr (kGains) gain_group(lut + 256 * l, v);
+    if constexpr (kGains && kChannels) gain_group<true>(lut + 768 * l, v);
+    else if constexpr (kGains) gain_group<false>(lut + 256 * l, v);
     s[0] += __byte_perm(v[0], 0u, 0x4140); s[1] += __byte_perm(v[0], 0u, 0x4342);
     s[2] += __byte_perm(v[1], 0u, 0x4140); s[3] += __byte_perm(v[1], 0u, 0x4342);
     s[4] += __byte_perm(v[2], 0u, 0x4140); s[5] += __byte_perm(v[2], 0u, 0x4342);
@@ -90,8 +92,9 @@ __global__ void __launch_bounds__(kLayerThreads) k_blend_layers(const __grid_con
   }
 }
 
+// lut: none (nullptr), [n][256] or (channels) [n][3][256]
 int launch_blend_layers(const long long *layers, int n_layers, int canvas_h, int canvas_w, const uint8_t *lut,
-                        uint8_t *out, cudaStream_t st) {
+                        bool channels, uint8_t *out, cudaStream_t st) {
   LayerParams p;
   for (int l = 0; l < n_layers; ++l) p.layer[l] = layer_desc(layers + 6 * l);
   p.out = out;
@@ -101,8 +104,9 @@ int launch_blend_layers(const long long *layers, int n_layers, int canvas_h, int
   p.segs_per_row = (canvas_w + kSegPx - 1) / kSegPx;
   const long long blocks = (long long)p.segs_per_row * canvas_h;
   if (blocks > 2147483647LL) return fail(APAP_E_TOOBIG, "blend_layers: canvas too large");
-  if (lut) k_blend_layers<true><<<(unsigned)blocks, kLayerThreads, 0, st>>>(p, lut);
-  else k_blend_layers<false><<<(unsigned)blocks, kLayerThreads, 0, st>>>(p, nullptr);
+  if (lut && channels) k_blend_layers<true, true><<<(unsigned)blocks, kLayerThreads, 0, st>>>(p, lut);
+  else if (lut) k_blend_layers<true, false><<<(unsigned)blocks, kLayerThreads, 0, st>>>(p, lut);
+  else k_blend_layers<false, false><<<(unsigned)blocks, kLayerThreads, 0, st>>>(p, nullptr);
   return check_cuda(cudaGetLastError(), "k_blend_layers launch");
 }
 
@@ -128,12 +132,20 @@ int check_blend_layers(const long long *layers, int n_layers, int canvas_h, int 
 extern "C" int apap_blend_layers(const long long *layers, int n_layers, int canvas_h, int canvas_w, uint8_t *out,
                                  size_t out_bytes, void *stream) {
   if (int rc = check_blend_layers(layers, n_layers, canvas_h, canvas_w, out, out_bytes)) return rc;
-  return launch_blend_layers(layers, n_layers, canvas_h, canvas_w, nullptr, out, static_cast<cudaStream_t>(stream));
+  return launch_blend_layers(layers, n_layers, canvas_h, canvas_w, nullptr, false, out,
+                             static_cast<cudaStream_t>(stream));
 }
 
 extern "C" int apap_blend_layers_gain(const long long *layers, int n_layers, int canvas_h, int canvas_w,
                                       const uint8_t *lut, uint8_t *out, size_t out_bytes, void *stream) {
   if (!lut) return fail(APAP_E_BADARG, "blend_layers_gain: null gain table");
   if (int rc = check_blend_layers(layers, n_layers, canvas_h, canvas_w, out, out_bytes)) return rc;
-  return launch_blend_layers(layers, n_layers, canvas_h, canvas_w, lut, out, static_cast<cudaStream_t>(stream));
+  return launch_blend_layers(layers, n_layers, canvas_h, canvas_w, lut, false, out, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int apap_blend_layers_channels(const long long *layers, int n_layers, int canvas_h, int canvas_w,
+                                          const uint8_t *lut, uint8_t *out, size_t out_bytes, void *stream) {
+  if (!lut) return fail(APAP_E_BADARG, "blend_layers_channels: null gain table");
+  if (int rc = check_blend_layers(layers, n_layers, canvas_h, canvas_w, out, out_bytes)) return rc;
+  return launch_blend_layers(layers, n_layers, canvas_h, canvas_w, lut, true, out, static_cast<cudaStream_t>(stream));
 }

@@ -17,7 +17,8 @@
 //   k_feather_blend one CTA per kSegPx-pixel canvas row segment, 4 pixels per thread (layers.cuh): a layer that does
 //                   not cover the segment adds exactly +0.0f and 0 and is skipped (uniform test).  kGains
 //                   (apap_feather_blend_gain): layer l's bytes go through its exposure-gain table lut[l][256]
-//                   first; the distances, made from the raw bytes, are unchanged.
+//                   first; the distances, made from the raw bytes, are unchanged.  kChannels
+//                   (apap_feather_blend_channels): the table is lut[l][3][256], one row per channel.
 // Distances are stored as min(D, cap) (apap_feather_distance_cap): cap is either the smallest integer with
 // fl(cap s) >= 1 -- float multiplication by s > 0 is monotone, so every D >= cap has weight 1 -- or, when that is
 // larger, W + H - 1, more than any finite distance in the canvas, so that only a layer with no empty pixel in the
@@ -201,7 +202,7 @@ __global__ void __launch_bounds__(kColThreadsX * kColSegs) k_feather_cols(const 
   }
 }
 
-template <bool kGains>
+template <bool kGains, bool kChannels>
 __global__ void __launch_bounds__(kLayerThreads) k_feather_blend(const __grid_constant__ FeatherParams p,
                                                                  const uint8_t *__restrict__ lut) {
   __shared__ __align__(16) uint32_t stage[kSegBytes / 4];
@@ -223,7 +224,8 @@ __global__ void __launch_bounds__(kLayerThreads) k_feather_blend(const __grid_co
     if ((unsigned)r >= (unsigned)R.ch || seg0 + seg_px <= R.cx0 || seg0 >= R.cx0 + R.cw) continue;   // uniform
     uint32_t v[3];
     fetch_group(p.layer[l], y, seg0, seg_px, x, n_px, v);
-    if constexpr (kGains) gain_group(lut + 256 * l, v);
+    if constexpr (kGains && kChannels) gain_group<true>(lut + 768 * l, v);
+    else if constexpr (kGains) gain_group<false>(lut + 256 * l, v);
     const uint16_t *row = R.dist + (size_t)r * (size_t)R.cw;
 #pragma unroll
     for (int k = 0; k < kLayerGroupPx; ++k) {
@@ -331,8 +333,9 @@ extern "C" int apap_feather_workspace_bytes(const long long *layers, int n_layer
   return 0;
 }
 
+// lut: none (nullptr), [n][256] or (channels) [n][3][256]
 static int feather_blend(const long long *layers, int n_layers, int canvas_h, int canvas_w, float sharpness,
-                         const uint8_t *lut, void *workspace, size_t workspace_bytes, uint8_t *out,
+                         const uint8_t *lut, bool channels, void *workspace, size_t workspace_bytes, uint8_t *out,
                          size_t out_bytes, cudaStream_t st) {
   if (!out || !workspace) return fail(APAP_E_BADARG, "feather_blend: null pointer");
   if (int rc = check_layers(layers, n_layers, canvas_h, canvas_w)) return rc;
@@ -370,15 +373,16 @@ static int feather_blend(const long long *layers, int n_layers, int canvas_h, in
                      dim3(kColThreadsX, kColSegs), 0, st>>>(p);
     if (int rc = check_cuda(cudaGetLastError(), "k_feather_cols launch")) return rc;
   }
-  if (lut) k_feather_blend<true><<<(unsigned)blocks, kLayerThreads, 0, st>>>(p, lut);
-  else k_feather_blend<false><<<(unsigned)blocks, kLayerThreads, 0, st>>>(p, nullptr);
+  if (lut && channels) k_feather_blend<true, true><<<(unsigned)blocks, kLayerThreads, 0, st>>>(p, lut);
+  else if (lut) k_feather_blend<true, false><<<(unsigned)blocks, kLayerThreads, 0, st>>>(p, lut);
+  else k_feather_blend<false, false><<<(unsigned)blocks, kLayerThreads, 0, st>>>(p, nullptr);
   return check_cuda(cudaGetLastError(), "k_feather_blend launch");
 }
 
 extern "C" int apap_feather_blend(const long long *layers, int n_layers, int canvas_h, int canvas_w, float sharpness,
                                   void *workspace, size_t workspace_bytes, uint8_t *out, size_t out_bytes,
                                   void *stream) {
-  return feather_blend(layers, n_layers, canvas_h, canvas_w, sharpness, nullptr, workspace, workspace_bytes, out,
+  return feather_blend(layers, n_layers, canvas_h, canvas_w, sharpness, nullptr, false, workspace, workspace_bytes, out,
                        out_bytes, static_cast<cudaStream_t>(stream));
 }
 
@@ -386,6 +390,14 @@ extern "C" int apap_feather_blend_gain(const long long *layers, int n_layers, in
                                        float sharpness, const uint8_t *lut, void *workspace, size_t workspace_bytes,
                                        uint8_t *out, size_t out_bytes, void *stream) {
   if (!lut) return fail(APAP_E_BADARG, "feather_blend_gain: null gain table");
-  return feather_blend(layers, n_layers, canvas_h, canvas_w, sharpness, lut, workspace, workspace_bytes, out,
+  return feather_blend(layers, n_layers, canvas_h, canvas_w, sharpness, lut, false, workspace, workspace_bytes, out,
+                       out_bytes, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int apap_feather_blend_channels(const long long *layers, int n_layers, int canvas_h, int canvas_w,
+                                           float sharpness, const uint8_t *lut, void *workspace,
+                                           size_t workspace_bytes, uint8_t *out, size_t out_bytes, void *stream) {
+  if (!lut) return fail(APAP_E_BADARG, "feather_blend_channels: null gain table");
+  return feather_blend(layers, n_layers, canvas_h, canvas_w, sharpness, lut, true, workspace, workspace_bytes, out,
                        out_bytes, static_cast<cudaStream_t>(stream));
 }

@@ -14,6 +14,11 @@
 // every thread's 4-bit mask of each in shared memory.  Then per ordered pair (a, b) of those layers that meets in
 // the segment (a second vote): the count (a <= b) and the limb sums of norm(P_a) over the intersection (a != b),
 // reduced per warp, then per CTA by thread 0, which adds them to global memory (fire-and-forget reductions).
+//
+// kChannels (apap_channel_stats, cv.detail.ChannelsCompensator): the three limbs of a pixel are its three channel
+// bytes instead, and the sums are per channel.  A thread sums at most 4 bytes per channel (< 2^10), a warp < 2^15,
+// the CTA < 2^18, so each CTA total goes to global memory as one 64-bit add per channel: at most 2^31 CTAs keep every
+// word below 2^49, and the words again do not depend on the schedule.
 #include "layers.cuh"
 
 namespace apap {
@@ -25,10 +30,11 @@ constexpr int kWarps = kLayerThreads / 32;
 struct GainStatsParams {
   LayerDesc layer[APAP_GAIN_MAX_LAYERS];
   unsigned long long *count;            // [n][n], i <= j
-  unsigned long long *sum;              // [3][n][n], i != j: 32-bit pieces of the exact sum
+  unsigned long long *sum;              // [3][n][n], i != j: 32-bit pieces of the exact sum (kChannels: channel sums)
   int n_layers, canvas_w, segs_per_row;
 };
 
+template <bool kChannels>
 __global__ void __launch_bounds__(kLayerThreads) k_gain_stats(const __grid_constant__ GainStatsParams p) {
   __shared__ uint8_t nib[APAP_GAIN_MAX_LAYERS / 2][kLayerThreads];   // 4-bit masks, two present layers per byte
   __shared__ short present[APAP_GAIN_MAX_LAYERS];
@@ -63,21 +69,29 @@ __global__ void __launch_bounds__(kLayerThreads) k_gain_stats(const __grid_const
     uint32_t w[3];
     fetch_group(p.layer[la], y, seg0, seg_px, x, n_px, w);
     const uint32_t ma = (nib[a >> 1][threadIdx.x] >> (4 * (a & 1))) & 15u;
-    uint32_t limb[3][kLayerGroupPx];            // sqrt(q) 2^52 in 25-bit limbs, 0 where empty
+    uint32_t limb[3][kLayerGroupPx];            // sqrt(q) 2^52 in 25-bit limbs (kChannels: the bytes), 0 where empty
 #pragma unroll
     for (int k = 0; k < kLayerGroupPx; ++k) {
-      uint32_t q = 0u;
+      if constexpr (kChannels) {
 #pragma unroll
-      for (int c = 0; c < 3; ++c) {
-        const int b = 3 * k + c;
-        const uint32_t v = (w[b >> 2] >> (8 * (b & 3))) & 0xffu;
-        q += v * v;
+        for (int c = 0; c < 3; ++c) {
+          const int b = 3 * k + c;
+          limb[c][k] = (w[b >> 2] >> (8 * (b & 3))) & 0xffu;
+        }
+      } else {
+        uint32_t q = 0u;
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+          const int b = 3 * k + c;
+          const uint32_t v = (w[b >> 2] >> (8 * (b & 3))) & 0xffu;
+          q += v * v;
+        }
+        const unsigned long long e =
+            q ? __double2ull_rn(__dmul_rn(__dsqrt_rn((double)q), 4503599627370496.0)) : 0ull;   // x 2^52, exact
+        limb[0][k] = (uint32_t)(e & kLimbMask);
+        limb[1][k] = (uint32_t)((e >> kLimbBits) & kLimbMask);
+        limb[2][k] = (uint32_t)(e >> (2 * kLimbBits));
       }
-      const unsigned long long e =
-          q ? __double2ull_rn(__dmul_rn(__dsqrt_rn((double)q), 4503599627370496.0)) : 0ull;   // x 2^52, exact
-      limb[0][k] = (uint32_t)(e & kLimbMask);
-      limb[1][k] = (uint32_t)((e >> kLimbBits) & kLimbMask);
-      limb[2][k] = (uint32_t)(e >> (2 * kLimbBits));
     }
     for (int b = 0; b < m; ++b) {
       const uint32_t inter = ma & (nib[b >> 1][threadIdx.x] >> (4 * (b & 1))) & 15u;
@@ -111,13 +125,20 @@ __global__ void __launch_bounds__(kLayerThreads) k_gain_stats(const __grid_const
         const int lb = present[b];
         if (a <= b) atomicAdd(p.count + (size_t)la * n + lb, t[3]);
         if (a != b) {
-          const unsigned __int128 total = (unsigned __int128)t[0] + ((unsigned __int128)t[1] << kLimbBits) +
-                                          ((unsigned __int128)t[2] << (2 * kLimbBits));
-          const size_t plane = (size_t)n * n, at = (size_t)la * n + lb;
+          if constexpr (kChannels) {
+            const size_t plane = (size_t)n * n, at = (size_t)la * n + lb;
 #pragma unroll
-          for (int i = 0; i < 3; ++i) {
-            const unsigned long long piece = (unsigned long long)(total >> (32 * i)) & 0xffffffffull;
-            if (piece) atomicAdd(p.sum + i * plane + at, piece);
+            for (int i = 0; i < 3; ++i)
+              if (t[i]) atomicAdd(p.sum + i * plane + at, t[i]);
+          } else {
+            const unsigned __int128 total = (unsigned __int128)t[0] + ((unsigned __int128)t[1] << kLimbBits) +
+                                            ((unsigned __int128)t[2] << (2 * kLimbBits));
+            const size_t plane = (size_t)n * n, at = (size_t)la * n + lb;
+#pragma unroll
+            for (int i = 0; i < 3; ++i) {
+              const unsigned long long piece = (unsigned long long)(total >> (32 * i)) & 0xffffffffull;
+              if (piece) atomicAdd(p.sum + i * plane + at, piece);
+            }
           }
         }
       }
@@ -125,15 +146,56 @@ __global__ void __launch_bounds__(kLayerThreads) k_gain_stats(const __grid_const
   }
 }
 
-int check_gain_layers(const long long *layers, int n_layers, int canvas_h, int canvas_w) {
-  if (!layers) return fail(APAP_E_BADARG, "gain_stats: null pointer");
-  if (int rc = check_layer_count_canvas("gain_stats", n_layers, APAP_GAIN_MAX_LAYERS, "APAP_GAIN_MAX_LAYERS", canvas_h,
+int check_gain_layers(const char *what, const long long *layers, int n_layers, int canvas_h, int canvas_w) {
+  char msg[160];
+  if (!layers) {
+    snprintf(msg, sizeof(msg), "%s: null pointer", what);
+    return fail(APAP_E_BADARG, msg);
+  }
+  if (int rc = check_layer_count_canvas(what, n_layers, APAP_GAIN_MAX_LAYERS, "APAP_GAIN_MAX_LAYERS", canvas_h,
                                         canvas_w))
     return rc;
-  return check_layer_descs("gain_stats", layers, n_layers);
+  return check_layer_descs(what, layers, n_layers);
 }
 
 size_t gain_stats_bytes(int n_layers) { return (size_t)4 * n_layers * n_layers * sizeof(unsigned long long); }
+
+// apap_gain_stats (kChannels false) and apap_channel_stats: the checks, one memset and one launch; messages start
+// with `what`
+template <bool kChannels>
+int overlap_stats(const char *what, const long long *layers, int n_layers, int canvas_h, int canvas_w, void *stats,
+                  size_t stats_bytes, cudaStream_t st) {
+  char msg[160];
+  const char *err = nullptr;
+  int code = APAP_E_BADARG;
+  if (!stats) err = "null pointer";
+  else if (int rc = check_gain_layers(what, layers, n_layers, canvas_h, canvas_w)) return rc;
+  else if (stats_bytes < gain_stats_bytes(n_layers)) err = "stats is smaller than apap_gain_stats_bytes";
+  else if (reinterpret_cast<uintptr_t>(stats) & 7u) {
+    err = "stats must be 8-byte aligned";
+    code = APAP_E_ALIGN;
+  }
+  if (err) {
+    snprintf(msg, sizeof(msg), "%s: %s", what, err);
+    return fail(code, msg);
+  }
+  GainStatsParams p;
+  for (int l = 0; l < n_layers; ++l) p.layer[l] = layer_desc(layers + 6 * l);
+  p.count = static_cast<unsigned long long *>(stats);
+  p.sum = p.count + (size_t)n_layers * n_layers;
+  p.n_layers = n_layers;
+  p.canvas_w = canvas_w;
+  p.segs_per_row = (canvas_w + kSegPx - 1) / kSegPx;
+  const long long blocks = (long long)p.segs_per_row * canvas_h;
+  if (blocks > 2147483647LL) {
+    snprintf(msg, sizeof(msg), "%s: canvas too large", what);
+    return fail(APAP_E_TOOBIG, msg);
+  }
+  snprintf(msg, sizeof(msg), "%s memset", what);
+  if (int rc = check_cuda(cudaMemsetAsync(stats, 0, gain_stats_bytes(n_layers), st), msg)) return rc;
+  k_gain_stats<kChannels><<<(unsigned)blocks, kLayerThreads, 0, st>>>(p);
+  return check_cuda(cudaGetLastError(), "k_gain_stats launch");
+}
 
 }  // namespace apap
 
@@ -149,22 +211,12 @@ extern "C" int apap_gain_stats_bytes(int n_layers, size_t *bytes) {
 
 extern "C" int apap_gain_stats(const long long *layers, int n_layers, int canvas_h, int canvas_w, void *stats,
                                size_t stats_bytes, void *stream) {
-  if (!stats) return fail(APAP_E_BADARG, "gain_stats: null pointer");
-  if (int rc = check_gain_layers(layers, n_layers, canvas_h, canvas_w)) return rc;
-  if (stats_bytes < gain_stats_bytes(n_layers))
-    return fail(APAP_E_BADARG, "gain_stats: stats is smaller than apap_gain_stats_bytes");
-  if (reinterpret_cast<uintptr_t>(stats) & 7u) return fail(APAP_E_ALIGN, "gain_stats: stats must be 8-byte aligned");
-  GainStatsParams p;
-  for (int l = 0; l < n_layers; ++l) p.layer[l] = layer_desc(layers + 6 * l);
-  p.count = static_cast<unsigned long long *>(stats);
-  p.sum = p.count + (size_t)n_layers * n_layers;
-  p.n_layers = n_layers;
-  p.canvas_w = canvas_w;
-  p.segs_per_row = (canvas_w + kSegPx - 1) / kSegPx;
-  const long long blocks = (long long)p.segs_per_row * canvas_h;
-  if (blocks > 2147483647LL) return fail(APAP_E_TOOBIG, "gain_stats: canvas too large");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (int rc = check_cuda(cudaMemsetAsync(stats, 0, gain_stats_bytes(n_layers), st), "gain_stats memset")) return rc;
-  k_gain_stats<<<(unsigned)blocks, kLayerThreads, 0, st>>>(p);
-  return check_cuda(cudaGetLastError(), "k_gain_stats launch");
+  return overlap_stats<false>("gain_stats", layers, n_layers, canvas_h, canvas_w, stats, stats_bytes,
+                              static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int apap_channel_stats(const long long *layers, int n_layers, int canvas_h, int canvas_w, void *stats,
+                                  size_t stats_bytes, void *stream) {
+  return overlap_stats<true>("channel_stats", layers, n_layers, canvas_h, canvas_w, stats, stats_bytes,
+                             static_cast<cudaStream_t>(stream));
 }

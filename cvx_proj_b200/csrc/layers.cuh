@@ -119,13 +119,22 @@ __device__ __forceinline__ void fetch_group(const LayerDesc &L, int y, int seg0,
 }
 
 // exposure gain of one group (the blends' kGains instantiations): every byte v becomes lut[v], the layer's
-// saturate(rint(v g)) table of apap_blend_layers_gain; lut[0] is 0, so absent pixels stay 0
+// saturate(rint(v g)) table of apap_blend_layers_gain; lut[0] is 0, so absent pixels stay 0.  kChannels: lut is the
+// layer's [3][256] table of apap_blend_layers_channels, and byte b of the group, channel b % 3, reads row b % 3
+template <bool kChannels>
 __device__ __forceinline__ void gain_group(const uint8_t *__restrict__ lut, uint32_t (&v)[3]) {
 #pragma unroll
   for (int i = 0; i < 3; ++i) {
     const uint32_t u = v[i];
-    v[i] = (uint32_t)__ldg(lut + (u & 0xffu)) | (uint32_t)__ldg(lut + ((u >> 8) & 0xffu)) << 8 |
-           (uint32_t)__ldg(lut + ((u >> 16) & 0xffu)) << 16 | (uint32_t)__ldg(lut + (u >> 24)) << 24;
+    if constexpr (kChannels) {
+      const uint8_t *t0 = lut + 256 * ((4 * i) % 3), *t1 = lut + 256 * ((4 * i + 1) % 3);
+      const uint8_t *t2 = lut + 256 * ((4 * i + 2) % 3), *t3 = lut + 256 * ((4 * i + 3) % 3);
+      v[i] = (uint32_t)__ldg(t0 + (u & 0xffu)) | (uint32_t)__ldg(t1 + ((u >> 8) & 0xffu)) << 8 |
+             (uint32_t)__ldg(t2 + ((u >> 16) & 0xffu)) << 16 | (uint32_t)__ldg(t3 + (u >> 24)) << 24;
+    } else {
+      v[i] = (uint32_t)__ldg(lut + (u & 0xffu)) | (uint32_t)__ldg(lut + ((u >> 8) & 0xffu)) << 8 |
+             (uint32_t)__ldg(lut + ((u >> 16) & 0xffu)) << 16 | (uint32_t)__ldg(lut + (u >> 24)) << 24;
+    }
   }
 }
 

@@ -21,7 +21,8 @@
 //   k_mb_down<kLevel0, kGains>  one launch per level i < nb for all layers (grid z = layer): X_{i+1} and G_{i+1} as
 //                               int16 {b, g, r, w} on the level i + 1 box.  Level 0 is never stored: it is read from
 //                               the layer bytes (the zero paste, the reflect pad, the weight from the raw bytes,
-//                               kGains: the bytes through the layer's exposure-gain table lut[k][256]).
+//                               kGains: the bytes through the layer's exposure-gain table lut[k][256], kChannels:
+//                               through its per-channel table lut[k][3][256]).
 //   k_mb_band<kLevel0, kTop, kGains>  one launch per level, nb down to 0: per pixel the layers' L, G summed in int32
 //                               registers (the per-layer Laplacians never leave the SM), normalised, pyrUp(R_{i+1})
 //                               added; R_i (i >= 1) is stored on the full level as int16 {b, g, r, 0}, level 0
@@ -45,7 +46,7 @@ struct MbParams {
   int4 rect[APAP_MULTIBAND_MAX_LAYERS];           // clipped rectangle [x0, x1) x [y0, y1) on the canvas
   MbWin lo[APAP_MULTIBAND_MAX_LAYERS];            // level i
   MbWin hi[APAP_MULTIBAND_MAX_LAYERS];            // level i + 1
-  const uint8_t *lut;                             // [n_layers][256] (kGains)
+  const uint8_t *lut;                             // [n_layers][256] (kGains), [n_layers][3][256] (kChannels)
   short4 *r_lo;                                   // R_i (k_mb_band, i >= 1), full level, row pitch lw
   const short4 *r_hi;                             // R_{i+1}, row pitch hw
   uint8_t *out;
@@ -68,7 +69,7 @@ __device__ __forceinline__ int mb_reflect_pad(int i, int n) {
 }
 
 // level 0 of layer l at padded position (x, y): X_0 {b, g, r} and G_0 in .w
-template <bool kGains>
+template <bool kGains, bool kChannels>
 __device__ __forceinline__ int4 mb_level0(const MbParams &p, int l, int x, int y) {
   const int4 R = p.rect[l];
   const bool in_canvas = x < p.canvas_w && y < p.canvas_h;
@@ -78,7 +79,12 @@ __device__ __forceinline__ int4 mb_level0(const MbParams &p, int l, int x, int y
   const uint8_t *q = L.addr + (long long)(cy - L.y0) * L.pitch + 3LL * (cx - L.x0);
   int b = __ldg(q), g = __ldg(q + 1), r = __ldg(q + 2);
   const int w = in_canvas && (b | g | r) ? 256 : 0;
-  if constexpr (kGains) {
+  if constexpr (kGains && kChannels) {
+    const uint8_t *lut = p.lut + 768 * l;
+    b = __ldg(lut + b);
+    g = __ldg(lut + 256 + g);
+    r = __ldg(lut + 512 + r);
+  } else if constexpr (kGains) {
     const uint8_t *lut = p.lut + 256 * l;
     b = __ldg(lut + b);
     g = __ldg(lut + g);
@@ -154,7 +160,7 @@ __device__ __forceinline__ int3 mb_up_full(const short4 *__restrict__ s, int n_x
   return make_int3(mb_sat16((t0 + 32) >> 6), mb_sat16((t1 + 32) >> 6), mb_sat16((t2 + 32) >> 6));
 }
 
-template <bool kLevel0, bool kGains>
+template <bool kLevel0, bool kGains, bool kChannels>
 __global__ void __launch_bounds__(kMbTileX *kMbTileY) k_mb_down(const __grid_constant__ MbParams p) {
   const int l = blockIdx.z;
   const MbWin &D = p.hi[l];
@@ -174,7 +180,7 @@ __global__ void __launch_bounds__(kMbTileX *kMbTileY) k_mb_down(const __grid_con
 #pragma unroll
     for (int c = 0; c < 5; ++c) {
       int4 v;
-      if constexpr (kLevel0) v = mb_level0<kGains>(p, l, ix[c], iy[a]);
+      if constexpr (kLevel0) v = mb_level0<kGains, kChannels>(p, l, ix[c], iy[a]);
       else v = mb_win_at(p.lo[l], ix[c], iy[a]);
       const int w = taps[a] * taps[c];
       s0 += w * v.x;
@@ -187,7 +193,7 @@ __global__ void __launch_bounds__(kMbTileX *kMbTileY) k_mb_down(const __grid_con
                                                    (short)mb_sat16((s2 + 128) >> 8), (short)mb_sat16((s3 + 128) >> 8));
 }
 
-template <bool kLevel0, bool kTop, bool kGains>
+template <bool kLevel0, bool kTop, bool kGains, bool kChannels>
 __global__ void __launch_bounds__(kMbTileX *kMbTileY) k_mb_band(const __grid_constant__ MbParams p) {
   const int tx0 = blockIdx.x * kMbTileX, ty0 = blockIdx.y * kMbTileY;
   const int x = tx0 + threadIdx.x, y = ty0 + threadIdx.y;
@@ -206,7 +212,7 @@ __global__ void __launch_bounds__(kMbTileX *kMbTileY) k_mb_band(const __grid_con
     if (bx1 <= tx0 || bx0 >= tx0 + kMbTileX || by1 <= ty0 || by0 >= ty0 + kMbTileY) continue;   // uniform
     if (!active || x < bx0 || x >= bx1 || y < by0 || y >= by1) continue;
     int4 v;
-    if constexpr (kLevel0) v = mb_level0<kGains>(p, l, x, y);
+    if constexpr (kLevel0) v = mb_level0<kGains, kChannels>(p, l, x, y);
     else v = mb_win_at(p.lo[l], x, y);
     if (v.w == 0) continue;
     if constexpr (!kTop) {
@@ -321,7 +327,7 @@ int mb_check(const char *what, const long long *layers, int n_layers, int canvas
   return 0;
 }
 
-template <bool kGains>
+template <bool kGains, bool kChannels>
 int mb_launch(const MbPlan &P, MbParams &p, cudaStream_t st) {
   const int nb = P.nb;
   const dim3 block(kMbTileX, kMbTileY);
@@ -346,8 +352,8 @@ int mb_launch(const MbPlan &P, MbParams &p, cudaStream_t st) {
     if (mw == 0) break;                           // every layer lies outside the canvas
     const dim3 grid((unsigned)((mw + kMbTileX - 1) / kMbTileX), (unsigned)((mh + kMbTileY - 1) / kMbTileY),
                     (unsigned)p.n_layers);
-    if (i == 0) k_mb_down<true, kGains><<<grid, block, 0, st>>>(p);
-    else k_mb_down<false, false><<<grid, block, 0, st>>>(p);
+    if (i == 0) k_mb_down<true, kGains, kChannels><<<grid, block, 0, st>>>(p);
+    else k_mb_down<false, false, false><<<grid, block, 0, st>>>(p);
     if (int rc = check_cuda(cudaGetLastError(), "k_mb_down launch")) return rc;
   }
   for (int i = nb; i >= 0; --i) {
@@ -356,17 +362,18 @@ int mb_launch(const MbPlan &P, MbParams &p, cudaStream_t st) {
     p.r_hi = i < nb ? P.r[i + 1] : nullptr;
     const int n_x = i == 0 ? p.canvas_w : p.lw, n_y = i == 0 ? p.canvas_h : p.lh;
     const dim3 grid((unsigned)((n_x + kMbTileX - 1) / kMbTileX), (unsigned)((n_y + kMbTileY - 1) / kMbTileY));
-    if (i == 0 && nb == 0) k_mb_band<true, true, kGains><<<grid, block, 0, st>>>(p);
-    else if (i == 0) k_mb_band<true, false, kGains><<<grid, block, 0, st>>>(p);
-    else if (i == nb) k_mb_band<false, true, false><<<grid, block, 0, st>>>(p);
-    else k_mb_band<false, false, false><<<grid, block, 0, st>>>(p);
+    if (i == 0 && nb == 0) k_mb_band<true, true, kGains, kChannels><<<grid, block, 0, st>>>(p);
+    else if (i == 0) k_mb_band<true, false, kGains, kChannels><<<grid, block, 0, st>>>(p);
+    else if (i == nb) k_mb_band<false, true, false, false><<<grid, block, 0, st>>>(p);
+    else k_mb_band<false, false, false, false><<<grid, block, 0, st>>>(p);
     if (int rc = check_cuda(cudaGetLastError(), "k_mb_band launch")) return rc;
   }
   return 0;
 }
 
+// lut: none (nullptr), [n][256] or (channels) [n][3][256]
 int multiband_blend(const char *what, const long long *layers, int n_layers, int canvas_h, int canvas_w, int bands,
-                    const uint8_t *lut, void *workspace, size_t workspace_bytes, uint8_t *out, size_t out_bytes,
+                    const uint8_t *lut, bool channels, void *workspace, size_t workspace_bytes, uint8_t *out, size_t out_bytes,
                     cudaStream_t st) {
   if (!out || !workspace) return mb_fail(APAP_E_BADARG, what, "null pointer");
   if (int rc = mb_check(what, layers, n_layers, canvas_h, canvas_w, bands)) return rc;
@@ -389,7 +396,8 @@ int multiband_blend(const char *what, const long long *layers, int n_layers, int
   p.canvas_h = canvas_h;
   p.wp = P.wp;
   p.hp = P.hp;
-  return lut ? mb_launch<true>(P, p, st) : mb_launch<false>(P, p, st);
+  if (lut && channels) return mb_launch<true, true>(P, p, st);
+  return lut ? mb_launch<true, false>(P, p, st) : mb_launch<false, false>(P, p, st);
 }
 
 }  // namespace
@@ -410,7 +418,7 @@ extern "C" int apap_multiband_workspace_bytes(const long long *layers, int n_lay
 extern "C" int apap_multiband_blend(const long long *layers, int n_layers, int canvas_h, int canvas_w, int bands,
                                     void *workspace, size_t workspace_bytes, uint8_t *out, size_t out_bytes,
                                     void *stream) {
-  return multiband_blend("multiband_blend", layers, n_layers, canvas_h, canvas_w, bands, nullptr, workspace,
+  return multiband_blend("multiband_blend", layers, n_layers, canvas_h, canvas_w, bands, nullptr, false, workspace,
                          workspace_bytes, out, out_bytes, static_cast<cudaStream_t>(stream));
 }
 
@@ -418,6 +426,14 @@ extern "C" int apap_multiband_blend_gain(const long long *layers, int n_layers, 
                                          const uint8_t *lut, void *workspace, size_t workspace_bytes, uint8_t *out,
                                          size_t out_bytes, void *stream) {
   if (!lut) return fail(APAP_E_BADARG, "multiband_blend_gain: null gain table");
-  return multiband_blend("multiband_blend_gain", layers, n_layers, canvas_h, canvas_w, bands, lut, workspace,
+  return multiband_blend("multiband_blend_gain", layers, n_layers, canvas_h, canvas_w, bands, lut, false, workspace,
                          workspace_bytes, out, out_bytes, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int apap_multiband_blend_channels(const long long *layers, int n_layers, int canvas_h, int canvas_w,
+                                             int bands, const uint8_t *lut, void *workspace, size_t workspace_bytes,
+                                             uint8_t *out, size_t out_bytes, void *stream) {
+  if (!lut) return fail(APAP_E_BADARG, "multiband_blend_channels: null gain table");
+  return multiband_blend("multiband_blend_channels", layers, n_layers, canvas_h, canvas_w, bands, lut, true,
+                         workspace, workspace_bytes, out, out_bytes, static_cast<cudaStream_t>(stream));
 }

@@ -219,18 +219,23 @@ def stitch_panorama(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops, *, mesh_s
     keeping its original mask.  With no other image it equals ``"none"``.  The gains are not part of the result; a
     caller who wants them calls ``exposure_gains`` on the layers.
 
+    ``exposure="channels"`` does the same with one gain per layer and colour channel, as OpenCV's
+    ``cv.detail.ChannelsCompensator`` (``--expos_comp channel``): ``utils.channel_gains`` over the same layers in the
+    same order, so a layer with a colour cast is evened out as well as a darker one.  Every field but ``panorama`` is
+    the ``"none"`` call's, and with no other image it equals ``"none"``.
+
     The layers are warped from the images the keypoint-pair producer already holds on the device and stay there; one
     blend call and one download make the panorama.  At most 255 other images (127 with ``"feather"``, 126 with
     ``"multiband"``); an unknown ``blend``, an unknown ``exposure``, too many images, a ``sharpness`` that
     ``feather_blend`` refuses for every canvas or (with ``"multiband"``) a ``bands`` that ``multiband_blend`` refuses
     raise ``ValueError`` before any keypoint work."""
     from . import _runtime as rt
-    from .utils import _BLENDERS, _device_image, exposure_gains
+    from .utils import _BLENDERS, _device_image, channel_gains, exposure_gains
 
     if blend not in tuple(_BLENDERS):                   # a tuple: an unhashable blend is a ValueError too
         raise ValueError(f"stitch_panorama: blend must be 'mean', 'feather' or 'multiband', got {blend!r}")
-    if exposure not in ("none", "gain"):
-        raise ValueError(f"stitch_panorama: exposure must be 'none' or 'gain', got {exposure!r}")
+    if exposure not in ("none", "gain", "channels"):
+        raise ValueError(f"stitch_panorama: exposure must be 'none', 'gain' or 'channels', got {exposure!r}")
     if warp_imgs is not None and len(warp_imgs) != len(other_imgs):
         raise ValueError(f"stitch_panorama: {len(other_imgs)} other images but {len(warp_imgs)} warp images")
     blend_fn, max_layers, param, check_param = _BLENDERS[blend]
@@ -261,6 +266,7 @@ def stitch_panorama(center_img, other_imgs, raw_kpts_cp, raw_kpts_ops, *, mesh_s
         layers.append(st.local_warp(warp_devs[i], local_h.copy(), meshes[i]))
     (width, height, ox, oy), origins = panorama_size([p.final_size for p in pairs])
     layers, places = layers + [blend_dev], [tuple(o) for o in origins] + [(ox, oy)]
-    gains = exposure_gains(layers, places, (width, height)) if exposure == "gain" else None
+    gain_fn = {"none": None, "gain": exposure_gains, "channels": channel_gains}[exposure]
+    gains = None if gain_fn is None else gain_fn(layers, places, (width, height))
     pano = blend_fn(layers, places, (width, height), gains=gains, **params)
     return PanoramaResult((width, height, ox, oy), origins, pairs, rt.to_host(torch, pano))

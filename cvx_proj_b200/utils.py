@@ -24,7 +24,8 @@ from . import _runtime as rt
 
 __all__ = ["image_warping", "warp_perspective", "warping_canvas", "invert3x3", "match_descriptors", "coarse_matching",
            "sift_describe", "equalize_hist", "keypoint_pairs", "keypoint_pairs_batch", "find_homography_ransac",
-           "find_homography_ransac_batch", "blend_layers", "feather_blend", "multiband_blend", "exposure_gains"]
+           "find_homography_ransac_batch", "blend_layers", "feather_blend", "multiband_blend", "exposure_gains",
+           "channel_gains"]
 
 
 def invert3x3(m) -> np.ndarray:
@@ -112,7 +113,9 @@ def blend_layers(layers, origins, size, device=None, gains=None):
 
     ``gains`` (one finite float per layer, e.g. from ``exposure_gains``): layer k's bytes ``v`` become
     ``saturate(rint(v g_k))`` before they are summed, as ``cv.detail.GainCompensator.apply`` does; ``n`` still counts
-    the layers non-empty before compensation.  ``None`` leaves the bytes as they are.
+    the layers non-empty before compensation.  Shape ``(n, 3)`` (e.g. from ``channel_gains``): byte ``v`` of channel
+    ``c`` becomes ``saturate(rint(v g_kc))``, as ``cv.detail.ChannelsCompensator.apply`` does.  ``None`` leaves the
+    bytes as they are.
 
     All numpy in -> numpy out (uploaded to ``device``); all CUDA tensors (one device) in -> a tensor on that device.
     Tensor layers are read in place when their pixels are packed (strides ``(pitch, 3, 1)``), so crops of a larger
@@ -203,7 +206,35 @@ def exposure_gains(layers, origins, size, device=None) -> np.ndarray:
 
     1 to 256 layers; ``layers``, ``origins``, ``size`` and the device rules as for ``blend_layers`` (tensor crops are
     read in place).  One launch and one download.  No CPU fallback."""
-    layers, origins, width, height, on_device, device = _check_layers("exposure_gains", layers, origins, size,
+    stats, n = _overlap_stats("exposure_gains", "apap_gain_stats", layers, origins, size, device)
+    return solve_gains(*gain_stats_ints(stats, n))
+
+
+def channel_gains(layers, origins, size, device=None) -> np.ndarray:
+    """Per-channel exposure-compensation gains of placed layers, float64 ``[n, 3]``: what
+    ``cv.detail.ChannelsCompensator()`` returns from ``getMatGains()`` (the first three entries per layer) after
+    ``feed([(0, 0)] * n, [P_k], [mask_k])``, with ``P_k`` and ``mask_k`` as for ``feather_blend``; column ``c`` belongs
+    to channel ``c`` of the layers.  Pass them as ``gains=`` to ``blend_layers``, ``feather_blend`` or
+    ``multiband_blend``.  Where ``exposure_gains`` evens out brightness only, these also even out a colour cast.
+
+    OpenCV solves ``GainCompensator``'s system once per channel, with ``I_c(i, j)`` the mean of channel ``c`` of
+    ``P_i`` over ``mask_i & mask_j`` (the masks and counts are ``exposure_gains``').  The per-pair channel sums are
+    byte sums, counted exactly on the GPU (``k_gain_stats<true>``); below ``2^53`` they are exact in double too, so
+    the result does not depend on the schedule.  ``solve_gains`` then runs once per channel.
+
+    1 to 256 layers; ``layers``, ``origins``, ``size`` and the device rules as for ``blend_layers`` (tensor crops are
+    read in place).  One launch and one download.  No CPU fallback."""
+    stats, n = _overlap_stats("channel_gains", "apap_channel_stats", layers, origins, size, device)
+    w = stats.view(np.uint64).reshape(4, n, n)
+    count = [[int(v) for v in row] for row in w[0]]
+    # solve_gains reads sums scaled by 2^52 (exposure_gains' fixed point); a byte sum below 2^53 scales exactly
+    return np.stack([solve_gains(count, [[int(v) << 52 for v in row] for row in w[1 + c]]) for c in range(3)], axis=1)
+
+
+def _overlap_stats(what, entry, layers, origins, size, device):
+    """``(stats, n)``: the uint64 ``[4][n][n]`` words of ``entry`` (``apap_gain_stats`` or ``apap_channel_stats``) for
+    placed layers checked as ``what``, as a host int64 array; one launch and one download."""
+    layers, origins, width, height, on_device, device = _check_layers(what, layers, origins, size,
                                                                        rt.GAIN_MAX_LAYERS, device)
     torch, device, lib, devs, desc_p = _placed_layers(layers, origins, on_device, device)
     n = len(devs)
@@ -211,10 +242,9 @@ def exposure_gains(layers, origins, size, device=None) -> np.ndarray:
     rt.check(lib.apap_gain_stats_bytes(n, ctypes.byref(nbytes)), "apap_gain_stats_bytes")
     stats = torch.empty(nbytes.value // 8, dtype=torch.int64, device=device)
     with torch.cuda.device(device):
-        rt.check(lib.apap_gain_stats(desc_p, n, height, width, stats.data_ptr(), stats.numel() * 8,
-                                     rt.stream_ptr(torch, device)), "apap_gain_stats")
-    count, sums = gain_stats_ints(rt.to_host(torch, stats), n)
-    return solve_gains(count, sums)
+        rt.check(getattr(lib, entry)(desc_p, n, height, width, stats.data_ptr(), stats.numel() * 8,
+                                     rt.stream_ptr(torch, device)), entry)
+    return rt.to_host(torch, stats), n
 
 
 def gain_stats_ints(stats, n):
@@ -267,15 +297,18 @@ def solve_gains(count, sums):
 
 
 def _gain_table(what, gains, n):
-    """``uint8 [n, 256]``: row k maps a byte ``v`` to ``saturate(rint(v g_k))`` in float64 (ties to even), what
-    ``GainCompensator.apply`` gives; ``ValueError`` unless ``gains`` holds one finite number per layer."""
+    """The gain tables of the blends' ``gains=``: ``gains`` of shape ``(n,)`` give ``uint8 [n, 256]``, row k mapping a
+    byte ``v`` to ``saturate(rint(v g_k))`` in float64 (ties to even), what ``GainCompensator.apply`` gives; shape
+    ``(n, 3)`` gives ``uint8 [n, 3, 256]``, row ``[k, c]`` for ``g_kc``, what ``ChannelsCompensator.apply`` gives.
+    ``ValueError`` for any other shape or a value that is not finite."""
     try:
         g = np.asarray(gains, dtype=np.float64)
     except (TypeError, ValueError):
         raise ValueError(f"{what}: gains must be {n} finite numbers") from None
-    if g.shape != (n,) or not np.isfinite(g).all():
-        raise ValueError(f"{what}: gains must be {n} finite numbers (one per layer), got shape {g.shape}")
-    return np.clip(np.rint(np.arange(256, dtype=np.float64)[None, :] * g[:, None]), 0, 255).astype(np.uint8)
+    if g.shape not in ((n,), (n, 3)) or not np.isfinite(g).all():
+        raise ValueError(f"{what}: gains must be {n} finite numbers (one per layer) or [{n}, 3] (one per layer and "
+                         f"channel), got shape {g.shape}")
+    return np.clip(np.rint(np.arange(256, dtype=np.float64) * g[..., None]), 0, 255).astype(np.uint8)
 
 
 def _feather_sharpness(what, sharpness):
@@ -358,8 +391,9 @@ def _placed_layers(layers, origins, on_device, device):
 
 def _blend(entry, params, workspace, layers, origins, width, height, on_device, device, lut):
     """A placed-layer blend after its checks: the layers described (``_placed_layers``), the workspace (``None``: the
-    blender needs none; else ``(query, its scalars)``), the canvas, and one call of ``entry`` -- or of ``entry +
-    "_gain"`` with the gain table ``lut`` uploaded when it is not ``None``.  The entries share one argument layout,
+    blender needs none; else ``(query, its scalars)``), the canvas, and one call of ``entry`` -- or, with the gain
+    table ``lut`` uploaded when it is not ``None``, of ``entry + "_gain"`` (``lut`` ``[n, 256]``) or ``entry +
+    "_channels"`` (``[n, 3, 256]``).  The entries share one argument layout,
     ``(desc, n, h, w, *params, [lut], [ws, ws_bytes], out, out_bytes, stream)`` with ``params`` the blender's
     scalars (none, ``sharpness`` or ``bands``), and the workspace queries ``(desc, n, h, w, *scalars, &bytes)``.
     numpy layers in -> numpy out, tensors in -> a tensor on their device."""
@@ -377,7 +411,7 @@ def _blend(entry, params, workspace, layers, origins, width, height, on_device, 
         st = rt.stream_ptr(torch, device)
         if lut is not None:
             lut_dev = rt.to_device(torch, device, lut)
-            entry, lut_args = entry + "_gain", (lut_dev.data_ptr(),)
+            entry, lut_args = entry + ("_channels" if lut.ndim == 3 else "_gain"), (lut_dev.data_ptr(),)
         rt.check(getattr(lib, entry)(*head, *params, *lut_args, *ws_args, out.data_ptr(), out.numel(), st), entry)
     return out if on_device else rt.to_host(torch, out)
 

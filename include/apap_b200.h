@@ -301,6 +301,30 @@ int apap_feather_blend_gain(const long long *layers, int n_layers, int canvas_h,
                             void *stream);
 
 /*
+ * Per-channel exposure compensation of placed layers (utils.channel_gains, driver.stitch_panorama(exposure=
+ * "channels")), as cv.detail.ChannelsCompensator (DESIGN.md section 3): GainCompensator's system once per channel.
+ *
+ * apap_channel_stats: its overlap statistics, exact.  stats as for apap_gain_stats (sized by apap_gain_stats_bytes)
+ * gets uint64 [4][n_layers][n_layers]:
+ *   plane 0 [i][j], i <= j    : |mask_i & mask_j|, as apap_gain_stats
+ *   plane 1 + c [i][j], i != j: the sum over mask_i & mask_j of byte c of layer i's pixels (c = 0, 1, 2)
+ *   the other entries are 0.  The result does not depend on the schedule.
+ * Arguments and checks as apap_gain_stats; one memset and one kernel (k_gain_stats<true>) on `stream`.
+ *
+ * apap_blend_layers_channels / apap_feather_blend_channels / apap_multiband_blend_channels: the _gain entries with
+ * byte v of channel c of layer k replaced by lut[k][c][v]; the masks still follow the raw bytes.
+ *   lut : device uint8 [n_layers][3][256], lut[k][c][0] = 0; for gains g_kc, saturate(rint(v g_kc)) in double
+ *         (ties to even); nullptr is APAP_E_BADARG
+ */
+int apap_channel_stats(const long long *layers, int n_layers, int canvas_h, int canvas_w, void *stats,
+                       size_t stats_bytes, void *stream);
+int apap_blend_layers_channels(const long long *layers, int n_layers, int canvas_h, int canvas_w, const uint8_t *lut,
+                               uint8_t *out, size_t out_bytes, void *stream);
+int apap_feather_blend_channels(const long long *layers, int n_layers, int canvas_h, int canvas_w, float sharpness,
+                                const uint8_t *lut, void *workspace, size_t workspace_bytes, uint8_t *out,
+                                size_t out_bytes, void *stream);
+
+/*
  * Multi-band blend of placed layers (utils.multiband_blend, driver.stitch_panorama(blend="multiband")): out [canvas_h]
  * [canvas_w][3] uint8 (device, any alignment, out_bytes >= canvas_h x canvas_w x 3) is bit for bit what
  * cv.detail.MultiBandBlender(0, bands, CV_16S) gives after prepare((0, 0, canvas_w, canvas_h)), feed(P_k as int16,
@@ -316,6 +340,7 @@ int apap_feather_blend_gain(const long long *layers, int n_layers, int canvas_h,
  * nb k_mb_down and nb + 1 k_mb_band launches on `stream`.
  * apap_multiband_blend_gain: layer k's bytes v replaced by lut[k][v] (as apap_blend_layers_gain) before the pyramids
  * are built; mask_k still follows the raw bytes, as OpenCV's pipeline feeds the blender the original masks.
+ * apap_multiband_blend_channels: the same with per-channel tables lut[k][c][v] (as apap_blend_layers_channels).
  */
 #define APAP_MULTIBAND_MAX_LAYERS 127
 int apap_multiband_workspace_bytes(const long long *layers, int n_layers, int canvas_h, int canvas_w, int bands,
@@ -325,6 +350,9 @@ int apap_multiband_blend(const long long *layers, int n_layers, int canvas_h, in
 int apap_multiband_blend_gain(const long long *layers, int n_layers, int canvas_h, int canvas_w, int bands,
                               const uint8_t *lut, void *workspace, size_t workspace_bytes, uint8_t *out,
                               size_t out_bytes, void *stream);
+int apap_multiband_blend_channels(const long long *layers, int n_layers, int canvas_h, int canvas_w, int bands,
+                                  const uint8_t *lut, void *workspace, size_t workspace_bytes, uint8_t *out,
+                                  size_t out_bytes, void *stream);
 
 /*
  * Input preparation on the device (what the host layer used to build in numpy; both reproduce their
